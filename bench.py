@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- batched LMPC solves/sec (build + QP) on B200, the metric BASELINE.json names.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--batch B] [--impl reference] [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[2], the one its metric is quoted on: C3, the walking CoM preview (3rd-order LIPM,
 6 states / 2 jerk controls, horizon 160, ZMP mixed inequalities), batch 16384, STRONG-scaled: at N GPUs (one process per GPU
@@ -17,8 +17,11 @@ batch.  There is no collective on the hot path; the only cross-GPU traffic is th
 `roofline`, `cpu_baseline`, `other_configs`: see DESIGN.md "Measurement".
 `--impl reference` times the CPU restatement (oracle port) of copra's Eigen + eigen-quadprog path -- the reference itself
 cannot be built offline -- on all host threads of this process's affinity mask, same config / metric.
+`--dump-outputs DIR` writes what the last timed step returned to the caller (see dump_sample) as DIR/<name>.npy, so that
+two builds can be compared output for output: the workloads are seeded, so the same arguments give the same inputs.
 """
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -157,8 +160,14 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "--query-gpu=" + self.FIELDS, "--format=csv,noheader,nounits",
                                           "-lms", "50", "-i", str(self.gpu)], stdout=open(self.path, "w"),
                                          stderr=subprocess.DEVNULL)
+            atexit.register(self.kill)  # an exception before stop() must not leave the sampler running
         except Exception:
             self.proc = None
+
+    def kill(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     def stop(self):
         out = dict(sm_mhz=None, sm_max_mhz=None, reasons=[], samples=0)
@@ -305,6 +314,27 @@ class Runner:
         self.eng.close()
 
 
+DUMP_BYTES = 64 * 1000 * 1000
+
+
+def dump_sample(run):
+    """float64 host copies of the result arrays copra_b200_lmpc_run filled in its last call (control, trajectory, status,
+    iters, nact, iact) for a fixed seeded sample of instances, small enough that the .npy files stay under DUMP_BYTES;
+    `instance` holds the sampled instance indices"""
+    torch, b = run.torch, run.batch
+    bufs = dict(control=run.d_control, trajectory=run.d_traj, status=run.d_status, iters=run.d_iters, nact=run.d_nact,
+                iact=run.d_iact)
+    per_instance = 8 * (1 + sum(t.numel() // b for t in bufs.values()))
+    keep = min(b, (DUMP_BYTES - 128 * (len(bufs) + 1)) // per_instance)  # 128: header of one .npy file
+    idx = np.arange(b) if keep == b else np.sort(np.random.default_rng(0).choice(b, keep, replace=False))
+    sel = torch.from_numpy(idx).to(run.dev)
+    out = dict(instance=idx.astype(np.float64))
+    for name, t in bufs.items():
+        a = t.view(b, -1).index_select(0, sel).to(torch.float64).cpu().numpy()
+        out[name] = a[:, 0] if a.shape[1] == 1 else a
+    return out
+
+
 def time_value(torch, runner, stream, flush, steps, barrier):
     """K timed steps, CUDA events on the launching stream, L2 flushed between steps; per-stage times of every step"""
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
@@ -435,8 +465,11 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary configurations (other_configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        raise SystemExit("--dump-outputs dumps the single-GPU b200 path: use it with --impl b200 on one GPU")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -489,6 +522,7 @@ def main():
     l0 = run.eng.launch_count()
     step_ms, stage, wall_timed = time_value(torch, run, stream, flush, args.steps, barrier)
     launches = run.eng.launch_count() - l0
+    dumped = dump_sample(run) if args.dump_outputs else None
     total_ms = sum(step_ms)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
@@ -660,6 +694,10 @@ def main():
             except Exception as ex:
                 extras["c1_raw_qp_latency"] = dict(error=repr(ex))
             line["other_configs"] = extras
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
