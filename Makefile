@@ -8,7 +8,7 @@ OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_th
 LIB := copra_b200/lib/libcopra_b200.so
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/copra_b200.h
 
-all: $(LIB) oracle tests/cpp/test_facade
+all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; false)
@@ -31,3 +31,9 @@ tests/cpp/test_facade: tests/cpp/test_facade.cpp tests/cpp/systems.hpp $(wildcar
 	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_facade.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
 
 facade-test: tests/cpp/test_facade
+
+# BatchedLMPC with per-step references and limits + retarget (needs the GPU to run)
+tests/cpp/test_per_step: tests/cpp/test_per_step.cpp $(wildcard include/copra/*) include/copra_b200.h $(LIB)
+	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_per_step.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
+
+per-step-test: tests/cpp/test_per_step

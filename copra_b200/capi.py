@@ -15,6 +15,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libcopra_b200.so")
 HOST, DEVICE = 0, 1
 FLAG_NO_REG = 1  # COPRA_B200_FLAG_NO_REG: no 1e-6 I regulariser (single cost evaluation)
 FLAG_STABLE_BOUND_PATTERN = 2  # device inputs: the +-inf pattern of trajectory bounds is unchanged since the last build
+PER_STEP = 2  # COPRA_B200_PER_STEP: step-size matrices, a vector per step (rows x steps entries, step-major)
 COST_KINDS = {"trajectory": 0, "target": 1, "control": 2, "mixed": 3}
 CSTR_KINDS = {"trajectory": 0, "control": 1, "mixed": 2, "trajectory_bound": 3, "control_bound": 4}
 GET = dict(Phi=0, Psi=1, xi=2, Q=3, c=4, Aeq=5, beq=6, Aineq=7, bineq=8, lb=9, ub=10)
@@ -71,7 +72,8 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_lmpc_built_sizes", "copra_b200_last_solver", "copra_b200_hessian_is_shared", "copra_b200_multi_create", "copra_b200_multi_destroy",
            "copra_b200_multi_last_error", "copra_b200_multi_size", "copra_b200_multi_shard", "copra_b200_multi_timing",
            "copra_b200_multi_launch_count", "copra_b200_multi_lmpc_run", "copra_b200_multi_lmpc_resolve",
-           "copra_b200_set_warm_start", "copra_b200_get_warm_start", "copra_b200_multi_set_warm_start"]
+           "copra_b200_set_warm_start", "copra_b200_get_warm_start", "copra_b200_multi_set_warm_start",
+           "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget"]
 
 _lib = None
 
@@ -112,6 +114,7 @@ def load():
         lib.copra_b200_lmpc_results.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_fp64_peaks.argtypes = [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double)]
         lib.copra_b200_lmpc_resolve.argtypes = [C.c_void_p, Array, C.c_int, C.POINTER(Results)]
+        lib.copra_b200_lmpc_retarget.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Results)]
         lib.copra_b200_dgemm_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_void_p, C.c_int,
                                                C.c_longlong, C.c_void_p, C.c_int, C.c_longlong, C.c_double, C.c_void_p, C.c_int,
                                                C.c_longlong, C.c_int, C.c_int]
@@ -133,6 +136,7 @@ def load():
         lib.copra_b200_multi_launch_count.restype = C.c_longlong
         lib.copra_b200_multi_lmpc_run.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Results)]
         lib.copra_b200_multi_lmpc_resolve.argtypes = [C.c_void_p, Array, C.POINTER(Results)]
+        lib.copra_b200_multi_lmpc_retarget.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Results)]
         lib.copra_b200_multi_set_warm_start.argtypes = [C.c_void_p, C.c_int]
         _lib = lib
     return _lib
@@ -146,9 +150,27 @@ def _colmajor(a, base_ndim):
     return np.ascontiguousarray(a)
 
 
+def _steps(kind, N):
+    """steps of the horizon a cost / constraint kind applies to: the length, in steps, of its per-step vector"""
+    return N + 1 if kind in ("trajectory", "trajectory_bound") else (1 if kind == "target" else N)
+
+
+def _rows_of(mat):
+    a = np.asarray(mat)
+    return int(a.shape[-2]) if a.ndim >= 2 else 1
+
+
+def _check_per_step(what, vec, rows, steps):
+    if np.asarray(vec).shape[-1] != rows * steps:
+        raise CopraB200Error(-1, "%s: a per-step vector holds rows x steps = %d x %d entries, got %d"
+                             % (what, rows, steps, np.asarray(vec).shape[-1]))
+
+
 class HostBatch:
     """A batch problem (copra_b200.workloads dict) packed into column-major host buffers + the ctypes
-    `Problem` describing them.  Buffers live as long as this object (pin=True: torch pinned memory)."""
+    `Problem` describing them.  Buffers live as long as this object (pin=True: torch pinned memory).
+    A cost or constraint dict with `per_step=True` is packed as COPRA_B200_PER_STEP: step-size matrices, and a p / f /
+    lower / upper of rows x steps entries (step-major) per instance."""
 
     _BASE = dict(A=2, B=2, d=1, x0=1, R=2, r=1, x0lb=1, x0ub=1, M=2, N=2, E=2, G=2, p=1, w=1, f=1, lower=1, upper=1)
 
@@ -168,17 +190,24 @@ class HostBatch:
             if bp.get(k) is not None:
                 setattr(p, k, self._arr(k, bp[k]))
         costs = (Cost * max(1, len(bp["costs"])))()
+        N_ = int(bp["N"])
         for i, c in enumerate(bp["costs"]):
             costs[i].kind = COST_KINDS[c["kind"]]
             pv = np.asarray(c["p"])
             costs[i].rows = int(pv.shape[-1])
             nx_, nu_ = int(bp["nx"]), int(bp["nu"])
+            per_step = bool(c.get("per_step", False))
+            if per_step:
+                costs[i].rows = _rows_of(c["M"] if c.get("M") is not None else c["N"])
+                _check_per_step("cost %d" % i, pv, costs[i].rows, _steps(c["kind"], N_))
             if c.get("M") is not None:
                 costs[i].M = self._arr("M", c["M"])
                 costs[i].full_size = int(np.asarray(c["M"]).shape[-1] != nx_)
             if c.get("N") is not None:
                 costs[i].N = self._arr("N", c["N"])
                 costs[i].full_size = int(np.asarray(c["N"]).shape[-1] != nu_) if c.get("M") is None else costs[i].full_size
+            if per_step:
+                costs[i].full_size = PER_STEP
             costs[i].p = self._arr("p", c["p"])
             w = c.get("w")
             w = np.ones(costs[i].rows) if w is None else np.asarray(w, dtype=np.float64)
@@ -193,9 +222,16 @@ class HostBatch:
         for i, c in enumerate(bp["constraints"]):
             cstrs[i].kind = CSTR_KINDS[c["kind"]]
             cstrs[i].is_ineq = int(bool(c.get("is_ineq", True)))
+            per_step = bool(c.get("per_step", False))
+            steps = _steps(c["kind"], N_)
             if c["kind"] in ("trajectory_bound", "control_bound"):
                 cstrs[i].rows = int(np.asarray(c["lower"]).shape[-1])
                 cstrs[i].full_size = int(cstrs[i].rows != (int(bp["nx"]) if c["kind"] == "trajectory_bound" else int(bp["nu"])))
+                if per_step:
+                    cstrs[i].rows = int(bp["nx"]) if c["kind"] == "trajectory_bound" else int(bp["nu"])
+                    cstrs[i].full_size = PER_STEP
+                    for k in ("lower", "upper"):
+                        _check_per_step("constraint %d %s" % (i, k), c[k], cstrs[i].rows, steps)
                 cstrs[i].lower = self._arr("lower", c["lower"])
                 cstrs[i].upper = self._arr("upper", c["upper"])
             else:
@@ -207,6 +243,10 @@ class HostBatch:
                     cstrs[i].G = self._arr("G", c["G"])
                     if c.get("E") is None:
                         cstrs[i].full_size = int(np.asarray(c["G"]).shape[-1] != int(bp["nu"]))
+                if per_step:
+                    cstrs[i].rows = _rows_of(c["E"] if c.get("E") is not None else c["G"])
+                    cstrs[i].full_size = PER_STEP
+                    _check_per_step("constraint %d" % i, c["f"], cstrs[i].rows, steps)
                 cstrs[i].f = self._arr("f", c["f"])
         self.keep.append(cstrs)
         p.ncstr, p.cstrs = len(bp["constraints"]), cstrs
@@ -236,6 +276,18 @@ class HostBatch:
         out.stride = size if batched else 0
         self.h2d_bytes += buf.nbytes
         return out
+
+
+def _result_buffers(B, s):
+    """host result arrays for B instances of sizes `s` and the Results struct pointing at them"""
+    out = dict(control=np.zeros((B, s["nU"])), trajectory=np.zeros((B, s["X"])), x=np.zeros((B, s["nvar"])),
+               status=np.full(B, -1, np.int32), iters=np.zeros((B, 2), np.int32), nact=np.zeros(B, np.int32),
+               iact=np.zeros((B, s["nvar"]), np.int32))
+    r = Results()
+    r.memory = HOST
+    for k, v in out.items():
+        setattr(r, k, v.ctypes.data)
+    return out, r
 
 
 class Engine:
@@ -406,6 +458,14 @@ class Engine:
         self._check(self.lib.copra_b200_lmpc_resolve(self.h, a, HOST, C.byref(r)))
         return out
 
+    def lmpc_retarget(self, bp_or_hb):
+        """receding-horizon step with new x0 and new vectors (p, f, lower / upper) on the resident build; the problem must
+        have the resident build's shape, its matrices are ignored (copra_b200_lmpc_retarget)"""
+        hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
+        out, r = _result_buffers(hb.problem.batch, self.sizes(hb))
+        self._check(self.lib.copra_b200_lmpc_retarget(self.h, C.byref(hb.problem), C.byref(r)))
+        return out
+
     def lmpc_build(self, hb):
         self._check(self.lib.copra_b200_lmpc_build(self.h, C.byref(hb.problem)))
 
@@ -501,6 +561,13 @@ class MultiEngine:
         rc = self.lib.copra_b200_multi_set_warm_start(self.m, 1 if on else 0)
         if rc:
             raise CopraB200Error("copra_b200_multi_set_warm_start failed (%d)" % rc)
+
+    def lmpc_retarget(self, bp_or_hb, sizes):
+        """copra_b200_lmpc_retarget on every shard of the last run"""
+        hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
+        out, r = _result_buffers(hb.problem.batch, sizes)
+        self._check(self.lib.copra_b200_multi_lmpc_retarget(self.m, C.byref(hb.problem), C.byref(r)))
+        return out
 
     def lmpc_resolve(self, x0, sizes):
         x0 = np.ascontiguousarray(np.asarray(x0, dtype=np.float64))

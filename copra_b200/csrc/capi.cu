@@ -20,6 +20,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <tuple>
 #include <vector>
 
 using namespace cb;
@@ -53,13 +54,17 @@ struct copra_b200_handle {
     bool ev_valid[8] = {};
     cudaEvent_t h2d_done = nullptr; // guards reuse of the pinned upload staging buffer
     bool h2d_pending = false;
-    // TrajectoryBound line selection cache for DEVICE inputs: (lower ptr, upper ptr, rows) -> lines
-    struct TbKey { const double* lo; const double* up; int rows; bool operator<(const TbKey& o) const { return lo != o.lo ? lo < o.lo : (up != o.up ? up < o.up : rows < o.rows); } };
+    // TrajectoryBound line selection cache for DEVICE inputs: (lower ptr, upper ptr, rows, full_size) -> lines
+    struct TbKey {
+        const double* lo; const double* up; int rows, full_size;
+        bool operator<(const TbKey& o) const { return std::tie(lo, up, rows, full_size) < std::tie(o.lo, o.up, o.rows, o.full_size); }
+    };
     std::map<TbKey, std::pair<std::vector<int>, std::vector<int>>> tb_cache;
     std::vector<double> sel_host; // last uploaded selector matrices / line lists
     std::vector<int> lines_host;
     // state of the last build
     bool built = false;
+    std::vector<int> shape;    // shape_key() of the last build: what copra_b200_lmpc_retarget must find unchanged
     bool factor_valid = false; // the thin solver's R^-1 of the last build is resident (re-solves skip the factorisation)
     bool rows_filled = false;  // Aeq / Aineq of the last build are materialised (the structured solver never reads them)
     bool use_thin = false;     // the last build is solved by the thin kernel (gi_thin.cuh)
@@ -254,11 +259,14 @@ int run_download(copra_b200_handle* h, Download& D, int memory)
 // ---- problem description -> families ----------------------------------------------------------
 struct Plan {
     Sizes sz;
-    struct CostMeta { int kind, rows, i0, i1, hasM, hasN, dense; };
-    struct FamMeta { int cstr, rows, i0, i1, hasE, hasG, is_eq, row_off, which, dense, gather; std::vector<int> lines; };
+    // vsteps: steps held by the vector (p, f, lower / upper) of a per-step entry, 1 otherwise; pstep / fstep: the
+    // family's stride between steps (0 = the same vector at every step)
+    struct CostMeta { int kind, rows, i0, i1, hasM, hasN, dense, vsteps, pstep; };
+    struct FamMeta { int cstr, rows, i0, i1, hasE, hasG, is_eq, row_off, which, dense, gather, fstep; std::vector<int> lines; };
     int cb_full = 0;
     std::vector<CostMeta> costs;
     std::vector<FamMeta> fams;
+    std::vector<int> cvsteps; // per constraint
     int bound_cstr = -1;
 };
 
@@ -273,12 +281,14 @@ int fetch_host(copra_b200_handle* h, const copra_b200_array& a, int count, int m
     return 0;
 }
 
-int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
+// vectors_only: the problem only supplies new vectors for a resident build (copra_b200_lmpc_retarget), so the matrices
+// may be absent
+int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl, bool vectors_only = false)
 {
     if (!p) return fail(h, COPRA_B200_E_ARG, "null problem");
     if (p->nx <= 0 || p->nu <= 0 || p->batch <= 0) return fail(h, COPRA_B200_E_ARG, "nx, nu and batch must be positive");
     if (p->N <= 0) return fail(h, COPRA_B200_E_ARG, "The number of step sould be a positive number!"); // PreviewSystem.cpp:31-33
-    if (!p->A.ptr || !p->B.ptr || !p->d.ptr || !p->x0.ptr) return fail(h, COPRA_B200_E_ARG, "A, B, d and x0 are required");
+    if (!p->x0.ptr || (!vectors_only && (!p->A.ptr || !p->B.ptr || !p->d.ptr))) return fail(h, COPRA_B200_E_ARG, "A, B, d and x0 are required");
     if (p->ncost < 0 || p->ncost > kMaxCost) return fail(h, COPRA_B200_E_ARG, "at most %d cost functions", kMaxCost);
     if (p->memory != COPRA_B200_HOST && p->memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
     const int nx = p->nx, nu = p->nu, N = p->N;
@@ -288,7 +298,8 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
     for (int i = 0; i < p->ncost; ++i) {
         const copra_b200_cost& c = p->costs[i];
         if (c.rows <= 0 || !c.p.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: rows must be positive and p given", i);
-        Plan::CostMeta m{ c.kind, c.rows, 0, 0, 0, 0, c.full_size ? 1 : 0 };
+        if (c.full_size < 0 || c.full_size > COPRA_B200_PER_STEP) return fail(h, COPRA_B200_E_ARG, "cost %d: full_size must be 0, 1 or COPRA_B200_PER_STEP", i);
+        Plan::CostMeta m{ c.kind, c.rows, 0, 0, 0, 0, c.full_size == 1 ? 1 : 0, 1, 0 };
         switch (c.kind) {
         case COPRA_B200_COST_TRAJECTORY: m.i0 = 0; m.i1 = N + 1; m.hasM = 1; break;
         case COPRA_B200_COST_TARGET: m.i0 = N; m.i1 = N + 1; m.hasM = 1; break;
@@ -296,9 +307,16 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
         case COPRA_B200_COST_MIXED: m.i0 = 0; m.i1 = N; m.hasM = 1; m.hasN = 1; break;
         default: return fail(h, COPRA_B200_E_ARG, "cost %d: unknown kind %d", i, c.kind);
         }
-        if (m.hasM && !c.M.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: M is required", i);
-        if (m.hasN && !c.N.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: N is required", i);
-        if (!c.w.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: weights are required (copra default: ones)", i);
+        if (!vectors_only) {
+            if (m.hasM && !c.M.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: M is required", i);
+            if (m.hasN && !c.N.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: N is required", i);
+            if (!c.w.ptr) return fail(h, COPRA_B200_E_ARG, "cost %d: weights are required (copra default: ones)", i);
+        }
+        if (c.full_size == COPRA_B200_PER_STEP) {
+            if (c.kind == COPRA_B200_COST_TARGET) return fail(h, COPRA_B200_E_ARG, "cost %d: a TargetCost has one step: it takes no per-step p", i);
+            m.vsteps = m.i1 - m.i0;
+            m.pstep = c.rows;
+        }
         if (m.dense) {
             if (c.kind == COPRA_B200_COST_TARGET) return fail(h, COPRA_B200_E_ARG, "cost %d: TargetCost takes a step-size M (xDim columns) only", i);
             m.i0 = 0; m.i1 = 1; // one stacked block
@@ -309,12 +327,18 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
     for (int i = 0; i < p->ncstr; ++i) {
         const copra_b200_constraint& c = p->cstrs[i];
         if (c.rows <= 0) return fail(h, COPRA_B200_E_ARG, "constraint %d: rows must be positive", i);
-        const bool full = c.full_size != 0;
+        if (c.full_size < 0 || c.full_size > COPRA_B200_PER_STEP)
+            return fail(h, COPRA_B200_E_ARG, "constraint %d: full_size must be 0, 1 or COPRA_B200_PER_STEP", i);
+        const bool full = c.full_size == 1, per_step = c.full_size == COPRA_B200_PER_STEP;
+        // steps of the horizon the constraint applies to: its vector holds that many copies when given per step
+        const int steps = (c.kind == COPRA_B200_CSTR_TRAJECTORY || c.kind == COPRA_B200_CSTR_TRAJECTORY_BOUND) ? N + 1 : N;
+        pl.cvsteps.push_back(per_step ? steps : 1);
         auto push = [&](int i0, int i1, int hasE, int hasG, bool iseq, int which, std::vector<int> lines) {
             Plan::FamMeta f;
             f.cstr = i; f.rows = lines.empty() ? c.rows : int(lines.size());
             f.dense = (full && which == 0) ? 1 : 0;
             f.gather = (full && which != 0) ? 1 : 0;
+            f.fstep = per_step ? c.rows : 0; // a trajectory bound's rows are nx: its vectors hold every line of a step
             if (full) { i0 = 0; i1 = 1; }
             f.i0 = i0; f.i1 = i1; f.hasE = hasE; f.hasG = hasG; f.is_eq = iseq ? 1 : 0; f.which = which;
             f.lines = std::move(lines);
@@ -325,25 +349,26 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
         };
         switch (c.kind) {
         case COPRA_B200_CSTR_TRAJECTORY:
-            if (!c.E.ptr || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: E and f are required", i);
+            if ((!vectors_only && !c.E.ptr) || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: E and f are required", i);
             push(0, N + 1, 1, 0, !c.is_ineq, 0, {});
             break;
         case COPRA_B200_CSTR_CONTROL:
-            if (!c.G.ptr || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: G and f are required", i);
+            if ((!vectors_only && !c.G.ptr) || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: G and f are required", i);
             push(0, N, 0, 1, !c.is_ineq, 0, {});
             break;
         case COPRA_B200_CSTR_MIXED:
-            if (!c.E.ptr || !c.G.ptr || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: E, G and f are required", i);
+            if ((!vectors_only && (!c.E.ptr || !c.G.ptr)) || !c.f.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: E, G and f are required", i);
             push(0, N, 1, 1, !c.is_ineq, 0, {});
             break;
         case COPRA_B200_CSTR_TRAJECTORY_BOUND: {
             if (!c.lower.ptr || !c.upper.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: lower and upper are required", i);
-            const int brows = full ? pl.sz.X : nx;
+            const int brows = full ? pl.sz.X : nx, count = brows * pl.cvsteps.back();
             if (c.rows != brows) return fail(h, COPRA_B200_E_ARG, "constraint %d: trajectory bounds must have xDim (or fullXDim) rows", i);
             // line selection (include/constraints.h:247-254) is part of the problem SHAPE: it is taken
-            // from instance 0 and, for host inputs, verified to be the same for every instance.
+            // from instance 0 and verified to be the same at every step of a per-step entry and, for host inputs, for every
+            // instance.
             std::vector<int> ll, ul;
-            copra_b200_handle::TbKey key{ c.lower.ptr, c.upper.ptr, brows };
+            copra_b200_handle::TbKey key{ c.lower.ptr, c.upper.ptr, brows, c.full_size };
             auto hit = h->tb_cache.find(key);
             // DEVICE inputs: the +-inf pattern is read back from instance 0 on EVERY build (one small D2H + sync) unless the
             // caller vouches with COPRA_B200_FLAG_STABLE_BOUND_PATTERN that it has not changed since the last build that
@@ -354,20 +379,21 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
                 ul = hit->second.second;
             } else {
                 std::vector<double> lo, up;
-                int rc = fetch_host(h, c.lower, brows, p->memory, lo);
+                int rc = fetch_host(h, c.lower, count, p->memory, lo);
                 if (rc) return rc;
-                rc = fetch_host(h, c.upper, brows, p->memory, up);
+                rc = fetch_host(h, c.upper, count, p->memory, up);
                 if (rc) return rc;
                 for (int l = 0; l < brows; ++l) if (lo[l] != -INFINITY) ll.push_back(l);
                 for (int l = 0; l < brows; ++l) if (up[l] != INFINITY) ul.push_back(l);
-                if (p->memory == COPRA_B200_HOST) {
-                    for (int b = 1; b < p->batch; ++b)
-                        for (int l = 0; l < brows; ++l) {
-                            const double a = c.lower.ptr[(long long)b * c.lower.stride + l], u = c.upper.ptr[(long long)b * c.upper.stride + l];
-                            if ((a != -INFINITY) != (lo[l] != -INFINITY) || (u != INFINITY) != (up[l] != INFINITY))
-                                return fail(h, COPRA_B200_E_ARG, "constraint %d: the set of infinite trajectory bounds must be the same for every instance", i);
-                        }
-                } else if (may_cache) {
+                const int nb = p->memory == COPRA_B200_HOST ? p->batch : 1;
+                for (int b = 0; b < nb; ++b)
+                    for (int l = 0; l < count; ++l) {
+                        const double a = b ? c.lower.ptr[(long long)b * c.lower.stride + l] : lo[l];
+                        const double u = b ? c.upper.ptr[(long long)b * c.upper.stride + l] : up[l];
+                        if ((a != -INFINITY) != (lo[l % brows] != -INFINITY) || (u != INFINITY) != (up[l % brows] != INFINITY))
+                            return fail(h, COPRA_B200_E_ARG, "constraint %d: the set of infinite trajectory bounds must be the same at every step and for every instance", i);
+                    }
+                if (may_cache) {
                     if (h->tb_cache.size() > 64) h->tb_cache.clear();
                     h->tb_cache[key] = std::make_pair(ll, ul);
                 }
@@ -378,7 +404,7 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
         case COPRA_B200_CSTR_CONTROL_BOUND:
             if (!c.lower.ptr || !c.upper.ptr) return fail(h, COPRA_B200_E_ARG, "constraint %d: lower and upper are required", i);
             if (c.rows != (full ? pl.sz.nU : nu)) return fail(h, COPRA_B200_E_ARG, "constraint %d: control bounds must have uDim (or fullUDim) rows", i);
-            pl.cb_full = full ? 1 : 0;
+            pl.cb_full = (full || per_step) ? 1 : 0; // a per-step lower / upper holds the nU entries of a full-size one
             if (pl.bound_cstr >= 0) return fail(h, COPRA_B200_E_UNSUPPORTED, "only one ControlBoundConstraint per controller (reference quirk Q8)");
             pl.bound_cstr = i;
             break;
@@ -390,6 +416,66 @@ int make_plan(copra_b200_handle* h, const copra_b200_problem* p, Plan& pl)
     pl.sz.mineq = in_off;
     pl.sz.q = eq_off + in_off + 2 * pl.sz.nvar;
     return 0;
+}
+
+// Everything a build fixes besides the matrices: dimensions, every entry's kind, rows, form and inequality sense, and the
+// trajectory-bound line selections.  A retarget must find it unchanged.
+std::vector<int> shape_key(const copra_b200_problem* p, const Plan& pl)
+{
+    std::vector<int> k{ p->nx, p->nu, p->N, p->batch, p->initial_state ? 1 : 0, p->ncost, p->ncstr };
+    for (int i = 0; i < p->ncost; ++i) k.insert(k.end(), { p->costs[i].kind, p->costs[i].rows, p->costs[i].full_size });
+    for (int i = 0; i < p->ncstr; ++i) {
+        const copra_b200_constraint& c = p->cstrs[i];
+        const bool rowcs = c.kind != COPRA_B200_CSTR_TRAJECTORY_BOUND && c.kind != COPRA_B200_CSTR_CONTROL_BOUND;
+        k.insert(k.end(), { c.kind, c.rows, c.full_size, rowcs ? (c.is_ineq ? 1 : 0) : 0 });
+    }
+    for (const auto& f : pl.fams) {
+        k.push_back(int(f.lines.size()));
+        k.insert(k.end(), f.lines.begin(), f.lines.end());
+    }
+    return k;
+}
+
+// The per-instance vectors of a problem: x0, every cost's p, every constraint's f / lower / upper (rows x steps doubles
+// per instance for a per-step entry).  A build uploads them with its matrices, a retarget alone.
+struct BoundArrs { std::vector<DArr> lower, upper; };
+
+void add_vectors(Upload& U, const copra_b200_problem* p, const Plan& pl, BuildParams& P, BoundArrs& ba)
+{
+    U.add(p->x0, P.nx, &P.x0);
+    for (int i = 0; i < P.ncost; ++i) {
+        const copra_b200_cost& c = p->costs[i];
+        U.add(c.p, size_t(c.rows) * pl.costs[i].vsteps, &P.cost[i].p);
+    }
+    // trajectory-bound families share the uploaded lower / upper vectors of their constraint
+    ba.lower.assign(p->ncstr, DArr{ nullptr, 0 });
+    ba.upper.assign(p->ncstr, DArr{ nullptr, 0 });
+    for (int i = 0; i < p->ncstr; ++i) {
+        const copra_b200_constraint& c = p->cstrs[i];
+        if (c.kind == COPRA_B200_CSTR_TRAJECTORY_BOUND || c.kind == COPRA_B200_CSTR_CONTROL_BOUND) {
+            U.add(c.lower, size_t(c.rows) * pl.cvsteps[i], &ba.lower[i]);
+            U.add(c.upper, size_t(c.rows) * pl.cvsteps[i], &ba.upper[i]);
+        }
+    }
+    for (int k = 0; k < P.nfam; ++k) {
+        const auto& f = pl.fams[k];
+        const copra_b200_constraint& c = p->cstrs[f.cstr];
+        if (f.which == 0) U.add(c.f, size_t(c.rows) * pl.cvsteps[f.cstr], &P.fam[k].f);
+    }
+}
+
+// after run_upload: point the bound families and the control bounds at the uploaded lower / upper
+void bind_bounds(const Plan& pl, BuildParams& P, const BoundArrs& ba)
+{
+    for (int k = 0; k < P.nfam; ++k) {
+        const auto& f = pl.fams[k];
+        if (f.which != 0) P.fam[k].f = f.which == 1 ? ba.lower[f.cstr] : ba.upper[f.cstr];
+    }
+    if (pl.bound_cstr >= 0) {
+        P.cb_lower = ba.lower[pl.bound_cstr];
+        P.cb_upper = ba.upper[pl.bound_cstr];
+        P.cb_full = pl.cb_full;
+    }
 }
 
 template <class T> int ws(copra_b200_handle* h, const char* name, size_t count, T** out)
@@ -689,7 +775,7 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
     bool q_shared = !p->initial_state && p->A.stride == 0 && p->B.stride == 0 && B > 1;
     for (int i = 0; i < p->ncost && q_shared; ++i) {
         const copra_b200_cost& c = p->costs[i];
-        if (c.full_size || (c.M.ptr && c.M.stride != 0) || (c.N.ptr && c.N.stride != 0) || c.w.stride != 0) q_shared = false;
+        if (c.full_size == 1 || (c.M.ptr && c.M.stride != 0) || (c.N.ptr && c.N.stride != 0) || c.w.stride != 0) q_shared = false;
     }
     if (getenv("COPRA_B200_NO_SHARED_HESSIAN")) q_shared = false;
     P.sQ = q_shared ? 0 : (long long)pl.sz.nvar * pl.sz.nvar;
@@ -729,7 +815,6 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
     U.add(p->A, size_t(nx) * nx, &P.A);
     U.add(p->B, size_t(nx) * nu, &P.B);
     U.add(p->d, nx, &P.d);
-    U.add(p->x0, nx, &P.x0);
     if (p->initial_state) {
         U.add(p->R, size_t(nx) * nx, &P.R);
         U.add(p->r, nx, &P.r);
@@ -741,33 +826,25 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
         CostFam& F = P.cost[i];
         F.rows = c.rows; F.i0 = pl.costs[i].i0; F.i1 = pl.costs[i].i1; F.hasM = pl.costs[i].hasM; F.hasN = pl.costs[i].hasN;
         F.dense = pl.costs[i].dense;
+        F.pstep = pl.costs[i].pstep;
         if (F.hasM) U.add(c.M, size_t(c.rows) * (F.dense ? pl.sz.X : nx), &F.M);
         if (F.hasN) U.add(c.N, size_t(c.rows) * (F.dense ? pl.sz.nU : nu), &F.N);
-        U.add(c.p, c.rows, &F.p);
         U.add(c.w, c.rows, &F.w);
-    }
-    // trajectory-bound families share the uploaded lower / upper vectors of their constraint
-    std::vector<DArr> lowerArr(p->ncstr), upperArr(p->ncstr);
-    for (int i = 0; i < p->ncstr; ++i) {
-        const copra_b200_constraint& c = p->cstrs[i];
-        if (c.kind == COPRA_B200_CSTR_TRAJECTORY_BOUND || c.kind == COPRA_B200_CSTR_CONTROL_BOUND) {
-            U.add(c.lower, c.rows, &lowerArr[i]);
-            U.add(c.upper, c.rows, &upperArr[i]);
-        }
     }
     for (int k = 0; k < P.nfam; ++k) {
         const auto& f = pl.fams[k];
         const copra_b200_constraint& c = p->cstrs[f.cstr];
         CstrFam& F = P.fam[k];
         F.rows = f.rows; F.i0 = f.i0; F.i1 = f.i1; F.hasE = f.hasE; F.hasG = f.hasG; F.is_eq = f.is_eq; F.row_off = f.row_off;
-        F.dense = f.dense; F.gather = f.gather;
+        F.dense = f.dense; F.gather = f.gather; F.fstep = f.fstep;
         F.fidx = nullptr;
         if (f.which == 0) {
             if (f.hasE) U.add(c.E, size_t(c.rows) * (f.dense ? pl.sz.X : nx), &F.E);
             if (f.hasG) U.add(c.G, size_t(c.rows) * (f.dense ? pl.sz.nU : nu), &F.G);
-            U.add(c.f, c.rows, &F.f);
         }
     }
+    BoundArrs ba;
+    add_vectors(U, p, pl, P, ba);
     rc = run_upload(h, U, B, p->memory, "params");
     if (rc) return rc;
     for (int k = 0; k < P.nfam; ++k) {
@@ -776,14 +853,9 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
         CstrFam& F = P.fam[k];
         F.E.p = f.gather ? nullptr : d_sel + sel_off[k];
         F.E.s = 0;
-        F.f = f.which == 1 ? lowerArr[f.cstr] : upperArr[f.cstr];
         F.fidx = d_lines + line_off[k];
     }
-    if (pl.bound_cstr >= 0) {
-        P.cb_lower = lowerArr[pl.bound_cstr];
-        P.cb_upper = upperArr[pl.bound_cstr];
-        P.cb_full = pl.cb_full;
-    }
+    bind_bounds(pl, P, ba);
     rc = record(h, 1);
     if (rc) return rc;
 
@@ -857,6 +929,7 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
     LAUNCHED(k2k4_assemble_launch(P, schur, schur_stride, h->sms, h->smem_optin, h->stream));
     if ((rc = record(h, 3))) return rc;
     h->sz = pl.sz;
+    h->shape = shape_key(p, pl);
     h->built = true;
     h->factor_valid = false;
     h->warm_valid = false;
@@ -1165,6 +1238,44 @@ int copra_b200_lmpc_resolve(copra_b200_handle* h, copra_b200_array x0, int memor
     if ((rc = run_upload(h, U, P.batch, memory, "params_x0"))) return rc; // its own buffer: the other parameters stay resident
     if ((rc = record(h, 1))) return rc;
     if ((rc = record(h, 2))) return rc;
+    LAUNCHED(k4_finalize_launch(P, h->sms, h->stream));
+    if ((rc = record(h, 3))) return rc;
+    h->in_resolve = true;
+    rc = do_solve(h, r);
+    h->in_resolve = false;
+    return rc;
+}
+
+int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, const copra_b200_results* r)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_retarget needs a previous build on this handle");
+    BuildParams& P = h->bp;
+    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget is defined for LMPC mode only");
+    for (int i = 0; i < P.ncost; ++i)
+        if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget: cost %d is a full-size entry (its f comes out of the dense GEMMs)", i);
+    for (int k = 0; k < P.nfam; ++k)
+        if (P.fam[k].dense || P.fam[k].gather)
+            return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget: a row constraint is a full-size entry (its b comes out of the dense GEMMs)");
+    // everything is validated before BuildParams changes: a refused retarget leaves the resident build usable
+    Plan pl;
+    int rc = make_plan(h, p, pl, true);
+    if (rc) return rc;
+    if (shape_key(p, pl) != h->shape)
+        return fail(h, COPRA_B200_E_ARG, "retarget: the problem's shape (dimensions, batch, entries, +-inf bound pattern) differs from the resident build");
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    for (bool& v : h->ev_valid) v = false;
+    if ((rc = record(h, 0))) return rc;
+    Upload U;
+    BoundArrs ba;
+    add_vectors(U, p, pl, P, ba);
+    // its own buffer: the matrices stay resident in the build's
+    if ((rc = run_upload(h, U, P.batch, p->memory, "params_vec"))) return rc;
+    bind_bounds(pl, P, ba);
+    if ((rc = record(h, 1))) return rc;
+    if ((rc = record(h, 2))) return rc;
+    LAUNCHED(k2_retarget_launch(P, h->sms, h->stream));
     LAUNCHED(k4_finalize_launch(P, h->sms, h->stream));
     if ((rc = record(h, 3))) return rc;
     h->in_resolve = true;

@@ -169,4 +169,26 @@ int copra_b200_multi_lmpc_resolve(copra_b200_multi* m, copra_b200_array x0, cons
     });
 }
 
+int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem* p, const copra_b200_results* r)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!p) return mfail(m, COPRA_B200_E_ARG, "null problem");
+    if (p->memory != COPRA_B200_HOST || (r && r->memory != COPRA_B200_HOST))
+        return mfail(m, COPRA_B200_E_ARG, "the multi-device entry takes HOST arrays (each shard is uploaded to its own device)");
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_retarget needs a previous run");
+    if (p->batch != m->hi.back()) return mfail(m, COPRA_B200_E_ARG, "retarget: the batch differs from the resident run's");
+    return run_shards(m, [&](int g) {
+        ProblemSlice q;
+        slice_problem(*p, m->lo[g], m->hi[g] - m->lo[g], q);
+        copra_b200_results rr{};
+        if (r) {
+            copra_b200_sizes sz{};
+            const int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+            if (rc) return rc;
+            rr = slice_results(*r, m->lo[g], sz);
+        }
+        return copra_b200_lmpc_retarget(m->h[g], &q.p, r ? &rr : nullptr);
+    });
+}
+
 } // extern "C"

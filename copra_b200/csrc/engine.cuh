@@ -9,6 +9,8 @@
 // which covers the four step-size costs (src/costFunctions.cpp:63-215) and the four step-size row
 // constraints (src/constraints.cpp:66-315); TrajectoryBoundConstraint becomes up to two selector
 // families (lower lines first, then upper lines -- quirk Q1 keeps the lower rows un-negated).
+// res_i = M xi_i - p_i and the right-hand side f_i may differ from step to step (COPRA_B200_PER_STEP: pstep / fstep); the
+// matrices, hence the Hessian and the rows, may not.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -28,6 +30,7 @@ struct DArr { // (pointer, batch stride) on the device
 
 struct CostFam {
     int dense;      // 1: full-size entry: M is rows x X, N rows x nU; evaluated by the DMMA GEMM path
+    int pstep;      // doubles between the p of consecutive steps (per-step vector, COPRA_B200_PER_STEP); 0 = one p for every step
     double* T;      // dense: rows x nU   T = M Psi (+ N)
     double* WT;     // dense: rows x nU   diag(w) T
     long long sT;
@@ -52,6 +55,7 @@ struct CstrFam {
     int hasE, hasG;
     int is_eq;
     int row_off;    // first row inside Aeq (is_eq) or Aineq
+    int fstep;      // doubles between the f of consecutive steps (per-step vector; nx for a trajectory bound); 0 = one f
     DArr E, G, f;
     const int* fidx; // optional gather of f (TrajectoryBound: line numbers), device, `rows` entries
     double* EGx;    // r x nu x (N+1): block k+1 = E A^k B, block 0 = G (or 0)
@@ -67,7 +71,7 @@ struct BuildParams {
     DArr A, B, d, x0;
     DArr R, r, x0lb, x0ub;        // initial-state mode (p may be null)
     DArr cb_lower, cb_upper;      // ControlBoundConstraint (p null = none)
-    int cb_full;                  // 1: lower/upper hold nU entries (full-size entry)
+    int cb_full;                  // 1: lower/upper hold nU entries (full-size or per-step entry)
     int skip_rows;                // 1: Aeq / Aineq are not materialised by the build (structured solver; filled on demand)
     double* PsiFull;              // X x nU per instance, only materialised when a full-size entry needs it
     // K1 outputs (workspace, per instance)

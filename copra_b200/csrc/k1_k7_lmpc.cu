@@ -225,7 +225,10 @@ int k1_psi_fill_launch(const double* Gs, long long sGs, double* Psi, int nx, int
 //   cstr  : EGx[kk] likewise with E/G ; Y rows = E Phi_i ; z rows = f - E xi_i
 // (reference: tmp = M_*Psi.block(..), M_*Phi.block(..), M_*xi.segment(..)-p_  src/costFunctions.cpp:74-78;
 //  E_*Psi.block, E_*Phi.block, f_-E_*xi.segment  src/constraints.cpp:77-81)
+// p and f are the only per-step inputs (pstep / fstep > 0: step i reads its own vector).  VEC_ONLY: res and z alone, for a
+// retarget of a resident build whose matrices did not change (MGx, MPhi, EGx and Y are kept).
 // ------------------------------------------------------------------------------------------------
+template <bool VEC_ONLY>
 __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
 {
     const int nx = P.nx, nu = P.nu, N = P.N, X = P.X;
@@ -245,7 +248,7 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
             double* MGx = F.MGx + (long long)b * F.sMGx;
             double* MPhi = F.MPhi + (long long)b * F.sMPhi;
             double* res = F.res + (long long)b * F.sres;
-            for (int t = tid; t < r * nu * (N + 1); t += T) {
+            for (int t = tid; t < r * nu * (N + 1) && !VEC_ONLY; t += T) {
                 const int l = t % r, bb = (t / r) % nu, kk = t / (r * nu);
                 double s = 0.0;
                 if (kk == 0) s = Nn ? Nn[l + bb * r] : 0.0;
@@ -255,7 +258,7 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
                 }
                 MGx[t] = s;
             }
-            for (int t = tid; t < r * nx * ns; t += T) {
+            for (int t = tid; t < r * nx * ns && !VEC_ONLY; t += T) {
                 const int l = t % r, sidx = (t / r) % nx, ii = t / (r * nx);
                 double s = 0.0;
                 if (M) {
@@ -266,12 +269,13 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
             }
             for (int t = tid; t < r * ns; t += T) {
                 const int l = t % r, ii = t / r;
+                const double pl = p[(F.i0 + ii) * F.pstep + l];
                 double s = 0.0;
                 if (M) {
                     const double* xv = xi + (long long)(F.i0 + ii) * nx;
                     for (int k = 0; k < nx; ++k) s = add_(s, mul_(M[l + k * r], xv[k]));
-                    s = add_(s, -p[l]);
-                } else s = -p[l];
+                    s = add_(s, -pl);
+                } else s = -pl;
                 res[t] = s;
             }
         }
@@ -286,7 +290,7 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
             const int mtot = F.is_eq ? P.meq : P.mineq;
             double* Y = (F.is_eq ? P.Yeq : P.Yin) + (long long)b * mtot * nx;
             double* z = (F.is_eq ? P.zeq : P.zin) + (long long)b * mtot;
-            for (int t = tid; t < r * nu * (N + 1); t += T) {
+            for (int t = tid; t < r * nu * (N + 1) && !VEC_ONLY; t += T) {
                 const int l = t % r, bb = (t / r) % nu, kk = t / (r * nu);
                 double s = 0.0;
                 if (kk == 0) s = G ? G[l + bb * r] : 0.0;
@@ -296,7 +300,7 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
                 }
                 EGx[t] = s;
             }
-            for (int t = tid; t < r * nx * ns; t += T) {
+            for (int t = tid; t < r * nx * ns && !VEC_ONLY; t += T) {
                 const int l = t % r, ii = (t / r) % ns, sidx = t / (r * ns);
                 double s = 0.0;
                 if (E) {
@@ -307,7 +311,7 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
             }
             for (int t = tid; t < r * ns; t += T) {
                 const int l = t % r, ii = t / r;
-                const double fl = f[F.fidx ? F.fidx[l] : l];
+                const double fl = f[(F.i0 + ii) * F.fstep + (F.fidx ? F.fidx[l] : l)];
                 double s = 0.0;
                 if (E) {
                     const double* xv = xi + (long long)(F.i0 + ii) * nx;
@@ -319,9 +323,9 @@ __device__ __forceinline__ void dev_precompute(const BuildParams& P, int b)
     }
 }
 
-__global__ void k2_precompute_kernel(const __grid_constant__ BuildParams P)
+template <bool VEC_ONLY> __global__ void k2_precompute_kernel(const __grid_constant__ BuildParams P)
 {
-    for (int b = blockIdx.x; b < P.batch; b += gridDim.x) dev_precompute(P, b);
+    for (int b = blockIdx.x; b < P.batch; b += gridDim.x) dev_precompute<VEC_ONLY>(P, b);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -533,15 +537,16 @@ __device__ __forceinline__ void dev_ef(const BuildParams& P, int b, int t, int c
     (void)nU;
 }
 
-// grid = (tiles over (nx+1) nU, batch, cost); STAGED: this cost's tables are first copied to shared memory
-template <bool STAGED> __global__ void k2_assemble_ef_kernel(const __grid_constant__ BuildParams P)
+// grid = (tiles over (nx+1) nU, batch, cost); STAGED: this cost's tables are first copied to shared memory.
+// f_all: every instance forms only f (a retarget: E is resident and unchanged)
+template <bool STAGED> __global__ void k2_assemble_ef_kernel(const __grid_constant__ BuildParams P, int f_all)
 {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int b = blockIdx.y, ci = blockIdx.z;
     const CostFam& F = P.cost[ci];
     if (F.dense) return;
     // batch-invariant E (sE == 0): instance 0 forms E and its f, every other instance only its nU entries of f
-    const bool f_only = F.sE == 0 && b > 0;
+    const bool f_only = (F.sE == 0 && b > 0) || f_all;
     if (f_only) {
         if (blockIdx.x * blockDim.x >= P.nU) return;
         t = (t < P.nU) ? t * (P.nx + 1) + P.nx : (P.nx + 1) * P.nU; // (s, col) = (nx, t)
@@ -900,6 +905,20 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
         launches += n_;                                \
     } while (0)
 
+// K2c for every step-size cost (f_all: f alone, see k2_assemble_ef_kernel)
+static int ef_launch(const BuildParams& P, int f_all, cudaStream_t st)
+{
+    size_t need = 0; // largest single cost: its M A^k B, M Phi_i, residual tables and weights
+    for (int i = 0; i < P.ncost; ++i)
+        if (!P.cost[i].dense)
+            need = std::max(need, size_t(P.cost[i].sMGx) + size_t(P.cost[i].sMPhi) + size_t(P.cost[i].sres) + P.cost[i].rows);
+    const dim3 grid(ceil_div(f_all ? P.nU : (P.nx + 1) * P.nU, 128), P.batch, P.ncost);
+    if (need * sizeof(double) <= 40 * 1024) k2_assemble_ef_kernel<true><<<grid, 128, need * sizeof(double), st>>>(P, f_all);
+    else k2_assemble_ef_kernel<false><<<grid, 128, 0, st>>>(P, f_all);
+    cudaError_t e = cudaGetLastError();
+    return e == cudaSuccess ? 1 : -int(e);
+}
+
 int k2k4_assemble_launch(const BuildParams& P, double* schur_ws, long long schur_stride, int sms, size_t smem_optin, cudaStream_t st)
 {
     int launches = 0;
@@ -910,7 +929,7 @@ int k2k4_assemble_launch(const BuildParams& P, double* schur_ws, long long schur
     bool any_dense = false;
     for (int i = 0; i < P.ncost; ++i) any_dense |= P.cost[i].dense && P.cost[i].hasM;
     for (int k = 0; k < P.nfam; ++k) any_dense |= P.fam[k].dense && P.fam[k].hasE;
-    k2_precompute_kernel<<<pgrid, 128, 0, st>>>(P);
+    k2_precompute_kernel<false><<<pgrid, 128, 0, st>>>(P);
     CB_CHECK_LAUNCH();
     if (any_dense) { // dense M / E blocks multiply the materialised Psi
         int n_ = k1_psi_fill_launch(P.Gs, (long long)P.N * nx * P.nu, P.PsiFull, nx, P.nu, P.N, nb, st);
@@ -950,14 +969,9 @@ int k2k4_assemble_launch(const BuildParams& P, double* schur_ws, long long schur
         CB_GEMM(1, 1, nU, R, 1.0, F.res, R, F.sres, F.WT, R, F.sT, 0.0, F.f, 1, F.sf, nb, st);
     }
     if (P.ncost > 0) {
-        size_t need = 0; // largest single cost: its M A^k B, M Phi_i, residual tables and weights
-        for (int i = 0; i < P.ncost; ++i)
-            if (!P.cost[i].dense)
-                need = std::max(need, size_t(P.cost[i].sMGx) + size_t(P.cost[i].sMPhi) + size_t(P.cost[i].sres) + P.cost[i].rows);
-        const dim3 grid(ceil_div((nx + 1) * nU, 128), nb, P.ncost);
-        if (need * sizeof(double) <= 40 * 1024) k2_assemble_ef_kernel<true><<<grid, 128, need * sizeof(double), st>>>(P);
-        else k2_assemble_ef_kernel<false><<<grid, 128, 0, st>>>(P);
-        CB_CHECK_LAUNCH();
+        const int n_ = ef_launch(P, 0, st);
+        if (n_ < 0) return n_;
+        launches += n_;
     }
     for (int fi = 0; fi < P.nfam; ++fi) { // full-size constraints: rows = E Psi (+G), Y = E Phi, z = f - E xi
         const CstrFam& F = P.fam[fi];
@@ -1008,6 +1022,20 @@ int k2k4_assemble_launch(const BuildParams& P, double* schur_ws, long long schur
         const int grid = std::min(P.batch, sms * per_sm);
         k4_schur_kernel<<<grid, threads, smem, st>>>(P, schur_ws, schur_stride, j_smem);
         CB_CHECK_LAUNCH();
+    }
+    return launches;
+}
+
+int k2_retarget_launch(const BuildParams& P, int sms, cudaStream_t st)
+{
+    if (P.batch > 65535) return -int(cudaErrorInvalidValue);
+    int launches = 0;
+    k2_precompute_kernel<true><<<std::min(P.batch, sms * 8), 128, 0, st>>>(P);
+    CB_CHECK_LAUNCH();
+    if (P.ncost > 0) {
+        const int n_ = ef_launch(P, 1, st);
+        if (n_ < 0) return n_;
+        launches += n_;
     }
     return launches;
 }

@@ -56,6 +56,8 @@ int dgemm_dmma_launch(int transA, int M, int N, int K, double alpha, const doubl
 int fp64_peaks_measure(int sms, double* scratch, cudaStream_t st, double* dfma_tflops, double* dmma_tflops);
 // K3 alone: materialise the step-size rows of Aeq / Aineq (skipped by builds whose solver evaluates them from the tables)
 int k3_fill_rows_launch(const BuildParams& P, cudaStream_t st);
+// K2 for new per-instance vectors on a resident build: res / z (K2a) and every cost's f (K2c); Q, E, Y, the tables stay
+int k2_retarget_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k4_finalize_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k7_results_launch(const BuildParams& P, const double* x, double* control, double* trajectory, cudaStream_t st);
 

@@ -10,6 +10,9 @@ A *batch problem* is a dict:
     costs       = [dict(kind, M, N, p, w)]          arrays carry a leading batch axis when they
     constraints = [dict(kind, E, G, f, lower, upper, is_ineq)]     differ per instance
     R, r, x0lb, x0ub (initial-state mode only)
+A cost or constraint with `per_step=True` keeps step-size matrices and holds one vector per step (p, f, lower / upper
+of rows x steps entries, step-major: COPRA_B200_PER_STEP); spanned() gives the same problem in copra's autoSpan'd
+full-size form.
 Matrices are in logical (rows, cols) shape; the C ABI / oracle wrappers do the column-major
 conversion.  Reference fixtures cited per config.
 """
@@ -194,6 +197,83 @@ def c5(batch=1024, seed_offset=0, N=200, T=0.01):
                dict(kind="control", N=np.eye(nu), p=np.zeros(nu), w=np.full(nu, 1e-3))],
         constraints=[dict(kind="trajectory", E=E, f=np.full(8, 0.6)),
                      dict(kind="control_bound", lower=np.full(nu, -5.0), upper=np.full(nu, 5.0))])
+
+
+def c3_walk(batch=16384, seed_offset=0, N=160, T=0.01, tick=0):
+    """C3 walking: c3(...) unchanged (same system, weights, E, x0 and draws) plus a footstep plan, so that the ZMP box and
+    the velocity reference move over the horizon as in a walking pattern generator.  Per instance, from config 6's stream:
+    a step period of 0.4-0.6 s, a step length of 0.10-0.20 m, a lateral offset of 0.02-0.05 m and the phase of the first
+    step (0.1 s plus up to one period).  The ZMP box stays centred at 0 until the first step (x0 is feasible at step 0);
+    from there its centre advances by one step length per step and alternates sides.  The forward velocity reference ramps
+    from 0 to the mean walking speed (step length / period) at the first step and stays there; the lateral one is 0.
+    The MixedConstraint's f and the TrajectoryCost's p are per-step entries.  `tick` > 0 is the same plan seen `tick` control
+    periods later (the next windows of a receding horizon; x0 stays c3's).  With these draws every instance of the default
+    batch solves (status 0)."""
+    bp = c3(batch, seed_offset, N, T)
+    rng = SplitMix64(_seed(6, seed_offset))
+    draws = rng.uniform(0.0, 1.0, (batch, 4))
+    period = 0.4 + 0.2 * draws[:, 0]
+    length = 0.10 + 0.10 * draws[:, 1]
+    lateral = 0.02 + 0.03 * draws[:, 2]
+    first = 0.1 + period * draws[:, 3]
+    t = (np.arange(N + 1) + tick) * T
+    k = np.where(t[None, :] < first[:, None], 0, 1 + np.floor((t[None, :] - first[:, None]) / period[:, None]))  # steps taken
+    cx = k * length[:, None]
+    cy = np.where(k == 0, 0.0, np.where(k % 2 == 1, 1.0, -1.0)) * lateral[:, None]
+    hw = np.asarray(bp["constraints"][0]["f"])[:, [0, 2]]
+    f = np.stack([hw[:, :1] + cx, hw[:, :1] - cx, hw[:, 1:] + cy, hw[:, 1:] - cy], axis=2)[:, :N]  # (batch, N, 4)
+    speed = length / period
+    vref = np.zeros((batch, N + 1, 2))
+    vref[:, :, 0] = speed[:, None] * np.minimum(1.0, t[None, :] / first[:, None])
+    bp["name"] = "C3-walk"
+    bp["costs"][0] = dict(bp["costs"][0], p=vref.reshape(batch, -1), per_step=True)
+    bp["constraints"][0] = dict(bp["constraints"][0], f=f.reshape(batch, -1), per_step=True)
+    return bp
+
+
+def _span(M, steps, add_cols=0):
+    """block-diagonal copies of the (..., r, c) step matrix M at `steps` steps, `add_cols` zero column blocks appended
+    (AutoSpan::spanMatrix)"""
+    M = np.asarray(M, dtype=np.float64)
+    M = M.reshape(M.shape[:-1] + (1, M.shape[-1])) if M.ndim == 1 else M
+    r, c = M.shape[-2:]
+    out = np.zeros(M.shape[:-2] + (r * steps, c * (steps + add_cols)))
+    for i in range(steps):
+        out[..., i * r:(i + 1) * r, i * c:(i + 1) * c] = M
+    return out
+
+
+def spanned(bp):
+    """The same batch problem with every per-step entry in copra's full-size form: autoSpan'd block-diagonal matrices,
+    weights tiled over the steps, and its full-length vector."""
+    N = bp["N"]
+    out = dict(bp)
+    costs = []
+    for c in bp["costs"]:
+        c = dict(c)
+        if c.pop("per_step", False):
+            steps = N + 1 if c["kind"] == "trajectory" else N
+            add = 1 if c["kind"] == "mixed" else 0
+            if c.get("M") is not None:
+                c["M"] = _span(c["M"], steps, add)
+            if c.get("N") is not None:
+                c["N"] = _span(c["N"], steps)
+            w = np.asarray(c["w"], dtype=np.float64)
+            c["w"] = np.tile(w, (1,) * (w.ndim - 1) + (steps,))
+        costs.append(c)
+    cstrs = []
+    for c in bp["constraints"]:
+        c = dict(c)
+        if c.pop("per_step", False) and c["kind"] not in ("trajectory_bound", "control_bound"):
+            steps = N + 1 if c["kind"] == "trajectory" else N
+            add = 1 if c["kind"] == "mixed" else 0
+            if c.get("E") is not None:
+                c["E"] = _span(c["E"], steps, add)
+            if c.get("G") is not None:
+                c["G"] = _span(c["G"], steps)
+        cstrs.append(c)
+    out["costs"], out["constraints"] = costs, cstrs
+    return out
 
 
 CONFIGS = {"c1": c1, "c2": c2, "c3": c3, "c4": c4, "c5": c5}

@@ -1060,6 +1060,9 @@ public:
     void system(copra_b200_array A, copra_b200_array B, copra_b200_array d, copra_b200_array x0) { p_.A = A; p_.B = B; p_.d = d; p_.x0 = x0; }
     void initialStateCost(copra_b200_array R, copra_b200_array r) { p_.R = R; p_.r = r; }
     void initialStateBounds(copra_b200_array lo, copra_b200_array up) { p_.x0lb = lo; p_.x0ub = up; }
+    // full_size = COPRA_B200_PER_STEP: step-size matrices and a p / f / lower / upper with one vector per step (rows x steps
+    // entries, step-major: the layout of AutoSpan::spanVector) -- references and limits that move over the horizon, on the
+    // kernels of a step-size entry.  The descriptors are kept: retarget() re-reads the vectors they point to.
     int addCost(const copra_b200_cost& c) { costs_.push_back(c); return int(costs_.size()) - 1; }
     int addConstraint(const copra_b200_constraint& c) { cstrs_.push_back(c); return int(cstrs_.size()) - 1; }
     ~BatchedLMPC() { if (multi_) copra_b200_multi_destroy(multi_); }
@@ -1147,6 +1150,32 @@ public:
         copra_b200_timing tm{};
         copra_b200_last_timing(b200::handle(), &tm);
         solveTime_ = tm.solve_ms * 1e-3;
+        solveAndBuildTime_ = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
+        return int(std::count(status_.begin(), status_.end(), 0));
+    }
+    // Receding-horizon step with new references and limits: new initial states, and the vectors (p, f, lower / upper) the
+    // cost and constraint descriptors point to are read again; the matrices of the resident build are reused
+    // (copra_b200_lmpc_retarget).  Falls back to solve() where resolve() does, and for full-size entries (their vector terms
+    // are part of the dense assembly).
+    int retarget(copra_b200_array x0)
+    {
+        p_.x0 = x0;
+        bool dense = false;
+        for (const auto& c : costs_) dense |= c.full_size == 1;
+        for (const auto& c : cstrs_) dense |= c.full_size == 1 && c.kind != COPRA_B200_CSTR_CONTROL_BOUND;
+        if (dense || p_.initial_state || p_.batch > 65535 || (multi_ ? !multiBuilt_ : myEpoch_ != b200::buildEpoch())) return solve();
+        const auto t0 = std::chrono::high_resolution_clock::now();
+        copra_b200_results R{};
+        R.control = controls_.data(); R.trajectory = trajectories_.data(); R.status = status_.data(); R.iters = iterations_.data();
+        R.nact = nact_.data(); R.iact = iact_.data(); R.memory = COPRA_B200_HOST;
+        if (multi_) {
+            if (copra_b200_multi_lmpc_retarget(multi_, finish(), &R)) throw std::runtime_error(copra_b200_multi_last_error(multi_));
+        } else {
+            b200::check(copra_b200_lmpc_retarget(b200::handle(), finish(), &R));
+            copra_b200_timing tm{};
+            copra_b200_last_timing(b200::handle(), &tm);
+            solveTime_ = tm.solve_ms * 1e-3;
+        }
         solveAndBuildTime_ = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
         return int(std::count(status_.begin(), status_.end(), 0));
     }
