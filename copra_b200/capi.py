@@ -59,6 +59,11 @@ class Results(C.Structure):
                 ("iters", C.c_void_p), ("nact", C.c_void_p), ("iact", C.c_void_p), ("memory", C.c_int)]
 
 
+class VjpOut(C.Structure):
+    _fields_ = [("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
+                ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
+
+
 class Timing(C.Structure):
     _fields_ = [(k, C.c_float) for k in ("h2d_ms", "condense_ms", "assemble_ms", "solve_ms", "rollout_ms", "d2h_ms",
                                          "total_ms")] + [("launches", C.c_longlong)]
@@ -73,7 +78,9 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_multi_last_error", "copra_b200_multi_size", "copra_b200_multi_shard", "copra_b200_multi_timing",
            "copra_b200_multi_launch_count", "copra_b200_multi_lmpc_run", "copra_b200_multi_lmpc_resolve",
            "copra_b200_set_warm_start", "copra_b200_get_warm_start", "copra_b200_multi_set_warm_start",
-           "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget"]
+           "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget", "copra_b200_lmpc_vjp",
+           "copra_b200_multi_lmpc_vjp"]
+VJP_WANT = ("x0", "p", "f", "lower", "upper")
 
 _lib = None
 
@@ -138,6 +145,8 @@ def load():
         lib.copra_b200_multi_lmpc_resolve.argtypes = [C.c_void_p, Array, C.POINTER(Results)]
         lib.copra_b200_multi_lmpc_retarget.argtypes = [C.c_void_p, C.POINTER(Problem), C.POINTER(Results)]
         lib.copra_b200_multi_set_warm_start.argtypes = [C.c_void_p, C.c_int]
+        lib.copra_b200_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut)]
+        lib.copra_b200_multi_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut)]
         _lib = lib
     return _lib
 
@@ -290,6 +299,78 @@ def _result_buffers(B, s):
     return out, r
 
 
+def vjp_lengths(bp):
+    """per-instance lengths of the gradients lmpc_vjp returns: nx, [p of every cost], [(f | lower / upper) of every
+    constraint] -- rows, or rows x steps for a per-step entry"""
+    plen = [int(np.asarray(c["p"]).shape[-1]) for c in bp["costs"]]
+    clen = [int(np.asarray(c["lower"] if c["kind"] in ("trajectory_bound", "control_bound") else c["f"]).shape[-1])
+            for c in bp["constraints"]]
+    return int(bp["nx"]), plen, clen
+
+
+def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
+    """allocate the wanted gradients (numpy, or torch tensors on the device of the torch cotangents), describe them in a
+    VjpOut and run `call(dcontrol_ptr, dtrajectory_ptr, memory, out)`.  With torch tensors the engine runs on its own stream:
+    the cotangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the
+    gradients (written, zero-initialised, by the engine itself) and the input copies are handed back."""
+    nx, plen, clen = vjp_lengths(bp)
+    dev = next((t.device for t in (dcontrol, dtrajectory) if t is not None and hasattr(t, "data_ptr")), None)
+    keep = []
+    if dev is not None:
+        import torch
+
+        def zeros(k):  # the engine zeroes every requested gradient on its stream
+            return torch.empty((B, k), dtype=torch.float64, device=dev)
+
+        def ptr(a):
+            return a.data_ptr()
+
+        def inp(a):
+            if a is None:
+                return None
+            a = a.detach().to(torch.float64).contiguous()
+            keep.append(a)
+            return a.data_ptr()
+        mem = DEVICE
+    else:
+        def zeros(k):
+            return np.zeros((B, k))
+
+        def ptr(a):
+            return a.ctypes.data
+
+        def inp(a):
+            if a is None:
+                return None
+            a = np.ascontiguousarray(np.asarray(a, dtype=np.float64))
+            keep.append(a)
+            return a.ctypes.data
+        mem = HOST
+    res = dict(x0=zeros(nx) if "x0" in want else None)
+    o = VjpOut()
+    o.x0 = ptr(res["x0"]) if res["x0"] is not None else None
+    kinds = [c["kind"] for c in bp["constraints"]]
+    bound = [k in ("trajectory_bound", "control_bound") for k in kinds]
+    lists = dict(p=[zeros(k) if "p" in want else None for k in plen],
+                 f=[zeros(k) if "f" in want and not b else None for k, b in zip(clen, bound)],
+                 lower=[zeros(k) if "lower" in want and b else None for k, b in zip(clen, bound)],
+                 upper=[zeros(k) if "upper" in want and b else None for k, b in zip(clen, bound)])
+    for key, arrs in lists.items():
+        ptrs = (C.c_void_p * max(1, len(arrs)))(*[ptr(a) if a is not None else None for a in arrs])
+        keep.append(ptrs)
+        setattr(o, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
+        res[key] = arrs
+    dc, dt = inp(dcontrol), inp(dtrajectory)
+    if dev is not None:
+        torch.cuda.synchronize(dev)
+    try:
+        call(dc, dt, mem, o)
+    finally:
+        if dev is not None and sync is not None:
+            sync()
+    return res
+
+
 class Engine:
     """One handle == one GPU + one stream (include/copra_b200.h)."""
 
@@ -298,6 +379,8 @@ class Engine:
         opt = Options()
         opt.device, opt.stream, opt.sm_limit = int(device), stream, int(sm_limit)
         self.h = C.c_void_p()
+        self.solve_count = 0  # solves run through this object (copra_b200.autograd detects a stale backward with it)
+        self._last_bp = None  # the problem of the resident build, for the shapes of lmpc_vjp's gradients
         rc = self.lib.copra_b200_create(C.byref(opt), C.byref(self.h))
         if rc != 0:
             raise CopraB200Error(rc, "copra_b200_create failed (no usable sm_100 CUDA device? there is no CPU fallback)")
@@ -419,7 +502,10 @@ class Engine:
         r.memory = HOST
         for k in want:
             setattr(r, k, out[k].ctypes.data)
+        self.solve_count += 1
+        self._last_bp = None
         self._check(self.lib.copra_b200_lmpc_run(self.h, C.byref(hb.problem), C.byref(r)))
+        self._last_bp = hb.bp
         out["sizes"] = s
         return {k: v for k, v in out.items() if k in want or k == "sizes"}
 
@@ -455,6 +541,7 @@ class Engine:
             setattr(r, k, v.ctypes.data)
         a = Array()
         a.ptr, a.stride = x0.ctypes.data, x0.shape[1]
+        self.solve_count += 1
         self._check(self.lib.copra_b200_lmpc_resolve(self.h, a, HOST, C.byref(r)))
         return out
 
@@ -463,10 +550,26 @@ class Engine:
         have the resident build's shape, its matrices are ignored (copra_b200_lmpc_retarget)"""
         hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
         out, r = _result_buffers(hb.problem.batch, self.sizes(hb))
+        self.solve_count += 1
         self._check(self.lib.copra_b200_lmpc_retarget(self.h, C.byref(hb.problem), C.byref(r)))
+        self._last_bp = hb.bp
         return out
 
+    def lmpc_vjp(self, dcontrol=None, dtrajectory=None, want=VJP_WANT):
+        """Vector-Jacobian product of the last solve (copra_b200_lmpc_vjp): dcontrol (batch, nU) = dL/dcontrol and / or
+        dtrajectory (batch, X) = dL/dtrajectory, numpy arrays or CUDA float64 tensors.  Returns dict(x0=(batch, nx),
+        p=[per cost], f=[per row constraint, None for bounds], lower=/upper=[per bound constraint, None otherwise]), each
+        gradient (batch, rows) or (batch, rows x steps) for a per-step entry, of the same kind as the cotangents; a gradient
+        not in `want` is None.  Instances whose status is not 0 get zeros."""
+        if self._last_bp is None:
+            raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run / lmpc_retarget on this engine")
+        bp = self._last_bp
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want,
+                         lambda dc, dt, mem, o: self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o))),
+                         sync=self.synchronize)
+
     def lmpc_build(self, hb):
+        self._last_bp = None
         self._check(self.lib.copra_b200_lmpc_build(self.h, C.byref(hb.problem)))
 
     def download(self, hb, what):
@@ -548,6 +651,7 @@ class MultiEngine:
         hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
         if results is not None:
             self._check(self.lib.copra_b200_multi_lmpc_run(self.m, C.byref(hb.problem), C.byref(results)))
+            self._last_bp = hb.bp
             return None
         out = self._outputs(hb.problem.batch, sizes)
         r = Results()
@@ -555,7 +659,18 @@ class MultiEngine:
         for k, v in out.items():
             setattr(r, k, v.ctypes.data)
         self._check(self.lib.copra_b200_multi_lmpc_run(self.m, C.byref(hb.problem), C.byref(r)))
+        self._last_bp = hb.bp
         return out
+
+    def lmpc_vjp(self, dcontrol=None, dtrajectory=None, want=VJP_WANT):
+        """Engine.lmpc_vjp over the shards of the last run (numpy arrays holding the whole batch)"""
+        bp = getattr(self, "_last_bp", None)
+        if bp is None:
+            raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run on this engine")
+        if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
+            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want,
+                         lambda dc, dt, mem, o: self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o))))
 
     def set_warm_start(self, on=True):
         rc = self.lib.copra_b200_multi_set_warm_start(self.m, 1 if on else 0)

@@ -71,6 +71,12 @@ struct copra_b200_handle {
     bool gs_j_valid = false;   // the small solver's per-instance factors of the resident build are cached (re-solves load them)
     bool warm_start = false;   // copra_b200_set_warm_start: re-solves seed the active set of the previous solve
     bool warm_valid = false;   // `warm_iact` holds the active sets of the last solve of the resident build
+    bool solved = false;       // res_status / res_nact / res_iact hold the last solve of the resident build (lmpc_vjp)
+    bool vjp_factor_valid = false; // vjp_Jt holds R^-1 of the resident build's Hessian(s) (builds the thin solver did not factor)
+    // per-instance vector lengths of the resident build (doubles): every cost's p, every constraint's f / lower / upper;
+    // the constraint and the side (0 f, 1 lower, 2 upper) of every family; the control-bound constraint (-1 = none)
+    std::vector<int> cost_len, cstr_len, fam_cstr, fam_which;
+    int bound_cstr = -1;
     bool in_resolve = false;
     bool lmpc_solve_active = false; // run_gi is called from do_solve (a resident LMPC build), not from the raw-QP entry
     bool gt_pform = false;     // ... in its shared-factor form (P = Jt Q1 kept, no factor mat-vec per pass)
@@ -930,8 +936,18 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
     if ((rc = record(h, 3))) return rc;
     h->sz = pl.sz;
     h->shape = shape_key(p, pl);
+    h->cost_len.clear();
+    for (int i = 0; i < P.ncost; ++i) h->cost_len.push_back(p->costs[i].rows * pl.costs[i].vsteps);
+    h->cstr_len.clear();
+    for (int i = 0; i < p->ncstr; ++i) h->cstr_len.push_back(p->cstrs[i].rows * pl.cvsteps[i]);
+    h->fam_cstr.clear();
+    h->fam_which.clear();
+    for (const auto& f : pl.fams) { h->fam_cstr.push_back(f.cstr); h->fam_which.push_back(f.which); }
+    h->bound_cstr = pl.bound_cstr;
     h->built = true;
+    h->solved = false;
     h->factor_valid = false;
+    h->vjp_factor_valid = false;
     h->warm_valid = false;
     h->gs_j_valid = false;
     h->rows_filled = !P.skip_rows;
@@ -941,6 +957,7 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
 int do_solve(copra_b200_handle* h, const copra_b200_results* r)
 {
     if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_solve called before a successful build");
+    h->solved = false;
     const BuildParams& P = h->bp;
     const size_t B = P.batch, nv = P.nvar;
     int rc;
@@ -954,6 +971,7 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
     if ((rc = ws(h, "res_iters", 2 * B, &iters))) return rc;
     if ((rc = ws(h, "res_nact", B, &nact))) return rc;
     if ((rc = ws(h, "res_iact", B * nv, &iact))) return rc;
+    int *ws_status = status, *ws_nact = nact, *ws_iact = iact;
     if (devres) { // write straight into the caller's device buffers where given
         if (r->x) x = r->x;
         if (r->control) control = r->control;
@@ -986,6 +1004,10 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
         if (rc) return rc;
     }
     if ((rc = record(h, 4))) return rc;
+    // the active sets of this solve stay in the workspace for copra_b200_lmpc_vjp
+    if (status != ws_status) CU(cudaMemcpyAsync(ws_status, status, B * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
+    if (nact != ws_nact) CU(cudaMemcpyAsync(ws_nact, nact, B * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
+    if (iact != ws_iact) CU(cudaMemcpyAsync(ws_iact, iact, B * nv * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
     const bool want_ct = !r || r->control || r->trajectory;
     if (want_ct) LAUNCHED(k7_results_launch(P, x, control, traj, h->stream));
     if ((rc = record(h, 5))) return rc;
@@ -1001,10 +1023,164 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
         if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
     }
     if ((rc = record(h, 6))) return rc;
+    h->solved = true;
+    return 0;
+}
+
+// K8 for the last solve (copra_b200_lmpc_vjp).  The batch is processed in chunks whose slab, Y and Gram workspace stay
+// under kVjpWsBytes; the outputs are zeroed first and every kernel only writes the entries it owns.
+constexpr size_t kVjpWsBytes = size_t(1) << 30;
+
+int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out)
+{
+    const BuildParams& P = h->bp;
+    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
+    const size_t B = P.batch, n = P.nvar, nx = P.nx;
+    int rc;
+    int *status = nullptr, *nact = nullptr, *iact = nullptr;
+    if ((rc = ws(h, "res_status", B, &status))) return rc;
+    if ((rc = ws(h, "res_nact", B, &nact))) return rc;
+    if ((rc = ws(h, "res_iact", B * n, &iact))) return rc;
+    // inputs
+    const double *dc = dcontrol, *dt = dtraj;
+    if (memory == COPRA_B200_HOST && (dcontrol || dtraj)) {
+        double* in = nullptr;
+        if ((rc = ws(h, "vjp_in", B * (P.nU + P.X), &in))) return rc;
+        if (dcontrol) CU(cudaMemcpyAsync(in, dcontrol, B * P.nU * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        if (dtraj) CU(cudaMemcpyAsync(in + B * P.nU, dtraj, B * P.X * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        dc = dcontrol ? in : nullptr;
+        dt = dtraj ? in + B * P.nU : nullptr;
+    }
+    // outputs: the caller's device buffers, or one workspace block downloaded at the end
+    VjpParams V{};
+    struct OutItem { double* host; double** dev; size_t len; };
+    std::vector<OutItem> items;
+    items.push_back({ out->x0, &V.dx0, nx });
+    for (int ci = 0; ci < P.ncost; ++ci) {
+        V.plen[ci] = h->cost_len[ci];
+        items.push_back({ out->p ? out->p[ci] : nullptr, &V.dp[ci], size_t(h->cost_len[ci]) });
+    }
+    for (int fi = 0; fi < P.nfam; ++fi) {
+        const int c = h->fam_cstr[fi], which = h->fam_which[fi];
+        double* const* arr = which == 0 ? out->f : (which == 1 ? out->lower : out->upper);
+        V.flen[fi] = h->cstr_len[c];
+        items.push_back({ arr ? arr[c] : nullptr, &V.df[fi], size_t(h->cstr_len[c]) });
+    }
+    if (h->bound_cstr >= 0) {
+        V.cblen = h->cstr_len[h->bound_cstr];
+        items.push_back({ out->lower ? out->lower[h->bound_cstr] : nullptr, &V.dlower, size_t(V.cblen) });
+        items.push_back({ out->upper ? out->upper[h->bound_cstr] : nullptr, &V.dupper, size_t(V.cblen) });
+    }
+    size_t total = 0;
+    for (auto& it : items) if (it.host) total += it.len * B;
+    double* oblk = nullptr;
+    if (memory == COPRA_B200_HOST && total && (rc = ws(h, "vjp_out", total, &oblk))) return rc;
+    total = 0;
+    for (auto& it : items) {
+        if (!it.host) continue;
+        *it.dev = memory == COPRA_B200_HOST ? oblk + total : it.host;
+        total += it.len * B;
+        if (memory == COPRA_B200_DEVICE) CU(cudaMemsetAsync(*it.dev, 0, it.len * B * sizeof(double), h->stream));
+    }
+    if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
+    // the largest active set of the solved instances sizes the slab
+    std::vector<int> hs(B), hn(B);
+    CU(cudaMemcpyAsync(hs.data(), status, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(hn.data(), nact, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    // the padded active-set width: the batch's largest sizes the workspace, each chunk uses its own largest
+    auto widest = [&](size_t lo, size_t hi) {
+        int w = 0;
+        for (size_t b = lo; b < hi; ++b) if (hs[b] == 0) w = std::max(w, hn[b]);
+        return w;
+    };
+    const int nm = widest(0, B);
+    // R^-1 of the Hessian(s): the thin solver's resident factor, else one factorisation kept until the next build
+    const int ldj = gt_even(int(n));
+    const size_t count = P.sQ ? B : 1;
+    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
+    const double* Jt = nullptr;
+    const int* qpd = nullptr;
+    if (h->use_thin && h->factor_valid) {
+        Jt = static_cast<const double*>(h->dev["gt_Jt"].p);
+        qpd = static_cast<const int*>(h->dev["gt_pd"].p);
+    } else {
+        double *J = nullptr, *JT = nullptr;
+        int* pd = nullptr;
+        if ((rc = ws(h, "vjp_Jt", count * ldj * n, &J))) return rc;
+        if ((rc = ws(h, "vjp_JtT", count * ldj * n, &JT))) return rc;
+        if ((rc = ws(h, "vjp_pd", count, &pd))) return rc;
+        if (!h->vjp_factor_valid) {
+            cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, int(n), ldj, int(count), J, JT, pd, sms, h->stream);
+            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+            h->launches += 1; h->call_launches += 1;
+            h->vjp_factor_valid = true;
+        }
+        Jt = J;
+        qpd = pd;
+    }
+    // chunked workspace
+    const size_t lds = size_t(ldj), m1 = size_t(nm) + 1, ldg = size_t(gt_even(nm));
+    const size_t per = 2 * lds * m1 + m1 * m1 + size_t(nm) * nm + 2 * ldg * nm + 2 * size_t(nm) + 2 * lds + 1;
+    const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kVjpWsBytes / (per * sizeof(double)))));
+    V.n = int(n); V.lds = int(lds); V.ldy = int(lds);
+    V.status = status; V.nact = nact; V.iact = iact;
+    V.qpd = qpd; V.qpd_stride = P.sQ ? 1 : 0;
+    V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
+    double* GJT = nullptr;
+    const size_t C = size_t(chunk);
+    if ((rc = ws(h, "vjp_slab", C * lds * m1, &V.slab))) return rc;
+    if ((rc = ws(h, "vjp_Y", C * lds * m1, &V.Y))) return rc;
+    if ((rc = ws(h, "vjp_Gf", C * m1 * m1, &V.Gf))) return rc;
+    if ((rc = ws(h, "vjp_Gq", C * nm * nm, &V.Gq))) return rc;
+    if ((rc = ws(h, "vjp_GJ", C * ldg * nm, const_cast<double**>(&V.GJ)))) return rc;
+    if ((rc = ws(h, "vjp_GJT", C * ldg * nm, &GJT))) return rc;
+    if ((rc = ws(h, "vjp_gpd", C, const_cast<int**>(&V.gpd)))) return rc;
+    if ((rc = ws(h, "vjp_rhs", C * nm, &V.rhs))) return rc;
+    if ((rc = ws(h, "vjp_mu", C * nm, &V.mu))) return rc;
+    if ((rc = ws(h, "vjp_W", C * lds, &V.W))) return rc;
+    if ((rc = ws(h, "vjp_V", C * lds, &V.V))) return rc;
+    const int N_ = int(n), L = int(lds);
+    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
+        const int nb = std::min(chunk, P.batch - b0);
+        const int nm = widest(size_t(b0), size_t(b0) + nb), M1 = nm + 1;
+        V.b0 = b0; V.nm = nm; V.ldg = gt_even(nm);
+        LAUNCHED(k8_gather_launch(P, V, nb, h->stream));
+        // Y = Jt' [A_act' | gbar]: one GEMM over the chunk for a shared factor
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * M1, N_, 1.0, Jt, ldj, 0, V.slab, L, 0, 0.0, V.Y, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(1, N_, M1, N_, 1.0, Jt + b0 * sJ, ldj, sJ, V.slab, L, (long long)L * M1, 0.0, V.Y, L,
+            (long long)L * M1, nb, h->stream));
+        if (nm > 0) {
+            LAUNCHED(dgemm_dmma_launch(1, M1, M1, N_, 1.0, V.Y, L, (long long)L * M1, V.Y, L, (long long)L * M1, 0.0, V.Gf, M1,
+                (long long)M1 * M1, nb, h->stream));
+            LAUNCHED(k8_gram_launch(V, nb, h->stream));
+            cudaError_t e = gt_factor_launch(DArr{ V.Gq, (long long)nm * nm }, nm, V.ldg, nb, const_cast<double*>(V.GJ), GJT,
+                const_cast<int*>(V.gpd), sms, h->stream);
+            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+            h->launches += 1; h->call_launches += 1;
+        }
+        LAUNCHED(k8_mu_launch(V, nb, h->stream));
+        // v = Jt w
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb, N_, 1.0, Jt, ldj, 0, V.W, L, 0, 0.0, V.V, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(0, N_, 1, N_, 1.0, Jt + b0 * sJ, ldj, sJ, V.W, L, L, 0.0, V.V, L, L, nb, h->stream));
+        LAUNCHED(k8_adjoint_launch(P, V, nb, h->stream));
+    }
+    if (memory == COPRA_B200_HOST) {
+        Download D;
+        for (auto& it : items) if (it.host) D.add(*it.dev, it.host, it.len * B * sizeof(double));
+        if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
+    }
     return 0;
 }
 
 } // namespace
+
+void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_len, std::vector<int>& cstr_len)
+{
+    nx = h->bp.nx;
+    cost_len = h->cost_len;
+    cstr_len = h->cstr_len;
+}
 
 // ===============================================================================================
 extern "C" {
@@ -1284,6 +1460,25 @@ int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, 
     return rc;
 }
 
+int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!out) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_vjp needs a solve of the resident build on this handle");
+    const BuildParams& P = h->bp;
+    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp is defined for LMPC mode only");
+    for (int i = 0; i < P.ncost; ++i)
+        if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp: cost %d is a full-size entry (its f comes out of the dense GEMMs)", i);
+    for (int k = 0; k < P.nfam; ++k)
+        if (P.fam[k].dense || P.fam[k].gather)
+            return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp: a row constraint is a full-size entry (its b comes out of the dense GEMMs)");
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_vjp(h, dcontrol, dtrajectory, memory, out);
+}
+
 int copra_b200_set_warm_start(copra_b200_handle* h, int on)
 {
     if (!h) return COPRA_B200_E_ARG;
@@ -1437,7 +1632,8 @@ int copra_b200_solve_qp_batch(copra_b200_handle* h, int n, int meq, int m, int b
     if ((meq > 0 && (!Aeq.ptr || !beq.ptr)) || (m > 0 && (!Aineq.ptr || !bineq.ptr))) return fail(h, COPRA_B200_E_ARG, "constraint matrices missing");
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
-    /* the last lmpc build stays valid: this entry uses its own workspace buffers */
+    /* the last lmpc build stays valid: this entry uses its own workspace buffers, except for the active sets */
+    h->solved = false;
     for (bool& v : h->ev_valid) v = false;
     int rc = record(h, 0);
     if (rc) return rc;

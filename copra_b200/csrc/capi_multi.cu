@@ -62,6 +62,9 @@ template <class F> int run_shards(copra_b200_multi* m, F body)
 
 } // namespace
 
+// per-instance lengths of x0 and of every cost's p / constraint's vector of the resident build (capi.cu)
+void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_len, std::vector<int>& cstr_len);
+
 extern "C" {
 
 int copra_b200_multi_create(const int* devices, int ndev, copra_b200_multi** out)
@@ -188,6 +191,38 @@ int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem
             rr = slice_results(*r, m->lo[g], sz);
         }
         return copra_b200_lmpc_retarget(m->h[g], &q.p, r ? &rr : nullptr);
+    });
+}
+
+int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out* out)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!out) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        std::vector<int> plen, clen;
+        int nx = 0;
+        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const long long lo = m->lo[g];
+        // every array of the whole batch, advanced to this shard's first instance
+        std::vector<double*> p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size());
+        for (size_t i = 0; i < plen.size(); ++i) p[i] = (out->p && out->p[i]) ? out->p[i] + lo * plen[i] : nullptr;
+        for (size_t i = 0; i < clen.size(); ++i) {
+            f[i] = (out->f && out->f[i]) ? out->f[i] + lo * clen[i] : nullptr;
+            lower[i] = (out->lower && out->lower[i]) ? out->lower[i] + lo * clen[i] : nullptr;
+            upper[i] = (out->upper && out->upper[i]) ? out->upper[i] + lo * clen[i] : nullptr;
+        }
+        copra_b200_vjp_out o{};
+        o.x0 = out->x0 ? out->x0 + lo * nx : nullptr;
+        o.p = out->p ? p.data() : nullptr;
+        o.f = out->f ? f.data() : nullptr;
+        o.lower = out->lower ? lower.data() : nullptr;
+        o.upper = out->upper ? upper.data() : nullptr;
+        return copra_b200_lmpc_vjp(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr, dtrajectory ? dtrajectory + lo * sz.X : nullptr,
+            COPRA_B200_HOST, &o);
     });
 }
 

@@ -61,4 +61,45 @@ int k2_retarget_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k4_finalize_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k7_results_launch(const BuildParams& P, const double* x, double* control, double* trajectory, cudaStream_t st);
 
+// K8 (k8_vjp.cu): vector-Jacobian product of the last solve, for the chunk of instances [b0, b0 + nb).  Buffers marked
+// "chunk" hold nb instances; the others are indexed by the instance number in the batch.
+struct VjpParams {
+    int n;                           // decision variables (nU: LMPC mode)
+    int nm;                          // the largest active-set size of the chunk (the padded width of slab, Y and G)
+    int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
+    int b0;
+    const int* status;
+    const int* nact;
+    const int* iact;                 // n per instance, 1-based [eq | ineq | upper | lower] indices
+    const int* qpd;                  // 1 = the Hessian's factor Jt is valid (positive definite), qpd_stride apart per instance
+    int qpd_stride;
+    const double* dcontrol;          // dL/dU (nU per instance, sdc apart), may be null
+    long long sdc;
+    const double* dtraj;             // dL/dtrajectory (X per instance, sdt apart), may be null
+    long long sdt;
+    double* slab;                    // chunk: lds x (nm + 1)   [A_act' | gbar]
+    double* Y;                       // chunk: ldy x (nm + 1)   Jt' slab
+    double* Gf;                      // chunk: (nm + 1)^2       Y'Y
+    double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
+    double* rhs;                     // chunk: nm               Y1' t
+    const double* GJ;                // chunk: ldg x nm         R_G^-1
+    const int* gpd;                  // chunk: 1 = G positive definite
+    double* mu;                      // chunk: nm               multipliers of the active rows (iact order)
+    double* W;                       // chunk: lds              t - Y1 mu
+    double* V;                       // chunk: lds              v = Jt W
+    // outputs (whole batch, zeroed by the caller; null = not wanted)
+    double* dx0;                     // nx per instance
+    double* dp[kMaxCost];            // plen[ci] per instance
+    int plen[kMaxCost];
+    double* df[kMaxFam];             // per family: its constraint's f, or a trajectory bound's lower / upper
+    int flen[kMaxFam];
+    double* dlower;                  // control bound, cblen per instance
+    double* dupper;
+    int cblen;
+};
+int k8_gather_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
+int k8_gram_launch(const VjpParams& V, int nb, cudaStream_t st);
+int k8_mu_launch(const VjpParams& V, int nb, cudaStream_t st);
+int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
+
 } // namespace cb

@@ -1179,6 +1179,26 @@ public:
         solveAndBuildTime_ = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
         return int(std::count(status_.begin(), status_.end(), 0));
     }
+    // Sensitivities of the last solve / resolve / retarget (copra_b200_lmpc_vjp): the vector-Jacobian product of the controls
+    // (dcontrol: nU x batch) and trajectories (dtrajectory: X x batch; either may be null) with respect to x0 and every entry's
+    // vectors, written where `out` points (HOST arrays, batch-major; null = not wanted).  std::domain_error for full-size
+    // entries other than the control bound and in initial-state mode; std::runtime_error when another controller has built
+    // on the shared engine since this one's last solve.
+    void vjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out)
+    {
+        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::vjp takes HOST arrays");
+        if (multi_) {
+            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::vjp needs a previous solve");
+            const int rc = copra_b200_multi_lmpc_vjp(multi_, dcontrol, dtrajectory, &out);
+            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
+            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
+            return;
+        }
+        if (myEpoch_ != b200::buildEpoch()) throw std::runtime_error("BatchedLMPC::vjp: another controller has built on the engine since this solve");
+        const int rc = copra_b200_lmpc_vjp(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out);
+        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
+        b200::check(rc);
+    }
     const std::vector<double>& controls() const { return controls_; }         // nU x batch, column-major
     const std::vector<double>& trajectories() const { return trajectories_; } // X x batch
     const std::vector<int>& status() const { return status_; }

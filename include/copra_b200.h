@@ -234,6 +234,28 @@ int copra_b200_lmpc_resolve(copra_b200_handle* h, copra_b200_array x0, int memor
  * row constraint or trajectory bound, whose vector terms come out of the dense GEMM epilogues (a full-size control bound is
  * fine). */
 int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, const copra_b200_results* r);
+/* Sensitivities of the last solve: the vector-Jacobian product of (control, trajectory) with respect to x0 and every
+ * cost's p and every constraint's f / lower / upper.  On the final active set the solution is an affine function of these
+ * vectors, so the product is exact (one adjoint KKT solve per instance, K8).  Gradients are per instance even for inputs
+ * given with stride 0; a step-size entry's gradient is the sum over its steps, a per-step entry's has its rows x steps layout.
+ * With x0 alone and a unit dcontrol this is a row of the local feedback gain d u / d x0.
+ * Instances whose status is not 0 get zero gradients.  NULL pointers (the arrays themselves or their entries) mark gradients
+ * that are not wanted; the arrays have ncost / ncstr entries of the resident build. */
+typedef struct {
+    double* x0;             /* nx per instance */
+    double* const* p;       /* [ncost]: rows (x steps for a per-step entry) per instance */
+    double* const* f;       /* [ncstr]: rows (x steps) per instance, row constraints */
+    double* const* lower;   /* [ncstr]: rows (x steps) per instance, trajectory and control bounds */
+    double* const* upper;
+} copra_b200_vjp_out;
+/* `dcontrol` holds nU doubles per instance (dL/dcontrol), `dtrajectory` X doubles (dL/dtrajectory); either may be NULL.
+ * They and every output pointer live in `memory`.  Refers to the last solve on the resident build (run, solve, resolve or
+ * retarget): E_STATE without one (also after a copra_b200_lmpc_run of more than 65535 instances); E_UNSUPPORTED in
+ * initial-state mode and for builds with a full-size (full_size = 1) cost, row constraint or trajectory bound, as for
+ * copra_b200_lmpc_retarget (a full-size control bound is fine).  Leaves the resident build, the factor caches and the
+ * warm-start seed untouched. */
+int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out);
 /* SolverInterface::SI_warmStart(bool) / SI_warmStart() (include/SolverInterface.h:42-45; QuadProg has none, the reference
  * prints "No warmStart() function for this qp").  Opt-in: with it on, copra_b200_lmpc_resolve seeds every instance with the
  * inequality / bound rows that were active at its previous solve on the resident build, solves that equality-constrained
@@ -279,6 +301,8 @@ int copra_b200_multi_lmpc_run(copra_b200_multi* m, const copra_b200_problem* p, 
 int copra_b200_multi_lmpc_resolve(copra_b200_multi* m, copra_b200_array x0, const copra_b200_results* r);
 /* copra_b200_lmpc_retarget on every shard of the last run (same batch) */
 int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem* p, const copra_b200_results* r);
+/* copra_b200_lmpc_vjp on every shard of the last run; HOST arrays holding the whole batch */
+int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out* out);
 /* copra_b200_set_warm_start on every shard's handle */
 int copra_b200_multi_set_warm_start(copra_b200_multi* m, int on);
 
