@@ -4,11 +4,11 @@ ARCH := -gencode arch=compute_100a,code=sm_100a
 EXTRA ?=
 NVFLAGS := $(ARCH) -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xptxas -v $(EXTRA)
 CSRC := copra_b200/csrc
-OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_thin_f1.o $(CSRC)/k6_thin_f2.o $(CSRC)/k6_thin_cluster.o $(CSRC)/k1_k7_lmpc.o $(CSRC)/dgemm_dmma.o $(CSRC)/fp64_peak.o $(CSRC)/k8_vjp.o $(CSRC)/capi.o $(CSRC)/capi_multi.o
+OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_thin_f1.o $(CSRC)/k6_thin_f2.o $(CSRC)/k6_thin_cluster.o $(CSRC)/k1_k7_lmpc.o $(CSRC)/dgemm_dmma.o $(CSRC)/fp64_peak.o $(CSRC)/k8_vjp.o $(CSRC)/k9_jvp.o $(CSRC)/capi.o $(CSRC)/capi_multi.o
 LIB := copra_b200/lib/libcopra_b200.so
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/copra_b200.h
 
-all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp
+all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp tests/cpp/test_jvp
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; false)
@@ -43,3 +43,9 @@ tests/cpp/test_vjp: tests/cpp/test_vjp.cpp $(wildcard include/copra/*) include/c
 	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_vjp.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
 
 vjp-test: tests/cpp/test_vjp
+
+# BatchedLMPC::feedbackGain / ::jvp against central differences of per-instance copra::LMPC solves, and their errors (GPU)
+tests/cpp/test_jvp: tests/cpp/test_jvp.cpp $(wildcard include/copra/*) include/copra_b200.h $(LIB)
+	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_jvp.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
+
+jvp-test: tests/cpp/test_jvp

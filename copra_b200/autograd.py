@@ -1,12 +1,14 @@
 """torch.autograd through a batch of LMPC solves: the forward runs copra_b200_lmpc_run on CUDA tensors, the backward the exact
-vector-Jacobian product of copra_b200_lmpc_vjp (K8) on the same engine.
+vector-Jacobian product of copra_b200_lmpc_vjp (K8) on the same engine, and forward-mode AD (torch.autograd.forward_ad) the
+exact Jacobian-vector product of copra_b200_lmpc_jvp (K9).
 
     ctrl, traj = copra_b200.autograd.lmpc(engine, bp, x0, p=[...], f=[...], lower=[...], upper=[...])
 
 `bp` is a workloads-style batch problem that fixes the matrices (A, B, d, M, N, w, E, G) and the kinds and shapes of every
 entry; the vectors are CUDA float64 tensors, batch-major (batch, length), one per cost (p) and one per constraint (f for row
 constraints, lower / upper for bounds; None keeps bp's value, which then gets no gradient).  Every instance gets its own
-gradient.  The backward raises if another solve ran on the engine since this forward: the engine keeps only the last solve.
+gradient.  The backward and the forward-mode tangent raise if another solve ran on the engine since this forward: the
+engine keeps only the last solve.
 """
 import ctypes as C
 
@@ -60,8 +62,24 @@ class _LMPC(torch.autograd.Function):
         engine._last_bp = problem
         engine.synchronize()
         ctx.engine, ctx.count, ctx.keys, ctx.present = engine, engine.solve_count, keys, [v is not None for v in vecs]
+        ctx.counts = (len(bp["costs"]), len(bp["constraints"]))
         ctx.mark_non_differentiable()
         return control, traj
+
+    @staticmethod
+    def jvp(ctx, _engine, _bp, _keys, dx0, *dvecs):
+        # forward mode: one tangent direction through copra_b200_lmpc_jvp (K9); the engine holds everything it needs
+        eng = ctx.engine
+        if eng.solve_count != ctx.count:
+            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the JVP needs the "
+                               "active sets of the solve being differentiated")
+        ncost, ncstr = ctx.counts
+        tangents = dict(p=[None] * ncost, f=[None] * ncstr, lower=[None] * ncstr, upper=[None] * ncstr)
+        for (kind, i), t in zip(ctx.keys, dvecs):
+            if t is not None:
+                tangents[kind][i] = t.unsqueeze(1)
+        du, dx = eng.lmpc_jvp(x0=dx0.unsqueeze(1) if dx0 is not None else None, **tangents)
+        return du[:, 0], dx[:, 0]
 
     @staticmethod
     def backward(ctx, dcontrol, dtraj):

@@ -64,6 +64,11 @@ class VjpOut(C.Structure):
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
 
 
+class JvpIn(C.Structure):
+    _fields_ = [("ndir", C.c_int), ("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
+                ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
+
+
 class Timing(C.Structure):
     _fields_ = [(k, C.c_float) for k in ("h2d_ms", "condense_ms", "assemble_ms", "solve_ms", "rollout_ms", "d2h_ms",
                                          "total_ms")] + [("launches", C.c_longlong)]
@@ -79,7 +84,8 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_multi_launch_count", "copra_b200_multi_lmpc_run", "copra_b200_multi_lmpc_resolve",
            "copra_b200_set_warm_start", "copra_b200_get_warm_start", "copra_b200_multi_set_warm_start",
            "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget", "copra_b200_lmpc_vjp",
-           "copra_b200_multi_lmpc_vjp"]
+           "copra_b200_multi_lmpc_vjp", "copra_b200_lmpc_jvp", "copra_b200_lmpc_feedback_gain",
+           "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
 
 _lib = None
@@ -147,6 +153,10 @@ def load():
         lib.copra_b200_multi_set_warm_start.argtypes = [C.c_void_p, C.c_int]
         lib.copra_b200_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut)]
         lib.copra_b200_multi_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut)]
+        lib.copra_b200_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_int, C.c_void_p, C.c_void_p]
+        lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
+        lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
+        lib.copra_b200_multi_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
         _lib = lib
     return _lib
 
@@ -371,6 +381,95 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
     return res
 
 
+def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None):
+    """describe the tangents (each (batch, k, len), numpy or CUDA float64 tensors; None = zero) in a JvpIn, allocate dU
+    (batch, k, nU) and dtrajectory (batch, k, X) of the same kind and run `call(jvp_in, memory, dU_ptr, dX_ptr)`.  With torch
+    tensors the engine runs on its own stream: the tangents are complete before the call (device synchronise) and `sync()`
+    waits for the engine's stream before the results are handed back."""
+    nx, plen, clen = vjp_lengths(bp)
+    kinds = [c["kind"] for c in bp["constraints"]]
+    bound = [kd in ("trajectory_bound", "control_bound") for kd in kinds]
+    lists = dict(p=list(p or []), f=list(f or []), lower=list(lower or []), upper=list(upper or []))
+    given = [x0] + [t for v in lists.values() for t in v]
+    given = [t for t in given if t is not None]
+    if not given:
+        raise CopraB200Error(-1, "lmpc_jvp needs at least one tangent")
+    k = int(given[0].shape[1]) if len(given[0].shape) == 3 else 0
+    dev = next((t.device for t in given if hasattr(t, "data_ptr")), None)
+    if dev is not None:
+        import torch
+    keep = []
+
+    def inp(a, n, what):
+        if a is None:
+            return None
+        if tuple(a.shape) != (B, k, n):
+            raise CopraB200Error(-1, "lmpc_jvp: the %s tangent has shape %s, expected (batch, k, len) = %s"
+                                 % (what, tuple(a.shape), (B, k, n)))
+        if dev is not None:
+            a = a.detach().to(device=dev, dtype=torch.float64).contiguous()
+            keep.append(a)
+            return a.data_ptr()
+        if hasattr(a, "data_ptr"):
+            raise CopraB200Error(-1, "lmpc_jvp: numpy and torch tangents cannot be mixed")
+        a = np.ascontiguousarray(np.asarray(a, dtype=np.float64))
+        keep.append(a)
+        return a.ctypes.data
+
+    t = JvpIn()
+    t.ndir = k
+    t.x0 = inp(x0, nx, "x0")
+    lens = dict(p=plen, f=clen, lower=clen, upper=clen)
+    for key, arrs in lists.items():
+        n = len(plen) if key == "p" else len(clen)
+        if len(arrs) > n:
+            raise CopraB200Error(-1, "lmpc_jvp: %d %s tangents for %d entries" % (len(arrs), key, n))
+        arrs = arrs + [None] * (n - len(arrs))
+        if key != "p":
+            for j, a in enumerate(arrs):
+                if a is not None and bound[j] == (key == "f"):
+                    raise CopraB200Error(-1, "lmpc_jvp: constraint %d has no %s vector" % (j, key))
+        ptrs = (C.c_void_p * max(1, n))(*[inp(a, lens[key][j], "%s[%d]" % (key, j)) for j, a in enumerate(arrs)])
+        keep.append(ptrs)
+        setattr(t, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
+    nU, X = int(bp["nu"]) * int(bp["N"]), nx * (int(bp["N"]) + 1)
+    if dev is not None:
+        du = torch.empty((B, k, nU), dtype=torch.float64, device=dev)
+        dx = torch.empty((B, k, X), dtype=torch.float64, device=dev)
+        torch.cuda.synchronize(dev)
+        ptr, mem = (lambda a: a.data_ptr()), DEVICE
+    else:
+        du, dx = np.zeros((B, k, nU)), np.zeros((B, k, X))
+        ptr, mem = (lambda a: a.ctypes.data), HOST
+    try:
+        call(t, mem, ptr(du), ptr(dx))
+    finally:
+        if dev is not None and sync is not None:
+            sync()
+    return du, dx
+
+
+def _gain_call(bp, B, steps, device, call, sync=None):
+    """allocate Ku / Kx (numpy, or CUDA tensors on `device`), run `call(steps, Ku_ptr, Kx_ptr, memory)` and return them as
+    (batch, nu*steps, nx) and (batch, nx*(steps+1), nx): the engine writes each instance's gain column-major"""
+    nx, nu = int(bp["nx"]), int(bp["nu"])
+    ru, rx = nu * int(steps), nx * (int(steps) + 1)
+    if device is not None:
+        import torch
+        ku = torch.empty((B, nx, max(ru, 0)), dtype=torch.float64, device=device)
+        kx = torch.empty((B, nx, max(rx, 0)), dtype=torch.float64, device=device)
+        torch.cuda.synchronize(device)
+        try:
+            call(int(steps), ku.data_ptr(), kx.data_ptr(), DEVICE)
+        finally:
+            if sync is not None:
+                sync()
+        return ku.transpose(1, 2).contiguous(), kx.transpose(1, 2).contiguous()
+    ku, kx = np.zeros((B, nx, max(ru, 0))), np.zeros((B, nx, max(rx, 0)))
+    call(int(steps), ku.ctypes.data, kx.ctypes.data, HOST)
+    return np.ascontiguousarray(ku.transpose(0, 2, 1)), np.ascontiguousarray(kx.transpose(0, 2, 1))
+
+
 class Engine:
     """One handle == one GPU + one stream (include/copra_b200.h)."""
 
@@ -568,6 +667,28 @@ class Engine:
                          lambda dc, dt, mem, o: self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o))),
                          sync=self.synchronize)
 
+    def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
+        """Jacobian-vector product of the last solve (copra_b200_lmpc_jvp) along k tangent directions: x0 (batch, k, nx) and
+        lists indexed by cost (p) / constraint (f for row constraints, lower / upper for bounds) of (batch, k, len) tangents,
+        len as the matching lmpc_vjp gradient; None entries are zero.  numpy arrays or CUDA float64 tensors.  Returns
+        (dcontrol (batch, k, nU), dtrajectory (batch, k, X)) of the same kind.  Instances whose status is not 0 get zeros."""
+        if self._last_bp is None:
+            raise CopraB200Error(-5, "lmpc_jvp needs a previous lmpc_run / lmpc_retarget on this engine")
+        bp = self._last_bp
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, mem, du, dx: self._check(self.lib.copra_b200_lmpc_jvp(self.h, C.byref(t), mem, du, dx)),
+                         sync=self.synchronize)
+
+    def lmpc_feedback_gain(self, steps=1, device=None):
+        """Local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): (Ku (batch, nu*steps, nx) = dU[:nu*steps]/dx0,
+        Kx (batch, nx*(steps+1), nx) = dtrajectory[:nx*(steps+1)]/dx0); numpy, or CUDA tensors on the torch `device`."""
+        if self._last_bp is None:
+            raise CopraB200Error(-5, "lmpc_feedback_gain needs a previous lmpc_run / lmpc_retarget on this engine")
+        bp = self._last_bp
+        return _gain_call(bp, int(bp["batch"]), steps, device,
+                          lambda st, ku, kx, mem: self._check(self.lib.copra_b200_lmpc_feedback_gain(self.h, st, ku, kx, mem)),
+                          sync=self.synchronize)
+
     def lmpc_build(self, hb):
         self._last_bp = None
         self._check(self.lib.copra_b200_lmpc_build(self.h, C.byref(hb.problem)))
@@ -671,6 +792,25 @@ class MultiEngine:
             raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
         return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want,
                          lambda dc, dt, mem, o: self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o))))
+
+    def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
+        """Engine.lmpc_jvp over the shards of the last run (numpy arrays holding the whole batch)"""
+        bp = getattr(self, "_last_bp", None)
+        if bp is None:
+            raise CopraB200Error(-5, "lmpc_jvp needs a previous lmpc_run on this engine")
+        tangents = [x0] + list(p or []) + list(f or []) + list(lower or []) + list(upper or [])
+        if any(hasattr(t, "data_ptr") for t in tangents):
+            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, mem, du, dx: self._check(self.lib.copra_b200_multi_lmpc_jvp(self.m, C.byref(t), du, dx)))
+
+    def lmpc_feedback_gain(self, steps=1):
+        """Engine.lmpc_feedback_gain over the shards of the last run (numpy arrays holding the whole batch)"""
+        bp = getattr(self, "_last_bp", None)
+        if bp is None:
+            raise CopraB200Error(-5, "lmpc_feedback_gain needs a previous lmpc_run on this engine")
+        return _gain_call(bp, int(bp["batch"]), steps, None,
+                          lambda st, ku, kx, mem: self._check(self.lib.copra_b200_multi_lmpc_feedback_gain(self.m, st, ku, kx)))
 
     def set_warm_start(self, on=True):
         rc = self.lib.copra_b200_multi_set_warm_start(self.m, 1 if on else 0)

@@ -1027,6 +1027,36 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
     return 0;
 }
 
+// R^-1 of the resident build's Hessian(s) for K8 / K9 (ld gt_even(n); one per instance when P.sQ, else one for the batch):
+// the thin solver's resident factor, else one factorisation kept until the next build
+int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
+{
+    const BuildParams& P = h->bp;
+    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
+    const size_t n = P.nvar, count = P.sQ ? size_t(P.batch) : 1;
+    const int ldj = gt_even(int(n));
+    int rc;
+    if (h->use_thin && h->factor_valid) {
+        *Jt = static_cast<const double*>(h->dev["gt_Jt"].p);
+        *qpd = static_cast<const int*>(h->dev["gt_pd"].p);
+        return 0;
+    }
+    double *J = nullptr, *JT = nullptr;
+    int* pd = nullptr;
+    if ((rc = ws(h, "vjp_Jt", count * ldj * n, &J))) return rc;
+    if ((rc = ws(h, "vjp_JtT", count * ldj * n, &JT))) return rc;
+    if ((rc = ws(h, "vjp_pd", count, &pd))) return rc;
+    if (!h->vjp_factor_valid) {
+        cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, int(n), ldj, int(count), J, JT, pd, sms, h->stream);
+        if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+        h->launches += 1; h->call_launches += 1;
+        h->vjp_factor_valid = true;
+    }
+    *Jt = J;
+    *qpd = pd;
+    return 0;
+}
+
 // K8 for the last solve (copra_b200_lmpc_vjp).  The batch is processed in chunks whose slab, Y and Gram workspace stay
 // under kVjpWsBytes; the outputs are zeroed first and every kernel only writes the entries it owns.
 constexpr size_t kVjpWsBytes = size_t(1) << 30;
@@ -1095,30 +1125,11 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
         return w;
     };
     const int nm = widest(0, B);
-    // R^-1 of the Hessian(s): the thin solver's resident factor, else one factorisation kept until the next build
     const int ldj = gt_even(int(n));
-    const size_t count = P.sQ ? B : 1;
     const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
     const double* Jt = nullptr;
     const int* qpd = nullptr;
-    if (h->use_thin && h->factor_valid) {
-        Jt = static_cast<const double*>(h->dev["gt_Jt"].p);
-        qpd = static_cast<const int*>(h->dev["gt_pd"].p);
-    } else {
-        double *J = nullptr, *JT = nullptr;
-        int* pd = nullptr;
-        if ((rc = ws(h, "vjp_Jt", count * ldj * n, &J))) return rc;
-        if ((rc = ws(h, "vjp_JtT", count * ldj * n, &JT))) return rc;
-        if ((rc = ws(h, "vjp_pd", count, &pd))) return rc;
-        if (!h->vjp_factor_valid) {
-            cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, int(n), ldj, int(count), J, JT, pd, sms, h->stream);
-            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
-            h->launches += 1; h->call_launches += 1;
-            h->vjp_factor_valid = true;
-        }
-        Jt = J;
-        qpd = pd;
-    }
+    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
     // chunked workspace
     const size_t lds = size_t(ldj), m1 = size_t(nm) + 1, ldg = size_t(gt_even(nm));
     const size_t per = 2 * lds * m1 + m1 * m1 + size_t(nm) * nm + 2 * ldg * nm + 2 * size_t(nm) + 2 * lds + 1;
@@ -1170,6 +1181,142 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
         for (auto& it : items) if (it.host) D.add(*it.dev, it.host, it.len * B * sizeof(double));
         if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
     }
+    return 0;
+}
+
+// K9 for the last solve (copra_b200_lmpc_jvp, copra_b200_lmpc_feedback_gain): k tangent directions described by `in`, or
+// (gain) the columns of the identity on x0.  Chunked like do_vjp; k9_output writes every entry of the first ru rows of dU
+// and the first rx rows of dtrajectory of each direction (zeros for an instance whose status is not 0).
+int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, int memory, double* dcontrol, int ru,
+    double* dtraj, int rx)
+{
+    const BuildParams& P = h->bp;
+    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
+    const size_t B = P.batch, n = P.nvar, nx = P.nx, K = size_t(k);
+    int rc;
+    JvpParams J{};
+    int *status = nullptr, *nact = nullptr, *iact = nullptr;
+    if ((rc = ws(h, "res_status", B, &status))) return rc;
+    if ((rc = ws(h, "res_nact", B, &nact))) return rc;
+    if ((rc = ws(h, "res_iact", B * n, &iact))) return rc;
+    // tangents: the caller's device arrays, or HOST arrays packed into the staging buffer and uploaded in one copy
+    Upload U;
+    DArr tx0{}, tp[kMaxCost]{}, tf[kMaxFam]{}, tlo{}, tup{};
+    auto add = [&](const double* a, size_t len, DArr* dst) { U.add(copra_b200_array{ a, (long long)(len * K) }, len * K, dst); };
+    if (in) {
+        add(in->x0, nx, &tx0);
+        for (int ci = 0; ci < P.ncost; ++ci) {
+            J.plen[ci] = h->cost_len[ci];
+            add(in->p ? in->p[ci] : nullptr, size_t(h->cost_len[ci]), &tp[ci]);
+        }
+        for (int fi = 0; fi < P.nfam; ++fi) {
+            const int c = h->fam_cstr[fi], which = h->fam_which[fi];
+            const double* const* arr = which == 0 ? in->f : (which == 1 ? in->lower : in->upper);
+            J.flen[fi] = h->cstr_len[c];
+            add(arr ? arr[c] : nullptr, size_t(h->cstr_len[c]), &tf[fi]);
+        }
+        if (h->bound_cstr >= 0) {
+            J.cblen = h->cstr_len[h->bound_cstr];
+            add(in->lower ? in->lower[h->bound_cstr] : nullptr, size_t(J.cblen), &tlo);
+            add(in->upper ? in->upper[h->bound_cstr] : nullptr, size_t(J.cblen), &tup);
+        }
+    }
+    if ((rc = run_upload(h, U, P.batch, memory, "jvp_in"))) return rc;
+    J.tx0 = tx0.p;
+    for (int ci = 0; ci < P.ncost; ++ci) J.tp[ci] = tp[ci].p;
+    for (int fi = 0; fi < P.nfam; ++fi) J.tf[fi] = tf[fi].p;
+    J.tlower = tlo.p;
+    J.tupper = tup.p;
+    // outputs: the caller's device buffers, or one workspace block downloaded at the end
+    J.ru = ru; J.rx = rx;
+    J.dcontrol = dcontrol; J.dtraj = dtraj;
+    if (memory == COPRA_B200_HOST && (dcontrol || dtraj)) {
+        double* oblk = nullptr;
+        if ((rc = ws(h, "jvp_out", B * (size_t(ru) + size_t(rx)) * K, &oblk))) return rc;
+        J.dcontrol = dcontrol ? oblk : nullptr;
+        J.dtraj = dtraj ? oblk + B * size_t(ru) * K : nullptr;
+    }
+    // the largest active set of the solved instances sizes the workspace, each chunk uses its own largest
+    std::vector<int> hs(B), hn(B);
+    CU(cudaMemcpyAsync(hs.data(), status, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(hn.data(), nact, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    auto widest = [&](size_t lo, size_t hi) {
+        int w = 0;
+        for (size_t b = lo; b < hi; ++b) if (hs[b] == 0) w = std::max(w, hn[b]);
+        return w;
+    };
+    const int nm = widest(0, B);
+    const int ldj = gt_even(int(n));
+    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
+    const double* Jt = nullptr;
+    const int* qpd = nullptr;
+    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
+    // chunked workspace
+    const size_t lds = size_t(ldj), mk = size_t(nm) + K, ldg = size_t(gt_even(nm));
+    const size_t per = 2 * lds * mk + mk * mk + size_t(nm) * nm + 2 * ldg * nm + size_t(nm) * K + 2 * lds * K + 1;
+    const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kVjpWsBytes / (per * sizeof(double)))));
+    J.n = int(n); J.k = k; J.gain = gain ? 1 : 0; J.lds = int(lds); J.ldy = int(lds);
+    J.status = status; J.nact = nact; J.iact = iact;
+    J.qpd = qpd; J.qpd_stride = P.sQ ? 1 : 0;
+    double* GJT = nullptr;
+    const size_t C = size_t(chunk);
+    if ((rc = ws(h, "vjp_slab", C * lds * mk, &J.slab))) return rc;
+    if ((rc = ws(h, "vjp_Y", C * lds * mk, &J.Y))) return rc;
+    if ((rc = ws(h, "vjp_Gf", C * mk * mk, &J.Gf))) return rc;
+    if ((rc = ws(h, "vjp_Gq", C * nm * nm, &J.Gq))) return rc;
+    if ((rc = ws(h, "vjp_GJ", C * ldg * nm, const_cast<double**>(&J.GJ)))) return rc;
+    if ((rc = ws(h, "vjp_GJT", C * ldg * nm, &GJT))) return rc;
+    if ((rc = ws(h, "vjp_gpd", C, const_cast<int**>(&J.gpd)))) return rc;
+    if ((rc = ws(h, "vjp_rhs", C * nm * K, &J.rhs))) return rc;
+    if ((rc = ws(h, "vjp_W", C * lds * K, &J.W))) return rc;
+    if ((rc = ws(h, "vjp_V", C * lds * K, &J.V))) return rc;
+    const int N_ = int(n), L = int(lds);
+    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
+        const int nb = std::min(chunk, P.batch - b0);
+        const int nm = widest(size_t(b0), size_t(b0) + nb), MK = nm + k;
+        J.b0 = b0; J.nm = nm; J.ldg = gt_even(nm);
+        LAUNCHED(k9_tangent_launch(P, J, nb, h->stream));
+        // Y = Jt' [A_act' | -cdot]: one GEMM over the chunk for a shared factor
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * MK, N_, 1.0, Jt, ldj, 0, J.slab, L, 0, 0.0, J.Y, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(1, N_, MK, N_, 1.0, Jt + b0 * sJ, ldj, sJ, J.slab, L, (long long)L * MK, 0.0, J.Y, L,
+            (long long)L * MK, nb, h->stream));
+        if (nm > 0) {
+            LAUNCHED(dgemm_dmma_launch(1, MK, MK, N_, 1.0, J.Y, L, (long long)L * MK, J.Y, L, (long long)L * MK, 0.0, J.Gf, MK,
+                (long long)MK * MK, nb, h->stream));
+            LAUNCHED(k9_gram_launch(J, nb, h->stream));
+            cudaError_t e = gt_factor_launch(DArr{ J.Gq, (long long)nm * nm }, nm, J.ldg, nb, const_cast<double*>(J.GJ), GJT,
+                const_cast<int*>(J.gpd), sms, h->stream);
+            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+            h->launches += 1; h->call_launches += 1;
+        }
+        LAUNCHED(k9_solve_launch(J, nb, h->stream));
+        // Udot = Jt W
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb * k, N_, 1.0, Jt, ldj, 0, J.W, L, 0, 0.0, J.V, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(0, N_, k, N_, 1.0, Jt + b0 * sJ, ldj, sJ, J.W, L, (long long)L * k, 0.0, J.V, L,
+            (long long)L * k, nb, h->stream));
+        LAUNCHED(k9_output_launch(P, J, nb, h->stream));
+    }
+    if (memory == COPRA_B200_HOST) {
+        Download D;
+        D.add(J.dcontrol, dcontrol, B * size_t(ru) * K * sizeof(double));
+        D.add(J.dtraj, dtraj, B * size_t(rx) * K * sizeof(double));
+        if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
+    }
+    return 0;
+}
+
+// the preconditions of the sensitivities of the last solve (copra_b200_lmpc_vjp, _jvp, _feedback_gain)
+int sens_check(copra_b200_handle* h, const char* name)
+{
+    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_%s needs a solve of the resident build on this handle", name);
+    const BuildParams& P = h->bp;
+    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s is defined for LMPC mode only", name);
+    for (int i = 0; i < P.ncost; ++i)
+        if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: cost %d is a full-size entry (its f comes out of the dense GEMMs)", name, i);
+    for (int k = 0; k < P.nfam; ++k)
+        if (P.fam[k].dense || P.fam[k].gather)
+            return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: a row constraint is a full-size entry (its b comes out of the dense GEMMs)", name);
     return 0;
 }
 
@@ -1477,6 +1624,32 @@ int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const doub
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
     return do_vjp(h, dcontrol, dtrajectory, memory, out);
+}
+
+int copra_b200_lmpc_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int memory, double* dcontrol, double* dtrajectory)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!in) return fail(h, COPRA_B200_E_ARG, "lmpc_jvp: null tangent description");
+    if (in->ndir < 1) return fail(h, COPRA_B200_E_ARG, "lmpc_jvp: ndir = %d, needs at least one direction", in->ndir);
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    int rc = sens_check(h, "lmpc_jvp");
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_jvp(h, in, in->ndir, false, memory, dcontrol, h->bp.nU, dtrajectory, h->bp.X);
+}
+
+int copra_b200_lmpc_feedback_gain(copra_b200_handle* h, int steps, double* Ku, double* Kx, int memory)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    int rc = sens_check(h, "lmpc_feedback_gain");
+    if (rc) return rc;
+    const BuildParams& P = h->bp;
+    if (steps < 1 || steps > P.N) return fail(h, COPRA_B200_E_ARG, "lmpc_feedback_gain: steps = %d outside [1, N = %d]", steps, P.N);
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_jvp(h, nullptr, P.nx, true, memory, Ku, P.nu * steps, Kx, P.nx * (steps + 1));
 }
 
 int copra_b200_set_warm_start(copra_b200_handle* h, int on)

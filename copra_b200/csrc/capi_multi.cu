@@ -226,4 +226,58 @@ int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const
     });
 }
 
+int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!in) return mfail(m, COPRA_B200_E_ARG, "lmpc_jvp: null tangent description");
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_jvp needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        std::vector<int> plen, clen;
+        int nx = 0;
+        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const long long lo = m->lo[g], k = in->ndir;
+        // every array of the whole batch (len x k per instance), advanced to this shard's first instance
+        auto at = [&](const double* const* arr, size_t i, int len) -> const double* {
+            return (arr && arr[i]) ? arr[i] + lo * len * k : nullptr;
+        };
+        std::vector<const double*> p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size());
+        for (size_t i = 0; i < plen.size(); ++i) p[i] = at(in->p, i, plen[i]);
+        for (size_t i = 0; i < clen.size(); ++i) {
+            f[i] = at(in->f, i, clen[i]);
+            lower[i] = at(in->lower, i, clen[i]);
+            upper[i] = at(in->upper, i, clen[i]);
+        }
+        copra_b200_jvp_in t = *in;
+        t.x0 = in->x0 ? in->x0 + lo * nx * k : nullptr;
+        t.p = in->p ? p.data() : nullptr;
+        t.f = in->f ? f.data() : nullptr;
+        t.lower = in->lower ? lower.data() : nullptr;
+        t.upper = in->upper ? upper.data() : nullptr;
+        return copra_b200_lmpc_jvp(m->h[g], &t, COPRA_B200_HOST, dcontrol ? dcontrol + lo * sz.nU * k : nullptr,
+            dtrajectory ? dtrajectory + lo * sz.X * k : nullptr);
+    });
+}
+
+int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_feedback_gain needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        std::vector<int> plen, clen;
+        int nx = 0;
+        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const int N = sz.X / nx - 1, nu = N > 0 ? sz.nU / N : 0;
+        if (steps < 1 || steps > N) return copra_b200_lmpc_feedback_gain(m->h[g], steps, nullptr, nullptr, COPRA_B200_HOST); // E_ARG
+        const long long lo = m->lo[g];
+        return copra_b200_lmpc_feedback_gain(m->h[g], steps, Ku ? Ku + lo * nu * steps * nx : nullptr,
+            Kx ? Kx + lo * nx * (steps + 1) * nx : nullptr, COPRA_B200_HOST);
+    });
+}
+
 } // extern "C"

@@ -16,6 +16,7 @@
 //               df / dlower / dupper: b^, lb^, ub^ scattered through the index maps of dev_precompute / dev_finalize
 // Instances whose status is not 0 keep an all-zero slab and their (pre-zeroed) gradients; a Hessian or Gram factorisation that
 // fails gives NaN gradients instead of silently wrong ones.
+#include "active_rows.cuh"
 #include "common.cuh"
 #include "engine.cuh"
 #include "launch.h"
@@ -27,20 +28,6 @@ namespace cb {
 namespace {
 
 constexpr int kVjpThreads = 256;
-
-// the family of general row `lrow` of Aeq (iseq) or Aineq, and its (step, line)
-__device__ __forceinline__ int vjp_family(const BuildParams& P, bool iseq, int lrow, int& step, int& line)
-{
-    for (int k = 0; k < P.nfam; ++k) {
-        const CstrFam& F = P.fam[k];
-        if ((F.is_eq != 0) == iseq && lrow >= F.row_off && lrow < F.row_off + F.rows * (F.i1 - F.i0)) {
-            step = F.i0 + (lrow - F.row_off) / F.rows;
-            line = (lrow - F.row_off) % F.rows;
-            return k;
-        }
-    }
-    return -1;
-}
 
 __device__ __forceinline__ int vjp_nact(const VjpParams& V, int b) { return V.status[b] == 0 ? V.nact[b] : 0; }
 
@@ -56,22 +43,7 @@ __global__ void __launch_bounds__(kVjpThreads) k8_gather_kernel(const __grid_con
     const int* iact = V.iact + (long long)b * n;
     for (int t = threadIdx.x; t < na * n; t += blockDim.x) {
         const int k = t / n, col = t % n;
-        const int idx = iact[k] - 1;
-        double v = 0.0;
-        if (idx < mg) {
-            const bool iseq = idx < P.meq;
-            int i, l;
-            const int fi = vjp_family(P, iseq, iseq ? idx : idx - P.meq, i, l);
-            if (fi >= 0) {
-                const CstrFam& F = P.fam[fi];
-                const int j = col / nu, bb = col % nu, kk = i - j;
-                if (kk >= 0) v = F.EGx[(long long)b * F.sEGx + l + F.rows * (bb + nu * kk)];
-            }
-        } else {
-            const int var = (idx - mg) % n; // upper rows first, then lower rows
-            v = (col == var) ? 1.0 : 0.0;
-        }
-        slab[col + (long long)k * V.lds] = v;
+        slab[col + (long long)k * V.lds] = active_row_entry(P, b, n, nu, mg, iact[k] - 1, col);
     }
     if (V.status[b] != 0) return;
     // gbar = dcontrol + Psi' dtraj, Psi' applied as the transposed block-Toeplitz product over the compact Gs

@@ -102,4 +102,47 @@ int k8_gram_launch(const VjpParams& V, int nb, cudaStream_t st);
 int k8_mu_launch(const VjpParams& V, int nb, cudaStream_t st);
 int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
+// K9 (k9_jvp.cu): Jacobian-vector products of the last solve for k tangent directions, for the chunk of instances
+// [b0, b0 + nb).  Buffers marked "chunk" hold nb instances; the others are indexed by the instance number in the batch.
+struct JvpParams {
+    int n;                           // decision variables (nU: LMPC mode)
+    int nm;                          // the largest active-set size of the chunk (the padded width of G)
+    int k;                           // tangent directions
+    int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
+    int b0;
+    int gain;                        // 1: the x0 tangents are the columns of the identity (k = nx), every other tangent zero
+    const int* status;
+    const int* nact;
+    const int* iact;                 // n per instance, 1-based [eq | ineq | upper | lower] indices
+    const int* qpd;                  // 1 = the Hessian's factor Jt is valid (positive definite), qpd_stride apart per instance
+    int qpd_stride;
+    // tangents (whole batch, len x k column-major per instance; null = zero), lengths as in VjpParams
+    const double* tx0;               // nx
+    const double* tp[kMaxCost];
+    int plen[kMaxCost];
+    const double* tf[kMaxFam];       // per family: its constraint's f, or a trajectory bound's lower / upper
+    int flen[kMaxFam];
+    const double* tlower;            // control bound, cblen
+    const double* tupper;
+    int cblen;
+    double* slab;                    // chunk: lds x (nm + k)   [A_act' | -cdot]
+    double* Y;                       // chunk: ldy x (nm + k)   Jt' slab = [Y1 | T]
+    double* Gf;                      // chunk: (nm + k)^2       Y'Y
+    double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
+    double* rhs;                     // chunk: nm x k           bdot_act, then Y1' T - bdot_act
+    const double* GJ;                // chunk: ldg x nm         R_G^-1
+    const int* gpd;                  // chunk: 1 = G positive definite
+    double* W;                       // chunk: lds x k          T - Y1 M
+    double* V;                       // chunk: lds x k          Udot = Jt W
+    // outputs (whole batch, every entry written; null = not wanted)
+    double* dcontrol;                // ru x k per instance: the first ru rows of Udot
+    int ru;
+    double* dtraj;                   // rx x k per instance: the first rx rows of Phi x0dot + Psi Udot
+    int rx;
+};
+int k9_tangent_launch(const BuildParams& P, const JvpParams& J, int nb, cudaStream_t st);
+int k9_gram_launch(const JvpParams& J, int nb, cudaStream_t st);
+int k9_solve_launch(const JvpParams& J, int nb, cudaStream_t st);
+int k9_output_launch(const BuildParams& P, const JvpParams& J, int nb, cudaStream_t st);
+
 } // namespace cb

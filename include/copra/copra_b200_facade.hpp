@@ -1199,6 +1199,43 @@ public:
         if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
         b200::check(rc);
     }
+    // Forward-mode sensitivities of the last solve (copra_b200_lmpc_jvp): dU (nU x k per instance) and dtrajectory (X x k)
+    // along the in.ndir tangent directions of x0 and every entry's vectors described by `in` (HOST arrays, batch-major; either
+    // output may be null).  Errors as vjp, plus std::domain_error for in.ndir < 1.
+    void jvp(const copra_b200_jvp_in& in, double* dcontrol, double* dtrajectory)
+    {
+        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::jvp takes HOST arrays");
+        if (multi_) {
+            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::jvp needs a previous solve");
+            const int rc = copra_b200_multi_lmpc_jvp(multi_, &in, dcontrol, dtrajectory);
+            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
+            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
+            return;
+        }
+        if (myEpoch_ != b200::buildEpoch()) throw std::runtime_error("BatchedLMPC::jvp: another controller has built on the engine since this solve");
+        const int rc = copra_b200_lmpc_jvp(b200::handle(), &in, COPRA_B200_HOST, dcontrol, dtrajectory);
+        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
+        b200::check(rc);
+    }
+    // The local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): Ku = dU[0 : nu*steps]/dx0 ((nu*steps) x nx
+    // per instance) and Kx = dtrajectory[0 : nx*(steps+1)]/dx0 ((nx*(steps+1)) x nx), column-major, batch-major HOST arrays;
+    // either may be null.  Errors as jvp, with std::domain_error for steps outside [1, N].
+    void feedbackGain(int steps, double* Ku, double* Kx)
+    {
+        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::feedbackGain takes HOST arrays");
+        if (multi_) {
+            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::feedbackGain needs a previous solve");
+            const int rc = copra_b200_multi_lmpc_feedback_gain(multi_, steps, Ku, Kx);
+            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
+            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
+            return;
+        }
+        if (myEpoch_ != b200::buildEpoch())
+            throw std::runtime_error("BatchedLMPC::feedbackGain: another controller has built on the engine since this solve");
+        const int rc = copra_b200_lmpc_feedback_gain(b200::handle(), steps, Ku, Kx, COPRA_B200_HOST);
+        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
+        b200::check(rc);
+    }
     const std::vector<double>& controls() const { return controls_; }         // nU x batch, column-major
     const std::vector<double>& trajectories() const { return trajectories_; } // X x batch
     const std::vector<int>& status() const { return status_; }

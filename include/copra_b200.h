@@ -256,6 +256,30 @@ typedef struct {
  * warm-start seed untouched. */
 int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
     const copra_b200_vjp_out* out);
+/* Forward-mode sensitivities of the last solve: the Jacobian-vector product of (control, trajectory) along `ndir` tangent
+ * directions of x0 and every cost's p and every constraint's f / lower / upper (one forward KKT solve per instance with
+ * ndir right-hand sides, K9; exact on the final active set, as the VJP).  Each tangent holds, per instance, ndir
+ * column-major vectors of the length of the matching copra_b200_vjp_out gradient (len x ndir); a step-size entry's tangent
+ * moves the value used at every step, a per-step entry's has its rows x steps layout.  NULL pointers (the arrays themselves
+ * or their entries) are zero tangents; the arrays have ncost / ncstr entries of the resident build. */
+typedef struct {
+    int ndir;                    /* k >= 1 tangent directions */
+    const double* x0;            /* nx x k per instance */
+    const double* const* p;      /* [ncost]: rows (x steps) x k per instance */
+    const double* const* f;      /* [ncstr]: row constraints */
+    const double* const* lower;  /* [ncstr]: trajectory and control bounds */
+    const double* const* upper;
+} copra_b200_jvp_in;
+/* `dcontrol` receives nU x k doubles per instance (dU), `dtrajectory` X x k (dtrajectory); either may be NULL.  The tangents
+ * and both outputs live in `memory`.  Instances whose status is not 0 get zeros; a Hessian or Gram factor that is not
+ * positive definite gives NaN.  Preconditions and error codes are those of copra_b200_lmpc_vjp, plus E_ARG for a NULL `in`
+ * or ndir < 1.  Leaves the resident build, the factor caches and the warm-start seed untouched. */
+int copra_b200_lmpc_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int memory, double* dcontrol, double* dtrajectory);
+/* The local feedback gain of the last solve, the JVP along the columns of the identity on x0 (the identity is never
+ * materialised): Ku = dU[0 : nu*steps] / dx0, (nu*steps) x nx per instance, and Kx = dtrajectory[0 : nx*(steps+1)] / dx0,
+ * (nx*(steps+1)) x nx, both column-major; either may be NULL.  A loop running faster than the MPC applies
+ * u0 + Ku (x - x0) with steps = 1.  E_ARG for steps outside [1, N]; otherwise as copra_b200_lmpc_jvp. */
+int copra_b200_lmpc_feedback_gain(copra_b200_handle* h, int steps, double* Ku, double* Kx, int memory);
 /* SolverInterface::SI_warmStart(bool) / SI_warmStart() (include/SolverInterface.h:42-45; QuadProg has none, the reference
  * prints "No warmStart() function for this qp").  Opt-in: with it on, copra_b200_lmpc_resolve seeds every instance with the
  * inequality / bound rows that were active at its previous solve on the resident build, solves that equality-constrained
@@ -303,6 +327,9 @@ int copra_b200_multi_lmpc_resolve(copra_b200_multi* m, copra_b200_array x0, cons
 int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem* p, const copra_b200_results* r);
 /* copra_b200_lmpc_vjp on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out* out);
+/* copra_b200_lmpc_jvp / copra_b200_lmpc_feedback_gain on every shard of the last run; HOST arrays holding the whole batch */
+int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory);
+int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx);
 /* copra_b200_set_warm_start on every shard's handle */
 int copra_b200_multi_set_warm_start(copra_b200_multi* m, int on);
 
