@@ -4,7 +4,7 @@ ARCH := -gencode arch=compute_100a,code=sm_100a
 EXTRA ?=
 NVFLAGS := $(ARCH) -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xptxas -v $(EXTRA)
 CSRC := copra_b200/csrc
-OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_thin_f1.o $(CSRC)/k6_thin_f2.o $(CSRC)/k6_thin_cluster.o $(CSRC)/k1_k7_lmpc.o $(CSRC)/dgemm_dmma.o $(CSRC)/fp64_peak.o $(CSRC)/k8_vjp.o $(CSRC)/k9_jvp.o $(CSRC)/capi.o $(CSRC)/capi_multi.o
+OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_thin_f1.o $(CSRC)/k6_thin_f2.o $(CSRC)/k6_thin_cluster.o $(CSRC)/k1_k7_lmpc.o $(CSRC)/dgemm_dmma.o $(CSRC)/fp64_peak.o $(CSRC)/k8_k9_sens.o $(CSRC)/capi.o $(CSRC)/capi_multi.o
 LIB := copra_b200/lib/libcopra_b200.so
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/copra_b200.h
 

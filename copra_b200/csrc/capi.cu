@@ -1057,20 +1057,91 @@ int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
     return 0;
 }
 
-// K8 for the last solve (copra_b200_lmpc_vjp).  The batch is processed in chunks whose slab, Y and Gram workspace stay
-// under kVjpWsBytes; the outputs are zeroed first and every kernel only writes the entries it owns.
-constexpr size_t kVjpWsBytes = size_t(1) << 30;
+// The active-set KKT solve of K8 / K9 for the last solve, with k right-hand sides per instance.  The batch is processed in
+// chunks whose slab, Y and Gram workspace stay under kSensWsBytes, each padded to its own largest active set.  `first(nb)`
+// writes a chunk's slab and rhs (the right-hand sides), `last(nb)` reads its V (and rhs = M); both launch one kernel.
+constexpr size_t kSensWsBytes = size_t(1) << 30;
 
-int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out)
+template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk& S, int k, First first, Last last)
 {
     const BuildParams& P = h->bp;
     const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
-    const size_t B = P.batch, n = P.nvar, nx = P.nx;
+    const size_t B = P.batch, n = P.nvar, K = size_t(k);
     int rc;
     int *status = nullptr, *nact = nullptr, *iact = nullptr;
     if ((rc = ws(h, "res_status", B, &status))) return rc;
     if ((rc = ws(h, "res_nact", B, &nact))) return rc;
     if ((rc = ws(h, "res_iact", B * n, &iact))) return rc;
+    // the largest active set of the solved instances sizes the workspace, each chunk uses its own largest
+    std::vector<int> hs(B), hn(B);
+    CU(cudaMemcpyAsync(hs.data(), status, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(hn.data(), nact, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    auto widest = [&](size_t lo, size_t hi) {
+        int w = 0;
+        for (size_t b = lo; b < hi; ++b) if (hs[b] == 0) w = std::max(w, hn[b]);
+        return w;
+    };
+    const int nm = widest(0, B);
+    const int ldj = gt_even(int(n));
+    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
+    const double* Jt = nullptr;
+    const int* qpd = nullptr;
+    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
+    // chunked workspace
+    const size_t lds = size_t(ldj), mk = size_t(nm) + K, ldg = size_t(gt_even(nm));
+    const size_t per = 2 * lds * mk + mk * mk + size_t(nm) * nm + 2 * ldg * nm + size_t(nm) * K + 2 * lds * K + 1;
+    const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kSensWsBytes / (per * sizeof(double)))));
+    S.n = int(n); S.k = k; S.lds = int(lds); S.ldy = int(lds);
+    S.status = status; S.nact = nact; S.iact = iact;
+    S.qpd = qpd; S.qpd_stride = P.sQ ? 1 : 0;
+    double* GJT = nullptr;
+    const size_t C = size_t(chunk);
+    if ((rc = ws(h, "vjp_slab", C * lds * mk, &S.slab))) return rc;
+    if ((rc = ws(h, "vjp_Y", C * lds * mk, &S.Y))) return rc;
+    if ((rc = ws(h, "vjp_Gf", C * mk * mk, &S.Gf))) return rc;
+    if ((rc = ws(h, "vjp_Gq", C * nm * nm, &S.Gq))) return rc;
+    if ((rc = ws(h, "vjp_GJ", C * ldg * nm, const_cast<double**>(&S.GJ)))) return rc;
+    if ((rc = ws(h, "vjp_GJT", C * ldg * nm, &GJT))) return rc;
+    if ((rc = ws(h, "vjp_gpd", C, const_cast<int**>(&S.gpd)))) return rc;
+    if ((rc = ws(h, "vjp_rhs", C * nm * K, &S.rhs))) return rc;
+    if ((rc = ws(h, "vjp_W", C * lds * K, &S.W))) return rc;
+    if ((rc = ws(h, "vjp_V", C * lds * K, &S.V))) return rc;
+    const int N_ = int(n), L = int(lds);
+    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
+        const int nb = std::min(chunk, P.batch - b0);
+        const int nm = widest(size_t(b0), size_t(b0) + nb), MK = nm + k;
+        S.b0 = b0; S.nm = nm; S.ldg = gt_even(nm);
+        LAUNCHED(first(nb));
+        // Y = Jt' slab: one GEMM over the chunk for a shared factor
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * MK, N_, 1.0, Jt, ldj, 0, S.slab, L, 0, 0.0, S.Y, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(1, N_, MK, N_, 1.0, Jt + b0 * sJ, ldj, sJ, S.slab, L, (long long)L * MK, 0.0, S.Y, L,
+            (long long)L * MK, nb, h->stream));
+        if (nm > 0) {
+            LAUNCHED(dgemm_dmma_launch(1, MK, MK, N_, 1.0, S.Y, L, (long long)L * MK, S.Y, L, (long long)L * MK, 0.0, S.Gf, MK,
+                (long long)MK * MK, nb, h->stream));
+            LAUNCHED(sens_gram_launch(S, nb, h->stream));
+            cudaError_t e = gt_factor_launch(DArr{ S.Gq, (long long)nm * nm }, nm, S.ldg, nb, const_cast<double*>(S.GJ), GJT,
+                const_cast<int*>(S.gpd), sms, h->stream);
+            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+            h->launches += 1; h->call_launches += 1;
+        }
+        LAUNCHED(sens_solve_launch(S, nb, h->stream));
+        // V = Jt W
+        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb * k, N_, 1.0, Jt, ldj, 0, S.W, L, 0, 0.0, S.V, L, 0, 1, h->stream));
+        else LAUNCHED(dgemm_dmma_launch(0, N_, k, N_, 1.0, Jt + b0 * sJ, ldj, sJ, S.W, L, (long long)L * k, 0.0, S.V, L,
+            (long long)L * k, nb, h->stream));
+        LAUNCHED(last(nb));
+    }
+    return 0;
+}
+
+// K8 for the last solve (copra_b200_lmpc_vjp): the outputs are zeroed first and k8_adjoint only writes the entries it owns.
+int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out)
+{
+    const BuildParams& P = h->bp;
+    const size_t B = P.batch, nx = P.nx;
+    int rc;
     // inputs
     const double *dc = dcontrol, *dt = dtraj;
     if (memory == COPRA_B200_HOST && (dcontrol || dtraj)) {
@@ -1113,69 +1184,10 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
         if (memory == COPRA_B200_DEVICE) CU(cudaMemsetAsync(*it.dev, 0, it.len * B * sizeof(double), h->stream));
     }
     if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
-    // the largest active set of the solved instances sizes the slab
-    std::vector<int> hs(B), hn(B);
-    CU(cudaMemcpyAsync(hs.data(), status, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(hn.data(), nact, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    // the padded active-set width: the batch's largest sizes the workspace, each chunk uses its own largest
-    auto widest = [&](size_t lo, size_t hi) {
-        int w = 0;
-        for (size_t b = lo; b < hi; ++b) if (hs[b] == 0) w = std::max(w, hn[b]);
-        return w;
-    };
-    const int nm = widest(0, B);
-    const int ldj = gt_even(int(n));
-    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
-    const double* Jt = nullptr;
-    const int* qpd = nullptr;
-    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
-    // chunked workspace
-    const size_t lds = size_t(ldj), m1 = size_t(nm) + 1, ldg = size_t(gt_even(nm));
-    const size_t per = 2 * lds * m1 + m1 * m1 + size_t(nm) * nm + 2 * ldg * nm + 2 * size_t(nm) + 2 * lds + 1;
-    const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kVjpWsBytes / (per * sizeof(double)))));
-    V.n = int(n); V.lds = int(lds); V.ldy = int(lds);
-    V.status = status; V.nact = nact; V.iact = iact;
-    V.qpd = qpd; V.qpd_stride = P.sQ ? 1 : 0;
     V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
-    double* GJT = nullptr;
-    const size_t C = size_t(chunk);
-    if ((rc = ws(h, "vjp_slab", C * lds * m1, &V.slab))) return rc;
-    if ((rc = ws(h, "vjp_Y", C * lds * m1, &V.Y))) return rc;
-    if ((rc = ws(h, "vjp_Gf", C * m1 * m1, &V.Gf))) return rc;
-    if ((rc = ws(h, "vjp_Gq", C * nm * nm, &V.Gq))) return rc;
-    if ((rc = ws(h, "vjp_GJ", C * ldg * nm, const_cast<double**>(&V.GJ)))) return rc;
-    if ((rc = ws(h, "vjp_GJT", C * ldg * nm, &GJT))) return rc;
-    if ((rc = ws(h, "vjp_gpd", C, const_cast<int**>(&V.gpd)))) return rc;
-    if ((rc = ws(h, "vjp_rhs", C * nm, &V.rhs))) return rc;
-    if ((rc = ws(h, "vjp_mu", C * nm, &V.mu))) return rc;
-    if ((rc = ws(h, "vjp_W", C * lds, &V.W))) return rc;
-    if ((rc = ws(h, "vjp_V", C * lds, &V.V))) return rc;
-    const int N_ = int(n), L = int(lds);
-    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
-        const int nb = std::min(chunk, P.batch - b0);
-        const int nm = widest(size_t(b0), size_t(b0) + nb), M1 = nm + 1;
-        V.b0 = b0; V.nm = nm; V.ldg = gt_even(nm);
-        LAUNCHED(k8_gather_launch(P, V, nb, h->stream));
-        // Y = Jt' [A_act' | gbar]: one GEMM over the chunk for a shared factor
-        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * M1, N_, 1.0, Jt, ldj, 0, V.slab, L, 0, 0.0, V.Y, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(1, N_, M1, N_, 1.0, Jt + b0 * sJ, ldj, sJ, V.slab, L, (long long)L * M1, 0.0, V.Y, L,
-            (long long)L * M1, nb, h->stream));
-        if (nm > 0) {
-            LAUNCHED(dgemm_dmma_launch(1, M1, M1, N_, 1.0, V.Y, L, (long long)L * M1, V.Y, L, (long long)L * M1, 0.0, V.Gf, M1,
-                (long long)M1 * M1, nb, h->stream));
-            LAUNCHED(k8_gram_launch(V, nb, h->stream));
-            cudaError_t e = gt_factor_launch(DArr{ V.Gq, (long long)nm * nm }, nm, V.ldg, nb, const_cast<double*>(V.GJ), GJT,
-                const_cast<int*>(V.gpd), sms, h->stream);
-            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
-            h->launches += 1; h->call_launches += 1;
-        }
-        LAUNCHED(k8_mu_launch(V, nb, h->stream));
-        // v = Jt w
-        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb, N_, 1.0, Jt, ldj, 0, V.W, L, 0, 0.0, V.V, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(0, N_, 1, N_, 1.0, Jt + b0 * sJ, ldj, sJ, V.W, L, L, 0.0, V.V, L, L, nb, h->stream));
-        LAUNCHED(k8_adjoint_launch(P, V, nb, h->stream));
-    }
+    rc = sens_run(h, V, 1, [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
+        [&](int nb) { return k8_adjoint_launch(P, V, nb, h->stream); });
+    if (rc) return rc;
     if (memory == COPRA_B200_HOST) {
         Download D;
         for (auto& it : items) if (it.host) D.add(*it.dev, it.host, it.len * B * sizeof(double));
@@ -1185,20 +1197,16 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
 }
 
 // K9 for the last solve (copra_b200_lmpc_jvp, copra_b200_lmpc_feedback_gain): k tangent directions described by `in`, or
-// (gain) the columns of the identity on x0.  Chunked like do_vjp; k9_output writes every entry of the first ru rows of dU
-// and the first rx rows of dtrajectory of each direction (zeros for an instance whose status is not 0).
+// (gain) the columns of the identity on x0.  k9_output writes every entry of the first ru rows of dU and the first rx rows of
+// dtrajectory of each direction (zeros for an instance whose status is not 0).
 int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, int memory, double* dcontrol, int ru,
     double* dtraj, int rx)
 {
     const BuildParams& P = h->bp;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
-    const size_t B = P.batch, n = P.nvar, nx = P.nx, K = size_t(k);
+    const size_t B = P.batch, nx = P.nx, K = size_t(k);
     int rc;
     JvpParams J{};
-    int *status = nullptr, *nact = nullptr, *iact = nullptr;
-    if ((rc = ws(h, "res_status", B, &status))) return rc;
-    if ((rc = ws(h, "res_nact", B, &nact))) return rc;
-    if ((rc = ws(h, "res_iact", B * n, &iact))) return rc;
+    J.gain = gain ? 1 : 0;
     // tangents: the caller's device arrays, or HOST arrays packed into the staging buffer and uploaded in one copy
     Upload U;
     DArr tx0{}, tp[kMaxCost]{}, tf[kMaxFam]{}, tlo{}, tup{};
@@ -1236,67 +1244,9 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
         J.dcontrol = dcontrol ? oblk : nullptr;
         J.dtraj = dtraj ? oblk + B * size_t(ru) * K : nullptr;
     }
-    // the largest active set of the solved instances sizes the workspace, each chunk uses its own largest
-    std::vector<int> hs(B), hn(B);
-    CU(cudaMemcpyAsync(hs.data(), status, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaMemcpyAsync(hn.data(), nact, B * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    auto widest = [&](size_t lo, size_t hi) {
-        int w = 0;
-        for (size_t b = lo; b < hi; ++b) if (hs[b] == 0) w = std::max(w, hn[b]);
-        return w;
-    };
-    const int nm = widest(0, B);
-    const int ldj = gt_even(int(n));
-    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
-    const double* Jt = nullptr;
-    const int* qpd = nullptr;
-    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
-    // chunked workspace
-    const size_t lds = size_t(ldj), mk = size_t(nm) + K, ldg = size_t(gt_even(nm));
-    const size_t per = 2 * lds * mk + mk * mk + size_t(nm) * nm + 2 * ldg * nm + size_t(nm) * K + 2 * lds * K + 1;
-    const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kVjpWsBytes / (per * sizeof(double)))));
-    J.n = int(n); J.k = k; J.gain = gain ? 1 : 0; J.lds = int(lds); J.ldy = int(lds);
-    J.status = status; J.nact = nact; J.iact = iact;
-    J.qpd = qpd; J.qpd_stride = P.sQ ? 1 : 0;
-    double* GJT = nullptr;
-    const size_t C = size_t(chunk);
-    if ((rc = ws(h, "vjp_slab", C * lds * mk, &J.slab))) return rc;
-    if ((rc = ws(h, "vjp_Y", C * lds * mk, &J.Y))) return rc;
-    if ((rc = ws(h, "vjp_Gf", C * mk * mk, &J.Gf))) return rc;
-    if ((rc = ws(h, "vjp_Gq", C * nm * nm, &J.Gq))) return rc;
-    if ((rc = ws(h, "vjp_GJ", C * ldg * nm, const_cast<double**>(&J.GJ)))) return rc;
-    if ((rc = ws(h, "vjp_GJT", C * ldg * nm, &GJT))) return rc;
-    if ((rc = ws(h, "vjp_gpd", C, const_cast<int**>(&J.gpd)))) return rc;
-    if ((rc = ws(h, "vjp_rhs", C * nm * K, &J.rhs))) return rc;
-    if ((rc = ws(h, "vjp_W", C * lds * K, &J.W))) return rc;
-    if ((rc = ws(h, "vjp_V", C * lds * K, &J.V))) return rc;
-    const int N_ = int(n), L = int(lds);
-    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
-        const int nb = std::min(chunk, P.batch - b0);
-        const int nm = widest(size_t(b0), size_t(b0) + nb), MK = nm + k;
-        J.b0 = b0; J.nm = nm; J.ldg = gt_even(nm);
-        LAUNCHED(k9_tangent_launch(P, J, nb, h->stream));
-        // Y = Jt' [A_act' | -cdot]: one GEMM over the chunk for a shared factor
-        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * MK, N_, 1.0, Jt, ldj, 0, J.slab, L, 0, 0.0, J.Y, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(1, N_, MK, N_, 1.0, Jt + b0 * sJ, ldj, sJ, J.slab, L, (long long)L * MK, 0.0, J.Y, L,
-            (long long)L * MK, nb, h->stream));
-        if (nm > 0) {
-            LAUNCHED(dgemm_dmma_launch(1, MK, MK, N_, 1.0, J.Y, L, (long long)L * MK, J.Y, L, (long long)L * MK, 0.0, J.Gf, MK,
-                (long long)MK * MK, nb, h->stream));
-            LAUNCHED(k9_gram_launch(J, nb, h->stream));
-            cudaError_t e = gt_factor_launch(DArr{ J.Gq, (long long)nm * nm }, nm, J.ldg, nb, const_cast<double*>(J.GJ), GJT,
-                const_cast<int*>(J.gpd), sms, h->stream);
-            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
-            h->launches += 1; h->call_launches += 1;
-        }
-        LAUNCHED(k9_solve_launch(J, nb, h->stream));
-        // Udot = Jt W
-        if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb * k, N_, 1.0, Jt, ldj, 0, J.W, L, 0, 0.0, J.V, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(0, N_, k, N_, 1.0, Jt + b0 * sJ, ldj, sJ, J.W, L, (long long)L * k, 0.0, J.V, L,
-            (long long)L * k, nb, h->stream));
-        LAUNCHED(k9_output_launch(P, J, nb, h->stream));
-    }
+    rc = sens_run(h, J, k, [&](int nb) { return k9_tangent_launch(P, J, nb, h->stream); },
+        [&](int nb) { return k9_output_launch(P, J, nb, h->stream); });
+    if (rc) return rc;
     if (memory == COPRA_B200_HOST) {
         Download D;
         D.add(J.dcontrol, dcontrol, B * size_t(ru) * K * sizeof(double));
@@ -1306,10 +1256,10 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
     return 0;
 }
 
-// the preconditions of the sensitivities of the last solve (copra_b200_lmpc_vjp, _jvp, _feedback_gain)
-int sens_check(copra_b200_handle* h, const char* name)
+// the resident build takes its vectors only through the vector part of K2 / K4, which retarget re-runs and the sensitivities
+// differentiate: LMPC mode, and no full-size entry other than the control bound
+int vector_inputs_check(copra_b200_handle* h, const char* name)
 {
-    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_%s needs a solve of the resident build on this handle", name);
     const BuildParams& P = h->bp;
     if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s is defined for LMPC mode only", name);
     for (int i = 0; i < P.ncost; ++i)
@@ -1318,6 +1268,13 @@ int sens_check(copra_b200_handle* h, const char* name)
         if (P.fam[k].dense || P.fam[k].gather)
             return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: a row constraint is a full-size entry (its b comes out of the dense GEMMs)", name);
     return 0;
+}
+
+// the preconditions of the sensitivities of the last solve (copra_b200_lmpc_vjp, _jvp, _feedback_gain)
+int sens_check(copra_b200_handle* h, const char* name)
+{
+    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_%s needs a solve of the resident build on this handle", name);
+    return vector_inputs_check(h, name);
 }
 
 } // namespace
@@ -1573,17 +1530,12 @@ int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, 
 {
     if (!h) return COPRA_B200_E_ARG;
     if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_retarget needs a previous build on this handle");
+    int rc = vector_inputs_check(h, "retarget");
+    if (rc) return rc;
     BuildParams& P = h->bp;
-    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget is defined for LMPC mode only");
-    for (int i = 0; i < P.ncost; ++i)
-        if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget: cost %d is a full-size entry (its f comes out of the dense GEMMs)", i);
-    for (int k = 0; k < P.nfam; ++k)
-        if (P.fam[k].dense || P.fam[k].gather)
-            return fail(h, COPRA_B200_E_UNSUPPORTED, "retarget: a row constraint is a full-size entry (its b comes out of the dense GEMMs)");
     // everything is validated before BuildParams changes: a refused retarget leaves the resident build usable
     Plan pl;
-    int rc = make_plan(h, p, pl, true);
-    if (rc) return rc;
+    if ((rc = make_plan(h, p, pl, true))) return rc;
     if (shape_key(p, pl) != h->shape)
         return fail(h, COPRA_B200_E_ARG, "retarget: the problem's shape (dimensions, batch, entries, +-inf bound pattern) differs from the resident build");
     CU(cudaSetDevice(h->device));
@@ -1613,14 +1565,8 @@ int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const doub
     if (!h) return COPRA_B200_E_ARG;
     if (!out) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
     if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
-    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_vjp needs a solve of the resident build on this handle");
-    const BuildParams& P = h->bp;
-    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp is defined for LMPC mode only");
-    for (int i = 0; i < P.ncost; ++i)
-        if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp: cost %d is a full-size entry (its f comes out of the dense GEMMs)", i);
-    for (int k = 0; k < P.nfam; ++k)
-        if (P.fam[k].dense || P.fam[k].gather)
-            return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp: a row constraint is a full-size entry (its b comes out of the dense GEMMs)");
+    int rc = sens_check(h, "lmpc_vjp");
+    if (rc) return rc;
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
     return do_vjp(h, dcontrol, dtrajectory, memory, out);

@@ -61,11 +61,13 @@ int k2_retarget_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k4_finalize_launch(const BuildParams& P, int sms, cudaStream_t st);
 int k7_results_launch(const BuildParams& P, const double* x, double* control, double* trajectory, cudaStream_t st);
 
-// K8 (k8_vjp.cu): vector-Jacobian product of the last solve, for the chunk of instances [b0, b0 + nb).  Buffers marked
-// "chunk" hold nb instances; the others are indexed by the instance number in the batch.
-struct VjpParams {
+// K8 / K9 (k8_k9_sens.cu): sensitivities of the last solve, one active-set KKT solve with k right-hand sides per instance, for
+// the chunk of instances [b0, b0 + nb).  Buffers marked "chunk" hold nb instances; the others are indexed by the instance
+// number in the batch.  SensChunk is what the VJP and the JVP share; per-instance vectors are len x k column-major.
+struct SensChunk {
     int n;                           // decision variables (nU: LMPC mode)
     int nm;                          // the largest active-set size of the chunk (the padded width of slab, Y and G)
+    int k;                           // right-hand sides: 1 for the VJP, the tangent directions for the JVP
     int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
     int b0;
     const int* status;
@@ -73,67 +75,47 @@ struct VjpParams {
     const int* iact;                 // n per instance, 1-based [eq | ineq | upper | lower] indices
     const int* qpd;                  // 1 = the Hessian's factor Jt is valid (positive definite), qpd_stride apart per instance
     int qpd_stride;
+    int plen[kMaxCost];              // per instance: each cost's p
+    int flen[kMaxFam];               // per family: its constraint's f, or a trajectory bound's lower / upper
+    int cblen;                       // the control bound's lower / upper
+    double* slab;                    // chunk: lds x (nm + k)   [A_act' | gbar] or [A_act' | -cdot]
+    double* Y;                       // chunk: ldy x (nm + k)   Jt' slab = [Y1 | T]
+    double* Gf;                      // chunk: (nm + k)^2       Y'Y
+    double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
+    double* rhs;                     // chunk: nm x k           bdot_act (0 for the VJP), then Y1' T - bdot_act (then mu for the VJP)
+    const double* GJ;                // chunk: ldg x nm         R_G^-1
+    const int* gpd;                  // chunk: 1 = G positive definite
+    double* W;                       // chunk: lds x k          T - Y1 M
+    double* V;                       // chunk: lds x k          Jt W (v for the VJP, Udot for the JVP)
+};
+int sens_gram_launch(const SensChunk& S, int nb, cudaStream_t st);
+int sens_solve_launch(const SensChunk& S, int nb, cudaStream_t st);
+
+// K8: the vector-Jacobian product (k = 1); sens_solve leaves the multipliers mu of the active rows (iact order) in rhs
+struct VjpParams : SensChunk {
     const double* dcontrol;          // dL/dU (nU per instance, sdc apart), may be null
     long long sdc;
     const double* dtraj;             // dL/dtrajectory (X per instance, sdt apart), may be null
     long long sdt;
-    double* slab;                    // chunk: lds x (nm + 1)   [A_act' | gbar]
-    double* Y;                       // chunk: ldy x (nm + 1)   Jt' slab
-    double* Gf;                      // chunk: (nm + 1)^2       Y'Y
-    double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
-    double* rhs;                     // chunk: nm               Y1' t
-    const double* GJ;                // chunk: ldg x nm         R_G^-1
-    const int* gpd;                  // chunk: 1 = G positive definite
-    double* mu;                      // chunk: nm               multipliers of the active rows (iact order)
-    double* W;                       // chunk: lds              t - Y1 mu
-    double* V;                       // chunk: lds              v = Jt W
     // outputs (whole batch, zeroed by the caller; null = not wanted)
     double* dx0;                     // nx per instance
-    double* dp[kMaxCost];            // plen[ci] per instance
-    int plen[kMaxCost];
-    double* df[kMaxFam];             // per family: its constraint's f, or a trajectory bound's lower / upper
-    int flen[kMaxFam];
-    double* dlower;                  // control bound, cblen per instance
+    double* dp[kMaxCost];
+    double* df[kMaxFam];
+    double* dlower;                  // control bound
     double* dupper;
-    int cblen;
 };
 int k8_gather_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
-int k8_gram_launch(const VjpParams& V, int nb, cudaStream_t st);
-int k8_mu_launch(const VjpParams& V, int nb, cudaStream_t st);
 int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
-// K9 (k9_jvp.cu): Jacobian-vector products of the last solve for k tangent directions, for the chunk of instances
-// [b0, b0 + nb).  Buffers marked "chunk" hold nb instances; the others are indexed by the instance number in the batch.
-struct JvpParams {
-    int n;                           // decision variables (nU: LMPC mode)
-    int nm;                          // the largest active-set size of the chunk (the padded width of G)
-    int k;                           // tangent directions
-    int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
-    int b0;
+// K9: Jacobian-vector products along k tangent directions, or the feedback gain
+struct JvpParams : SensChunk {
     int gain;                        // 1: the x0 tangents are the columns of the identity (k = nx), every other tangent zero
-    const int* status;
-    const int* nact;
-    const int* iact;                 // n per instance, 1-based [eq | ineq | upper | lower] indices
-    const int* qpd;                  // 1 = the Hessian's factor Jt is valid (positive definite), qpd_stride apart per instance
-    int qpd_stride;
-    // tangents (whole batch, len x k column-major per instance; null = zero), lengths as in VjpParams
+    // tangents (whole batch; null = zero)
     const double* tx0;               // nx
     const double* tp[kMaxCost];
-    int plen[kMaxCost];
-    const double* tf[kMaxFam];       // per family: its constraint's f, or a trajectory bound's lower / upper
-    int flen[kMaxFam];
-    const double* tlower;            // control bound, cblen
+    const double* tf[kMaxFam];
+    const double* tlower;            // control bound
     const double* tupper;
-    int cblen;
-    double* slab;                    // chunk: lds x (nm + k)   [A_act' | -cdot]
-    double* Y;                       // chunk: ldy x (nm + k)   Jt' slab = [Y1 | T]
-    double* Gf;                      // chunk: (nm + k)^2       Y'Y
-    double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
-    double* rhs;                     // chunk: nm x k           bdot_act, then Y1' T - bdot_act
-    const double* GJ;                // chunk: ldg x nm         R_G^-1
-    const int* gpd;                  // chunk: 1 = G positive definite
-    double* W;                       // chunk: lds x k          T - Y1 M
-    double* V;                       // chunk: lds x k          Udot = Jt W
     // outputs (whole batch, every entry written; null = not wanted)
     double* dcontrol;                // ru x k per instance: the first ru rows of Udot
     int ru;
@@ -141,8 +123,6 @@ struct JvpParams {
     int rx;
 };
 int k9_tangent_launch(const BuildParams& P, const JvpParams& J, int nb, cudaStream_t st);
-int k9_gram_launch(const JvpParams& J, int nb, cudaStream_t st);
-int k9_solve_launch(const JvpParams& J, int nb, cudaStream_t st);
 int k9_output_launch(const BuildParams& P, const JvpParams& J, int nb, cudaStream_t st);
 
 } // namespace cb
