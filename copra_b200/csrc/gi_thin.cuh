@@ -103,7 +103,7 @@ struct GtBatch {
     // solver stores P = Jt Q1 INSTEAD of Q1 (P' Q P = I) and never touches the factor in the iterations:
     //   h = Jt d = H a (nx + nu column reads of Hpsi / H)      d1 = Q1' d = P' R' Jt' a = P' a      z = Jt zt = h - P d1
     //   |zt|^2 = d' zt = a' z      |d|^2 = a' h      ADD: P gains z / |zt|      DROP: the same reflection, applied to P
-    // -- two sweeps over P and one over S per pass, nothing else.  Null: the general form (Q1, z = Jt zt).
+    // -- one sweep over P (gt_pass_fused; two for n > 320) and one over S per pass, nothing else.  Null: the general form (Q1, z = Jt zt).
     const double* Hpsi;
     const double* Hm;
     const double* Qs;   // the shared Hessian (n x n), only for the rare second orthogonalisation pass (v = P' Q z)
@@ -520,6 +520,43 @@ __device__ __forceinline__ void gt_row_dots(const CL& cl, const double* __restri
 }
 
 // ---- the pass of the shared-factor form (GtBatch::Hpsi) -----------------------------------------------------------------------
+// Partial sums of r = S vec over the active rows for gt_pass_fused: lanes along rows, the columns split over GS = T / round32(nact)
+// thread groups, group g's sums in partS[g * rs + row] (at most T doubles); gt_s_rows_sum adds the groups up in fixed order.
+// Requires nact <= T.  The same arithmetic as the S half of gt_pass_rows, which keeps its inline copy: calling this from there
+// too made ptxas spill more in the 2-CTA/SM kernel of FORM 1.
+__device__ __forceinline__ void gt_s_rows_part(const GtWork& W, int nact, const double* __restrict__ vec, const double* __restrict__ S,
+    size_t lds, double* __restrict__ partS)
+{
+    const int tid = threadIdx.x, T = blockDim.x;
+    const int rs = max(32, round32(nact)), GS = max(1, T / rs);
+    const int g = tid / rs, r_ = tid - g * rs;
+    if (g < GS && r_ < nact) {
+        const size_t cs = size_t(GS) * lds;
+        const double* sr = S + W.rowmap[r_] + size_t(g) * lds;
+        const double* vp = vec + g;
+        double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
+        int c = g;
+        for (; c + 3 * GS < nact; c += 4 * GS, sr += 4 * cs, vp += 4 * GS) {
+            const double m0 = sr[0], m1 = sr[cs], m2 = sr[2 * cs], m3 = sr[3 * cs];
+            s0 = fma(m0, vp[0], s0); s1 = fma(m1, vp[GS], s1); s2 = fma(m2, vp[2 * GS], s2); s3 = fma(m3, vp[3 * GS], s3);
+        }
+        if (c < nact) {
+            const bool h1 = c + GS < nact, h2 = c + 2 * GS < nact;
+            const double m0 = sr[0], m1 = h1 ? sr[cs] : 0.0, m2 = h2 ? sr[2 * cs] : 0.0;
+            s0 = fma(m0, vp[0], s0); s1 = fma(m1, h1 ? vp[GS] : 0.0, s1); s2 = fma(m2, h2 ? vp[2 * GS] : 0.0, s2);
+        }
+        partS[g * rs + r_] = (s0 + s1) + (s2 + s3);
+    }
+}
+
+__device__ __forceinline__ double gt_s_rows_sum(int nact, const double* __restrict__ partS, int i)
+{
+    const int rs = max(32, round32(nact)), GS = max(1, int(blockDim.x) / rs);
+    double s = partS[i];
+    for (int k = 1; k < GS; ++k) s += partS[k * rs + i];
+    return s;
+}
+
 // outw = P vec (a thread per row PAIR, the column range split over G = T / round32(ld / 2) thread groups; P is stored where the
 // general form keeps Q1) and, when outr != null, outr = S vec over the active rows (lanes along rows, columns split over
 // thread groups); all partial sums meet in `part` in fixed order.  Requires n <= blockDim.x.  ONE __syncthreads inside; the
@@ -603,6 +640,107 @@ __device__ __forceinline__ void gt_pass_rows(const GtWork& W, int ld, int q1s, i
         for (int k = 1; k < GS; ++k) s += partS[k * rs + tid];
         outr[tid] = s;
     }
+}
+
+// The pass of the shared-factor form in ONE read of P[:, :nact]: d1 = P' y and w = P d1 (P[:, c] d1[c] needs column c only).
+// Warp wp owns the columns c = wp, wp + nw, ... in ascending order; lane l holds the rows 2 l + 64 k (k < kFusedKP: one 128-bit
+// load each, all issued before the dot) of the current column, forms d1[c] with a fixed butterfly of shuffles and adds
+// P[:, c] d1[c] to its own partials of w from the same registers.  Entries of y past `supp` are exact zeros and are skipped by
+// the dot; for a bound row (bj >= 0) d1[c] = bsign P[bj, c] comes from the lane that holds row bj and y is not read.
+// Behind the one barrier d1 needs, r = S d1 when want_r (gt_s_rows_part).  The nw x ld warp partials of w do not fit in `part`, so
+// they meet there in two fixed-order stages: warp wp + nw/2 stores its partial in slot wp before the barrier, warp wp adds its
+// own to that slot after it; gt_pass_fused_w sums the nw/2 slots in order.  `part` takes (nw/2) ld doubles of slots and T of
+// S partials: (T / 64) ld + T <= 6 T (gt_layout) exactly when ld <= 320, whatever T (a multiple of 64).  Fixed summation order
+// throughout, no atomics: deterministic.  Two __syncthreads inside; afterwards gt_pass_fused_w / gt_pass_fused_r read w and r
+// straight from `part`, and every thread reads back only the rows it owns before the next barrier.
+constexpr int kFusedKP = 5; // ld <= 320: 10 doubles of the column and 10 of w partials per thread, within 64 registers (2 CTAs/SM)
+
+__device__ __forceinline__ void gt_pass_fused(const GtWork& W, int ld, int nact, const double* __restrict__ y, int supp, int bj,
+    double bsign, double* __restrict__ d1, const double* __restrict__ S, size_t lds, bool want_r, double* __restrict__ part)
+{
+    constexpr int KP = kFusedKP;
+    const int lane = lane_id(), wp = warp_id(), nw = blockDim.x >> 5, half = nw >> 1;
+    double2 w[KP];
+#pragma unroll
+    for (int u = 0; u < KP; ++u) w[u] = make_double2(0.0, 0.0);
+    const int nin = min(KP, (ld - 2 * lane + 63) >> 6);           // chunks of this lane inside the column
+    const int ndot = min(nin, (supp + 63) >> 6);                   // ... and inside the support of y
+    auto sweep = [&](auto dot) {
+        const double* col = W.Q1 + size_t(wp) * ld + 2 * lane;
+        double* d1p = d1 + wp;
+#pragma unroll 1
+        for (int c = wp; c < nact; c += nw, col += size_t(nw) * ld, d1p += nw) {
+            double2 p[KP];
+#pragma unroll
+            for (int u = 0; u < KP; ++u)
+                p[u] = (u < nin) ? *reinterpret_cast<const double2*>(col + 64 * u) : make_double2(0.0, 0.0);
+            const double s = dot(p);
+            if (lane == 0) *d1p = s;
+#pragma unroll
+            for (int u = 0; u < KP; ++u) { w[u].x = fma(p[u].x, s, w[u].x); w[u].y = fma(p[u].y, s, w[u].y); }
+        }
+    };
+    if (bj >= 0) {
+        const int rb = bj - 2 * lane, src = (bj & 63) >> 1; // row bj relative to this lane's first row; the lane that holds it
+        sweep([&](const double2 (&p)[KP]) {
+            double v = 0.0;
+#pragma unroll
+            for (int u = 0; u < KP; ++u) {
+                v = (rb == 64 * u) ? p[u].x : v;
+                v = (rb == 64 * u + 1) ? p[u].y : v;
+            }
+            return bsign * __shfl_sync(0xffffffffu, v, src);
+        });
+    } else {
+        sweep([&](const double2 (&p)[KP]) {
+            double s = 0.0;
+#pragma unroll
+            for (int u = 0; u < KP; ++u) {
+                if (u < ndot) {
+                    const double2 a = *reinterpret_cast<const double2*>(y + 2 * lane + 64 * u);
+                    s = fma(p[u].y, a.y, fma(p[u].x, a.x, s));
+                }
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+            return s;
+        });
+    }
+    if (wp >= half) {
+        double* slot = part + size_t(wp - half) * ld + 2 * lane;
+#pragma unroll
+        for (int u = 0; u < KP; ++u)
+            if (u < nin) *reinterpret_cast<double2*>(slot + 64 * u) = w[u];
+    }
+    __syncthreads();
+    if (wp < half) {
+        double* slot = part + size_t(wp) * ld + 2 * lane;
+#pragma unroll
+        for (int u = 0; u < KP; ++u) {
+            if (u < nin) {
+                double2 o = *reinterpret_cast<const double2*>(slot + 64 * u);
+                o.x = w[u].x + o.x; o.y = w[u].y + o.y;
+                *reinterpret_cast<double2*>(slot + 64 * u) = o;
+            }
+        }
+    }
+    if (want_r) gt_s_rows_part(W, nact, d1, S, lds, part + size_t(half) * ld);
+    __syncthreads();
+}
+
+// w[k] after gt_pass_fused
+__device__ __forceinline__ double gt_pass_fused_w(const double* __restrict__ part, int ld, int k)
+{
+    const int half = blockDim.x >> 6;
+    double s = part[k];
+    for (int q = 1; q < half; ++q) s += part[size_t(q) * ld + k];
+    return s;
+}
+
+// r[i] after gt_pass_fused(want_r)
+__device__ __forceinline__ double gt_pass_fused_r(const double* __restrict__ part, int ld, int nact, int i)
+{
+    return gt_s_rows_sum(nact, part + size_t(blockDim.x >> 6) * ld, i);
 }
 
 // Two right-hand sides in one sweep (the warm-start seed adds its rows two at a time): out0[c] = P[:, c] . v0, out1[c] = P[:, c] . v1
@@ -1012,6 +1150,8 @@ __device__ inline int gt_solve(const CL& cl, const GtBatch& B, const GtWork& W, 
     const double* gAin = B.Aineq.p ? B.Aineq.at(b) : nullptr;
     auto q1col = [&](int c) -> double* { return (c < q1s ? W.Q1s : W.Q1) + size_t(c) * ld; };
     constexpr bool pform = FORM >= 1; // shared-factor form: z = H a - P d1 (see GtBatch::Hpsi)
+    // its pass reads P once (gt_pass_fused) up to n = 320; larger n keep the two sweeps (gt_q1_col_dots, then gt_pass_rows)
+    [[maybe_unused]] const bool fused = pform && ld <= 64 * kFusedKP;
     const bool use_ss = (FORM == 2) ? true : (B.ss != 0);                // compile-time in the hot kernel: the other row paths vanish
     const bool structured = (FORM == 2) ? true : (B.structured != 0);
 
@@ -1538,7 +1678,9 @@ __device__ inline int gt_solve(const CL& cl, const GtBatch& B, const GtWork& W, 
                 if (pform) {
                     // ---- shared-factor form: d1 = P' a ; [w, r] = [P, S] d1 ; z = h - w ; |zt|^2 = a'z ; |d|^2 = a'h -----------------
                     load_h(); // every thread reads back only the entries it wrote: the loads overlap with the sweeps below
-                    if (nact > 0) {
+                    if (nact > 0 && fused) {
+                        gt_pass_fused(W, ld, nact, W.av, supp, bj, bsign, W.d1, S, ldn, true, W.part);
+                    } else if (nact > 0) {
                         if (bj >= 0) {
                             for (int c = tid; c < nact; c += T) W.d1[c] = bsign * q1col(c)[bj];
                         } else {
@@ -1556,12 +1698,13 @@ __device__ inline int gt_solve(const CL& cl, const GtBatch& B, const GtWork& W, 
                             double zk = W.z[k];
                             if (first) {
                                 a_dn = fma(ak, zk, a_dn); // W.z still holds h
-                                if (nact > 0) { zk -= W.w[k]; W.z[k] = zk; }
+                                if (nact > 0) { zk -= fused ? gt_pass_fused_w(W.part, ld, k) : W.w[k]; W.z[k] = zk; }
                             }
                             a_zz = fma(zk, zk, a_zz); a_za = fma(ak, zk, a_za);
                         }
                         MinIdx tc; tc.v = 0.0; tc.i = -1;
                         for (int i = tid; i < nact; i += T) {
+                            if (first && fused) W.r[i] = gt_pass_fused_r(W.part, ld, nact, i);
                             if (W.iact[i] - 1 >= meq && W.r[i] > 0.0) {
                                 MinIdx c; c.v = W.u[i] / W.r[i]; c.i = i;
                                 tc = better(tc, c);
@@ -1587,11 +1730,16 @@ __device__ inline int gt_solve(const CL& cl, const GtBatch& B, const GtWork& W, 
                         }
                         for (int k = n + tid; k < np; k += T) W.zt[k] = 0.0;
                         __syncthreads();
-                        gt_q1_col_dots(cl, W, n, ld, q1s, nact, W.zt, W.v);
-                        __syncthreads();
-                        gt_pass_rows(W, ld, q1s, nact, W.v, W.w, S, ldn, nullptr, W.part);
-                        __syncthreads();
-                        for (int k = tid; k < n; k += T) W.z[k] -= W.w[k];
+                        if (fused) {
+                            gt_pass_fused(W, ld, nact, W.zt, n, -1, 0.0, W.v, S, ldn, false, W.part);
+                            for (int k = tid; k < n; k += T) W.z[k] -= gt_pass_fused_w(W.part, ld, k);
+                        } else {
+                            gt_q1_col_dots(cl, W, n, ld, q1s, nact, W.zt, W.v);
+                            __syncthreads();
+                            gt_pass_rows(W, ld, q1s, nact, W.v, W.w, S, ldn, nullptr, W.part);
+                            __syncthreads();
+                            for (int k = tid; k < n; k += T) W.z[k] -= W.w[k];
+                        }
                         for (int k = tid; k < nact; k += T) W.d1[k] += W.v[k];
                         __syncthreads();
                         gt_row_dots(cl, S, ldn, nact, 0, nact, [&](int r_) { return size_t(W.rowmap[r_]); }, W.d1, W.r, W.part);
