@@ -25,7 +25,8 @@ _ip = C.POINTER(C.c_int)
 
 
 class Options(C.Structure):
-    _fields_ = [("device", C.c_int), ("stream", C.c_void_p), ("sm_limit", C.c_int), ("reserved", C.c_int * 5)]
+    _fields_ = [("device", C.c_int), ("stream", C.c_void_p), ("sm_limit", C.c_int), ("small_variant", C.c_int),
+                ("reserved", C.c_int * 4)]
 
 
 class Array(C.Structure):
@@ -473,10 +474,10 @@ def _gain_call(bp, B, steps, device, call, sync=None):
 class Engine:
     """One handle == one GPU + one stream (include/copra_b200.h)."""
 
-    def __init__(self, device=0, stream=None, sm_limit=0):
+    def __init__(self, device=0, stream=None, sm_limit=0, small_variant=0):
         self.lib = load()
         opt = Options()
-        opt.device, opt.stream, opt.sm_limit = int(device), stream, int(sm_limit)
+        opt.device, opt.stream, opt.sm_limit, opt.small_variant = int(device), stream, int(sm_limit), int(small_variant)
         self.h = C.c_void_p()
         self.solve_count = 0  # solves run through this object (copra_b200.autograd detects a stale backward with it)
         self._last_bp = None  # the problem of the resident build, for the shapes of lmpc_vjp's gradients

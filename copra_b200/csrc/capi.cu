@@ -44,7 +44,8 @@ struct copra_b200_handle {
     bool own_stream = false;
     int sms = 148;
     size_t smem_optin = 227 * 1024;
-    int sm_limit = 0;
+    int plan_sms = 148;     // SMs the solver planners size their grids for: sms, or copra_b200_options::sm_limit if smaller
+    int small_variant = 0;  // copra_b200_options::small_variant
     std::string err;
     long long launches = 0;
     long long call_launches = 0;
@@ -79,6 +80,7 @@ struct copra_b200_handle {
     int bound_cstr = -1;
     bool in_resolve = false;
     bool lmpc_solve_active = false; // run_gi is called from do_solve (a resident LMPC build), not from the raw-QP entry
+    bool gt_shared = false;    // ... with a batch-invariant system and Hessian (one factor, the Dpsi / Hpsi tables)
     bool gt_pform = false;     // ... in its shared-factor form (P = Jt Q1 kept, no factor mat-vec per pass)
     const char* solver = "";   // K5+K6 kernel(s) of the last solve
     bool nvtx_open = false;    // an NVTX stage range is open on the calling thread
@@ -497,8 +499,7 @@ template <class T> int ws(copra_b200_handle* h, const char* name, size_t count, 
 int run_gi(copra_b200_handle* h, GiBatch& G)
 {
     int rc;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
-    GiPlan plan = gi_plan(G.n, G.meq, G.m, G.batch, sms, h->smem_optin);
+    GiPlan plan = gi_plan(G.n, G.meq, G.m, G.batch, h->plan_sms, h->smem_optin, h->small_variant);
     int* counter = nullptr;
     if ((rc = ws(h, "counter", 2, &counter))) return rc;
     CU(cudaMemsetAsync(counter, 0, 2 * sizeof(int), h->stream));
@@ -509,7 +510,7 @@ int run_gi(copra_b200_handle* h, GiBatch& G)
     G.ws = nullptr; G.ws_stride = plan.ws_stride;
     h->solver = plan.small ? "gi_small_kernel" : "gi_batch_kernel";
     G.jcache = nullptr; G.jflag = nullptr; G.jmode = 0;
-    if (plan.small && h->lmpc_solve_active && !getenv("COPRA_B200_NO_FACTOR_CACHE")) {
+    if (plan.small && h->lmpc_solve_active) {
         // re-solves of a resident LMPC build: the first one stores every instance's factor, the following ones load it
         // (<= 2 GB of cache; a plain build + solve pays nothing)
         const int n2e = (G.n + 1) & ~1;
@@ -540,7 +541,7 @@ int run_gi(copra_b200_handle* h, GiBatch& G)
         plan.threads = 512; plan.j_smem = plan.s_smem = plan.a_smem = 0;
         plan.smem_bytes = gi_layout(G.n, G.meq, G.m, 512, 0, 0, 0).bytes;
         plan.ws_stride = 2LL * odd_ld(G.n) * G.n;
-        plan.grid = std::max(1, std::min(G.batch, sms));
+        plan.grid = std::max(1, std::min(G.batch, h->plan_sms));
         G.j_smem = G.s_smem = G.a_smem = 0;
         G.ws_stride = plan.ws_stride;
     }
@@ -557,14 +558,13 @@ bool plan_thin(copra_b200_handle* h)
 {
     const BuildParams& P = h->bp;
     h->use_thin = false;
-    if (getenv("COPRA_B200_LEGACY_SOLVER")) return false;
     if (P.initial_state) return false;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
-    const GiPlan legacy = gi_plan(P.nvar, P.meq, P.mineq, P.batch, sms, h->smem_optin);
+    const int sms = h->plan_sms;
+    const GiPlan legacy = gi_plan(P.nvar, P.meq, P.mineq, P.batch, sms, h->smem_optin, h->small_variant);
     if (legacy.small) return false;
     // a handful of instances: the cluster kernel spreads ONE instance over several SMs (latency); the thin kernel is the
     // throughput design (one SM per instance) and wins as soon as the clusters would not cover the batch in one wave
-    if (legacy.cluster > 0 && P.batch * legacy.cluster * 2 <= sms && !getenv("COPRA_B200_THIN_SOLVER")) return false;
+    if (legacy.cluster > 0 && P.batch * legacy.cluster * 2 <= sms) return false;
     GtBatch& T = h->gt;
     std::memset(&T, 0, sizeof T);
     T.n = P.nvar; T.meq = P.meq; T.m = P.mineq; T.batch = P.batch;
@@ -581,20 +581,19 @@ bool plan_thin(copra_b200_handle* h)
     T.tab_doubles = tab;
     T.ldk = (P.N + 1) | 1;
     T.ld = gt_even(T.n);
-    const char* re = getenv("COPRA_B200_THIN_REORTH");
-    T.reorth = re ? atof(re) : 1e-2;
+    T.reorth = 1e-2;
     // state-space evaluation of the general rows (chunks of 16 steps) when its tables fit next to everything else
     T.nx = P.nx; T.X = P.X;
-    { const char* le = getenv("COPRA_B200_THIN_SS_CHUNK"); T.ssL = le ? std::max(2, atoi(le)) : 16; }
+    T.ssL = 16;
     T.ssC = (P.N + T.ssL - 1) / T.ssL;
     int eg = 0;
     for (int k = 0; k < P.nfam; ++k) eg += P.fam[k].rows * ((P.fam[k].hasE ? P.nx : 0) + (P.fam[k].hasG ? P.nu : 0));
     T.ss_doubles = gt_ss_layout(P.nx, P.nu, P.N, T.ssL, T.ssC, eg).total;
-    T.ss = (P.meq + P.mineq > 0 && !getenv("COPRA_B200_THIN_NO_SS")) ? 1 : 0;
+    T.ss = P.meq + P.mineq > 0 ? 1 : 0;
     if (!T.ss) T.ss_doubles = 0;
     // batch-invariant system AND Hessian: Dpsi / Hpsi tables and the P form of the pass (see GtBatch)
-    const bool shared_all = P.sQ == 0 && P.A.s == 0 && P.B.s == 0 && !getenv("COPRA_B200_THIN_NO_DPSI");
-    GtShape shape{ T.n, T.meq, T.m, tab, T.ldk, T.ld, T.ss_doubles, (shared_all && !getenv("COPRA_B200_THIN_NO_PFORM")) ? 1 : 0 };
+    const bool shared = P.sQ == 0 && P.A.s == 0 && P.B.s == 0;
+    GtShape shape{ T.n, T.meq, T.m, tab, T.ldk, T.ld, T.ss_doubles, shared ? 1 : 0 };
     h->gtplan = gt_plan(shape, T.batch, sms, h->smem_optin);
     if (shape.pform && T.n > h->gtplan.threads) { shape.pform = 0; h->gtplan = gt_plan(shape, T.batch, sms, h->smem_optin); }
     if (T.ss && !h->gtplan.ok) { // does not fit: convolution form
@@ -603,21 +602,18 @@ bool plan_thin(copra_b200_handle* h)
     }
     // Per-instance factors and big streams (n >= 512) in a batch of only a few waves: the step is the latency of its heaviest
     // instance, which is bound by what ONE SM can stream -- give every instance a thread-block cluster instead.
-    {
-        const char* ce = getenv("COPRA_B200_THIN_CLUSTER");
-        // 16 CTAs per instance (a non-portable cluster size: one cluster per GPC) when the device schedules them, else 8:
-        // C5's heaviest instance takes 0.39 s on 16 CTAs, 0.53 s on 8, 2.3 s on one
-        const int want = ce ? atoi(ce) : ((!shared_all && P.sQ != 0 && T.n >= 512 && P.batch <= 16 * sms) ? 16 : 0);
-        for (int csize = want; csize > 1 && h->gtplan.ok; csize >>= 1) {
-            if ((csize & (csize - 1)) != 0 || csize > 16) break;
+    // 16 CTAs per instance (a non-portable cluster size: one cluster per GPC) when the device schedules them, else 8:
+    // C5's heaviest instance takes 0.39 s on 16 CTAs, 0.53 s on 8, 2.3 s on one
+    if (P.sQ != 0 && T.n >= 512 && P.batch <= 16 * sms) {
+        for (int csize = 16; csize > 1 && h->gtplan.ok; csize >>= 1) {
             GtShape cs = shape;
             cs.cluster = csize; cs.pform = 0; cs.ss_doubles = 0;
             const GtPlan cp = gt_plan(cs, T.batch, sms, h->smem_optin);
             if (cp.ok) { h->gtplan = cp; shape = cs; T.ss = 0; T.ss_doubles = 0; break; }
-            if (ce) break; // an explicit request is not silently replaced
         }
     }
     if (!h->gtplan.ok) return false;
+    h->gt_shared = shared;
     h->gt_pform = shape.pform != 0;
     T.lay = gt_layout(T.n, T.meq, T.m, T.tab_doubles, h->gtplan.threads, h->gtplan.q1s, T.ss_doubles);
     T.ssl = gt_ss_layout(P.nx, P.nu, P.N, T.ssL, T.ssC, eg);
@@ -631,7 +627,6 @@ int run_gt(copra_b200_handle* h, double* x, int* status, int* iters, int* nact, 
     const BuildParams& P = h->bp;
     GtBatch& T = h->gt;
     const GtPlan& plan = h->gtplan;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
     const size_t n = P.nvar, ldj = size_t(T.ld), count = P.sQ ? size_t(P.batch) : 1;
     int rc;
     double *Jt = nullptr, *JtT = nullptr, *wsp = nullptr;
@@ -642,8 +637,7 @@ int run_gt(copra_b200_handle* h, double* x, int* status, int* iters, int* nact, 
     if ((rc = ws(h, "gt_ws", size_t(plan.grid) * plan.ws_stride, &wsp))) return rc;
     if ((rc = ws(h, "counter", 2, &counter))) return rc;
     // batch-invariant system and Hessian: Dpsi = Jt' Psi' once per build (one Toeplitz fill + one DMMA GEMM)
-    const bool use_dpsi = P.sQ == 0 && P.A.s == 0 && P.B.s == 0 && !getenv("COPRA_B200_THIN_NO_DPSI");
-    const bool pform = use_dpsi && h->gt_pform;
+    const bool use_dpsi = h->gt_shared, pform = h->gt_pform;
     double *psit = nullptr, *dpsi = nullptr, *hpsi = nullptr, *hm = nullptr;
     if (use_dpsi) {
         if ((rc = ws(h, "gt_psit", n * size_t(P.X), &psit))) return rc;
@@ -654,7 +648,7 @@ int run_gt(copra_b200_handle* h, double* x, int* status, int* iters, int* nact, 
         if ((rc = ws(h, "gt_hm", ldj * n, &hm))) return rc;
     }
     if (!h->factor_valid) {
-        cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, P.nvar, T.ld, int(count), Jt, JtT, pd, sms, h->stream);
+        cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, P.nvar, T.ld, int(count), Jt, JtT, pd, h->plan_sms, h->stream);
         if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
         h->launches += 1; h->call_launches += 1;
         if (use_dpsi) {
@@ -711,7 +705,7 @@ int run_gt(copra_b200_handle* h, double* x, int* status, int* iters, int* nact, 
     if (h->warm_start && pform && (rc = ws(h, "warm_iact", size_t(P.batch) * n, &warm_iact))) return rc;
     T.warm = (h->warm_start && pform && h->in_resolve && h->warm_valid) ? warm_iact : nullptr;
     const int slots = plan.cluster > 1 ? plan.grid / plan.cluster : plan.grid; // instances in flight
-    const bool lpt = P.batch > slots && (P.batch <= 24 * slots || plan.cluster > 1) && !getenv("COPRA_B200_THIN_NO_LPT");
+    const bool lpt = P.batch > slots && (P.batch <= 24 * slots || plan.cluster > 1);
     cudaError_t e;
     if (lpt) {
         int *keys = nullptr, *keys2 = nullptr, *idx = nullptr, *order = nullptr;
@@ -729,7 +723,7 @@ int run_gt(copra_b200_handle* h, double* x, int* status, int* iters, int* nact, 
         CU(cudaMemsetAsync(counter, 0, 2 * sizeof(int), h->stream));
         T.prekey = nullptr; T.preidx = nullptr; T.order = order;
         // clusters for the head of the longest-first queue only (the heavy tail of the iteration counts)
-        if (plan.cluster > 1) { const char* kh = getenv("COPRA_B200_THIN_HEAVY"); T.kheavy = kh ? atoi(kh) : std::max(1, P.batch / 16); }
+        if (plan.cluster > 1) T.kheavy = std::max(1, P.batch / 16);
     }
     e = gt_launch(T, plan, h->stream);
     if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_launch: %s", cudaGetErrorString(e));
@@ -783,7 +777,6 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
         const copra_b200_cost& c = p->costs[i];
         if (c.full_size == 1 || (c.M.ptr && c.M.stride != 0) || (c.N.ptr && c.N.stride != 0) || c.w.stride != 0) q_shared = false;
     }
-    if (getenv("COPRA_B200_NO_SHARED_HESSIAN")) q_shared = false;
     P.sQ = q_shared ? 0 : (long long)pl.sz.nvar * pl.sz.nvar;
 
     // selector matrices + line indices for TrajectoryBound families (tiny, shared by all instances)
@@ -892,8 +885,7 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
         F.sMGx = r * nu * (N + 1); F.sMPhi = r * nx * ns; F.sres = r * ns; F.sE = size_t(nx) * nU; F.sf = nU;
         // E = (M Phi)' W (M Psi + N) does not depend on p, x0 or d: one copy for the batch when A, B, M, N, w are shared
         // (src/costFunctions.cpp:77,105,210) -- the per-instance part of the assembly is f alone
-        const bool e_shared = !F.dense && P.A.s == 0 && P.B.s == 0 && (!F.hasM || F.M.s == 0) && (!F.hasN || F.N.s == 0) && F.w.s == 0 &&
-            !getenv("COPRA_B200_NO_SHARED_HESSIAN");
+        const bool e_shared = !F.dense && P.A.s == 0 && P.B.s == 0 && (!F.hasM || F.M.s == 0) && (!F.hasN || F.N.s == 0) && F.w.s == 0;
         if (e_shared) F.sE = 0;
         snprintf(nm, sizeof nm, "MGx%d", i); if ((rc = ws(h, nm, Bz * F.sMGx, &F.MGx))) return rc;
         snprintf(nm, sizeof nm, "MPhi%d", i); if ((rc = ws(h, nm, Bz * F.sMPhi, &F.MPhi))) return rc;
@@ -1032,7 +1024,6 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
 int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
 {
     const BuildParams& P = h->bp;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
     const size_t n = P.nvar, count = P.sQ ? size_t(P.batch) : 1;
     const int ldj = gt_even(int(n));
     int rc;
@@ -1047,7 +1038,7 @@ int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
     if ((rc = ws(h, "vjp_JtT", count * ldj * n, &JT))) return rc;
     if ((rc = ws(h, "vjp_pd", count, &pd))) return rc;
     if (!h->vjp_factor_valid) {
-        cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, int(n), ldj, int(count), J, JT, pd, sms, h->stream);
+        cudaError_t e = gt_factor_launch(DArr{ P.Q, P.sQ }, int(n), ldj, int(count), J, JT, pd, h->plan_sms, h->stream);
         if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
         h->launches += 1; h->call_launches += 1;
         h->vjp_factor_valid = true;
@@ -1065,7 +1056,6 @@ constexpr size_t kSensWsBytes = size_t(1) << 30;
 template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk& S, int k, First first, Last last)
 {
     const BuildParams& P = h->bp;
-    const int sms = h->sm_limit > 0 ? std::min(h->sm_limit, h->sms) : h->sms;
     const size_t B = P.batch, n = P.nvar, K = size_t(k);
     int rc;
     int *status = nullptr, *nact = nullptr, *iact = nullptr;
@@ -1122,7 +1112,7 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
                 (long long)MK * MK, nb, h->stream));
             LAUNCHED(sens_gram_launch(S, nb, h->stream));
             cudaError_t e = gt_factor_launch(DArr{ S.Gq, (long long)nm * nm }, nm, S.ldg, nb, const_cast<double*>(S.GJ), GJT,
-                const_cast<int*>(S.gpd), sms, h->stream);
+                const_cast<int*>(S.gpd), h->plan_sms, h->stream);
             if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
             h->launches += 1; h->call_launches += 1;
         }
@@ -1314,7 +1304,8 @@ int copra_b200_create(const copra_b200_options* opt, copra_b200_handle** out)
     h->device = dev;
     h->sms = prop.multiProcessorCount;
     h->smem_optin = prop.sharedMemPerBlockOptin;
-    h->sm_limit = opt ? opt->sm_limit : 0;
+    h->plan_sms = (opt && opt->sm_limit > 0) ? std::min(opt->sm_limit, h->sms) : h->sms;
+    h->small_variant = opt ? opt->small_variant : 0;
     h->vsmall = gi_vsmall();
     if (opt && opt->stream) h->stream = static_cast<cudaStream_t>(opt->stream);
     else {

@@ -26,7 +26,6 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 
 namespace cb {
 
@@ -347,9 +346,8 @@ int dgemm_dmma_launch(int transA, int M, int N, int K, double alpha, const doubl
         g.B = B + (long long)b0 * sB; g.ldb = ldb; g.sB = sB;
         g.C = C + (long long)b0 * sC; g.ldc = ldc; g.sC = sC;
         // tensor-map TMA pipeline when the operands qualify (16-byte aligned, even leading dimensions / batch strides)
-        static const bool no_tma = getenv("COPRA_B200_DGEMM_NO_TMA") != nullptr;
         CUtensorMap ta, tb;
-        const bool tma = !no_tma && K >= 1 &&
+        const bool tma = K >= 1 &&
             (transA ? make_map(&ta, g.A, K, M, lda, sA, nb, PK, PM) : make_map(&ta, g.A, M, K, lda, sA, nb, 16, PK)) &&
             make_map(&tb, g.B, K, N, ldb, sB, nb, PK, PN);
         cudaError_t e;

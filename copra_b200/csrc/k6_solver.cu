@@ -6,7 +6,6 @@
 #include "launch.h"
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace cb {
 
@@ -132,14 +131,7 @@ double gi_vsmall()
     return vsmall;
 }
 
-static int gi_cluster_threads()
-{
-    const char* e = getenv("COPRA_B200_CLUSTER_THREADS"); // tuning knob
-    const int t = e ? atoi(e) : 512;
-    return (t == 128 || t == 256 || t == 512) ? t : 512;
-}
-
-GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin)
+GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin, int small_variant)
 {
     GiPlan p;
     p.small = 0;
@@ -158,12 +150,10 @@ GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin)
             if (per_sm > best_per_sm) { best = v; best_per_sm = per_sm; best_bytes = b; }
             if (per_sm >= kSmMinB) break;
         }
-        if (const char* e = getenv("COPRA_B200_SMALL_VARIANT")) { // tuning knob: force a residency variant
-            const int v = atoi(e);
-            if (v >= 0 && v < 3) {
-                const size_t b = gs_layout(n, meq, m, v < 1, v < 2).bytes;
-                if (b + 2048 <= smem_optin) { best = v; best_bytes = b; best_per_sm = int(std::min<size_t>(kSmMinB, (smem_optin + 1024) / (b + 1024))); }
-            }
+        if (small_variant >= 1 && small_variant <= 3) { // testing: force residency variant small_variant - 1 when it fits
+            const int v = small_variant - 1;
+            const size_t b = gs_layout(n, meq, m, v < 1, v < 2).bytes;
+            if (b + 2048 <= smem_optin) { best = v; best_bytes = b; best_per_sm = int(std::min<size_t>(kSmMinB, (smem_optin + 1024) / (b + 1024))); }
         }
         if (best >= 0) {
             p.small = 1;
@@ -178,11 +168,10 @@ GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin)
     // n too large for one SM's shared memory: a cluster of C CTAs shares J through DSMEM
     if (size_t(odd_ld(n)) * n * sizeof(double) + 24 * 1024 > smem_optin) {
         for (int C = 2; C <= kClMaxC; C *= 2) {
-            const int cth = gi_cluster_threads();
-            const size_t b = gc_layout(n, meq, m, C, cth).bytes;
+            const size_t b = gc_layout(n, meq, m, C, 512).bytes;
             if (b + 2048 <= smem_optin) {
                 p.cluster = C;
-                p.threads = cth;
+                p.threads = 512;
                 p.smem_bytes = b;
                 p.j_smem = 1; p.s_smem = 0; p.a_smem = 0;
                 p.ws_stride = 0;

@@ -6,7 +6,6 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include <algorithm>
-#include <cstdlib>
 
 namespace cb {
 
@@ -74,18 +73,11 @@ cudaError_t gt_psit_fill_launch(const double* Gs, double* PsiT, int nx, int nu, 
     return cudaGetLastError();
 }
 
-static int gt_env_int(const char* name, int dflt)
-{
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
-
 int gt_cluster_capacity(const GtPlan& plan, int csize); // k6_thin_cluster.cu
 
 GtPlan gt_plan(const GtShape& sh, int batch, int sms, size_t smem_optin)
 {
     GtPlan p{};
-    p.threads = gt_env_int("COPRA_B200_THIN_THREADS", 512);
     // 512 threads per instance: 256 (47.7 k solves/s on C3) and 1024 x 1 CTA/SM (51.1 k) were measured against 512 x 2 (63.0 k) and
     // dropped -- every extra instantiation of the solver costs minutes of compile time
     p.threads = 512;
@@ -104,20 +96,17 @@ GtPlan gt_plan(const GtShape& sh, int batch, int sms, size_t smem_optin)
         p.grid = std::max(1, std::min(batch, cap)) * sh.cluster;
         return p;
     }
-    // one CTA per SM; whatever shared memory the vectors and tables leave holds the head columns of Q1
-    int per_sm = std::max(1, gt_env_int("COPRA_B200_THIN_CTAS_PER_SM", 2));
-    per_sm = std::min(per_sm, 2048 / p.threads);
-    per_sm = std::min<int>(per_sm, int((smem_optin + 1024) / (base + 1024)));
+    // one CTA per instance, two per SM when their shared memory fits; whatever shared memory the vectors and tables leave
+    // holds the head columns of Q1
+    const int per_sm = std::min<int>(2, int((smem_optin + 1024) / (base + 1024)));
     const size_t budget = (smem_optin + 1024) / per_sm - 1024 - 1024; // per CTA, minus static shared memory headroom
     int q1s = budget > base ? int((budget - base) / (size_t(sh.ld) * sizeof(double))) : 0;
     q1s = std::min(q1s, sh.n);
-    q1s = std::min(q1s, std::max(0, gt_env_int("COPRA_B200_THIN_Q1S", sh.n)));
     if (sh.pform) q1s = 0; // the shared-factor kernels are compiled without the shared-memory head of P
     p.q1s = q1s;
     p.smem_bytes = gt_layout(sh.n, sh.meq, sh.m, sh.tab_doubles, p.threads, q1s, sh.ss_doubles).bytes;
     p.per_sm = per_sm;
     p.grid = std::max(1, std::min(batch, sms * per_sm));
-    p.grid = std::max(1, std::min(p.grid, gt_env_int("COPRA_B200_THIN_GRID", p.grid)));
     p.ws_stride = (long long)sh.ld * sh.n + (long long)sh.n * sh.n; // Q1 (or P), S
     return p;
 }

@@ -35,8 +35,9 @@ struct GiPlan {
     long long ws_stride; // doubles per CTA of global workspace
 };
 
-// choose threads / smem residency / grid for a (n, meq, m) shape on a device with `sms` SMs
-GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin);
+// choose threads / smem residency / grid for a (n, meq, m) shape on a device with `sms` SMs; small_variant is
+// copra_b200_options::small_variant (0 = the planner's choice)
+GiPlan gi_plan(int n, int meq, int m, int batch, int sms, size_t smem_optin, int small_variant);
 cudaError_t gi_launch(const GiBatch& B, const GiPlan& plan, cudaStream_t st);
 double gi_vsmall();
 // cluster path (gi_cluster.cuh): S workspace of odd_ld(n)*n doubles per cluster, sized by the caller

@@ -51,7 +51,9 @@ typedef struct {
     int device;          /* CUDA device ordinal */
     void* stream;        /* cudaStream_t to launch on; NULL = the handle creates its own */
     int sm_limit;        /* 0 = use every SM; otherwise cap the persistent grids (testing) */
-    int reserved[5];
+    int small_variant;   /* testing: 0 = planner's choice, 1..3 force shared-memory residency variant 0..2 of the small-n
+                            kernel (gi_small_kernel) when it fits */
+    int reserved[4];
 } copra_b200_options;
 
 typedef struct {

@@ -104,10 +104,11 @@ def test_resolve_against_the_oracle(engine, make, shift):
     assert np.array_equal(back["control"], first["control"]) and np.array_equal(back["iact"], first["iact"])
 
 
-def test_c1_fixture_batched_through_the_thin_solver(engine, monkeypatch):
+def test_c1_fixture_batched_with_shared_and_per_instance_weights(engine):
     """the BoundedSystem fixture (n = 300, single input: odd Toeplitz supports, 112 active trajectory-bound rows, cond(Q) ~ 3e4)
-    as a batch with perturbed x0 -> thin solver with a shared factor; and the same instances with the factor forced
-    per-instance (COPRA_B200_NO_SHARED_HESSIAN) must give identical results"""
+    as a batch with perturbed x0 -> thin solver with a shared factor; and the same instances with per-instance weights (the
+    same values for every instance, so the Hessian and every cost's E are assembled and factored per instance) must give
+    identical results"""
     base = wl.c1("target")
     rng = np.random.default_rng(5)
     B = 24
@@ -118,8 +119,7 @@ def test_c1_fixture_batched_through_the_thin_solver(engine, monkeypatch):
     assert w["iter_diff"] == 0
     shared = engine.lmpc_run(bp)
     assert engine.hessian_is_shared() and "gi_thin_kernel" in engine.last_solver()
-    monkeypatch.setenv("COPRA_B200_NO_SHARED_HESSIAN", "1")
-    own = engine.lmpc_run(bp)
+    own = engine.lmpc_run(dict(bp, costs=[dict(c, w=np.tile(c["w"], (B, 1))) for c in bp["costs"]]))
     assert not engine.hessian_is_shared()
     assert np.array_equal(shared["iact"], own["iact"]) and np.abs(shared["x"] - own["x"]).max() <= 1e-9
 

@@ -117,10 +117,11 @@ def test_c3(engine):
     assert w.get("excused_rows", 0) == 0 and w["iter_diff"] == 0
 
 
-def test_c3_cluster_kernel(engine, monkeypatch):
-    """the same shape through the latency-oriented cluster kernel (what a handful of instances use)"""
-    monkeypatch.setenv("COPRA_B200_LEGACY_SOLVER", "1")
+def test_c3_cluster_kernel(engine):
+    """the same shape through the latency-oriented cluster kernel (what a handful of instances use: 4 clusters of at most 8
+    CTAs cover the batch twice over on 148 SMs)"""
     check_batch(engine, wl.c3(batch=4))
+    assert engine.last_solver() == "gi_cluster_kernel"
 
 
 def test_c4_initial_state(engine):
@@ -132,35 +133,62 @@ def test_c5(engine):
     check_batch(engine, wl.c5(batch=8))
 
 
-def test_c5_single_cta_kernel(engine, monkeypatch):
-    """the same shape with one CTA per instance (what batches of many waves use)"""
-    monkeypatch.setenv("COPRA_B200_THIN_CLUSTER", "1")
-    check_batch(engine, wl.c5(batch=4))
+def test_c5_single_cta_kernel():
+    """the same shape with one CTA per instance (what batches of many waves use): the planner gives each instance a cluster
+    only while the batch is at most 16 instances per SM, so 17 instances on one SM take the single-CTA kernel"""
+    eng = capi.Engine(0, sm_limit=1)
+    try:
+        check_batch(eng, wl.c5(batch=17), instances=range(4))
+        assert eng.last_solver() == "gt_factor_kernel + gi_thin_kernel"
+    finally:
+        eng.close()
 
 
-def test_c5_hybrid_cluster_queue(engine, monkeypatch):
-    """longest-first queue whose head is solved by whole clusters and whose tail by single CTAs: every placement gives the
-    same iterates (identical counts and active sets, x to rounding) as the all-single-CTA run, and the oracle's on a sample"""
-    bp = wl.c5(batch=40)
+def test_c5_hybrid_cluster_queue(engine):
+    """longest-first queue whose head (batch / 16 = 5 instances) is solved by whole clusters and whose tail by single CTAs:
+    every placement gives the same iterates (identical counts and active sets, x to rounding) as the all-single-CTA run (80
+    instances on 4 SMs), and the oracle's on a sample"""
+    bp = wl.c5(batch=80)
     want = ("status", "iters", "control", "iact", "nact")
-    monkeypatch.setenv("COPRA_B200_THIN_HEAVY", "5")
     hyb = engine.lmpc_run(bp, want=want)
     assert "thin" in engine.last_solver()
-    monkeypatch.setenv("COPRA_B200_THIN_CLUSTER", "1")
-    solo = engine.lmpc_run(bp, want=want)
+    eng = capi.Engine(0, sm_limit=4)
+    try:
+        solo = eng.lmpc_run(bp, want=want)
+        assert "thin" in eng.last_solver()
+    finally:
+        eng.close()
     assert np.array_equal(hyb["status"], solo["status"]) and np.array_equal(hyb["iters"], solo["iters"])
     assert np.array_equal(hyb["iact"], solo["iact"])
     assert np.abs(hyb["control"] - solo["control"]).max() <= 1e-9
     heavy = np.argsort(-hyb["iters"].sum(axis=1))[:2]
-    for i in list(heavy) + [0, 39]:
+    for i in list(heavy) + [0, 79]:
         o = po.lmpc(wl.instance(bp, int(i)))
         assert x_err(hyb["control"][i], o["control"]) < 1e-6
         assert active_set(hyb["iact"][i]) == active_set(o["iact"]) and tuple(hyb["iters"][i]) == tuple(o["iter"])
 
 
-def test_c5_general_kernel(engine, monkeypatch):
-    monkeypatch.setenv("COPRA_B200_LEGACY_SOLVER", "1")
-    check_batch(engine, wl.c5(batch=1))
+def test_c5_general_kernel(engine):
+    """C5's QP (n = 800, more than the cluster kernel holds) through the raw-QP entry, whose planner sends it to the
+    single-CTA general kernel"""
+    bp = wl.c5(batch=1)
+    hb = capi.HostBatch(bp)
+    engine.lmpc_run(hb)
+    st = {k: engine.download(hb, k) for k in STAGES}
+    o = po.lmpc(wl.instance(bp, 0))
+    for k in STAGES:
+        assert rel_err(st[k][0], o[k]) <= 1e-10, (k, rel_err(st[k][0], o[k]))
+        assert zeros_preserved(st[k][0], o[k]), (k, "structural zeros")
+    eq = st["Aeq"].shape[1] > 0
+    r = engine.solve_qp_batch(st["Q"], st["c"], st["Aeq"] if eq else None, st["beq"] if eq else None, st["Aineq"], st["bineq"],
+                              st["lb"], st["ub"])
+    assert engine.last_solver() == "gi_batch_kernel"
+    assert r["status"][0] == o["fail"] == 0
+    # LMPC mode: the decision variables are the controls
+    assert x_err(r["x"][0], o["x"]) <= 1e-6 and x_err(r["x"][0], o["control"]) <= 1e-6
+    excused = active_set_excused(active_set(r["iact"][0], r["nact"][0]), o)
+    assert tuple(r["iters"][0]) == tuple(o["iter"]), (r["iters"][0], o["iter"])
+    print(bp["name"], {"excused_rows": excused})
 
 
 # ---- committed golden fixtures (tests/golden/make_golden.py) -------------------------------------------
@@ -392,7 +420,7 @@ def test_receding_horizon_resolve(engine):
     assert not np.array_equal(again["control"], first["control"])
 
 
-def test_small_solver_residency_variants(engine, monkeypatch):
+def test_small_solver_residency_variants():
     """gi_small_kernel keeps S and the general rows in shared memory or in global memory (L2) depending on how many
     instances fit an SM; every variant runs the same algorithm (same pivots, same active sets; the compiler may
     contract a*b+c*d differently per instantiation, so x agrees to rounding, not bit for bit)"""
@@ -413,10 +441,13 @@ def test_small_solver_residency_variants(engine, monkeypatch):
         cases.append((Q, c, Aeq if meq else None, beq if meq else None, Aineq, bineq, lb, ub))
     bp = wl.c2(batch=48)
     ref = None
-    for v in ("0", "1", "2"):
-        monkeypatch.setenv("COPRA_B200_SMALL_VARIANT", v)
-        out = [engine.solve_qp_batch(*cs) for cs in cases]
-        mpc = engine.lmpc_run(bp)
+    for v in range(3):
+        eng = capi.Engine(0, small_variant=v + 1)
+        try:
+            out = [eng.solve_qp_batch(*cs) for cs in cases]
+            mpc = eng.lmpc_run(bp)
+        finally:
+            eng.close()
         if ref is None:
             ref = (out, mpc)
             for cs, r in zip(cases, out):  # variant 0 against the oracle
