@@ -8,7 +8,7 @@ OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_th
 LIB := copra_b200/lib/libcopra_b200.so
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/copra_b200.h
 
-all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp tests/cpp/test_jvp
+all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp tests/cpp/test_jvp tests/cpp/test_vjp_costs
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; false)
@@ -49,3 +49,9 @@ tests/cpp/test_jvp: tests/cpp/test_jvp.cpp $(wildcard include/copra/*) include/c
 	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_jvp.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
 
 jvp-test: tests/cpp/test_jvp
+
+# BatchedLMPC::vjp with the cost gradients: writes them for tests/test_vjp_costs_gpu.py, checks its errors (GPU)
+tests/cpp/test_vjp_costs: tests/cpp/test_vjp_costs.cpp $(wildcard include/copra/*) include/copra_b200.h $(LIB)
+	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_vjp_costs.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
+
+vjp-costs-test: tests/cpp/test_vjp_costs

@@ -2,13 +2,16 @@
 vector-Jacobian product of copra_b200_lmpc_vjp (K8) on the same engine, and forward-mode AD (torch.autograd.forward_ad) the
 exact Jacobian-vector product of copra_b200_lmpc_jvp (K9).
 
-    ctrl, traj = copra_b200.autograd.lmpc(engine, bp, x0, p=[...], f=[...], lower=[...], upper=[...])
+    ctrl, traj = copra_b200.autograd.lmpc(engine, bp, x0, p=[...], f=[...], lower=[...], upper=[...], w=[...], M=[...], N=[...])
 
 `bp` is a workloads-style batch problem that fixes the matrices (A, B, d, M, N, w, E, G) and the kinds and shapes of every
 entry; the vectors are CUDA float64 tensors, batch-major (batch, length), one per cost (p) and one per constraint (f for row
 constraints, lower / upper for bounds; None keeps bp's value, which then gets no gradient).  Every instance gets its own
-gradient.  The backward and the forward-mode tangent raise if another solve ran on the engine since this forward: the
-engine keeps only the last solve.
+gradient.  The cost weights and matrices w (rows), M (rows, nx) and N (rows, nu) may be given per cost as CUDA float64
+tensors too, in reverse mode only (copra_b200_lmpc_vjp_costs): a batched tensor (leading batch axis) gets per-instance
+gradients; an unbatched one is shared by the batch (stride 0: the Hessian stays batch-invariant) and its gradient is the sum
+over the batch.  A non-zero forward-mode tangent on them raises NotImplementedError.  The backward and the forward-mode
+tangent raise if another solve ran on the engine since this forward: the engine keeps only the last solve.
 """
 import ctypes as C
 
@@ -23,7 +26,29 @@ def _vec_entries(bp):
     keys = [("p", i) for i in range(len(bp["costs"]))]
     for j, c in enumerate(bp["constraints"]):
         keys += [("lower", j), ("upper", j)] if c["kind"] in ("trajectory_bound", "control_bound") else [("f", j)]
-    return keys
+    return keys + [(k, i) for i in range(len(bp["costs"])) for k in _COST_KEYS]
+
+
+_COST_KEYS = ("w", "M", "N")
+_BASE_NDIM = dict(w=1, M=2, N=2)
+
+
+def _patch_cost_matrix(problem, pr, kind, i, t):
+    """point cost i's `kind` (w, M or N) of the packed problem at the tensor t (batched or shared, logical row-major)"""
+    rows, has_m, has_n = capi.cost_shapes(problem)[i]
+    if (kind == "M" and not has_m) or (kind == "N" and not has_n):
+        raise ValueError("cost %d (%s) has no %s" % (i, problem["costs"][i]["kind"], kind))
+    base = _BASE_NDIM[kind]
+    if t.dim() not in (base, base + 1) or t.shape[-base] != rows:
+        raise ValueError("cost %d: %s has shape %s, expected %d rows (with an optional leading batch axis)"
+                         % (i, kind, tuple(t.shape), rows))
+    t = t.detach().to(torch.float64)
+    if base == 2:
+        t = t.transpose(-1, -2)  # the engine reads M / N column-major
+    t = t.contiguous()
+    arr = getattr(pr.costs[i], kind)
+    arr.ptr, arr.stride = t.data_ptr(), (t[0].numel() if t.dim() > base else 0)
+    return t
 
 
 class _LMPC(torch.autograd.Function):
@@ -37,13 +62,16 @@ class _LMPC(torch.autograd.Function):
         problem["x0"] = np.zeros((B, int(bp["nx"])))
         for (kind, i), v in zip(keys, vecs):
             if v is not None:  # shape only: the tensor itself is patched in below
-                (problem["costs"] if kind == "p" else problem["constraints"])[i][kind] = np.zeros(tuple(v.shape))
+                (problem["costs"] if kind in ("p",) + _COST_KEYS else problem["constraints"])[i][kind] = np.zeros(tuple(v.shape))
         hb = capi.HostBatch(problem, device_tensors=dev)
         live = [x0.detach().contiguous()]
         pr = hb.problem
         pr.x0.ptr, pr.x0.stride = live[0].data_ptr(), live[0].shape[1]
         for (kind, i), v in zip(keys, vecs):
             if v is None:
+                continue
+            if kind in _COST_KEYS:
+                live.append(_patch_cost_matrix(problem, pr, kind, i, v))
                 continue
             t = v.detach().contiguous()
             live.append(t)
@@ -62,6 +90,9 @@ class _LMPC(torch.autograd.Function):
         engine._last_bp = problem
         engine.synchronize()
         ctx.engine, ctx.count, ctx.keys, ctx.present = engine, engine.solve_count, keys, [v is not None for v in vecs]
+        # the build reads x0, w, M and N where they live: the VJP of the cost matrices reads them again
+        ctx.live = (hb, live)
+        ctx.shared = [v is not None and kind in _COST_KEYS and v.dim() == _BASE_NDIM[kind] for (kind, _), v in zip(keys, vecs)]
         ctx.counts = (len(bp["costs"]), len(bp["constraints"]))
         ctx.mark_non_differentiable()
         return control, traj
@@ -76,6 +107,11 @@ class _LMPC(torch.autograd.Function):
         ncost, ncstr = ctx.counts
         tangents = dict(p=[None] * ncost, f=[None] * ncstr, lower=[None] * ncstr, upper=[None] * ncstr)
         for (kind, i), t in zip(ctx.keys, dvecs):
+            if kind in _COST_KEYS:
+                if t is not None and bool(torch.count_nonzero(t)):
+                    raise NotImplementedError("copra_b200.autograd: forward-mode derivatives with respect to the cost weights "
+                                              "and matrices (w, M, N) are not implemented; reverse mode (backward) is")
+                continue
             if t is not None:
                 tangents[kind][i] = t.unsqueeze(1)
         du, dx = eng.lmpc_jvp(x0=dx0.unsqueeze(1) if dx0 is not None else None, **tangents)
@@ -87,17 +123,21 @@ class _LMPC(torch.autograd.Function):
         if eng.solve_count != ctx.count:
             raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the VJP needs the "
                                "active sets of the solve being differentiated")
-        g = eng.lmpc_vjp(dcontrol=dcontrol, dtrajectory=dtraj)  # ordered against torch's stream on both sides
+        want = capi.VJP_WANT + tuple(k for k in _COST_KEYS
+                                     if any(p and kind == k for (kind, _), p in zip(ctx.keys, ctx.present)))
+        g = eng.lmpc_vjp(dcontrol=dcontrol, dtrajectory=dtraj, want=want)  # ordered against torch's stream on both sides
         grads = [g["x0"]]
-        for (kind, i), present in zip(ctx.keys, ctx.present):
-            grads.append(g[kind][i] if present else None)
+        for (kind, i), present, shared in zip(ctx.keys, ctx.present, ctx.shared):
+            grad = g[kind][i] if present else None
+            grads.append(grad.sum(0) if shared else grad)  # a shared input's gradient sums its instances'
         return (None, None, None, *grads)
 
 
-def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None):
-    """(control, trajectory) of the batch problem `bp` with the given vector inputs, differentiable with respect to x0 and
-    every vector given (lists indexed by cost / constraint, None entries keep bp's values)."""
+def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None, w=None, M=None, N=None):
+    """(control, trajectory) of the batch problem `bp` with the given inputs, differentiable with respect to x0 and every
+    vector, weight and cost matrix given (lists indexed by cost / constraint, None entries keep bp's values).  w, M and N
+    are (rows,), (rows, nx) and (rows, nu) per cost, or with a leading batch axis; reverse mode only."""
     keys = _vec_entries(bp)
-    given = dict(p=p or [], f=f or [], lower=lower or [], upper=upper or [])
+    given = dict(p=p or [], f=f or [], lower=lower or [], upper=upper or [], w=w or [], M=M or [], N=N or [])
     vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
     return _LMPC.apply(engine, bp, keys, x0, *vecs)

@@ -65,6 +65,10 @@ class VjpOut(C.Structure):
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
 
 
+class VjpCostOut(C.Structure):
+    _fields_ = [("w", C.POINTER(C.c_void_p)), ("M", C.POINTER(C.c_void_p)), ("N", C.POINTER(C.c_void_p))]
+
+
 class JvpIn(C.Structure):
     _fields_ = [("ndir", C.c_int), ("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
@@ -86,8 +90,10 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_set_warm_start", "copra_b200_get_warm_start", "copra_b200_multi_set_warm_start",
            "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget", "copra_b200_lmpc_vjp",
            "copra_b200_multi_lmpc_vjp", "copra_b200_lmpc_jvp", "copra_b200_lmpc_feedback_gain",
-           "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain"]
+           "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain", "copra_b200_lmpc_vjp_costs",
+           "copra_b200_multi_lmpc_vjp_costs"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
+VJP_COST_WANT = ("w", "M", "N")  # gradients with respect to the cost weights and matrices: requested by name only
 
 _lib = None
 
@@ -154,6 +160,10 @@ def load():
         lib.copra_b200_multi_set_warm_start.argtypes = [C.c_void_p, C.c_int]
         lib.copra_b200_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut)]
         lib.copra_b200_multi_lmpc_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut)]
+        lib.copra_b200_lmpc_vjp_costs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut),
+                                                  C.POINTER(VjpCostOut)]
+        lib.copra_b200_multi_lmpc_vjp_costs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
+                                                        C.POINTER(VjpCostOut)]
         lib.copra_b200_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_int, C.c_void_p, C.c_void_p]
         lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
@@ -319,9 +329,22 @@ def vjp_lengths(bp):
     return int(bp["nx"]), plen, clen
 
 
+def cost_shapes(bp):
+    """(rows, has_M, has_N) of every cost: the shapes of the w, M and N gradients lmpc_vjp returns"""
+    out = []
+    for c in bp["costs"]:
+        if c.get("per_step"):
+            rows = _rows_of(c["M"] if c.get("M") is not None else c["N"])
+        else:
+            rows = int(np.asarray(c["p"]).shape[-1])
+        out.append((rows, c["kind"] in ("trajectory", "target", "mixed"), c["kind"] in ("control", "mixed")))
+    return out
+
+
 def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
     """allocate the wanted gradients (numpy, or torch tensors on the device of the torch cotangents), describe them in a
-    VjpOut and run `call(dcontrol_ptr, dtrajectory_ptr, memory, out)`.  With torch tensors the engine runs on its own stream:
+    VjpOut (and, when w, M or N are wanted, a VjpCostOut) and run `call(dcontrol_ptr, dtrajectory_ptr, memory, out,
+    cost_out)`, cost_out None unless cost gradients are wanted.  With torch tensors the engine runs on its own stream:
     the cotangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the
     gradients (written, zero-initialised, by the engine itself) and the input copies are handed back."""
     nx, plen, clen = vjp_lengths(bp)
@@ -371,14 +394,32 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
         keep.append(ptrs)
         setattr(o, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
         res[key] = arrs
+    co = None
+    if any(k in want for k in VJP_COST_WANT):
+        # the engine writes M (rows x nx) and N (rows x nu) column-major: allocated as (batch, cols, rows)
+        nu = int(bp["nu"])
+        shapes = cost_shapes(bp)
+        raw = dict(w=[zeros(r) if "w" in want else None for r, _, _ in shapes],
+                   M=[zeros(nx * r).reshape(B, nx, r) if "M" in want and hm else None for r, hm, _ in shapes],
+                   N=[zeros(nu * r).reshape(B, nu, r) if "N" in want and hn else None for r, _, hn in shapes])
+        co = VjpCostOut()
+        for key, arrs in raw.items():
+            ptrs = (C.c_void_p * max(1, len(arrs)))(*[ptr(a) if a is not None else None for a in arrs])
+            keep.append(ptrs)
+            setattr(co, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
     dc, dt = inp(dcontrol), inp(dtrajectory)
     if dev is not None:
         torch.cuda.synchronize(dev)
     try:
-        call(dc, dt, mem, o)
+        call(dc, dt, mem, o, co)
     finally:
         if dev is not None and sync is not None:
             sync()
+    if co is not None:
+        res["w"] = raw["w"]
+        for key in ("M", "N"):
+            res[key] = [None if a is None else (a.transpose(1, 2).contiguous() if dev is not None
+                                                else np.ascontiguousarray(a.transpose(0, 2, 1))) for a in raw[key]]
     return res
 
 
@@ -660,13 +701,19 @@ class Engine:
         dtrajectory (batch, X) = dL/dtrajectory, numpy arrays or CUDA float64 tensors.  Returns dict(x0=(batch, nx),
         p=[per cost], f=[per row constraint, None for bounds], lower=/upper=[per bound constraint, None otherwise]), each
         gradient (batch, rows) or (batch, rows x steps) for a per-step entry, of the same kind as the cotangents; a gradient
-        not in `want` is None.  Instances whose status is not 0 get zeros."""
+        not in `want` is None.  Instances whose status is not 0 get zeros.
+        With "w", "M" or "N" in `want` (copra_b200_lmpc_vjp_costs, the same KKT solve) it also returns w=[(batch, rows)],
+        M=[(batch, rows, nx)] and N=[(batch, rows, nu)] per cost, None where a cost has no such matrix."""
         if self._last_bp is None:
             raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run / lmpc_retarget on this engine")
         bp = self._last_bp
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want,
-                         lambda dc, dt, mem, o: self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o))),
-                         sync=self.synchronize)
+
+        def call(dc, dt, mem, o, co):
+            if co is None:
+                self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o)))
+            else:
+                self._check(self.lib.copra_b200_lmpc_vjp_costs(self.h, dc, dt, mem, C.byref(o), C.byref(co)))
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want, call, sync=self.synchronize)
 
     def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
         """Jacobian-vector product of the last solve (copra_b200_lmpc_jvp) along k tangent directions: x0 (batch, k, nx) and
@@ -791,8 +838,13 @@ class MultiEngine:
             raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run on this engine")
         if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
             raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want,
-                         lambda dc, dt, mem, o: self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o))))
+
+        def call(dc, dt, mem, o, co):
+            if co is None:
+                self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o)))
+            else:
+                self._check(self.lib.copra_b200_multi_lmpc_vjp_costs(self.m, dc, dt, C.byref(o), C.byref(co)))
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want, call)
 
     def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
         """Engine.lmpc_jvp over the shards of the last run (numpy arrays holding the whole batch)"""

@@ -72,7 +72,7 @@ struct copra_b200_handle {
     bool gs_j_valid = false;   // the small solver's per-instance factors of the resident build are cached (re-solves load them)
     bool warm_start = false;   // copra_b200_set_warm_start: re-solves seed the active set of the previous solve
     bool warm_valid = false;   // `warm_iact` holds the active sets of the last solve of the resident build
-    bool solved = false;       // res_status / res_nact / res_iact hold the last solve of the resident build (lmpc_vjp)
+    bool solved = false;       // res_x / res_status / res_nact / res_iact hold the last solve of the resident build (lmpc_vjp)
     bool vjp_factor_valid = false; // vjp_Jt holds R^-1 of the resident build's Hessian(s) (builds the thin solver did not factor)
     // per-instance vector lengths of the resident build (doubles): every cost's p, every constraint's f / lower / upper;
     // the constraint and the side (0 f, 1 lower, 2 upper) of every family; the control-bound constraint (-1 = none)
@@ -963,6 +963,7 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
     if ((rc = ws(h, "res_iters", 2 * B, &iters))) return rc;
     if ((rc = ws(h, "res_nact", B, &nact))) return rc;
     if ((rc = ws(h, "res_iact", B * nv, &iact))) return rc;
+    double* ws_x = x;
     int *ws_status = status, *ws_nact = nact, *ws_iact = iact;
     if (devres) { // write straight into the caller's device buffers where given
         if (r->x) x = r->x;
@@ -996,7 +997,8 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
         if (rc) return rc;
     }
     if ((rc = record(h, 4))) return rc;
-    // the active sets of this solve stay in the workspace for copra_b200_lmpc_vjp
+    // the solution and the active sets of this solve stay in the workspace for copra_b200_lmpc_vjp
+    if (x != ws_x) CU(cudaMemcpyAsync(ws_x, x, B * nv * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
     if (status != ws_status) CU(cudaMemcpyAsync(ws_status, status, B * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
     if (nact != ws_nact) CU(cudaMemcpyAsync(ws_nact, nact, B * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
     if (iact != ws_iact) CU(cudaMemcpyAsync(ws_iact, iact, B * nv * sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
@@ -1126,12 +1128,16 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
     return 0;
 }
 
-// K8 for the last solve (copra_b200_lmpc_vjp): the outputs are zeroed first and k8_adjoint only writes the entries it owns.
-int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out)
+// K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs): the outputs are zeroed first and k8_adjoint only writes the
+// entries it owns; with `costs`, k8_cost_grad follows k8_adjoint on each chunk and writes the cost gradients.
+int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out,
+    const copra_b200_vjp_cost_out* costs)
 {
     const BuildParams& P = h->bp;
-    const size_t B = P.batch, nx = P.nx;
+    const size_t B = P.batch, nx = P.nx, nu = P.nu;
     int rc;
+    static const copra_b200_vjp_out none{};
+    if (!out) out = &none;
     // inputs
     const double *dc = dcontrol, *dt = dtraj;
     if (memory == COPRA_B200_HOST && (dcontrol || dtraj)) {
@@ -1162,6 +1168,17 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
         items.push_back({ out->lower ? out->lower[h->bound_cstr] : nullptr, &V.dlower, size_t(V.cblen) });
         items.push_back({ out->upper ? out->upper[h->bound_cstr] : nullptr, &V.dupper, size_t(V.cblen) });
     }
+    bool want_costs = false;
+    if (costs) {
+        for (int ci = 0; ci < P.ncost; ++ci) {
+            const size_t r = P.cost[ci].rows;
+            items.push_back({ costs->w ? costs->w[ci] : nullptr, &V.dw[ci], r });
+            items.push_back({ costs->M ? costs->M[ci] : nullptr, &V.dM[ci], r * nx });
+            items.push_back({ costs->N ? costs->N[ci] : nullptr, &V.dN[ci], r * nu });
+            want_costs |= (costs->w && costs->w[ci]) || (costs->M && costs->M[ci]) || (costs->N && costs->N[ci]);
+        }
+        if (want_costs && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
+    }
     size_t total = 0;
     for (auto& it : items) if (it.host) total += it.len * B;
     double* oblk = nullptr;
@@ -1176,7 +1193,12 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
     if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
     V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
     rc = sens_run(h, V, 1, [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
-        [&](int nb) { return k8_adjoint_launch(P, V, nb, h->stream); });
+        [&](int nb) {
+            const int n1 = k8_adjoint_launch(P, V, nb, h->stream);
+            if (n1 < 0 || !want_costs) return n1;
+            const int n2 = k8_cost_grad_launch(P, V, nb, h->stream);
+            return n2 < 0 ? n2 : n1 + n2;
+        });
     if (rc) return rc;
     if (memory == COPRA_B200_HOST) {
         Download D;
@@ -1274,6 +1296,13 @@ void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_
     nx = h->bp.nx;
     cost_len = h->cost_len;
     cstr_len = h->cstr_len;
+}
+
+void cb_cost_shapes(const copra_b200_handle* h, int& nu, std::vector<int>& rows)
+{
+    nu = h->bp.nu;
+    rows.clear();
+    for (int i = 0; i < h->bp.ncost; ++i) rows.push_back(h->bp.cost[i].rows);
 }
 
 // ===============================================================================================
@@ -1553,14 +1582,32 @@ int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, 
 int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
     const copra_b200_vjp_out* out)
 {
+    return copra_b200_lmpc_vjp_costs(h, dcontrol, dtrajectory, memory, out, nullptr);
+}
+
+int copra_b200_lmpc_vjp_costs(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs)
+{
     if (!h) return COPRA_B200_E_ARG;
-    if (!out) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (!out && !costs) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
     if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
     int rc = sens_check(h, "lmpc_vjp");
     if (rc) return rc;
+    if (costs) {
+        const BuildParams& P = h->bp;
+        for (int ci = 0; ci < P.ncost; ++ci) {
+            if (costs->M && costs->M[ci] && !P.cost[ci].hasM)
+                return fail(h, COPRA_B200_E_ARG, "lmpc_vjp_costs: cost %d has no M (a ControlCost)", ci);
+            if (costs->N && costs->N[ci] && !P.cost[ci].hasN)
+                return fail(h, COPRA_B200_E_ARG, "lmpc_vjp_costs: cost %d has no N (a TrajectoryCost or TargetCost)", ci);
+        }
+        if (k8_cost_grad_smem(P) > h->smem_optin)
+            return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp_costs: the horizon needs %zu bytes of shared memory per instance, "
+                "the device allows %zu", k8_cost_grad_smem(P), h->smem_optin);
+    }
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
-    return do_vjp(h, dcontrol, dtrajectory, memory, out);
+    return do_vjp(h, dcontrol, dtrajectory, memory, out, costs);
 }
 
 int copra_b200_lmpc_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int memory, double* dcontrol, double* dtrajectory)
@@ -1610,8 +1657,8 @@ int copra_b200_lmpc_results(copra_b200_handle* h, const double* x, double* contr
     const double* dx = x;
     double *dc = control, *dt = trajectory;
     if (memory == COPRA_B200_HOST) {
-        double* tmp = nullptr;
-        if ((rc = ws(h, "res_x", B * P.nvar, &tmp))) return rc;
+        double* tmp = nullptr; // not res_x: that holds the solution of the last solve, for copra_b200_lmpc_vjp_costs
+        if ((rc = ws(h, "results_x", B * P.nvar, &tmp))) return rc;
         CU(cudaMemcpyAsync(tmp, x, B * P.nvar * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         dx = tmp;
         if ((rc = ws(h, "res_control", B * P.nU, &dc))) return rc;

@@ -64,6 +64,8 @@ template <class F> int run_shards(copra_b200_multi* m, F body)
 
 // per-instance lengths of x0 and of every cost's p / constraint's vector of the resident build (capi.cu)
 void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_len, std::vector<int>& cstr_len);
+// nu and the rows of every cost of the resident build (capi.cu)
+void cb_cost_shapes(const copra_b200_handle* h, int& nu, std::vector<int>& rows);
 
 extern "C" {
 
@@ -196,8 +198,16 @@ int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem
 
 int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out* out)
 {
+    return copra_b200_multi_lmpc_vjp_costs(m, dcontrol, dtrajectory, out, nullptr);
+}
+
+int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs)
+{
     if (!m) return COPRA_B200_E_ARG;
-    if (!out) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (!out && !costs) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    static const copra_b200_vjp_out none{};
+    if (!out) out = &none;
     if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp needs a previous run");
     return run_shards(m, [&](int g) {
         copra_b200_sizes sz{};
@@ -221,8 +231,24 @@ int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const
         o.f = out->f ? f.data() : nullptr;
         o.lower = out->lower ? lower.data() : nullptr;
         o.upper = out->upper ? upper.data() : nullptr;
-        return copra_b200_lmpc_vjp(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr, dtrajectory ? dtrajectory + lo * sz.X : nullptr,
-            COPRA_B200_HOST, &o);
+        // the cost gradients likewise: rows, rows x nx and rows x nu per instance
+        int nu = 0;
+        std::vector<int> rows;
+        cb_cost_shapes(m->h[g], nu, rows);
+        std::vector<double*> cw(rows.size()), cM(rows.size()), cN(rows.size());
+        for (size_t i = 0; i < rows.size() && costs; ++i) {
+            cw[i] = (costs->w && costs->w[i]) ? costs->w[i] + lo * rows[i] : nullptr;
+            cM[i] = (costs->M && costs->M[i]) ? costs->M[i] + lo * rows[i] * nx : nullptr;
+            cN[i] = (costs->N && costs->N[i]) ? costs->N[i] + lo * rows[i] * nu : nullptr;
+        }
+        copra_b200_vjp_cost_out co{};
+        if (costs) {
+            co.w = costs->w ? cw.data() : nullptr;
+            co.M = costs->M ? cM.data() : nullptr;
+            co.N = costs->N ? cN.data() : nullptr;
+        }
+        return copra_b200_lmpc_vjp_costs(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
+            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &o, costs ? &co : nullptr);
     });
 }
 

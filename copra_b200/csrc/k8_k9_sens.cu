@@ -19,7 +19,11 @@
 //   k8_adjoint  the transpose of the vector part of K2 / K4 (what a retarget re-runs):
 //               dx0 = sum_costs E c^ - Yeq' b^eq - Yin' b^in + Phi' dtraj,  dp_i = -W T_i c^,
 //               df / dlower / dupper: b^, lb^, ub^ scattered through the index maps of dev_precompute / dev_finalize
-//   k9_output   the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
+//   k8_cost_grad the cost weights and matrices, which enter the objective only: dL/dtheta = c^' (dQ/dtheta U + dc/dtheta).
+//               With x^ = Psi c^, the solution's states x_i and controls u_i, e_i = M x_i + N u_i - p_i and
+//               t_i = T_i c^ = M x^_i + N c^_i:  dw_l = sum_i t_il e_il,  dM = sum_i W (e_i x^_i' + t_i x_i'),
+//               dN = sum_i W (e_i c^_i' + t_i u_i')
+//   k9_output  the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
 // Every sum runs in a fixed order.  Instances whose status is not 0 get zeros; a Hessian or Gram factorisation that failed
 // gives NaN instead of silently wrong results.
 #include "common.cuh"
@@ -385,6 +389,106 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
     }
 }
 
+// dw, dM and dN of every requested cost (see the file comment), one CTA per instance of the chunk.  Shared memory: c^ and U
+// (n each), x^ = Psi c^ and xd = Phi x0 + Psi U (X each; x_i = xd_i + xi_i), then e and t of one cost (rows x steps each).
+// e_i = res_i + M xd_i + N u_i with the resident res_i = M xi_i - p_i.  Every sum runs in a fixed order; an instance whose
+// status is not 0 keeps the zeros its outputs were initialised to, a failed factorisation reaches the outputs as NaN through v.
+__global__ void __launch_bounds__(kSensThreads) k8_cost_grad_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ VjpParams V)
+{
+    extern __shared__ double sens_sm[];
+    const int lb = blockIdx.x, b = V.b0 + lb;
+    if (V.status[b] != 0) return;
+    const int n = V.n, nx = P.nx, nu = P.nu, N = P.N, X = P.X, NX = N * nx;
+    const int tid = threadIdx.x, T = blockDim.x;
+    double* ch = sens_sm;  // n  c^ = -v
+    double* u = ch + n;    // n  U
+    double* xh = u + n;    // X  Psi c^
+    double* xd = xh + X;   // X  Phi x0 + Psi U
+    double* et = xd + X;   // 2 x rows x steps: e, then t, of one cost
+    for (int t = tid; t < n; t += T) {
+        ch[t] = -V.V[(long long)lb * V.lds + t];
+        u[t] = V.U[(long long)b * n + t];
+    }
+    __syncthreads();
+    const double* Phi = P.Phi + (long long)b * X * nx;
+    const double* Gs = P.Gs + (long long)b * NX * nu;
+    const double* xi = P.xi + (long long)b * X;
+    const double* x0 = P.x0.at(b);
+    for (int row = tid; row < X; row += T) {
+        const int i = row / nx, r = row % nx;
+        double sh = 0.0, su = 0.0;
+        int go = (i - 1) * nx + r; // G_{i-1-j}[r, :]
+        for (int j = 0; j < i; ++j, go -= nx)
+            for (int cc = 0; cc < nu; ++cc) {
+                const double g = Gs[go + (long long)cc * NX];
+                sh += g * ch[j * nu + cc];
+                su += g * u[j * nu + cc];
+            }
+        double s0 = 0.0;
+        for (int a = 0; a < nx; ++a) s0 += Phi[row + (long long)a * X] * x0[a];
+        xh[row] = sh;
+        xd[row] = s0 + su;
+    }
+    for (int ci = 0; ci < P.ncost; ++ci) {
+        double *ow = V.dw[ci], *oM = V.dM[ci], *oN = V.dN[ci];
+        if (!ow && !oM && !oN) continue;
+        const CostFam& F = P.cost[ci];
+        const int r = F.rows, ns = F.i1 - F.i0, len = r * ns;
+        const double* M = F.hasM ? F.M.at(b) : nullptr; // r x nx
+        const double* Nm = F.hasN ? F.N.at(b) : nullptr; // r x nu
+        const double* w = F.w.at(b);
+        const double* res = F.res + (long long)b * F.sres;
+        __syncthreads(); // xh / xd complete; the previous cost's e / t are no longer read
+        for (int t = tid; t < len; t += T) {
+            const int l = t % r, i = F.i0 + t / r;
+            double e = res[t], tt = 0.0;
+            if (M)
+                for (int a = 0; a < nx; ++a) {
+                    const double m = M[l + r * a];
+                    e += m * xd[i * nx + a];
+                    tt += m * xh[i * nx + a];
+                }
+            if (Nm && i < N)
+                for (int bb = 0; bb < nu; ++bb) {
+                    const double m = Nm[l + r * bb];
+                    e += m * u[i * nu + bb];
+                    tt += m * ch[i * nu + bb];
+                }
+            et[t] = e;
+            et[len + t] = tt;
+        }
+        __syncthreads();
+        const double* e = et;
+        const double* tv = et + len;
+        if (ow)
+            for (int l = tid; l < r; l += T) {
+                double acc = 0.0;
+                for (int s = 0; s < ns; ++s) acc += tv[s * r + l] * e[s * r + l];
+                ow[(long long)b * r + l] = acc;
+            }
+        if (oM)
+            for (int q = tid; q < r * nx; q += T) {
+                const int l = q % r, a = q / r;
+                double acc = 0.0;
+                for (int s = 0; s < ns; ++s) {
+                    const int k = (F.i0 + s) * nx + a;
+                    acc += e[s * r + l] * xh[k] + tv[s * r + l] * (xd[k] + xi[k]);
+                }
+                oM[(long long)b * r * nx + q] = w[l] * acc;
+            }
+        if (oN)
+            for (int q = tid; q < r * nu; q += T) {
+                const int l = q % r, bb = q / r;
+                double acc = 0.0;
+                for (int s = 0; s < ns && F.i0 + s < N; ++s) {
+                    const int k = (F.i0 + s) * nu + bb;
+                    acc += e[s * r + l] * ch[k] + tv[s * r + l] * u[k];
+                }
+                oN[(long long)b * r * nu + q] = w[l] * acc;
+            }
+    }
+}
+
 // dcontrol = the first ru rows of Udot; dtraj = the first rx rows of Phi x0dot + Psi Udot, Psi applied as the block-Toeplitz
 // product over the compact Gs (K7 without xi).  Zeros for an instance whose status is not 0.
 __global__ void __launch_bounds__(kSensThreads) k9_output_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ JvpParams J)
@@ -468,6 +572,22 @@ int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStre
     cudaError_t e = cudaFuncSetAttribute(k8_adjoint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return -int(e);
     k8_adjoint_kernel<<<nb, kSensThreads, smem, st>>>(P, V);
+    return launched(cudaGetLastError());
+}
+
+size_t k8_cost_grad_smem(const BuildParams& P)
+{
+    int et = 1;
+    for (int ci = 0; ci < P.ncost; ++ci) et = std::max(et, 2 * P.cost[ci].rows * (P.cost[ci].i1 - P.cost[ci].i0));
+    return sizeof(double) * (2 * size_t(P.nvar) + 2 * size_t(P.X) + size_t(et));
+}
+
+int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st)
+{
+    const size_t smem = k8_cost_grad_smem(P);
+    cudaError_t e = cudaFuncSetAttribute(k8_cost_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return -int(e);
+    k8_cost_grad_kernel<<<nb, kSensThreads, smem, st>>>(P, V);
     return launched(cudaGetLastError());
 }
 

@@ -92,7 +92,8 @@ struct SensChunk {
 int sens_gram_launch(const SensChunk& S, int nb, cudaStream_t st);
 int sens_solve_launch(const SensChunk& S, int nb, cudaStream_t st);
 
-// K8: the vector-Jacobian product (k = 1); sens_solve leaves the multipliers mu of the active rows (iact order) in rhs
+// K8: the vector-Jacobian product (k = 1); sens_solve leaves the multipliers mu of the active rows (iact order) in rhs.
+// k8_cost_grad adds the gradients with respect to each cost's w, M and N from the same v.
 struct VjpParams : SensChunk {
     const double* dcontrol;          // dL/dU (nU per instance, sdc apart), may be null
     long long sdc;
@@ -104,9 +105,17 @@ struct VjpParams : SensChunk {
     double* df[kMaxFam];
     double* dlower;                  // control bound
     double* dupper;
+    // cost gradients (k8_cost_grad; whole batch, zeroed by the caller; null = not wanted)
+    const double* U;                 // the solution being differentiated, n per instance
+    double* dw[kMaxCost];            // rows per instance
+    double* dM[kMaxCost];            // rows x nx per instance, column-major
+    double* dN[kMaxCost];            // rows x nu per instance, column-major
 };
 int k8_gather_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
+// shared memory of k8_cost_grad for the resident build (the caller checks it against the device's opt-in limit)
+size_t k8_cost_grad_smem(const BuildParams& P);
+int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
 // K9: Jacobian-vector products along k tangent directions, or the feedback gain
 struct JvpParams : SensChunk {

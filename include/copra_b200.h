@@ -258,6 +258,24 @@ typedef struct {
  * warm-start seed untouched. */
 int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
     const copra_b200_vjp_out* out);
+/* The same vector-Jacobian product, and with it the gradients with respect to every cost's weights and matrices: one adjoint
+ * KKT solve serves both (with costs = NULL this is copra_b200_lmpc_vjp).  These inputs enter the objective only, so on the
+ * final active set  dL/dtheta = c^' (dQ/dtheta U + dc/dtheta)  with c^ = dL/dc; per cost, with the solution's states x_i and
+ * controls u_i, e_i = M x_i + N u_i - p_i, x^ = Psi c^ and t_i = M x^_i + N c^_i over the steps i the cost covers:
+ *   dL/dw_l = sum_i (t_i)_l (e_i)_l,  dL/dM = sum_i W (e_i x^_i' + t_i x_i'),  dL/dN = sum_i W (e_i c^_i' + t_i u_i').
+ * Gradients are per instance even for inputs given with stride 0.  NULL pointers (the arrays themselves or their entries)
+ * mark gradients that are not wanted; `out` may be NULL when only cost gradients are wanted.  With DEVICE inputs, the x0,
+ * M, N and w arrays the resident build (or its last retarget / resolve) was given are read again: they must still hold
+ * those values.  Preconditions and error codes are those of copra_b200_lmpc_vjp, plus E_ARG for an M entry of a cost
+ * without M (CONTROL) or an N entry of a cost without N (TRAJECTORY, TARGET), and E_UNSUPPORTED for a horizon whose
+ * 2 nU + 2 X + 2 rows x steps doubles exceed the device's shared memory per block. */
+typedef struct {
+    double* const* w;   /* [ncost]: rows per instance */
+    double* const* M;   /* [ncost]: rows x nx per instance, column-major; must be NULL for a cost without M */
+    double* const* N;   /* [ncost]: rows x nu per instance, column-major; must be NULL for a cost without N */
+} copra_b200_vjp_cost_out;
+int copra_b200_lmpc_vjp_costs(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out /* may be NULL */, const copra_b200_vjp_cost_out* costs);
 /* Forward-mode sensitivities of the last solve: the Jacobian-vector product of (control, trajectory) along `ndir` tangent
  * directions of x0 and every cost's p and every constraint's f / lower / upper (one forward KKT solve per instance with
  * ndir right-hand sides, K9; exact on the final active set, as the VJP).  Each tangent holds, per instance, ndir
@@ -329,6 +347,9 @@ int copra_b200_multi_lmpc_resolve(copra_b200_multi* m, copra_b200_array x0, cons
 int copra_b200_multi_lmpc_retarget(copra_b200_multi* m, const copra_b200_problem* p, const copra_b200_results* r);
 /* copra_b200_lmpc_vjp on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out* out);
+/* copra_b200_lmpc_vjp_costs on every shard of the last run; HOST arrays holding the whole batch */
+int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs);
 /* copra_b200_lmpc_jvp / copra_b200_lmpc_feedback_gain on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory);
 int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx);
