@@ -8,7 +8,7 @@ OBJS := $(CSRC)/k6_solver.o $(CSRC)/k6_thin.o $(CSRC)/k6_thin_f0.o $(CSRC)/k6_th
 LIB := copra_b200/lib/libcopra_b200.so
 HDRS := $(wildcard $(CSRC)/*.cuh) $(wildcard $(CSRC)/*.h) include/copra_b200.h
 
-all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp tests/cpp/test_jvp tests/cpp/test_vjp_costs
+all: $(LIB) oracle tests/cpp/test_facade tests/cpp/test_per_step tests/cpp/test_vjp tests/cpp/test_jvp tests/cpp/test_vjp_costs tests/cpp/test_vjp_model
 
 $(CSRC)/%.o: $(CSRC)/%.cu $(HDRS)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $@.ptxas.log || (cat $@.ptxas.log; false)
@@ -55,3 +55,9 @@ tests/cpp/test_vjp_costs: tests/cpp/test_vjp_costs.cpp $(wildcard include/copra/
 	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_vjp_costs.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
 
 vjp-costs-test: tests/cpp/test_vjp_costs
+
+# BatchedLMPC::vjp with the model gradients against central differences of copra::LMPC, and its errors (GPU)
+tests/cpp/test_vjp_model: tests/cpp/test_vjp_model.cpp $(wildcard include/copra/*) include/copra_b200.h $(LIB)
+	g++ -std=c++14 -O1 -Wall -Wextra -pthread -Iinclude -o $@ tests/cpp/test_vjp_model.cpp -Lcopra_b200/lib -lcopra_b200 -Wl,-rpath,'$$ORIGIN/../../copra_b200/lib'
+
+vjp-model-test: tests/cpp/test_vjp_model

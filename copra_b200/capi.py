@@ -69,6 +69,11 @@ class VjpCostOut(C.Structure):
     _fields_ = [("w", C.POINTER(C.c_void_p)), ("M", C.POINTER(C.c_void_p)), ("N", C.POINTER(C.c_void_p))]
 
 
+class VjpModelOut(C.Structure):
+    _fields_ = [("A", C.c_void_p), ("B", C.c_void_p), ("d", C.c_void_p), ("E", C.POINTER(C.c_void_p)),
+                ("G", C.POINTER(C.c_void_p))]
+
+
 class JvpIn(C.Structure):
     _fields_ = [("ndir", C.c_int), ("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
@@ -91,9 +96,10 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget", "copra_b200_lmpc_vjp",
            "copra_b200_multi_lmpc_vjp", "copra_b200_lmpc_jvp", "copra_b200_lmpc_feedback_gain",
            "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain", "copra_b200_lmpc_vjp_costs",
-           "copra_b200_multi_lmpc_vjp_costs"]
+           "copra_b200_multi_lmpc_vjp_costs", "copra_b200_lmpc_vjp_model", "copra_b200_multi_lmpc_vjp_model"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
 VJP_COST_WANT = ("w", "M", "N")  # gradients with respect to the cost weights and matrices: requested by name only
+VJP_MODEL_WANT = ("A", "B", "d", "E", "G")  # ... and to the dynamics and the row constraints' matrices: by name only
 
 _lib = None
 
@@ -164,6 +170,10 @@ def load():
                                                   C.POINTER(VjpCostOut)]
         lib.copra_b200_multi_lmpc_vjp_costs.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
                                                         C.POINTER(VjpCostOut)]
+        lib.copra_b200_lmpc_vjp_model.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut),
+                                                  C.POINTER(VjpCostOut), C.POINTER(VjpModelOut)]
+        lib.copra_b200_multi_lmpc_vjp_model.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
+                                                        C.POINTER(VjpCostOut), C.POINTER(VjpModelOut)]
         lib.copra_b200_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_int, C.c_void_p, C.c_void_p]
         lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
@@ -341,10 +351,21 @@ def cost_shapes(bp):
     return out
 
 
+def cstr_shapes(bp):
+    """(rows, has_E, has_G) of every constraint: the shapes of the E and G gradients lmpc_vjp returns (0 rows for a bound)"""
+    out = []
+    for c in bp["constraints"]:
+        has_e, has_g = c["kind"] in ("trajectory", "mixed"), c["kind"] in ("control", "mixed")
+        rows = _rows_of(c["E"] if has_e else c["G"]) if has_e or has_g else 0
+        out.append((rows, has_e, has_g))
+    return out
+
+
 def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
     """allocate the wanted gradients (numpy, or torch tensors on the device of the torch cotangents), describe them in a
-    VjpOut (and, when w, M or N are wanted, a VjpCostOut) and run `call(dcontrol_ptr, dtrajectory_ptr, memory, out,
-    cost_out)`, cost_out None unless cost gradients are wanted.  With torch tensors the engine runs on its own stream:
+    VjpOut (and, when w, M or N are wanted, a VjpCostOut; when A, B, d, E or G are, a VjpModelOut) and run
+    `call(dcontrol_ptr, dtrajectory_ptr, memory, out, cost_out, model_out)`, cost_out / model_out None unless such gradients
+    are wanted.  With torch tensors the engine runs on its own stream:
     the cotangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the
     gradients (written, zero-initialised, by the engine itself) and the input copies are handed back."""
     nx, plen, clen = vjp_lengths(bp)
@@ -407,11 +428,28 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
             ptrs = (C.c_void_p * max(1, len(arrs)))(*[ptr(a) if a is not None else None for a in arrs])
             keep.append(ptrs)
             setattr(co, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
+    mo = None
+    if any(k in want for k in VJP_MODEL_WANT):
+        # column-major matrices again: A as (batch, nx, nx) transposed, B (batch, nu, nx), E (batch, nx, rows), G (batch, nu, rows)
+        nu = int(bp["nu"])
+        shapes = cstr_shapes(bp)
+        mraw = dict(A=zeros(nx * nx).reshape(B, nx, nx) if "A" in want else None,
+                    B=zeros(nx * nu).reshape(B, nu, nx) if "B" in want else None,
+                    d=zeros(nx) if "d" in want else None,
+                    E=[zeros(nx * r).reshape(B, nx, r) if "E" in want and he else None for r, he, _ in shapes],
+                    G=[zeros(nu * r).reshape(B, nu, r) if "G" in want and hg else None for r, _, hg in shapes])
+        mo = VjpModelOut()
+        for key in ("A", "B", "d"):
+            setattr(mo, key, ptr(mraw[key]) if mraw[key] is not None else None)
+        for key in ("E", "G"):
+            ptrs = (C.c_void_p * max(1, len(mraw[key])))(*[ptr(a) if a is not None else None for a in mraw[key]])
+            keep.append(ptrs)
+            setattr(mo, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
     dc, dt = inp(dcontrol), inp(dtrajectory)
     if dev is not None:
         torch.cuda.synchronize(dev)
     try:
-        call(dc, dt, mem, o, co)
+        call(dc, dt, mem, o, co, mo)
     finally:
         if dev is not None and sync is not None:
             sync()
@@ -420,6 +458,14 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
         for key in ("M", "N"):
             res[key] = [None if a is None else (a.transpose(1, 2).contiguous() if dev is not None
                                                 else np.ascontiguousarray(a.transpose(0, 2, 1))) for a in raw[key]]
+
+    def logical(a):  # (batch, cols, rows) column-major -> (batch, rows, cols)
+        if a is None:
+            return None
+        return a.transpose(1, 2).contiguous() if dev is not None else np.ascontiguousarray(a.transpose(0, 2, 1))
+    if mo is not None:
+        res["A"], res["B"], res["d"] = logical(mraw["A"]), logical(mraw["B"]), mraw["d"]
+        res["E"], res["G"] = [logical(a) for a in mraw["E"]], [logical(a) for a in mraw["G"]]
     return res
 
 
@@ -703,13 +749,20 @@ class Engine:
         gradient (batch, rows) or (batch, rows x steps) for a per-step entry, of the same kind as the cotangents; a gradient
         not in `want` is None.  Instances whose status is not 0 get zeros.
         With "w", "M" or "N" in `want` (copra_b200_lmpc_vjp_costs, the same KKT solve) it also returns w=[(batch, rows)],
-        M=[(batch, rows, nx)] and N=[(batch, rows, nu)] per cost, None where a cost has no such matrix."""
+        M=[(batch, rows, nx)] and N=[(batch, rows, nu)] per cost, None where a cost has no such matrix.
+        With "A", "B", "d", "E" or "G" in `want` (copra_b200_lmpc_vjp_model, the same KKT solve with the forward solve as a
+        second right-hand side) it also returns A=(batch, nx, nx), B=(batch, nx, nu), d=(batch, nx), and E=[(batch, rows, nx)]
+        and G=[(batch, rows, nu)] per constraint, None where a constraint has no such matrix (a trajectory bound's selector
+        has no gradient)."""
         if self._last_bp is None:
             raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run / lmpc_retarget on this engine")
         bp = self._last_bp
 
-        def call(dc, dt, mem, o, co):
-            if co is None:
+        def call(dc, dt, mem, o, co, mo):
+            if mo is not None:
+                self._check(self.lib.copra_b200_lmpc_vjp_model(self.h, dc, dt, mem, C.byref(o), co and C.byref(co),
+                                                               C.byref(mo)))
+            elif co is None:
                 self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o)))
             else:
                 self._check(self.lib.copra_b200_lmpc_vjp_costs(self.h, dc, dt, mem, C.byref(o), C.byref(co)))
@@ -839,8 +892,11 @@ class MultiEngine:
         if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
             raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
 
-        def call(dc, dt, mem, o, co):
-            if co is None:
+        def call(dc, dt, mem, o, co, mo):
+            if mo is not None:
+                self._check(self.lib.copra_b200_multi_lmpc_vjp_model(self.m, dc, dt, C.byref(o), co and C.byref(co),
+                                                                     C.byref(mo)))
+            elif co is None:
                 self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o)))
             else:
                 self._check(self.lib.copra_b200_multi_lmpc_vjp_costs(self.m, dc, dt, C.byref(o), C.byref(co)))

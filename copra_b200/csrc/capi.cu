@@ -1128,10 +1128,12 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
     return 0;
 }
 
-// K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs): the outputs are zeroed first and k8_adjoint only writes the
-// entries it owns; with `costs`, k8_cost_grad follows k8_adjoint on each chunk and writes the cost gradients.
+// K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs, _vjp_model): the outputs are zeroed first and k8_adjoint only
+// writes the entries it owns; with `costs`, k8_cost_grad follows k8_adjoint on each chunk and writes the cost gradients;
+// with `model`, the KKT solve takes the forward solve as a second right-hand side (its multipliers) and k8_model_grad
+// follows them and writes the model gradients.
 int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out,
-    const copra_b200_vjp_cost_out* costs)
+    const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model)
 {
     const BuildParams& P = h->bp;
     const size_t B = P.batch, nx = P.nx, nu = P.nu;
@@ -1177,8 +1179,25 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
             items.push_back({ costs->N ? costs->N[ci] : nullptr, &V.dN[ci], r * nu });
             want_costs |= (costs->w && costs->w[ci]) || (costs->M && costs->M[ci]) || (costs->N && costs->N[ci]);
         }
-        if (want_costs && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
     }
+    bool want_model = false;
+    if (model) {
+        items.push_back({ model->A, &V.dA, nx * nx });
+        items.push_back({ model->B, &V.dB, nx * nu });
+        items.push_back({ model->d, &V.dd, nx });
+        want_model = model->A || model->B || model->d;
+        for (int fi = 0; fi < P.nfam; ++fi) {
+            if (h->fam_which[fi] != 0) continue; // a trajectory bound's E is the engine's selector
+            const int c = h->fam_cstr[fi];
+            const size_t r = P.fam[fi].rows;
+            double* E = model->E ? model->E[c] : nullptr;
+            double* G = model->G ? model->G[c] : nullptr;
+            items.push_back({ E, &V.dE[fi], r * nx });
+            items.push_back({ G, &V.dG[fi], r * nu });
+            want_model |= E || G;
+        }
+    }
+    if ((want_costs || want_model) && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
     size_t total = 0;
     for (auto& it : items) if (it.host) total += it.len * B;
     double* oblk = nullptr;
@@ -1192,12 +1211,21 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
     }
     if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
     V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
-    rc = sens_run(h, V, 1, [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
+    rc = sens_run(h, V, want_model ? 2 : 1, [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
         [&](int nb) {
-            const int n1 = k8_adjoint_launch(P, V, nb, h->stream);
-            if (n1 < 0 || !want_costs) return n1;
-            const int n2 = k8_cost_grad_launch(P, V, nb, h->stream);
-            return n2 < 0 ? n2 : n1 + n2;
+            int n = k8_adjoint_launch(P, V, nb, h->stream);
+            if (n < 0) return n;
+            if (want_costs) {
+                const int n2 = k8_cost_grad_launch(P, V, nb, h->stream);
+                if (n2 < 0) return n2;
+                n += n2;
+            }
+            if (want_model) {
+                const int n3 = k8_model_grad_launch(P, V, nb, h->stream);
+                if (n3 < 0) return n3;
+                n += n3;
+            }
+            return n;
         });
     if (rc) return rc;
     if (memory == COPRA_B200_HOST) {
@@ -1303,6 +1331,13 @@ void cb_cost_shapes(const copra_b200_handle* h, int& nu, std::vector<int>& rows)
     nu = h->bp.nu;
     rows.clear();
     for (int i = 0; i < h->bp.ncost; ++i) rows.push_back(h->bp.cost[i].rows);
+}
+
+void cb_cstr_rows(const copra_b200_handle* h, std::vector<int>& rows)
+{
+    rows.assign(h->cstr_len.size(), 0);
+    for (int fi = 0; fi < h->bp.nfam; ++fi)
+        if (h->fam_which[fi] == 0) rows[h->fam_cstr[fi]] = h->bp.fam[fi].rows;
 }
 
 // ===============================================================================================
@@ -1588,8 +1623,14 @@ int copra_b200_lmpc_vjp(copra_b200_handle* h, const double* dcontrol, const doub
 int copra_b200_lmpc_vjp_costs(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
     const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs)
 {
+    return copra_b200_lmpc_vjp_model(h, dcontrol, dtrajectory, memory, out, costs, nullptr);
+}
+
+int copra_b200_lmpc_vjp_model(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model)
+{
     if (!h) return COPRA_B200_E_ARG;
-    if (!out && !costs) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (!out && !costs && !model) return fail(h, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
     if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
     int rc = sens_check(h, "lmpc_vjp");
     if (rc) return rc;
@@ -1605,9 +1646,28 @@ int copra_b200_lmpc_vjp_costs(copra_b200_handle* h, const double* dcontrol, cons
             return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp_costs: the horizon needs %zu bytes of shared memory per instance, "
                 "the device allows %zu", k8_cost_grad_smem(P), h->smem_optin);
     }
+    if (model) {
+        const BuildParams& P = h->bp;
+        const int ncstr = int(h->cstr_len.size());
+        std::vector<int> hasE(ncstr, 0), hasG(ncstr, 0);
+        for (int fi = 0; fi < P.nfam; ++fi)
+            if (h->fam_which[fi] == 0) {
+                hasE[h->fam_cstr[fi]] = P.fam[fi].hasE;
+                hasG[h->fam_cstr[fi]] = P.fam[fi].hasG;
+            }
+        for (int c = 0; c < ncstr; ++c) {
+            if (model->E && model->E[c] && !hasE[c])
+                return fail(h, COPRA_B200_E_ARG, "lmpc_vjp_model: constraint %d has no E (a ControlConstraint or a bound)", c);
+            if (model->G && model->G[c] && !hasG[c])
+                return fail(h, COPRA_B200_E_ARG, "lmpc_vjp_model: constraint %d has no G (a TrajectoryConstraint or a bound)", c);
+        }
+        if (k8_model_grad_smem(P) > h->smem_optin)
+            return fail(h, COPRA_B200_E_UNSUPPORTED, "lmpc_vjp_model: the horizon needs %zu bytes of shared memory per instance, "
+                "the device allows %zu", k8_model_grad_smem(P), h->smem_optin);
+    }
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
-    return do_vjp(h, dcontrol, dtrajectory, memory, out, costs);
+    return do_vjp(h, dcontrol, dtrajectory, memory, out, costs, model);
 }
 
 int copra_b200_lmpc_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int memory, double* dcontrol, double* dtrajectory)

@@ -66,6 +66,8 @@ template <class F> int run_shards(copra_b200_multi* m, F body)
 void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_len, std::vector<int>& cstr_len);
 // nu and the rows of every cost of the resident build (capi.cu)
 void cb_cost_shapes(const copra_b200_handle* h, int& nu, std::vector<int>& rows);
+// the rows of every row constraint's E / G of the resident build, 0 for a bound (capi.cu)
+void cb_cstr_rows(const copra_b200_handle* h, std::vector<int>& rows);
 
 extern "C" {
 
@@ -204,8 +206,14 @@ int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const
 int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
     const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs)
 {
+    return copra_b200_multi_lmpc_vjp_model(m, dcontrol, dtrajectory, out, costs, nullptr);
+}
+
+int copra_b200_multi_lmpc_vjp_model(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model)
+{
     if (!m) return COPRA_B200_E_ARG;
-    if (!out && !costs) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
+    if (!out && !costs && !model) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
     static const copra_b200_vjp_out none{};
     if (!out) out = &none;
     if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp needs a previous run");
@@ -247,8 +255,24 @@ int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol,
             co.M = costs->M ? cM.data() : nullptr;
             co.N = costs->N ? cN.data() : nullptr;
         }
-        return copra_b200_lmpc_vjp_costs(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
-            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &o, costs ? &co : nullptr);
+        // and the model gradients: nx x nx, nx x nu, nx, and rows x nx / rows x nu per row constraint
+        std::vector<int> crows;
+        cb_cstr_rows(m->h[g], crows);
+        std::vector<double*> mE(crows.size()), mG(crows.size());
+        for (size_t i = 0; i < crows.size() && model; ++i) {
+            mE[i] = (model->E && model->E[i]) ? model->E[i] + lo * crows[i] * nx : nullptr;
+            mG[i] = (model->G && model->G[i]) ? model->G[i] + lo * crows[i] * nu : nullptr;
+        }
+        copra_b200_vjp_model_out mo{};
+        if (model) {
+            mo.A = model->A ? model->A + lo * nx * nx : nullptr;
+            mo.B = model->B ? model->B + lo * nx * nu : nullptr;
+            mo.d = model->d ? model->d + lo * nx : nullptr;
+            mo.E = model->E ? mE.data() : nullptr;
+            mo.G = model->G ? mG.data() : nullptr;
+        }
+        return copra_b200_lmpc_vjp_model(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
+            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &o, costs ? &co : nullptr, model ? &mo : nullptr);
     });
 }
 

@@ -23,6 +23,14 @@
 //               With x^ = Psi c^, the solution's states x_i and controls u_i, e_i = M x_i + N u_i - p_i and
 //               t_i = T_i c^ = M x^_i + N c^_i:  dw_l = sum_i t_il e_il,  dM = sum_i W (e_i x^_i' + t_i x_i'),
 //               dN = sum_i W (e_i c^_i' + t_i u_i')
+//   k8_model_grad the dynamics A, B, d and the row constraints' E, G.  These also move the active rows, so the forward
+//               multipliers lambda enter: the VJP then runs with k = 2, the second right-hand side being the forward solve
+//               (-c in the slab, beta of the active rows in rhs), which leaves lambda in rhs column 1.  With gx_i = dtraj_i +
+//               sum_costs M'W t_i - sum_rows mu_j E_l', gh_i = sum_costs M'W e_i + sum_rows lambda_j E_l' (rows j at step i,
+//               line l), rho_N = gx_N, rho_i = gx_i + A' rho_{i+1} and rho^ the same from gh:
+//               dA = sum_{i<N} rho_{i+1} x_i' + rho^_{i+1} x^_i',  dB = sum_{i<N} rho_{i+1} u_i' + rho^_{i+1} c^_i',
+//               dd = sum_{i<N} rho_{i+1},  dE_l = sum_i lambda_(i,l) x^_i' - mu_(i,l) x_i',  dG_l = sum_i lambda_(i,l) c^_i' -
+//               mu_(i,l) u_i'  (rho_0 is dx0)
 //   k9_output  the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
 // Every sum runs in a fixed order.  Instances whose status is not 0 get zeros; a Hessian or Gram factorisation that failed
 // gives NaN instead of silently wrong results.
@@ -99,8 +107,24 @@ __global__ void __launch_bounds__(kSensThreads) k8_gather_kernel(const __grid_co
     const int n = V.n, nu = P.nu, N = P.N, nx = P.nx, nm = V.nm;
     const long long NX = (long long)N * nx;
     double* slab = sens_gather(P, V, lb, b);
-    for (int i = threadIdx.x; i < nm; i += blockDim.x) V.rhs[(long long)lb * nm + i] = 0.0; // a cotangent has bdot_act = 0
+    // a cotangent has bdot_act = 0; the forward solve's right-hand side (k = 2) is beta of the active rows, in their natural
+    // orientation: beq | bineq | ub | lb in the solver's index space
+    const int na = sens_nact(V, b), mg = P.meq + P.mineq;
+    const int* iact = V.iact + (long long)b * n;
+    for (int t = threadIdx.x; t < nm * V.k; t += blockDim.x) {
+        const int a = t % nm;
+        double v = 0.0;
+        if (t >= nm && a < na) {
+            const int idx = iact[a] - 1;
+            v = idx < P.meq ? P.beq[(long long)b * P.meq + idx]
+              : idx < mg ? P.bineq[(long long)b * P.mineq + idx - P.meq]
+              : idx < mg + n ? P.ub[(long long)b * P.nvar + idx - mg] : P.lb[(long long)b * P.nvar + idx - mg - n];
+        }
+        V.rhs[(long long)lb * nm * V.k + t] = v;
+    }
     if (V.status[b] != 0) return;
+    if (V.k == 2)
+        for (int col = threadIdx.x; col < n; col += blockDim.x) slab[col + (long long)(nm + 1) * V.lds] = -P.c[(long long)b * P.nvar + col];
     // gbar = dcontrol + Psi' dtraj, Psi' applied as the transposed block-Toeplitz product over the compact Gs
     const double* Gs = P.Gs + (long long)b * NX * nu;
     for (int col = threadIdx.x; col < n; col += blockDim.x) {
@@ -206,8 +230,9 @@ __global__ void sens_gram_kernel(const __grid_constant__ SensChunk S)
     }
 }
 
-// M = J_G J_G' rhs (J_G = R_G^-1) and W = T - Y1 M for every right-hand side, TILE per pass: 1 when k = 1, so a single
-// right-hand side does not pay for kDirTile predicated lanes, else kDirTile.  A Gram matrix that is not positive definite
+// M = J_G J_G' rhs (J_G = R_G^-1) and W = T - Y1 M for every right-hand side, TILE per pass: k when k <= 2, so one or two
+// right-hand sides do not pay for kDirTile predicated lanes, else kDirTile.  Each column's arithmetic is the same for every
+// TILE.  With TILE <= 2 (the VJP) M goes back to rhs.  A Gram matrix that is not positive definite
 // (linearly dependent active rows) or a Hessian factor that failed gives NaN rather than silently wrong results.
 template <int TILE> __global__ void __launch_bounds__(kSensThreads) sens_solve_kernel(const __grid_constant__ SensChunk S)
 {
@@ -259,7 +284,9 @@ template <int TILE> __global__ void __launch_bounds__(kSensThreads) sens_solve_k
                     if (dd < kt) {
                         const double m = (ok && qok) ? acc[dd] : CUDART_NAN;
                         rm[i + dd * nm] = m;
-                        if (TILE == 1) rhs[i] = m; // the VJP's multipliers, for k8_adjoint
+                        // the VJP's multipliers mu (and, k = 2, the forward lambda), for k8_adjoint / k8_model_grad;
+                        // TILE <= 2 is launched with k = TILE, so d0 = 0
+                        if (TILE <= 2) rhs[i + dd * nm] = m;
                     }
             }
             __syncthreads();
@@ -298,11 +325,11 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
     double* ch = sens_sm;          // n    c^ = -v
     double* bh = ch + n;           // mg + 2n: b^eq | b^in | ub^ | lb^  (the solver's constraint index space)
     double* tmp = bh + mg + 2 * n; // per-step partials of one cost
-    for (int t = tid; t < n; t += T) ch[t] = -V.V[(long long)lb * V.lds + t];
+    for (int t = tid; t < n; t += T) ch[t] = -V.V[(long long)lb * V.lds * V.k + t];
     for (int t = tid; t < mg + 2 * n; t += T) bh[t] = 0.0;
     __syncthreads();
     const int* iact = V.iact + (long long)b * n;
-    for (int k = tid; k < na; k += T) bh[iact[k] - 1] = V.rhs[(long long)lb * nm + k]; // mu, from sens_solve
+    for (int k = tid; k < na; k += T) bh[iact[k] - 1] = V.rhs[(long long)lb * nm * V.k + k]; // mu, from sens_solve
     __syncthreads();
     // dx0 = sum_costs E c^ - Yeq' b^eq - Yin' b^in + Phi' dtraj
     if (V.dx0) {
@@ -406,7 +433,7 @@ __global__ void __launch_bounds__(kSensThreads) k8_cost_grad_kernel(const __grid
     double* xd = xh + X;   // X  Phi x0 + Psi U
     double* et = xd + X;   // 2 x rows x steps: e, then t, of one cost
     for (int t = tid; t < n; t += T) {
-        ch[t] = -V.V[(long long)lb * V.lds + t];
+        ch[t] = -V.V[(long long)lb * V.lds * V.k + t];
         u[t] = V.U[(long long)b * n + t];
     }
     __syncthreads();
@@ -489,6 +516,170 @@ __global__ void __launch_bounds__(kSensThreads) k8_cost_grad_kernel(const __grid
     }
 }
 
+// dA, dB, dd and the dE / dG of every requested row constraint (see the file comment), one CTA per instance of the chunk.
+// Shared memory: c^ and U (n each); x^ = Psi c^ and x = Phi x0 + Psi U + xi (X each); gx, then rho, and gh, then rho^ (X
+// each); mu and lambda spread over the general rows [eq | ineq] (mg each: the bound rows do not depend on the model).  A is
+// Phi's block 1 and B is Gs's block 0.  Every sum runs in a fixed order; an instance whose status is not 0 keeps the zeros its
+// outputs were initialised to, a failed factorisation reaches the outputs as NaN through v, mu and lambda.
+__global__ void __launch_bounds__(kSensThreads) k8_model_grad_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ VjpParams V)
+{
+    extern __shared__ double sens_sm[];
+    const int lb = blockIdx.x, b = V.b0 + lb;
+    if (V.status[b] != 0) return;
+    const int n = V.n, nx = P.nx, nu = P.nu, N = P.N, X = P.X, NX = N * nx, meq = P.meq, mg = meq + P.mineq, nm = V.nm;
+    const int na = V.nact[b];
+    const int tid = threadIdx.x, T = blockDim.x;
+    double* ch = sens_sm;    // n   c^ = -v
+    double* u = ch + n;      // n   U
+    double* xh = u + n;      // X   Psi c^
+    double* x = xh + X;      // X   Phi x0 + Psi U + xi
+    double* rho = x + X;     // X   gx, then rho
+    double* rhoh = rho + X;  // X   gh, then rho^
+    double* mu = rhoh + X;   // mg  the adjoint's multipliers
+    double* lam = mu + mg;   // mg  the forward solve's multipliers
+    const double* v = V.V + (long long)lb * V.lds * V.k;
+    for (int t = tid; t < n; t += T) {
+        ch[t] = -v[t];
+        u[t] = V.U[(long long)b * n + t];
+    }
+    for (int t = tid; t < mg; t += T) mu[t] = lam[t] = 0.0;
+    __syncthreads();
+    const int* iact = V.iact + (long long)b * n;
+    const double* rhs = V.rhs + (long long)lb * nm * V.k;
+    for (int a = tid; a < na; a += T) {
+        const int idx = iact[a] - 1;
+        if (idx < mg) {
+            mu[idx] = rhs[a];
+            lam[idx] = rhs[nm + a];
+        }
+    }
+    const double* Phi = P.Phi + (long long)b * X * nx;
+    const double* Gs = P.Gs + (long long)b * NX * nu;
+    const double* xi = P.xi + (long long)b * X;
+    const double* x0 = P.x0.at(b);
+    for (int row = tid; row < X; row += T) {
+        const int i = row / nx, r = row % nx;
+        double sh = 0.0, su = 0.0;
+        int go = (i - 1) * nx + r; // G_{i-1-j}[r, :]
+        for (int j = 0; j < i; ++j, go -= nx)
+            for (int cc = 0; cc < nu; ++cc) {
+                const double g = Gs[go + (long long)cc * NX];
+                sh += g * ch[j * nu + cc];
+                su += g * u[j * nu + cc];
+            }
+        double s0 = 0.0;
+        for (int a = 0; a < nx; ++a) s0 += Phi[row + (long long)a * X] * x0[a];
+        xh[row] = sh;
+        x[row] = s0 + su + xi[row];
+    }
+    __syncthreads();
+    // gx_i = dtraj_i + sum_costs M'W t_i - sum_rows mu E_l',  gh_i = sum_costs M'W e_i + sum_rows lambda E_l'
+    const double* dt = V.dtraj ? V.dtraj + (long long)b * V.sdt : nullptr;
+    for (int row = tid; row < X; row += T) {
+        const int i = row / nx, r = row % nx;
+        double gx = dt ? dt[row] : 0.0, gh = 0.0;
+        for (int ci = 0; ci < P.ncost; ++ci) {
+            const CostFam& F = P.cost[ci];
+            if (!F.hasM || i < F.i0 || i >= F.i1) continue;
+            const int rr = F.rows;
+            const double* M = F.M.at(b);
+            const double* Nm = F.hasN && i < N ? F.N.at(b) : nullptr;
+            const double* w = F.w.at(b);
+            const double* res = F.res + (long long)b * F.sres + (long long)(i - F.i0) * rr; // M xi_i - p_i
+            for (int l = 0; l < rr; ++l) {
+                double e = res[l], tt = 0.0;
+                for (int a = 0; a < nx; ++a) {
+                    const double m = M[l + rr * a];
+                    e += m * (x[i * nx + a] - xi[i * nx + a]);
+                    tt += m * xh[i * nx + a];
+                }
+                if (Nm)
+                    for (int bb = 0; bb < nu; ++bb) {
+                        const double m = Nm[l + rr * bb];
+                        e += m * u[i * nu + bb];
+                        tt += m * ch[i * nu + bb];
+                    }
+                const double mw = M[l + rr * r] * w[l];
+                gx += mw * tt;
+                gh += mw * e;
+            }
+        }
+        for (int fi = 0; fi < P.nfam; ++fi) {
+            const CstrFam& F = P.fam[fi];
+            if (!F.hasE || i < F.i0 || i >= F.i1) continue;
+            const double* E = F.E.at(b); // a trajectory bound's selector: quirk Q1 keeps its lower rows as x <= lower
+            const int j0 = (F.is_eq ? 0 : meq) + F.row_off + (i - F.i0) * F.rows;
+            for (int l = 0; l < F.rows; ++l) {
+                const double ev = E[l + F.rows * r];
+                gx -= ev * mu[j0 + l];
+                gh += ev * lam[j0 + l];
+            }
+        }
+        rho[row] = gx;
+        rhoh[row] = gh;
+    }
+    // rho_N = gx_N, rho_i = gx_i + A' rho_{i+1} (and rho^ from gh) down to rho_1: the outputs need no rho_0 (= dx0)
+    for (int i = N - 1; i >= 1; --i) {
+        __syncthreads();
+        for (int r = tid; r < nx; r += T) {
+            double s = 0.0, sh = 0.0;
+            for (int a = 0; a < nx; ++a) {
+                const double A = Phi[nx + a + (long long)r * X]; // A[a, r]
+                s += A * rho[(i + 1) * nx + a];
+                sh += A * rhoh[(i + 1) * nx + a];
+            }
+            rho[i * nx + r] += s;
+            rhoh[i * nx + r] += sh;
+        }
+    }
+    __syncthreads();
+    if (V.dA)
+        for (int q = tid; q < nx * nx; q += T) {
+            const int r = q % nx, a = q / nx;
+            double acc = 0.0;
+            for (int i = 0; i < N; ++i) acc += rho[(i + 1) * nx + r] * x[i * nx + a] + rhoh[(i + 1) * nx + r] * xh[i * nx + a];
+            V.dA[(long long)b * nx * nx + q] = acc;
+        }
+    if (V.dB)
+        for (int q = tid; q < nx * nu; q += T) {
+            const int r = q % nx, cc = q / nx;
+            double acc = 0.0;
+            for (int i = 0; i < N; ++i) acc += rho[(i + 1) * nx + r] * u[i * nu + cc] + rhoh[(i + 1) * nx + r] * ch[i * nu + cc];
+            V.dB[(long long)b * nx * nu + q] = acc;
+        }
+    if (V.dd)
+        for (int r = tid; r < nx; r += T) {
+            double acc = 0.0;
+            for (int i = 0; i < N; ++i) acc += rho[(i + 1) * nx + r];
+            V.dd[(long long)b * nx + r] = acc;
+        }
+    // dE_l = sum_i lambda_(i,l) x^_i' - mu_(i,l) x_i',  dG_l = sum_i lambda_(i,l) c^_i' - mu_(i,l) u_i'
+    for (int fi = 0; fi < P.nfam; ++fi) {
+        const CstrFam& F = P.fam[fi];
+        const int rr = F.rows, j0 = (F.is_eq ? 0 : meq) + F.row_off;
+        if (V.dE[fi])
+            for (int q = tid; q < rr * nx; q += T) {
+                const int l = q % rr, a = q / rr;
+                double acc = 0.0;
+                for (int i = F.i0; i < F.i1; ++i) {
+                    const int j = j0 + (i - F.i0) * rr + l;
+                    acc += lam[j] * xh[i * nx + a] - mu[j] * x[i * nx + a];
+                }
+                V.dE[fi][(long long)b * rr * nx + q] = acc;
+            }
+        if (V.dG[fi])
+            for (int q = tid; q < rr * nu; q += T) {
+                const int l = q % rr, cc = q / rr;
+                double acc = 0.0;
+                for (int i = F.i0; i < F.i1 && i < N; ++i) {
+                    const int j = j0 + (i - F.i0) * rr + l;
+                    acc += lam[j] * ch[i * nu + cc] - mu[j] * u[i * nu + cc];
+                }
+                V.dG[fi][(long long)b * rr * nu + q] = acc;
+            }
+    }
+}
+
 // dcontrol = the first ru rows of Udot; dtraj = the first rx rows of Phi x0dot + Psi Udot, Psi applied as the block-Toeplitz
 // product over the compact Gs (K7 without xi).  Zeros for an instance whose status is not 0.
 __global__ void __launch_bounds__(kSensThreads) k9_output_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ JvpParams J)
@@ -550,8 +741,8 @@ int sens_gram_launch(const SensChunk& S, int nb, cudaStream_t st)
 
 int sens_solve_launch(const SensChunk& S, int nb, cudaStream_t st)
 {
-    const int tile = S.k == 1 ? 1 : kDirTile;
-    const auto kernel = S.k == 1 ? sens_solve_kernel<1> : sens_solve_kernel<kDirTile>;
+    const int tile = S.k <= 2 ? S.k : kDirTile;
+    const auto kernel = S.k == 1 ? sens_solve_kernel<1> : S.k == 2 ? sens_solve_kernel<2> : sens_solve_kernel<kDirTile>;
     const size_t smem = sizeof(double) * 2 * std::min(S.k, tile) * size_t(std::max(S.nm, 1));
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return -int(e);
@@ -588,6 +779,20 @@ int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaSt
     cudaError_t e = cudaFuncSetAttribute(k8_cost_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return -int(e);
     k8_cost_grad_kernel<<<nb, kSensThreads, smem, st>>>(P, V);
+    return launched(cudaGetLastError());
+}
+
+size_t k8_model_grad_smem(const BuildParams& P)
+{
+    return sizeof(double) * (2 * size_t(P.nvar) + 4 * size_t(P.X) + 2 * size_t(P.meq + P.mineq));
+}
+
+int k8_model_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st)
+{
+    const size_t smem = k8_model_grad_smem(P);
+    cudaError_t e = cudaFuncSetAttribute(k8_model_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return -int(e);
+    k8_model_grad_kernel<<<nb, kSensThreads, smem, st>>>(P, V);
     return launched(cudaGetLastError());
 }
 

@@ -68,7 +68,7 @@ int k7_results_launch(const BuildParams& P, const double* x, double* control, do
 struct SensChunk {
     int n;                           // decision variables (nU: LMPC mode)
     int nm;                          // the largest active-set size of the chunk (the padded width of slab, Y and G)
-    int k;                           // right-hand sides: 1 for the VJP, the tangent directions for the JVP
+    int k;                           // right-hand sides: 1 for the VJP (2 with model gradients), the tangent directions for the JVP
     int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
     int b0;
     const int* status;
@@ -83,7 +83,7 @@ struct SensChunk {
     double* Y;                       // chunk: ldy x (nm + k)   Jt' slab = [Y1 | T]
     double* Gf;                      // chunk: (nm + k)^2       Y'Y
     double* Gq;                      // chunk: nm x nm          G with 1 on the padded diagonal
-    double* rhs;                     // chunk: nm x k           bdot_act (0 for the VJP), then Y1' T - bdot_act (then mu for the VJP)
+    double* rhs;                     // chunk: nm x k           bdot_act (VJP: 0 | beta), then Y1' T - bdot_act (then VJP: mu | lambda)
     const double* GJ;                // chunk: ldg x nm         R_G^-1
     const int* gpd;                  // chunk: 1 = G positive definite
     double* W;                       // chunk: lds x k          T - Y1 M
@@ -93,7 +93,9 @@ int sens_gram_launch(const SensChunk& S, int nb, cudaStream_t st);
 int sens_solve_launch(const SensChunk& S, int nb, cudaStream_t st);
 
 // K8: the vector-Jacobian product (k = 1); sens_solve leaves the multipliers mu of the active rows (iact order) in rhs.
-// k8_cost_grad adds the gradients with respect to each cost's w, M and N from the same v.
+// k8_cost_grad adds the gradients with respect to each cost's w, M and N from the same v.  With model gradients k = 2: the
+// second right-hand side is the forward solve itself (slab column nm + 1 = -c, rhs column 1 = beta of the active rows), so
+// rhs column 1 ends up holding the forward multipliers lambda that k8_model_grad needs next to mu.
 struct VjpParams : SensChunk {
     const double* dcontrol;          // dL/dU (nU per instance, sdc apart), may be null
     long long sdc;
@@ -110,12 +112,21 @@ struct VjpParams : SensChunk {
     double* dw[kMaxCost];            // rows per instance
     double* dM[kMaxCost];            // rows x nx per instance, column-major
     double* dN[kMaxCost];            // rows x nu per instance, column-major
+    // model gradients (k8_model_grad; whole batch, zeroed by the caller; null = not wanted; needs U and k = 2)
+    double* dA;                      // nx x nx per instance, column-major
+    double* dB;                      // nx x nu per instance, column-major
+    double* dd;                      // nx per instance
+    double* dE[kMaxFam];             // per row family (not the trajectory-bound selectors): rows x nx per instance, column-major
+    double* dG[kMaxFam];             // rows x nu per instance, column-major
 };
 int k8_gather_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 // shared memory of k8_cost_grad for the resident build (the caller checks it against the device's opt-in limit)
 size_t k8_cost_grad_smem(const BuildParams& P);
 int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
+// the same for k8_model_grad
+size_t k8_model_grad_smem(const BuildParams& P);
+int k8_model_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
 // K9: Jacobian-vector products along k tangent directions, or the feedback gain
 struct JvpParams : SensChunk {

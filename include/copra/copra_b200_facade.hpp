@@ -1186,7 +1186,7 @@ public:
     // on the shared engine since this one's last solve.
     void vjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out)
     {
-        vjpImpl(dcontrol, dtrajectory, out, nullptr);
+        vjpImpl(dcontrol, dtrajectory, out, nullptr, nullptr);
     }
     // The same product together with the gradients with respect to every cost's weights and matrices
     // (copra_b200_lmpc_vjp_costs): costs.w / .M / .N per cost, rows, rows x nx and rows x nu per instance (column-major),
@@ -1194,7 +1194,17 @@ public:
     // of a TrajectoryCost / TargetCost.
     void vjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out, const copra_b200_vjp_cost_out& costs)
     {
-        vjpImpl(dcontrol, dtrajectory, out, &costs);
+        vjpImpl(dcontrol, dtrajectory, out, &costs, nullptr);
+    }
+    // The same products together with the gradients with respect to the dynamics and the row constraints' matrices
+    // (copra_b200_lmpc_vjp_model): model.A / .B / .d, nx x nx, nx x nu and nx per instance, model.E / .G per constraint, rows x
+    // nx and rows x nu per instance (column-major), batch-major HOST arrays; null = not wanted; `costs` may be null.  Errors
+    // as vjp, plus std::domain_error for an E of a constraint without E (ControlConstraint, bounds) or a G of one without G
+    // (TrajectoryConstraint, bounds).
+    void vjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out, const copra_b200_vjp_cost_out* costs,
+        const copra_b200_vjp_model_out& model)
+    {
+        vjpImpl(dcontrol, dtrajectory, out, costs, &model);
     }
     // Forward-mode sensitivities of the last solve (copra_b200_lmpc_jvp): dU (nU x k per instance) and dtrajectory (X x k)
     // along the in.ndir tangent directions of x0 and every entry's vectors described by `in` (HOST arrays, batch-major; either
@@ -1249,21 +1259,20 @@ private:
         p_.ncstr = int(cstrs_.size()); p_.cstrs = cstrs_.data();
         return &p_;
     }
-    // costs null: copra_b200_lmpc_vjp; otherwise copra_b200_lmpc_vjp_costs (one KKT solve for both)
-    void vjpImpl(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out, const copra_b200_vjp_cost_out* costs)
+    // copra_b200_lmpc_vjp_model (one KKT solve for all of them); costs and model null is copra_b200_lmpc_vjp
+    void vjpImpl(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out, const copra_b200_vjp_cost_out* costs,
+        const copra_b200_vjp_model_out* model)
     {
         if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::vjp takes HOST arrays");
         if (multi_) {
             if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::vjp needs a previous solve");
-            const int rc = costs ? copra_b200_multi_lmpc_vjp_costs(multi_, dcontrol, dtrajectory, &out, costs)
-                                 : copra_b200_multi_lmpc_vjp(multi_, dcontrol, dtrajectory, &out);
+            const int rc = copra_b200_multi_lmpc_vjp_model(multi_, dcontrol, dtrajectory, &out, costs, model);
             if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
             if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
             return;
         }
         if (myEpoch_ != b200::buildEpoch()) throw std::runtime_error("BatchedLMPC::vjp: another controller has built on the engine since this solve");
-        const int rc = costs ? copra_b200_lmpc_vjp_costs(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, costs)
-                             : copra_b200_lmpc_vjp(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out);
+        const int rc = copra_b200_lmpc_vjp_model(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, costs, model);
         if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
         b200::check(rc);
     }

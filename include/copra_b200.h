@@ -276,6 +276,33 @@ typedef struct {
 } copra_b200_vjp_cost_out;
 int copra_b200_lmpc_vjp_costs(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
     const copra_b200_vjp_out* out /* may be NULL */, const copra_b200_vjp_cost_out* costs);
+/* The same products, and with them the gradients with respect to the dynamics A, B, d and every row constraint's E and G
+ * (with model = NULL this is copra_b200_lmpc_vjp_costs).  These inputs also move the active rows a_j' U = beta_j, so the
+ * multipliers lambda of the forward solve enter: the adjoint KKT solve takes the forward solve as a second right-hand side.
+ * With the adjoint (c^ = -v, mu) of copra_b200_lmpc_vjp, the states x_i and controls u_i of the solution, x^ = Psi c^,
+ * e_i and t_i of every cost as above, and the active rows j at step i and line l of a constraint (E x_i + G u_i <=/= f):
+ *   gx_i = dL/dtrajectory_i + sum_costs M'W t_i - sum_j mu_j E_l',  gh_i = sum_costs M'W e_i + sum_j lambda_j E_l',
+ *   rho_N = gx_N, rho_i = gx_i + A' rho_{i+1}, and rho^ the same from gh;
+ *   dL/dA = sum_{i<N} rho_{i+1} x_i' + rho^_{i+1} x^_i',  dL/dB = sum_{i<N} rho_{i+1} u_i' + rho^_{i+1} c^_i',
+ *   dL/dd = sum_{i<N} rho_{i+1},  dL/dE_l = sum_i lambda_(i,l) x^_i' - mu_(i,l) x_i',  dL/dG_l = sum_i lambda_(i,l) c^_i' -
+ *   mu_(i,l) u_i'  (inactive rows have lambda = mu = 0; rho_0 is dL/dx0).
+ * A trajectory bound takes part through its multipliers (its E is the engine's line selector; quirk Q1: lower rows are
+ * x <= lower) but has no E gradient.  Gradients are per instance even for inputs given with stride 0.  NULL pointers mark
+ * gradients that are not wanted; `out` and `costs` may be NULL.  With DEVICE inputs, the E arrays the resident build was
+ * given are read again, as are x0, M, N and w: they must still hold those values.  Preconditions and error codes are those
+ * of copra_b200_lmpc_vjp_costs, plus E_ARG for an E entry of a constraint without E (CONTROL, bounds) or a G entry of one
+ * without G (TRAJECTORY, bounds), and E_UNSUPPORTED for a horizon whose 2 nU + 4 X + 2 (meq + mineq) doubles exceed the
+ * device's shared memory per block. */
+typedef struct {
+    double* A;          /* nx x nx per instance, column-major */
+    double* B;          /* nx x nu per instance, column-major */
+    double* d;          /* nx per instance */
+    double* const* E;   /* [ncstr]: rows x nx per instance, column-major; must be NULL for a constraint without E */
+    double* const* G;   /* [ncstr]: rows x nu per instance, column-major; must be NULL for a constraint without G */
+} copra_b200_vjp_model_out;
+int copra_b200_lmpc_vjp_model(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out /* may be NULL */, const copra_b200_vjp_cost_out* costs /* may be NULL */,
+    const copra_b200_vjp_model_out* model);
 /* Forward-mode sensitivities of the last solve: the Jacobian-vector product of (control, trajectory) along `ndir` tangent
  * directions of x0 and every cost's p and every constraint's f / lower / upper (one forward KKT solve per instance with
  * ndir right-hand sides, K9; exact on the final active set, as the VJP).  Each tangent holds, per instance, ndir
@@ -350,6 +377,9 @@ int copra_b200_multi_lmpc_vjp(copra_b200_multi* m, const double* dcontrol, const
 /* copra_b200_lmpc_vjp_costs on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
     const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs);
+/* copra_b200_lmpc_vjp_model on every shard of the last run; HOST arrays holding the whole batch */
+int copra_b200_multi_lmpc_vjp_model(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model);
 /* copra_b200_lmpc_jvp / copra_b200_lmpc_feedback_gain on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory);
 int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx);
