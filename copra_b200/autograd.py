@@ -15,6 +15,16 @@ over the batch.  The dynamics A (nx, nx), B (nx, nu), d (nx,) and every row cons
 given the same way (copra_b200_lmpc_vjp_model), with the same batched / shared rule.  A non-zero forward-mode tangent on any
 of these matrices raises NotImplementedError.  The backward and the forward-mode tangent raise if another solve ran on the
 engine since this forward: the engine keeps only the last solve.
+
+A batch of raw QPs  min 1/2 x'Qx + c'x  s.t.  Aeq x = beq, Aineq x <= bineq, lb <= x <= ub  is differentiable the same way, in
+reverse mode (copra_b200_qp_vjp), with respect to every tensor given:
+
+    x, status = copra_b200.autograd.qp(engine, Q, c, Aeq=..., beq=..., Aineq=..., bineq=..., lb=..., ub=...)
+
+Each input is a CUDA float64 tensor with an optional leading batch axis: a batched tensor gets per-instance gradients, an
+unbatched one is shared by the batch (stride 0) and its gradient is the sum over the batch.  lb / ub default to -inf / +inf.
+Q is read as a symmetric matrix, so its gradient is the symmetric one.  `status` is not differentiable; instances whose status
+is not 0 get zero gradients.
 """
 import ctypes as C
 
@@ -178,3 +188,50 @@ def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None, w=None, M=None,
                  d=[d], E=E or [], G=G or [])
     vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
     return _LMPC.apply(engine, bp, keys, x0, *vecs)
+
+
+class _QP(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, engine, keys, *arrs):
+        live = [a.detach() for a in arrs]
+        given = dict(zip(keys, live))
+        r = engine.solve_qp_batch(*[given.get(k) for k in capi.QP_VJP_WANT])  # keeps its device inputs alive for the VJP
+        ctx.engine, ctx.count, ctx.keys = engine, engine.solve_count, keys
+        ctx.shared = [a.dim() == capi.QP_BASE_NDIM[k] for k, a in zip(keys, arrs)]
+        ctx.mark_non_differentiable(r["status"])
+        ctx.x_like = (tuple(r["x"].shape), r["x"].device)
+        return r["x"], r["status"]
+
+    @staticmethod
+    def jvp(ctx, _engine, _keys, *tangents):
+        if any(t is not None and bool(torch.count_nonzero(t)) for t in tangents):
+            raise NotImplementedError("copra_b200.autograd.qp: forward-mode derivatives of a raw QP batch are not implemented; "
+                                      "reverse mode (backward) is")
+        shape, dev = ctx.x_like
+        return torch.zeros(shape, dtype=torch.float64, device=dev), None
+
+    @staticmethod
+    def backward(ctx, dx, _dstatus):
+        eng = ctx.engine
+        if eng.solve_count != ctx.count:
+            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the VJP needs the "
+                               "active sets of the solve being differentiated")
+        want = tuple(k for k, need in zip(ctx.keys, ctx.needs_input_grad[2:]) if need)
+        if not want:
+            return (None,) * (2 + len(ctx.keys))
+        g = eng.qp_vjp(dx, want=want)  # ordered against torch's stream on both sides
+        grads = [None if g[k] is None else (g[k].sum(0) if shared else g[k]) for k, shared in zip(ctx.keys, ctx.shared)]
+        return (None, None, *grads)
+
+
+def qp(engine, Q, c, Aeq=None, beq=None, Aineq=None, bineq=None, lb=None, ub=None):
+    """(x, status) of the batch of raw QPs given as CUDA float64 tensors (see the module docstring), differentiable with
+    respect to every tensor given; lb / ub default to -inf / +inf"""
+    n = Q.shape[-1]
+    if lb is None:
+        lb = torch.full((n,), -torch.inf, dtype=torch.float64, device=Q.device)
+    if ub is None:
+        ub = torch.full((n,), torch.inf, dtype=torch.float64, device=Q.device)
+    given = dict(Q=Q, c=c, Aeq=Aeq, beq=beq, Aineq=Aineq, bineq=bineq, lb=lb, ub=ub)
+    keys = tuple(k for k in capi.QP_VJP_WANT if given[k] is not None)
+    return _QP.apply(engine, keys, *[given[k] for k in keys])

@@ -74,6 +74,10 @@ class VjpModelOut(C.Structure):
                 ("G", C.POINTER(C.c_void_p))]
 
 
+class QpVjpOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")]
+
+
 class JvpIn(C.Structure):
     _fields_ = [("ndir", C.c_int), ("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
@@ -96,10 +100,13 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_lmpc_retarget", "copra_b200_multi_lmpc_retarget", "copra_b200_lmpc_vjp",
            "copra_b200_multi_lmpc_vjp", "copra_b200_lmpc_jvp", "copra_b200_lmpc_feedback_gain",
            "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain", "copra_b200_lmpc_vjp_costs",
-           "copra_b200_multi_lmpc_vjp_costs", "copra_b200_lmpc_vjp_model", "copra_b200_multi_lmpc_vjp_model"]
+           "copra_b200_multi_lmpc_vjp_costs", "copra_b200_lmpc_vjp_model", "copra_b200_multi_lmpc_vjp_model",
+           "copra_b200_qp_vjp"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
 VJP_COST_WANT = ("w", "M", "N")  # gradients with respect to the cost weights and matrices: requested by name only
 VJP_MODEL_WANT = ("A", "B", "d", "E", "G")  # ... and to the dynamics and the row constraints' matrices: by name only
+QP_VJP_WANT = ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")  # gradients of a raw QP batch (copra_b200_qp_vjp)
+QP_BASE_NDIM = dict(Q=2, c=1, Aeq=2, beq=1, Aineq=2, bineq=1, lb=1, ub=1)
 
 _lib = None
 
@@ -174,6 +181,7 @@ def load():
                                                   C.POINTER(VjpCostOut), C.POINTER(VjpModelOut)]
         lib.copra_b200_multi_lmpc_vjp_model.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
                                                         C.POINTER(VjpCostOut), C.POINTER(VjpModelOut)]
+        lib.copra_b200_qp_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(QpVjpOut)]
         lib.copra_b200_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_int, C.c_void_p, C.c_void_p]
         lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
@@ -568,6 +576,7 @@ class Engine:
         self.h = C.c_void_p()
         self.solve_count = 0  # solves run through this object (copra_b200.autograd detects a stale backward with it)
         self._last_bp = None  # the problem of the resident build, for the shapes of lmpc_vjp's gradients
+        self._last_qp = None  # the shape (and DEVICE inputs) of the last raw QP batch, for qp_vjp
         rc = self.lib.copra_b200_create(C.byref(opt), C.byref(self.h))
         if rc != 0:
             raise CopraB200Error(rc, "copra_b200_create failed (no usable sm_100 CUDA device? there is no CPU fallback)")
@@ -643,33 +652,95 @@ class Engine:
 
     # ---- K5+K6 ----
     def solve_qp_batch(self, Q, c, Aeq, beq, Aineq, bineq, lb, ub):
-        """Arrays with a leading batch axis (or shared, without).  Returns dict(x, status, iters, nact, iact)."""
-        Q = np.asarray(Q, float)
-        n = Q.shape[-1]
-        arrs = dict(Q=(Q, 2), c=(c, 1), Aeq=(Aeq, 2), beq=(beq, 1), Aineq=(Aineq, 2), bineq=(bineq, 1), lb=(lb, 1), ub=(ub, 1))
+        """Arrays with a leading batch axis (or shared, without).  Returns dict(x, status, iters, nact, iact).  numpy arrays
+        (HOST memory), or CUDA float64 tensors (DEVICE memory: the results are tensors on the same device, and the inputs are
+        kept alive on this engine because qp_vjp reads them again)."""
+        arrs = dict(Q=Q, c=c, Aeq=Aeq, beq=beq, Aineq=Aineq, bineq=bineq, lb=lb, ub=ub)
+        dev = next((a.device for a in arrs.values() if hasattr(a, "data_ptr")), None)
+        if dev is not None:
+            import torch
+            arrs = {k: None if a is None else torch.as_tensor(a, dtype=torch.float64, device=dev) for k, a in arrs.items()}
+        else:
+            arrs = {k: None if a is None else np.asarray(a, float) for k, a in arrs.items()}
+        n = arrs["Q"].shape[-1]
         batch = 1
-        for k, (a, base) in arrs.items():
-            if a is not None and np.asarray(a).ndim > base:
-                batch = np.asarray(a).shape[0]
-        meq = 0 if Aeq is None else np.asarray(Aeq).reshape(-1, np.asarray(Aeq).shape[-2], n).shape[1]
-        m = 0 if Aineq is None else np.asarray(Aineq).reshape(-1, np.asarray(Aineq).shape[-2], n).shape[1]
+        for k, a in arrs.items():
+            if a is not None and a.ndim > QP_BASE_NDIM[k]:
+                batch = a.shape[0]
+        def size(a):
+            return 0 if a is None else (a.numel() if dev is not None else a.size)
+        rows = {k: int(arrs[k].shape[-2]) if size(arrs[k]) else 0 for k in ("Aeq", "Aineq")}
+        meq, m = rows["Aeq"], rows["Aineq"]
         keep, cargs = [], []
-        for k in ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub"):
-            a, base = arrs[k]
+        for k in QP_VJP_WANT:
+            a, base = arrs[k], QP_BASE_NDIM[k]
             o = Array()
-            if a is not None and np.asarray(a).size > 0:
-                a = np.asarray(a, float)
-                buf = _colmajor(a, base)
+            if size(a) and rows.get(k, 1) > 0:
+                if dev is not None:
+                    buf = (a.transpose(-1, -2) if base == 2 else a).contiguous()
+                    o.ptr = buf.data_ptr()
+                    o.stride = buf[0].numel() if a.dim() > base else 0
+                else:
+                    buf = _colmajor(a, base)
+                    o.ptr = buf.ctypes.data
+                    o.stride = int(np.prod(buf.shape[1:])) if a.ndim > base else 0
                 keep.append(buf)
-                o.ptr = buf.ctypes.data
-                o.stride = int(np.prod(buf.shape[1:])) if a.ndim > base else 0
             cargs.append(o)
-        x = np.zeros((batch, n))
-        status, iters = np.zeros(batch, np.int32), np.zeros((batch, 2), np.int32)
-        nact, iact = np.zeros(batch, np.int32), np.zeros((batch, n), np.int32)
-        self._check(self.lib.copra_b200_solve_qp_batch(self.h, n, meq, m, batch, *cargs, x.ctypes.data, status.ctypes.data,
-                                                       iters.ctypes.data, nact.ctypes.data, iact.ctypes.data, HOST))
+        self.solve_count += 1
+        self._last_qp = None
+        if dev is not None:
+            x = torch.empty((batch, n), dtype=torch.float64, device=dev)
+            status, iters = torch.empty(batch, dtype=torch.int32, device=dev), torch.empty((batch, 2), dtype=torch.int32, device=dev)
+            nact, iact = torch.empty(batch, dtype=torch.int32, device=dev), torch.empty((batch, n), dtype=torch.int32, device=dev)
+            torch.cuda.synchronize(dev)
+            try:
+                self._check(self.lib.copra_b200_solve_qp_batch(self.h, n, meq, m, batch, *cargs, x.data_ptr(), status.data_ptr(),
+                                                               iters.data_ptr(), nact.data_ptr(), iact.data_ptr(), DEVICE))
+            finally:
+                self.synchronize()
+        else:
+            x = np.zeros((batch, n))
+            status, iters = np.zeros(batch, np.int32), np.zeros((batch, 2), np.int32)
+            nact, iact = np.zeros(batch, np.int32), np.zeros((batch, n), np.int32)
+            self._check(self.lib.copra_b200_solve_qp_batch(self.h, n, meq, m, batch, *cargs, x.ctypes.data, status.ctypes.data,
+                                                           iters.ctypes.data, nact.ctypes.data, iact.ctypes.data, HOST))
+        # DEVICE inputs are read again by qp_vjp: they stay alive until the next raw QP batch
+        self._last_qp = dict(n=n, meq=meq, m=m, batch=batch, live=keep if dev is not None else None)
         return dict(x=x, status=status, iters=iters, nact=nact, iact=iact)
+
+    def qp_vjp(self, dx, want=QP_VJP_WANT):
+        """Vector-Jacobian product of the last raw QP batch (copra_b200_qp_vjp): dx (batch, n) = dL/dx, a numpy array or a
+        CUDA float64 tensor.  Returns dict(Q=(batch, n, n), c=(batch, n), Aeq=(batch, meq, n), beq=(batch, meq),
+        Aineq=(batch, m, n), bineq=(batch, m), lb=(batch, n), ub=(batch, n)) of the same kind as dx, per instance even for
+        inputs given shared; a gradient not in `want` is None, and those of absent rows (meq or m = 0) are empty.  dQ is the
+        gradient along symmetric perturbations of Q.  Instances whose status is not 0 get zeros."""
+        if getattr(self, "_last_qp", None) is None:
+            raise CopraB200Error(-5, "qp_vjp needs a previous solve_qp_batch on this engine")
+        q = self._last_qp
+        n, meq, m, B = q["n"], q["meq"], q["m"], q["batch"]
+        # the engine writes each instance's matrices column-major: allocated as (batch, cols, rows)
+        shapes = dict(Q=(n, n), c=(n,), Aeq=(n, meq), beq=(meq,), Aineq=(n, m), bineq=(m,), lb=(n,), ub=(n,))
+        dev = dx.device if hasattr(dx, "data_ptr") else None
+        o = QpVjpOut()
+        if dev is not None:
+            import torch
+            d = dx.detach().to(torch.float64).contiguous()
+            raw = {k: torch.empty((B,) + shapes[k], dtype=torch.float64, device=dev) if k in want else None for k in shapes}
+            for k, a in raw.items():
+                setattr(o, k, a.data_ptr() if a is not None and a.numel() else None)
+            torch.cuda.synchronize(dev)
+            try:
+                self._check(self.lib.copra_b200_qp_vjp(self.h, d.data_ptr(), DEVICE, C.byref(o)))
+            finally:
+                self.synchronize()
+            return {k: None if a is None else (a.transpose(1, 2).contiguous() if a.dim() == 3 else a) for k, a in raw.items()}
+        d = np.ascontiguousarray(np.asarray(dx, dtype=np.float64))
+        raw = {k: np.zeros((B,) + shapes[k]) if k in want else None for k in shapes}
+        for k, a in raw.items():
+            setattr(o, k, a.ctypes.data if a is not None and a.size else None)
+        self._check(self.lib.copra_b200_qp_vjp(self.h, d.ctypes.data, HOST, C.byref(o)))
+        return {k: None if a is None else (np.ascontiguousarray(a.transpose(0, 2, 1)) if a.ndim == 3 else a)
+                for k, a in raw.items()}
 
     # ---- K1..K7 ----
     def sizes(self, hb):

@@ -74,6 +74,10 @@ struct copra_b200_handle {
     bool warm_valid = false;   // `warm_iact` holds the active sets of the last solve of the resident build
     bool solved = false;       // res_x / res_status / res_nact / res_iact hold the last solve of the resident build (lmpc_vjp)
     bool vjp_factor_valid = false; // vjp_Jt holds R^-1 of the resident build's Hessian(s) (builds the thin solver did not factor)
+    // the last raw QP batch (copra_b200_qp_vjp): its shape and input arrays (the caller's device arrays, or the qp_params
+    // staging buffer), its solution in res_x / res_status / res_nact / res_iact; any LMPC call clears qp_solved
+    bool qp_solved = false;
+    GiBatch qp{};
     // per-instance vector lengths of the resident build (doubles): every cost's p, every constraint's f / lower / upper;
     // the constraint and the side (0 f, 1 lower, 2 upper) of every family; the control-bound constraint (-1 = none)
     std::vector<int> cost_len, cstr_len, fam_cstr, fam_which;
@@ -751,6 +755,7 @@ int ensure_rows(copra_b200_handle* h)
 
 int do_build(copra_b200_handle* h, const copra_b200_problem* p)
 {
+    h->qp_solved = false;
     Plan pl;
     int rc = make_plan(h, p, pl);
     if (rc) return rc;
@@ -948,6 +953,7 @@ int do_build(copra_b200_handle* h, const copra_b200_problem* p)
 
 int do_solve(copra_b200_handle* h, const copra_b200_results* r)
 {
+    h->qp_solved = false;
     if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_solve called before a successful build");
     h->solved = false;
     const BuildParams& P = h->bp;
@@ -1021,6 +1027,15 @@ int do_solve(copra_b200_handle* h, const copra_b200_results* r)
     return 0;
 }
 
+// Where the K8 / K9 core finds R^-1 (ld gt_even(n)) of the Hessian of a chunk of instances: Jt of the chunk's first instance,
+// sJ doubles apart (0 = one factor for the batch), and the positive-definiteness flags of the whole batch, qpd_stride apart
+struct SensFactor {
+    const double* Jt;
+    long long sJ;
+    const int* qpd;
+    int qpd_stride;
+};
+
 // R^-1 of the resident build's Hessian(s) for K8 / K9 (ld gt_even(n); one per instance when P.sQ, else one for the batch):
 // the thin solver's resident factor, else one factorisation kept until the next build
 int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
@@ -1050,15 +1065,17 @@ int sens_factor(copra_b200_handle* h, const double** Jt, const int** qpd)
     return 0;
 }
 
-// The active-set KKT solve of K8 / K9 for the last solve, with k right-hand sides per instance.  The batch is processed in
-// chunks whose slab, Y and Gram workspace stay under kSensWsBytes, each padded to its own largest active set.  `first(nb)`
+// The active-set KKT solve of K8 / K9 for the last solve (n variables, `batch` instances; res_status / res_nact / res_iact
+// hold its status and active sets), with k right-hand sides per instance.  The batch is processed in chunks whose slab, Y and
+// Gram workspace, plus `factor_per` doubles per instance for a factor made per chunk, stay under kSensWsBytes, each padded to
+// its own largest active set.  `factor(b0, nb, F)` provides the chunk's Hessian factor, launching what it needs; `first(nb)`
 // writes a chunk's slab and rhs (the right-hand sides), `last(nb)` reads its V (and rhs = M); both launch one kernel.
 constexpr size_t kSensWsBytes = size_t(1) << 30;
 
-template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk& S, int k, First first, Last last)
+template <class Factor, class First, class Last>
+int sens_run(copra_b200_handle* h, SensChunk& S, int n_, int batch, int k, size_t factor_per, Factor factor, First first, Last last)
 {
-    const BuildParams& P = h->bp;
-    const size_t B = P.batch, n = P.nvar, K = size_t(k);
+    const size_t B = batch, n = n_, K = size_t(k);
     int rc;
     int *status = nullptr, *nact = nullptr, *iact = nullptr;
     if ((rc = ws(h, "res_status", B, &status))) return rc;
@@ -1076,17 +1093,12 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
     };
     const int nm = widest(0, B);
     const int ldj = gt_even(int(n));
-    const long long sJ = P.sQ ? (long long)ldj * (long long)n : 0;
-    const double* Jt = nullptr;
-    const int* qpd = nullptr;
-    if ((rc = sens_factor(h, &Jt, &qpd))) return rc;
     // chunked workspace
     const size_t lds = size_t(ldj), mk = size_t(nm) + K, ldg = size_t(gt_even(nm));
-    const size_t per = 2 * lds * mk + mk * mk + size_t(nm) * nm + 2 * ldg * nm + size_t(nm) * K + 2 * lds * K + 1;
+    const size_t per = 2 * lds * mk + mk * mk + size_t(nm) * nm + 2 * ldg * nm + size_t(nm) * K + 2 * lds * K + 1 + factor_per;
     const int chunk = int(std::max<size_t>(1, std::min<size_t>(B, kSensWsBytes / (per * sizeof(double)))));
     S.n = int(n); S.k = k; S.lds = int(lds); S.ldy = int(lds);
     S.status = status; S.nact = nact; S.iact = iact;
-    S.qpd = qpd; S.qpd_stride = P.sQ ? 1 : 0;
     double* GJT = nullptr;
     const size_t C = size_t(chunk);
     if ((rc = ws(h, "vjp_slab", C * lds * mk, &S.slab))) return rc;
@@ -1100,14 +1112,19 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
     if ((rc = ws(h, "vjp_W", C * lds * K, &S.W))) return rc;
     if ((rc = ws(h, "vjp_V", C * lds * K, &S.V))) return rc;
     const int N_ = int(n), L = int(lds);
-    for (int b0 = 0; b0 < P.batch; b0 += chunk) {
-        const int nb = std::min(chunk, P.batch - b0);
+    for (int b0 = 0; b0 < batch; b0 += chunk) {
+        const int nb = std::min(chunk, batch - b0);
         const int nm = widest(size_t(b0), size_t(b0) + nb), MK = nm + k;
+        SensFactor F{};
+        if ((rc = factor(b0, nb, F))) return rc;
+        const double* Jt = F.Jt;
+        const long long sJ = F.sJ;
+        S.qpd = F.qpd; S.qpd_stride = F.qpd_stride;
         S.b0 = b0; S.nm = nm; S.ldg = gt_even(nm);
         LAUNCHED(first(nb));
         // Y = Jt' slab: one GEMM over the chunk for a shared factor
         if (sJ == 0) LAUNCHED(dgemm_dmma_launch(1, N_, nb * MK, N_, 1.0, Jt, ldj, 0, S.slab, L, 0, 0.0, S.Y, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(1, N_, MK, N_, 1.0, Jt + b0 * sJ, ldj, sJ, S.slab, L, (long long)L * MK, 0.0, S.Y, L,
+        else LAUNCHED(dgemm_dmma_launch(1, N_, MK, N_, 1.0, Jt, ldj, sJ, S.slab, L, (long long)L * MK, 0.0, S.Y, L,
             (long long)L * MK, nb, h->stream));
         if (nm > 0) {
             LAUNCHED(dgemm_dmma_launch(1, MK, MK, N_, 1.0, S.Y, L, (long long)L * MK, S.Y, L, (long long)L * MK, 0.0, S.Gf, MK,
@@ -1121,11 +1138,54 @@ template <class First, class Last> int sens_run(copra_b200_handle* h, SensChunk&
         LAUNCHED(sens_solve_launch(S, nb, h->stream));
         // V = Jt W
         if (sJ == 0) LAUNCHED(dgemm_dmma_launch(0, N_, nb * k, N_, 1.0, Jt, ldj, 0, S.W, L, 0, 0.0, S.V, L, 0, 1, h->stream));
-        else LAUNCHED(dgemm_dmma_launch(0, N_, k, N_, 1.0, Jt + b0 * sJ, ldj, sJ, S.W, L, (long long)L * k, 0.0, S.V, L,
+        else LAUNCHED(dgemm_dmma_launch(0, N_, k, N_, 1.0, Jt, ldj, sJ, S.W, L, (long long)L * k, 0.0, S.V, L,
             (long long)L * k, nb, h->stream));
         LAUNCHED(last(nb));
     }
     return 0;
+}
+
+// the factor source of the resident LMPC build: sens_factor's, made once and kept until the next build
+int lmpc_factor(copra_b200_handle* h, int b0, SensFactor& F)
+{
+    const BuildParams& P = h->bp;
+    const double* Jt = nullptr;
+    int rc = sens_factor(h, &Jt, &F.qpd);
+    if (rc) return rc;
+    F.sJ = P.sQ ? (long long)gt_even(P.nvar) * P.nvar : 0;
+    F.Jt = Jt + b0 * F.sJ;
+    F.qpd_stride = P.sQ ? 1 : 0;
+    return 0;
+}
+
+// the gradients a VJP writes: the caller's device buffers, or (HOST) one workspace block downloaded by download_outputs;
+// every wanted one is zeroed on the stream first (the kernels write only the entries they own)
+struct OutItem { double* host; double** dev; size_t len; };
+
+int bind_outputs(copra_b200_handle* h, std::vector<OutItem>& items, size_t B, int memory)
+{
+    int rc;
+    size_t total = 0;
+    for (auto& it : items) if (it.host) total += it.len * B;
+    double* oblk = nullptr;
+    if (memory == COPRA_B200_HOST && total && (rc = ws(h, "vjp_out", total, &oblk))) return rc;
+    total = 0;
+    for (auto& it : items) {
+        if (!it.host) continue;
+        *it.dev = memory == COPRA_B200_HOST ? oblk + total : it.host;
+        total += it.len * B;
+        if (memory == COPRA_B200_DEVICE) CU(cudaMemsetAsync(*it.dev, 0, it.len * B * sizeof(double), h->stream));
+    }
+    if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
+    return 0;
+}
+
+int download_outputs(copra_b200_handle* h, const std::vector<OutItem>& items, size_t B, int memory)
+{
+    if (memory != COPRA_B200_HOST) return 0;
+    Download D;
+    for (auto& it : items) if (it.host) D.add(*it.dev, it.host, it.len * B * sizeof(double));
+    return run_download(h, D, COPRA_B200_HOST);
 }
 
 // K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs, _vjp_model): the outputs are zeroed first and k8_adjoint only
@@ -1152,7 +1212,6 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
     }
     // outputs: the caller's device buffers, or one workspace block downloaded at the end
     VjpParams V{};
-    struct OutItem { double* host; double** dev; size_t len; };
     std::vector<OutItem> items;
     items.push_back({ out->x0, &V.dx0, nx });
     for (int ci = 0; ci < P.ncost; ++ci) {
@@ -1198,20 +1257,10 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
         }
     }
     if ((want_costs || want_model) && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
-    size_t total = 0;
-    for (auto& it : items) if (it.host) total += it.len * B;
-    double* oblk = nullptr;
-    if (memory == COPRA_B200_HOST && total && (rc = ws(h, "vjp_out", total, &oblk))) return rc;
-    total = 0;
-    for (auto& it : items) {
-        if (!it.host) continue;
-        *it.dev = memory == COPRA_B200_HOST ? oblk + total : it.host;
-        total += it.len * B;
-        if (memory == COPRA_B200_DEVICE) CU(cudaMemsetAsync(*it.dev, 0, it.len * B * sizeof(double), h->stream));
-    }
-    if (oblk) CU(cudaMemsetAsync(oblk, 0, total * sizeof(double), h->stream));
+    if ((rc = bind_outputs(h, items, B, memory))) return rc;
     V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
-    rc = sens_run(h, V, want_model ? 2 : 1, [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
+    rc = sens_run(h, V, P.nvar, P.batch, want_model ? 2 : 1, 0, [&](int b0, int, SensFactor& F) { return lmpc_factor(h, b0, F); },
+        [&](int nb) { return k8_gather_launch(P, V, nb, h->stream); },
         [&](int nb) {
             int n = k8_adjoint_launch(P, V, nb, h->stream);
             if (n < 0) return n;
@@ -1228,12 +1277,7 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
             return n;
         });
     if (rc) return rc;
-    if (memory == COPRA_B200_HOST) {
-        Download D;
-        for (auto& it : items) if (it.host) D.add(*it.dev, it.host, it.len * B * sizeof(double));
-        if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
-    }
-    return 0;
+    return download_outputs(h, items, B, memory);
 }
 
 // K9 for the last solve (copra_b200_lmpc_jvp, copra_b200_lmpc_feedback_gain): k tangent directions described by `in`, or
@@ -1284,7 +1328,8 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
         J.dcontrol = dcontrol ? oblk : nullptr;
         J.dtraj = dtraj ? oblk + B * size_t(ru) * K : nullptr;
     }
-    rc = sens_run(h, J, k, [&](int nb) { return k9_tangent_launch(P, J, nb, h->stream); },
+    rc = sens_run(h, J, P.nvar, P.batch, k, 0, [&](int b0, int, SensFactor& F) { return lmpc_factor(h, b0, F); },
+        [&](int nb) { return k9_tangent_launch(P, J, nb, h->stream); },
         [&](int nb) { return k9_output_launch(P, J, nb, h->stream); });
     if (rc) return rc;
     if (memory == COPRA_B200_HOST) {
@@ -1294,6 +1339,62 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
         if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
     }
     return 0;
+}
+
+// K8 for the last raw QP batch (copra_b200_qp_vjp): the same KKT core, fed by qp_gather and finished by qp_grad.  Its factor
+// of Q has workspace of its own, so the resident LMPC build's factors survive: one factorisation for a stride-0 Q, else one
+// per chunk (counted in the chunk's bytes instead of 2 ld n doubles for the whole batch).  With dAeq / dAineq the forward
+// solve is the second right-hand side (k = 2) and its multipliers lambda enter.
+int do_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b200_qp_vjp_out* out)
+{
+    const GiBatch& G = h->qp;
+    const size_t B = G.batch, n = G.n, meq = G.meq, m = G.m;
+    const int ldj = gt_even(G.n);
+    int rc;
+    const double* d = dx;
+    if (memory == COPRA_B200_HOST) {
+        double* in = nullptr;
+        if ((rc = ws(h, "qpv_in", B * n, &in))) return rc;
+        CU(cudaMemcpyAsync(in, dx, B * n * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        d = in;
+    }
+    QpVjpParams V{};
+    std::vector<OutItem> items{ { out->Q, &V.dQ, n * n }, { out->c, &V.dc, n }, { out->Aeq, &V.dAeq, meq * n },
+        { out->beq, &V.dbeq, meq }, { out->Aineq, &V.dAineq, m * n }, { out->bineq, &V.dbineq, m }, { out->lb, &V.dlb, n },
+        { out->ub, &V.dub, n } };
+    if ((rc = bind_outputs(h, items, B, memory))) return rc;
+    V.meq = G.meq; V.m = G.m;
+    V.c = G.c; V.Aeq = G.Aeq; V.beq = G.beq; V.Aineq = G.Aineq; V.bineq = G.bineq; V.lb = G.lb; V.ub = G.ub;
+    V.dx = d;
+    double* x = nullptr;
+    if ((rc = ws(h, "res_x", B * n, &x))) return rc;
+    V.x = x;
+    const bool shared_q = G.Q.s == 0;
+    auto factor = [&](int b0, int nb, SensFactor& F) {
+        double *J = nullptr, *JT = nullptr;
+        int* pd = nullptr;
+        const size_t count = shared_q ? 1 : size_t(nb); // the first chunk is the largest: later ones reuse its workspace
+        int rc2;
+        if ((rc2 = ws(h, "qpv_Jt", count * ldj * n, &J))) return rc2;
+        if ((rc2 = ws(h, "qpv_JtT", count * ldj * n, &JT))) return rc2;
+        if ((rc2 = ws(h, "qpv_pd", shared_q ? 1 : B, &pd))) return rc2;
+        if (!shared_q || b0 == 0) {
+            cudaError_t e = gt_factor_launch(DArr{ G.Q.at(shared_q ? 0 : b0), G.Q.s }, G.n, ldj, int(count), J, JT,
+                shared_q ? pd : pd + b0, h->plan_sms, h->stream);
+            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+            h->launches += 1; h->call_launches += 1;
+        }
+        F.Jt = J;
+        F.sJ = shared_q ? 0 : (long long)ldj * (long long)n;
+        F.qpd = pd;
+        F.qpd_stride = shared_q ? 0 : 1;
+        return 0;
+    };
+    const bool want_rows = out->Aeq || out->Aineq;
+    rc = sens_run(h, V, G.n, G.batch, want_rows ? 2 : 1, shared_q ? 0 : 2 * size_t(ldj) * n, factor,
+        [&](int nb) { return qp_gather_launch(V, nb, h->stream); }, [&](int nb) { return qp_grad_launch(V, nb, h->stream); });
+    if (rc) return rc;
+    return download_outputs(h, items, B, memory);
 }
 
 // the resident build takes its vectors only through the vector part of K2 / K4, which retarget re-runs and the sensitivities
@@ -1512,6 +1613,7 @@ int copra_b200_lmpc_run(copra_b200_handle* h, const copra_b200_problem* p, const
 {
     if (!h) return COPRA_B200_E_ARG;
     h->built = false;
+    h->qp_solved = false;
     if (!p) return fail(h, COPRA_B200_E_ARG, "null problem");
     const int kChunk = 32768;
     if (p->batch <= 65535) {
@@ -1559,6 +1661,7 @@ int copra_b200_fp64_peaks(copra_b200_handle* h, double* dfma_tflops, double* dmm
 int copra_b200_lmpc_resolve(copra_b200_handle* h, copra_b200_array x0, int memory, const copra_b200_results* r)
 {
     if (!h) return COPRA_B200_E_ARG;
+    h->qp_solved = false;
     if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_resolve needs a previous build on this handle");
     BuildParams& P = h->bp;
     if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "re-solve with new x0 is defined for LMPC mode only");
@@ -1584,6 +1687,7 @@ int copra_b200_lmpc_resolve(copra_b200_handle* h, copra_b200_array x0, int memor
 int copra_b200_lmpc_retarget(copra_b200_handle* h, const copra_b200_problem* p, const copra_b200_results* r)
 {
     if (!h) return COPRA_B200_E_ARG;
+    h->qp_solved = false;
     if (!h->built) return fail(h, COPRA_B200_E_STATE, "copra_b200_lmpc_retarget needs a previous build on this handle");
     int rc = vector_inputs_check(h, "retarget");
     if (rc) return rc;
@@ -1851,6 +1955,7 @@ int copra_b200_solve_qp_batch(copra_b200_handle* h, int n, int meq, int m, int b
     h->call_launches = 0;
     /* the last lmpc build stays valid: this entry uses its own workspace buffers, except for the active sets */
     h->solved = false;
+    h->qp_solved = false;
     for (bool& v : h->ev_valid) v = false;
     int rc = record(h, 0);
     if (rc) return rc;
@@ -1876,6 +1981,18 @@ int copra_b200_solve_qp_batch(copra_b200_handle* h, int n, int meq, int m, int b
     if ((rc = record(h, 3))) return rc;
     if ((rc = run_gi(h, G))) return rc;
     if ((rc = record(h, 4))) return rc;
+    // the solution and the active sets stay in the workspace for copra_b200_qp_vjp
+    const auto keep = [&](const char* name, void* src, size_t bytes) {
+        void* dst = nullptr;
+        int rc2 = dev_reserve(h, name, bytes, &dst);
+        if (rc2 || dst == src) return rc2;
+        CU(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, h->stream));
+        return 0;
+    };
+    if ((rc = keep("res_x", G.x, B * n * sizeof(double)))) return rc;
+    if ((rc = keep("res_status", G.status, B * sizeof(int)))) return rc;
+    if ((rc = keep("res_nact", G.nact, B * sizeof(int)))) return rc;
+    if ((rc = keep("res_iact", G.iact, B * n * sizeof(int)))) return rc;
     if ((rc = record(h, 5))) return rc;
     if (!dv) {
         Download D;
@@ -1887,7 +2004,31 @@ int copra_b200_solve_qp_batch(copra_b200_handle* h, int n, int meq, int m, int b
         if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
     }
     if ((rc = record(h, 6))) return rc;
+    h->qp = G;
+    h->qp_solved = true;
     return 0;
+}
+
+int copra_b200_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b200_qp_vjp_out* out)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!h->qp_solved)
+        return fail(h, COPRA_B200_E_STATE, "copra_b200_qp_vjp needs a raw QP batch (copra_b200_solve_qp_batch) as the last solve on this handle");
+    if (!dx) return fail(h, COPRA_B200_E_ARG, "qp_vjp: dx is required");
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    const GiBatch& G = h->qp;
+    if (!out) return 0;
+    if ((out->Aeq || out->beq) && G.meq == 0) return fail(h, COPRA_B200_E_ARG, "qp_vjp: dAeq / dbeq requested for a batch without equality rows");
+    if ((out->Aineq || out->bineq) && G.m == 0) return fail(h, COPRA_B200_E_ARG, "qp_vjp: dAineq / dbineq requested for a batch without inequality rows");
+    const int k = (out->Aeq || out->Aineq) ? 2 : 1;
+    // qp_grad holds v and x, sens_solve up to 2 k n doubles (the active set has at most n rows), gt_factor Q's scratch
+    const size_t smem = std::max(std::max(qp_grad_smem(G.n), sizeof(double) * 2 * k * size_t(G.n)), gt_factor_smem(G.n));
+    if (smem > h->smem_optin)
+        return fail(h, COPRA_B200_E_UNSUPPORTED, "qp_vjp: n = %d needs %zu bytes of shared memory per block, the device allows %zu",
+            G.n, smem, h->smem_optin);
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_qp_vjp(h, dx, memory, out);
 }
 
 } // extern "C"

@@ -31,6 +31,9 @@
 //               dA = sum_{i<N} rho_{i+1} x_i' + rho^_{i+1} x^_i',  dB = sum_{i<N} rho_{i+1} u_i' + rho^_{i+1} c^_i',
 //               dd = sum_{i<N} rho_{i+1},  dE_l = sum_i lambda_(i,l) x^_i' - mu_(i,l) x_i',  dG_l = sum_i lambda_(i,l) c^_i' -
 //               mu_(i,l) u_i'  (rho_0 is dx0)
+//   qp_gather / qp_grad  the same VJP for a raw QP batch (copra_b200_qp_vjp): the active rows come from the caller's dense
+//               Aeq / Aineq, and dc = -v, dQ = -(v x' + x v') / 2, dbeta_j = mu_j, da_j = -lambda_j v - mu_j x (k = 2 when the
+//               Aeq / Aineq gradients are wanted, lambda again from the forward solve as second right-hand side)
 //   k9_output  the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
 // Every sum runs in a fixed order.  Instances whose status is not 0 get zeros; a Hessian or Gram factorisation that failed
 // gives NaN instead of silently wrong results.
@@ -63,65 +66,69 @@ __device__ __forceinline__ int active_row_family(const BuildParams& P, bool iseq
     return -1;
 }
 
-// entry `col` of constraint `idx` (0-based in the solver's [eq | ineq | upper | lower] index space) of instance b;
-// n = nU, nu = P.nu, mg = P.meq + P.mineq
-__device__ __forceinline__ double active_row_entry(const BuildParams& P, int b, int n, int nu, int mg, int idx, int col)
+// entry `col` of general row `idx` (0-based in the solver's [eq | ineq] index space, idx < P.meq + P.mineq) of instance b;
+// nu = P.nu
+__device__ __forceinline__ double general_row_entry(const BuildParams& P, int b, int nu, int idx, int col)
 {
     double v = 0.0;
-    if (idx < mg) {
-        const bool iseq = idx < P.meq;
-        int i, l;
-        const int fi = active_row_family(P, iseq, iseq ? idx : idx - P.meq, i, l);
-        if (fi >= 0) {
-            const CstrFam& F = P.fam[fi];
-            const int j = col / nu, bb = col % nu, kk = i - j;
-            if (kk >= 0) v = F.EGx[(long long)b * F.sEGx + l + F.rows * (bb + nu * kk)];
-        }
-    } else {
-        const int var = (idx - mg) % n; // upper rows first, then lower rows
-        v = (col == var) ? 1.0 : 0.0;
+    const bool iseq = idx < P.meq;
+    int i, l;
+    const int fi = active_row_family(P, iseq, iseq ? idx : idx - P.meq, i, l);
+    if (fi >= 0) {
+        const CstrFam& F = P.fam[fi];
+        const int j = col / nu, bb = col % nu, kk = i - j;
+        if (kk >= 0) v = F.EGx[(long long)b * F.sEGx + l + F.rows * (bb + nu * kk)];
     }
     return v;
 }
 
-// zero the lds x (nm + k) slab of chunk instance lb (batch instance b) and write its active rows as the first nact columns;
-// the caller writes the k right-hand-side columns
-__device__ __forceinline__ double* sens_gather(const BuildParams& P, const SensChunk& S, int lb, int b)
+// zero the lds x (nm + k) slab of chunk instance lb (batch instance b) and write its active rows as the first nact columns:
+// row(idx, col) gives entry `col` of general row idx < mg, a bound row (upper rows first, then lower rows) is a unit vector.
+// The caller writes the k right-hand-side columns
+template <class Row> __device__ __forceinline__ double* sens_gather(const SensChunk& S, int lb, int b, int mg, Row row)
 {
-    const int n = S.n, nu = P.nu, mg = P.meq + P.mineq;
+    const int n = S.n;
     double* slab = S.slab + (long long)lb * S.lds * (S.nm + S.k);
     const int na = sens_nact(S, b);
     for (long long t = threadIdx.x; t < (long long)S.lds * (S.nm + S.k); t += blockDim.x) slab[t] = 0.0;
     __syncthreads();
     const int* iact = S.iact + (long long)b * n;
     for (int t = threadIdx.x; t < na * n; t += blockDim.x) {
-        const int a = t / n, col = t % n;
-        slab[col + (long long)a * S.lds] = active_row_entry(P, b, n, nu, mg, iact[a] - 1, col);
+        const int a = t / n, col = t % n, idx = iact[a] - 1;
+        slab[col + (long long)a * S.lds] = idx < mg ? row(idx, col) : ((idx - mg) % n == col ? 1.0 : 0.0);
     }
     return slab;
+}
+
+// rhs of a VJP (nm x k): a cotangent has bdot_act = 0; the forward solve's right-hand side (k = 2) is beta(idx) of the active
+// rows, in their natural orientation
+template <class Beta> __device__ __forceinline__ void vjp_rhs(const SensChunk& S, int lb, int b, Beta beta)
+{
+    const int na = sens_nact(S, b), nm = S.nm;
+    const int* iact = S.iact + (long long)b * S.n;
+    for (int t = threadIdx.x; t < nm * S.k; t += blockDim.x) {
+        const int a = t % nm;
+        S.rhs[(long long)lb * nm * S.k + t] = (t >= nm && a < na) ? beta(iact[a] - 1) : 0.0;
+    }
+}
+
+// beta of row idx in the solver's index space: beq | bineq | ub | lb (per-instance pointers)
+__device__ __forceinline__ double active_beta(int idx, int meq, int mg, int n, const double* beq, const double* bineq,
+    const double* ub, const double* lb)
+{
+    return idx < meq ? beq[idx] : idx < mg ? bineq[idx - meq] : idx < mg + n ? ub[idx - mg] : lb[idx - mg - n];
 }
 
 __global__ void __launch_bounds__(kSensThreads) k8_gather_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ VjpParams V)
 {
     const int lb = blockIdx.x, b = V.b0 + lb;
-    const int n = V.n, nu = P.nu, N = P.N, nx = P.nx, nm = V.nm;
+    const int n = V.n, nu = P.nu, N = P.N, nx = P.nx, nm = V.nm, mg = P.meq + P.mineq;
     const long long NX = (long long)N * nx;
-    double* slab = sens_gather(P, V, lb, b);
-    // a cotangent has bdot_act = 0; the forward solve's right-hand side (k = 2) is beta of the active rows, in their natural
-    // orientation: beq | bineq | ub | lb in the solver's index space
-    const int na = sens_nact(V, b), mg = P.meq + P.mineq;
-    const int* iact = V.iact + (long long)b * n;
-    for (int t = threadIdx.x; t < nm * V.k; t += blockDim.x) {
-        const int a = t % nm;
-        double v = 0.0;
-        if (t >= nm && a < na) {
-            const int idx = iact[a] - 1;
-            v = idx < P.meq ? P.beq[(long long)b * P.meq + idx]
-              : idx < mg ? P.bineq[(long long)b * P.mineq + idx - P.meq]
-              : idx < mg + n ? P.ub[(long long)b * P.nvar + idx - mg] : P.lb[(long long)b * P.nvar + idx - mg - n];
-        }
-        V.rhs[(long long)lb * nm * V.k + t] = v;
-    }
+    double* slab = sens_gather(V, lb, b, mg, [&](int idx, int col) { return general_row_entry(P, b, nu, idx, col); });
+    vjp_rhs(V, lb, b, [&](int idx) {
+        return active_beta(idx, P.meq, mg, n, P.beq + (long long)b * P.meq, P.bineq + (long long)b * P.mineq,
+            P.ub + (long long)b * P.nvar, P.lb + (long long)b * P.nvar);
+    });
     if (V.status[b] != 0) return;
     if (V.k == 2)
         for (int col = threadIdx.x; col < n; col += blockDim.x) slab[col + (long long)(nm + 1) * V.lds] = -P.c[(long long)b * P.nvar + col];
@@ -154,7 +161,7 @@ __global__ void __launch_bounds__(kSensThreads) k9_tangent_kernel(const __grid_c
 {
     const int lb = blockIdx.x, b = J.b0 + lb;
     const int n = J.n, nu = P.nu, nx = P.nx, mg = P.meq + P.mineq, nm = J.nm, k = J.k;
-    double* slab = sens_gather(P, J, lb, b);
+    double* slab = sens_gather(J, lb, b, mg, [&](int idx, int col) { return general_row_entry(P, b, nu, idx, col); });
     if (J.status[b] != 0) return;
     const int na = J.nact[b];
     const int* iact = J.iact + (long long)b * n;
@@ -680,6 +687,79 @@ __global__ void __launch_bounds__(kSensThreads) k8_model_grad_kernel(const __gri
     }
 }
 
+// The raw QP (copra_b200_qp_vjp): [A_act' | dx] into the zero-padded slab, A_act read from the caller's column-major Aeq /
+// Aineq through iact; with row-matrix gradients (k = 2) also -c in slab column nm + 1 and beta of the active rows in rhs
+// column 1, as k8_gather
+__global__ void __launch_bounds__(kSensThreads) qp_gather_kernel(const __grid_constant__ QpVjpParams V)
+{
+    const int lb = blockIdx.x, b = V.b0 + lb;
+    const int n = V.n, meq = V.meq, m = V.m, mg = meq + m, nm = V.nm;
+    const double* Aeq = V.Aeq.at(b);
+    const double* Aineq = V.Aineq.at(b);
+    double* slab = sens_gather(V, lb, b, mg, [&](int idx, int col) {
+        return idx < meq ? Aeq[idx + (long long)meq * col] : Aineq[idx - meq + (long long)m * col];
+    });
+    vjp_rhs(V, lb, b, [&](int idx) { return active_beta(idx, meq, mg, n, V.beq.at(b), V.bineq.at(b), V.ub.at(b), V.lb.at(b)); });
+    if (V.status[b] != 0) return;
+    const double* c = V.c.at(b);
+    const double* dx = V.dx + (long long)b * n;
+    for (int col = threadIdx.x; col < n; col += blockDim.x) {
+        slab[col + (long long)nm * V.lds] = dx[col];
+        if (V.k == 2) slab[col + (long long)(nm + 1) * V.lds] = -c[col];
+    }
+}
+
+// The raw QP's gradients from v (S.V), mu (rhs column 0), lambda (rhs column 1, k = 2) and the solution x, one CTA per
+// instance: dc = -v, dQ = -(v x' + x v') / 2, dbeta_j = mu_j at active row j's index (beq | bineq | ub | lb), and the row of
+// dAeq / dAineq of an active general row j = -lambda_j v - mu_j x.  Shared memory: v and x (n each).  An instance whose status
+// is not 0 keeps the zeros its outputs were initialised to; a failed factorisation reaches the outputs as NaN through v, mu
+// and lambda.
+__global__ void __launch_bounds__(kSensThreads) qp_grad_kernel(const __grid_constant__ QpVjpParams V)
+{
+    extern __shared__ double sens_sm[];
+    const int lb = blockIdx.x, b = V.b0 + lb;
+    if (V.status[b] != 0) return;
+    const int n = V.n, meq = V.meq, m = V.m, mg = meq + m, nm = V.nm, na = V.nact[b];
+    const int tid = threadIdx.x, T = blockDim.x;
+    double* v = sens_sm; // n
+    double* x = v + n;   // n
+    const double* Vb = V.V + (long long)lb * V.lds * V.k;
+    for (int t = tid; t < n; t += T) {
+        v[t] = Vb[t];
+        x[t] = V.x[(long long)b * n + t];
+    }
+    __syncthreads();
+    if (V.dc)
+        for (int t = tid; t < n; t += T) V.dc[(long long)b * n + t] = -v[t];
+    if (V.dQ)
+        for (int q = tid; q < n * n; q += T) {
+            const int i = q % n, j = q / n;
+            // no contraction, so that dQ is exactly symmetric
+            V.dQ[(long long)b * n * n + q] = -0.5 * __dadd_rn(__dmul_rn(v[i], x[j]), __dmul_rn(x[i], v[j]));
+        }
+    const int* iact = V.iact + (long long)b * n;
+    const double* rhs = V.rhs + (long long)lb * nm * V.k;
+    for (int a = tid; a < na; a += T) {
+        const int idx = iact[a] - 1;
+        double* out = idx < meq ? (V.dbeq ? V.dbeq + (long long)b * meq + idx : nullptr)
+                    : idx < mg ? (V.dbineq ? V.dbineq + (long long)b * m + idx - meq : nullptr)
+                    : idx < mg + n ? (V.dub ? V.dub + (long long)b * n + idx - mg : nullptr)
+                    : (V.dlb ? V.dlb + (long long)b * n + idx - mg - n : nullptr);
+        if (out) *out = rhs[a];
+    }
+    if (V.k == 2)
+        for (int t = tid; t < na * n; t += T) {
+            const int a = t / n, j = t % n, idx = iact[a] - 1;
+            if (idx >= mg) continue;
+            const double g = -rhs[nm + a] * v[j] - rhs[a] * x[j];
+            if (idx < meq) {
+                if (V.dAeq) V.dAeq[(long long)b * meq * n + idx + (long long)meq * j] = g;
+            } else if (V.dAineq) {
+                V.dAineq[(long long)b * m * n + idx - meq + (long long)m * j] = g;
+            }
+        }
+}
+
 // dcontrol = the first ru rows of Udot; dtraj = the first rx rows of Phi x0dot + Psi Udot, Psi applied as the block-Toeplitz
 // product over the compact Gs (K7 without xi).  Zeros for an instance whose status is not 0.
 __global__ void __launch_bounds__(kSensThreads) k9_output_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ JvpParams J)
@@ -799,6 +879,23 @@ int k8_model_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaS
 int k9_output_launch(const BuildParams& P, const JvpParams& J, int nb, cudaStream_t st)
 {
     k9_output_kernel<<<nb, kSensThreads, 0, st>>>(P, J);
+    return launched(cudaGetLastError());
+}
+
+int qp_gather_launch(const QpVjpParams& V, int nb, cudaStream_t st)
+{
+    qp_gather_kernel<<<nb, kSensThreads, 0, st>>>(V);
+    return launched(cudaGetLastError());
+}
+
+size_t qp_grad_smem(int n) { return sizeof(double) * 2 * size_t(n); }
+
+int qp_grad_launch(const QpVjpParams& V, int nb, cudaStream_t st)
+{
+    const size_t smem = qp_grad_smem(V.n);
+    cudaError_t e = cudaFuncSetAttribute(qp_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+    if (e != cudaSuccess) return -int(e);
+    qp_grad_kernel<<<nb, kSensThreads, smem, st>>>(V);
     return launched(cudaGetLastError());
 }
 

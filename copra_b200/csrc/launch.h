@@ -128,6 +128,20 @@ int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaSt
 size_t k8_model_grad_smem(const BuildParams& P);
 int k8_model_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
+// K8 for a raw QP batch (copra_b200_qp_vjp): the same KKT core with the active rows read from the caller's dense Aeq / Aineq
+// (column-major, meq x n / m x n per instance).  k = 1, or 2 with dAeq / dAineq: then rhs column 1 holds lambda, as above.
+struct QpVjpParams : SensChunk {
+    int meq, m;
+    DArr c, Aeq, beq, Aineq, bineq, lb, ub; // the inputs of the solve
+    const double* dx;                // dL/dx, n per instance (whole batch)
+    const double* x;                 // the solution, n per instance
+    // outputs (whole batch, zeroed by the caller; null = not wanted), the layouts of copra_b200_solve_qp_batch's inputs
+    double *dQ, *dc, *dAeq, *dbeq, *dAineq, *dbineq, *dlb, *dub;
+};
+int qp_gather_launch(const QpVjpParams& V, int nb, cudaStream_t st);
+size_t qp_grad_smem(int n);
+int qp_grad_launch(const QpVjpParams& V, int nb, cudaStream_t st);
+
 // K9: Jacobian-vector products along k tangent directions, or the feedback gain
 struct JvpParams : SensChunk {
     int gain;                        // 1: the x0 tangents are the columns of the identity (k = nx), every other tangent zero

@@ -197,6 +197,37 @@ int copra_b200_solve_qp_batch(copra_b200_handle* h, int n, int meq, int m, int b
     copra_b200_array Aineq, copra_b200_array bineq, copra_b200_array lb, copra_b200_array ub,
     double* x, int* status, int* iters, int* nact, int* iact, int memory);
 
+/* Sensitivities of the last raw QP batch (copra_b200_solve_qp_batch): the vector-Jacobian product of its solutions x with
+ * respect to every input, exact on the final active set.  Write the active rows as equalities a_j'x = beta_j in their natural
+ * orientation (an Aeq row with beq, an Aineq row with bineq, e_k with ub_k for an upper row and with lb_k for a lower row).  With
+ * dx = dL/dx, one adjoint KKT solve per instance, [Q A_act'; A_act 0] [v; mu] = [dx; 0], gives
+ *   dL/dc = -v,  dL/dbeta_j = mu_j (dbeq, dbineq, dub, dlb at the row's index; 0 for inactive rows),
+ *   dL/dQ = -(v x' + x v') / 2,  dL/da_j = -lambda_j v - mu_j x (the row of dAeq / dAineq; 0 for inactive rows),
+ * with lambda the multipliers of the forward solve, [Q A_act'; A_act 0] [x; lambda] = [-c; beta]: the KKT solve takes the
+ * forward solve as a second right-hand side only when dAeq or dAineq is wanted.  Q is read as a symmetric matrix, so dQ is the
+ * gradient along symmetric perturbations of Q.  A weakly active row gives the one-sided derivative on the final active set.
+ * Each gradient has, per instance, the layout copra_b200_solve_qp_batch takes for its input (Q n x n, Aeq meq x n, Aineq
+ * m x n, column-major); gradients are per instance even for inputs given with stride 0.  NULL marks a gradient that is not
+ * wanted. */
+typedef struct {
+    double* Q;
+    double* c;
+    double* Aeq;
+    double* beq;
+    double* Aineq;
+    double* bineq;
+    double* lb;
+    double* ub;
+} copra_b200_qp_vjp_out;
+/* `dx` holds n doubles per instance; it and every output pointer live in `memory`.  Instances whose status is not 0 get
+ * zeros; a Q or a Gram matrix of the active rows that is not positive definite (linearly dependent active rows) gives NaN.
+ * With DEVICE inputs the solve's input arrays are read again: the caller leaves them unchanged until this call.  E_STATE when
+ * the last solve on the handle was not a raw QP batch (none yet, or an LMPC build, solve, resolve or retarget since); E_ARG for
+ * a NULL dx, or for dAeq / dbeq with meq = 0 or dAineq / dbineq with m = 0; E_UNSUPPORTED when n needs more shared memory per
+ * block than the device allows.  A NULL `out` returns 0 after these checks.  Leaves a resident LMPC build, its factor caches
+ * and its warm-start seed untouched. */
+int copra_b200_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b200_qp_vjp_out* out);
+
 /* Dense assembly primitive -- batched FP64 GEMM on the tensor cores (DMMA m8n8k4 fed through shared memory, TMA
  * bulk loads for aligned operands): C[b] = alpha * op(A[b]) * B[b] + beta * C[b], column-major, strides in doubles.
  * It is what full-size (autoSpan'd) entries use for M*Psi, T'WT, E*Psi (src/costFunctions.cpp:65-69,
