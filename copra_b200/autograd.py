@@ -16,6 +16,16 @@ given the same way (copra_b200_lmpc_vjp_model), with the same batched / shared r
 of these matrices raises NotImplementedError.  The backward and the forward-mode tangent raise if another solve ran on the
 engine since this forward: the engine keeps only the last solve.
 
+An initial-state build (copra::InitialStateLMPC: x0 is optimised inside the box [x0lb, x0ub] with the cost
+1/2 x0'R x0 + r'x0) is differentiable the same way, in reverse and in forward mode (copra_b200_lmpc_vjp_initial_state /
+_jvp_initial_state), with respect to x0 and the vectors and to R, r, x0lb and x0ub:
+
+    ctrl, traj = copra_b200.autograd.initial_state_lmpc(engine, bp, x0, R=..., r=..., x0lb=..., x0ub=..., p=[...], ...)
+
+R (nx, nx), r, x0lb and x0ub (nx,) follow the batched / shared rule above; R is read through its symmetric part, so its
+gradient is symmetric.  x0 enters such a build only as the default of an x0 bound that is not given, so its gradient is
+zero when both x0lb and x0ub are.
+
 A batch of raw QPs  min 1/2 x'Qx + c'x  s.t.  Aeq x = beq, Aineq x <= bineq, lb <= x <= ub  is differentiable the same way, in
 reverse mode (copra_b200_qp_vjp), with respect to every tensor given:
 
@@ -188,6 +198,117 @@ def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None, w=None, M=None,
                  d=[d], E=E or [], G=G or [])
     vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
     return _LMPC.apply(engine, bp, keys, x0, *vecs)
+
+
+_INITIAL_BASE = dict(R=2, r=1, x0lb=1, x0ub=1)
+
+
+def _initial_entries(bp):
+    """(kind, index) of every input after x0 of an initial-state build: R, r, x0lb, x0ub, then the vectors"""
+    keys = [(k, 0) for k in capi.INITIAL_KEYS] + [("p", i) for i in range(len(bp["costs"]))]
+    for j, c in enumerate(bp["constraints"]):
+        keys += [("lower", j), ("upper", j)] if c["kind"] in ("trajectory_bound", "control_bound") else [("f", j)]
+    return keys
+
+
+class _InitialStateLMPC(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, engine, bp, keys, x0, *vecs):
+        B, nx = int(bp["batch"]), int(bp["nx"])
+        dev = x0.device
+        problem = dict(bp)
+        problem["costs"] = [dict(c) for c in bp["costs"]]
+        problem["constraints"] = [dict(c) for c in bp["constraints"]]
+        problem["x0"] = np.zeros((B, nx))
+        for (kind, i), v in zip(keys, vecs):
+            if v is None:  # shape only: the tensor itself is patched in below
+                continue
+            if kind in _INITIAL_BASE:
+                problem[kind] = np.zeros(tuple(v.shape))
+            else:
+                (problem["costs"] if kind == "p" else problem["constraints"])[i][kind] = np.zeros(tuple(v.shape))
+        hb = capi.HostBatch(problem, device_tensors=dev)
+        live = [x0.detach().contiguous()]
+        pr = hb.problem
+        pr.x0.ptr, pr.x0.stride = live[0].data_ptr(), live[0].shape[1]
+        for (kind, i), v in zip(keys, vecs):
+            if v is None:
+                continue
+            if kind in _INITIAL_BASE:
+                base = _INITIAL_BASE[kind]
+                if v.dim() not in (base, base + 1) or tuple(v.shape[v.dim() - base:]) != (nx,) * base:
+                    raise ValueError("%s has shape %s, expected %s (with an optional leading batch axis)"
+                                     % (kind, tuple(v.shape), (nx,) * base))
+                live.append(_point(getattr(pr, kind), v, base))
+                continue
+            t = v.detach().contiguous()
+            live.append(t)
+            arr = getattr(pr.costs[i] if kind == "p" else pr.cstrs[i], kind)
+            arr.ptr, arr.stride = t.data_ptr(), t.shape[1]
+        s = engine.sizes(hb)
+        control = torch.empty((B, s["nU"]), dtype=torch.float64, device=dev)
+        traj = torch.empty((B, s["X"]), dtype=torch.float64, device=dev)
+        r = capi.Results()
+        r.memory = capi.DEVICE
+        r.control, r.trajectory = control.data_ptr(), traj.data_ptr()
+        torch.cuda.synchronize(dev)
+        engine.solve_count += 1
+        engine._last_bp = None
+        engine._check(engine.lib.copra_b200_lmpc_run(engine.h, C.byref(pr), C.byref(r)))
+        engine._last_bp = problem
+        engine.synchronize()
+        ctx.engine, ctx.count, ctx.keys, ctx.present = engine, engine.solve_count, keys, [v is not None for v in vecs]
+        ctx.live = (hb, live)
+        ctx.shared = [v is not None and kind in _INITIAL_BASE and v.dim() == _INITIAL_BASE[kind] for (kind, _), v in zip(keys, vecs)]
+        ctx.counts = (B, len(bp["costs"]), len(bp["constraints"]))
+        ctx.mark_non_differentiable()
+        return control, traj
+
+    @staticmethod
+    def jvp(ctx, _engine, _bp, _keys, dx0, *dvecs):
+        # forward mode: one tangent direction through copra_b200_lmpc_jvp_initial_state (K9)
+        eng = ctx.engine
+        if eng.solve_count != ctx.count:
+            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the JVP needs the "
+                               "active sets of the solve being differentiated")
+        B, ncost, ncstr = ctx.counts
+        tangents = dict(p=[None] * ncost, f=[None] * ncstr, lower=[None] * ncstr, upper=[None] * ncstr)
+        init = {}
+        for (kind, i), t, shared in zip(ctx.keys, dvecs, ctx.shared):
+            if t is None:
+                continue
+            if kind in _INITIAL_BASE:
+                init[kind] = (t.expand(B, *t.shape) if shared else t).unsqueeze(1)
+            else:
+                tangents[kind][i] = t.unsqueeze(1)
+        du, dx = eng.initial_state_jvp(x0=dx0.unsqueeze(1) if dx0 is not None else None, **init, **tangents)
+        return du[:, 0], dx[:, 0]
+
+    @staticmethod
+    def backward(ctx, dcontrol, dtraj):
+        eng = ctx.engine
+        if eng.solve_count != ctx.count:
+            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the VJP needs the "
+                               "active sets of the solve being differentiated")
+        want = capi.VJP_WANT + tuple(k for (k, _), p in zip(ctx.keys, ctx.present) if p and k in _INITIAL_BASE)
+        g = eng.initial_state_vjp(dcontrol=dcontrol, dtrajectory=dtraj, want=want)  # ordered against torch's stream
+        grads = [g["x0"]]
+        for (kind, i), present, shared in zip(ctx.keys, ctx.present, ctx.shared):
+            grad = (g[kind] if kind in _INITIAL_BASE else g[kind][i]) if present else None
+            grads.append(grad.sum(0) if shared else grad)  # a shared input's gradient sums its instances'
+        return (None, None, None, *grads)
+
+
+def initial_state_lmpc(engine, bp, x0, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
+    """(control, trajectory) of the initial-state batch problem `bp` with the given inputs, differentiable in reverse and in
+    forward mode with respect to x0, R (nx, nx), r, x0lb, x0ub (nx,) (each with an optional leading batch axis) and every
+    vector given (lists indexed by cost / constraint, as lmpc); None keeps bp's value, which then gets no gradient"""
+    if not bp.get("initial_state"):
+        raise ValueError("initial_state_lmpc takes an initial-state problem; copra_b200.autograd.lmpc takes LMPC-mode ones")
+    keys = _initial_entries(bp)
+    given = dict(R=[R], r=[r], x0lb=[x0lb], x0ub=[x0ub], p=p or [], f=f or [], lower=lower or [], upper=upper or [])
+    vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
+    return _InitialStateLMPC.apply(engine, bp, keys, x0, *vecs)
 
 
 class _QP(torch.autograd.Function):

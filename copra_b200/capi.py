@@ -83,6 +83,14 @@ class JvpIn(C.Structure):
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
 
 
+class VjpInitialOut(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("R", "r", "x0lb", "x0ub")]
+
+
+class JvpInitialIn(C.Structure):
+    _fields_ = [(k, C.c_void_p) for k in ("R", "r", "x0lb", "x0ub")]
+
+
 class Timing(C.Structure):
     _fields_ = [(k, C.c_float) for k in ("h2d_ms", "condense_ms", "assemble_ms", "solve_ms", "rollout_ms", "d2h_ms",
                                          "total_ms")] + [("launches", C.c_longlong)]
@@ -101,11 +109,13 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_multi_lmpc_vjp", "copra_b200_lmpc_jvp", "copra_b200_lmpc_feedback_gain",
            "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain", "copra_b200_lmpc_vjp_costs",
            "copra_b200_multi_lmpc_vjp_costs", "copra_b200_lmpc_vjp_model", "copra_b200_multi_lmpc_vjp_model",
-           "copra_b200_qp_vjp"]
+           "copra_b200_qp_vjp", "copra_b200_lmpc_vjp_initial_state", "copra_b200_lmpc_jvp_initial_state",
+           "copra_b200_multi_lmpc_vjp_initial_state", "copra_b200_multi_lmpc_jvp_initial_state"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
 VJP_COST_WANT = ("w", "M", "N")  # gradients with respect to the cost weights and matrices: requested by name only
 VJP_MODEL_WANT = ("A", "B", "d", "E", "G")  # ... and to the dynamics and the row constraints' matrices: by name only
 QP_VJP_WANT = ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")  # gradients of a raw QP batch (copra_b200_qp_vjp)
+INITIAL_KEYS = ("R", "r", "x0lb", "x0ub")  # initial-state builds: the x0 cost and box (copra_b200_lmpc_vjp_initial_state)
 QP_BASE_NDIM = dict(Q=2, c=1, Aeq=2, beq=1, Aineq=2, bineq=1, lb=1, ub=1)
 
 _lib = None
@@ -186,6 +196,14 @@ def load():
         lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
         lib.copra_b200_multi_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+        lib.copra_b200_lmpc_vjp_initial_state.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(VjpOut),
+                                                          C.POINTER(VjpInitialOut)]
+        lib.copra_b200_multi_lmpc_vjp_initial_state.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
+                                                                C.POINTER(VjpInitialOut)]
+        lib.copra_b200_lmpc_jvp_initial_state.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.POINTER(JvpInitialIn), C.c_int,
+                                                          C.c_void_p, C.c_void_p]
+        lib.copra_b200_multi_lmpc_jvp_initial_state.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.POINTER(JvpInitialIn),
+                                                                C.c_void_p, C.c_void_p]
         _lib = lib
     return _lib
 
@@ -369,11 +387,18 @@ def cstr_shapes(bp):
     return out
 
 
-def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
+def initial_want(bp):
+    """the gradients Engine.initial_state_vjp returns by default: x0 and the vectors, and R, r, x0lb, x0ub where the build
+    was given them"""
+    return VJP_WANT + tuple(k for k in INITIAL_KEYS if bp.get(k) is not None)
+
+
+def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None, initial=False):
     """allocate the wanted gradients (numpy, or torch tensors on the device of the torch cotangents), describe them in a
     VjpOut (and, when w, M or N are wanted, a VjpCostOut; when A, B, d, E or G are, a VjpModelOut) and run
     `call(dcontrol_ptr, dtrajectory_ptr, memory, out, cost_out, model_out)`, cost_out / model_out None unless such gradients
-    are wanted.  With torch tensors the engine runs on its own stream:
+    are wanted.  With `initial` (an initial-state build) it runs `call(dcontrol_ptr, dtrajectory_ptr, memory, out, init_out)`
+    instead, init_out a VjpInitialOut for R, r, x0lb and x0ub.  With torch tensors the engine runs on its own stream:
     the cotangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the
     gradients (written, zero-initialised, by the engine itself) and the input copies are handed back."""
     nx, plen, clen = vjp_lengths(bp)
@@ -453,11 +478,25 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
             ptrs = (C.c_void_p * max(1, len(mraw[key])))(*[ptr(a) if a is not None else None for a in mraw[key]])
             keep.append(ptrs)
             setattr(mo, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
+    io = None
+    if initial:
+        if co is not None or mo is not None:
+            raise CopraB200Error(-4, "initial-state builds have no gradients with respect to w, M, N, A, B, d, E or G")
+        # R is written column-major; it is symmetric, so its logical layout is the same
+        iraw = dict(R=zeros(nx * nx).reshape(B, nx, nx) if "R" in want else None,
+                    **{k: zeros(nx) if k in want else None for k in ("r", "x0lb", "x0ub")})
+        io = VjpInitialOut()
+        for key, a in iraw.items():
+            setattr(io, key, ptr(a) if a is not None else None)
+            res[key] = a
     dc, dt = inp(dcontrol), inp(dtrajectory)
     if dev is not None:
         torch.cuda.synchronize(dev)
     try:
-        call(dc, dt, mem, o, co, mo)
+        if initial:
+            call(dc, dt, mem, o, io)
+        else:
+            call(dc, dt, mem, o, co, mo)
     finally:
         if dev is not None and sync is not None:
             sync()
@@ -477,16 +516,24 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None):
     return res
 
 
-def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None):
+def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None, init=None):
     """describe the tangents (each (batch, k, len), numpy or CUDA float64 tensors; None = zero) in a JvpIn, allocate dU
-    (batch, k, nU) and dtrajectory (batch, k, X) of the same kind and run `call(jvp_in, memory, dU_ptr, dX_ptr)`.  With torch
-    tensors the engine runs on its own stream: the tangents are complete before the call (device synchronise) and `sync()`
-    waits for the engine's stream before the results are handed back."""
+    (batch, k, nU) and dtrajectory (batch, k, X) of the same kind and run `call(jvp_in, memory, dU_ptr, dX_ptr)`.  With
+    `init` (a dict of the R (batch, k, nx, nx), r, x0lb and x0ub (batch, k, nx) tangents of an initial-state build) it runs
+    `call(jvp_in, jvp_initial_in, memory, dU_ptr, dX_ptr)` instead.  With torch tensors the engine runs on its own stream: the
+    tangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the results
+    are handed back."""
     nx, plen, clen = vjp_lengths(bp)
     kinds = [c["kind"] for c in bp["constraints"]]
     bound = [kd in ("trajectory_bound", "control_bound") for kd in kinds]
     lists = dict(p=list(p or []), f=list(f or []), lower=list(lower or []), upper=list(upper or []))
-    given = [x0] + [t for v in lists.values() for t in v]
+    initial = init is not None
+    init = dict(init or {})
+    R = init.get("R")
+    if R is not None and len(R.shape) == 4:  # (batch, k, nx, nx) -> column-major nx x nx per direction
+        R = R.transpose(2, 3) if hasattr(R, "data_ptr") else np.swapaxes(np.asarray(R, dtype=np.float64), 2, 3)
+        init["R"] = R.reshape(R.shape[0], R.shape[1], nx * nx)
+    given = [x0] + [t for v in lists.values() for t in v] + [t for t in init.values()]
     given = [t for t in given if t is not None]
     if not given:
         raise CopraB200Error(-1, "lmpc_jvp needs at least one tangent")
@@ -528,6 +575,9 @@ def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None):
         ptrs = (C.c_void_p * max(1, n))(*[inp(a, lens[key][j], "%s[%d]" % (key, j)) for j, a in enumerate(arrs)])
         keep.append(ptrs)
         setattr(t, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
+    ti = JvpInitialIn()
+    for key in INITIAL_KEYS:
+        setattr(ti, key, inp(init.get(key), nx * nx if key == "R" else nx, key))
     nU, X = int(bp["nu"]) * int(bp["N"]), nx * (int(bp["N"]) + 1)
     if dev is not None:
         du = torch.empty((B, k, nU), dtype=torch.float64, device=dev)
@@ -538,7 +588,10 @@ def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None):
         du, dx = np.zeros((B, k, nU)), np.zeros((B, k, X))
         ptr, mem = (lambda a: a.ctypes.data), HOST
     try:
-        call(t, mem, ptr(du), ptr(dx))
+        if initial:
+            call(t, ti, mem, ptr(du), ptr(dx))
+        else:
+            call(t, mem, ptr(du), ptr(dx))
     finally:
         if dev is not None and sync is not None:
             sync()
@@ -851,6 +904,31 @@ class Engine:
                          lambda t, mem, du, dx: self._check(self.lib.copra_b200_lmpc_jvp(self.h, C.byref(t), mem, du, dx)),
                          sync=self.synchronize)
 
+    def initial_state_vjp(self, dcontrol=None, dtrajectory=None, want=None):
+        """Vector-Jacobian product of the last solve of an initial-state build (copra_b200_lmpc_vjp_initial_state): as
+        lmpc_vjp, with R=(batch, nx, nx), r=, x0lb=, x0ub=(batch, nx) as well.  x0 receives the multipliers of the x0 bounds
+        that defaulted to x0 (zeros when the build was given both x0lb and x0ub).  `want` defaults to x0, the vectors, and
+        those of R, r, x0lb and x0ub the build was given; asking for one it was not given raises (E_ARG)."""
+        if self._last_bp is None:
+            raise CopraB200Error(-5, "initial_state_vjp needs a previous lmpc_run on this engine")
+        bp = self._last_bp
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, initial_want(bp) if want is None else want,
+                         lambda dc, dt, mem, o, io: self._check(self.lib.copra_b200_lmpc_vjp_initial_state(
+                             self.h, dc, dt, mem, C.byref(o), C.byref(io))),
+                         sync=self.synchronize, initial=True)
+
+    def initial_state_jvp(self, x0=None, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
+        """Jacobian-vector product of the last solve of an initial-state build (copra_b200_lmpc_jvp_initial_state): as
+        lmpc_jvp, with tangents R (batch, k, nx, nx), r, x0lb and x0ub (batch, k, nx) as well.  The x0 tangent moves the x0
+        bounds the build was not given.  Returns (dcontrol (batch, k, nU), dtrajectory (batch, k, X))."""
+        if self._last_bp is None:
+            raise CopraB200Error(-5, "initial_state_jvp needs a previous lmpc_run on this engine")
+        bp = self._last_bp
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, ti, mem, du, dx: self._check(self.lib.copra_b200_lmpc_jvp_initial_state(
+                             self.h, C.byref(t), C.byref(ti), mem, du, dx)),
+                         sync=self.synchronize, init=dict(R=R, r=r, x0lb=x0lb, x0ub=x0ub))
+
     def lmpc_feedback_gain(self, steps=1, device=None):
         """Local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): (Ku (batch, nu*steps, nx) = dU[:nu*steps]/dx0,
         Kx (batch, nx*(steps+1), nx) = dtrajectory[:nx*(steps+1)]/dx0); numpy, or CUDA tensors on the torch `device`."""
@@ -983,6 +1061,29 @@ class MultiEngine:
             raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
         return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
                          lambda t, mem, du, dx: self._check(self.lib.copra_b200_multi_lmpc_jvp(self.m, C.byref(t), du, dx)))
+
+    def initial_state_vjp(self, dcontrol=None, dtrajectory=None, want=None):
+        """Engine.initial_state_vjp over the shards of the last run (numpy arrays holding the whole batch)"""
+        bp = getattr(self, "_last_bp", None)
+        if bp is None:
+            raise CopraB200Error(-5, "initial_state_vjp needs a previous lmpc_run on this engine")
+        if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
+            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, initial_want(bp) if want is None else want,
+                         lambda dc, dt, mem, o, io: self._check(self.lib.copra_b200_multi_lmpc_vjp_initial_state(
+                             self.m, dc, dt, C.byref(o), C.byref(io))), initial=True)
+
+    def initial_state_jvp(self, x0=None, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
+        """Engine.initial_state_jvp over the shards of the last run (numpy arrays holding the whole batch)"""
+        bp = getattr(self, "_last_bp", None)
+        if bp is None:
+            raise CopraB200Error(-5, "initial_state_jvp needs a previous lmpc_run on this engine")
+        tangents = [x0, R, r, x0lb, x0ub] + list(p or []) + list(f or []) + list(lower or []) + list(upper or [])
+        if any(hasattr(t, "data_ptr") for t in tangents):
+            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, ti, mem, du, dx: self._check(self.lib.copra_b200_multi_lmpc_jvp_initial_state(
+                             self.m, C.byref(t), C.byref(ti), du, dx)), init=dict(R=R, r=r, x0lb=x0lb, x0ub=x0ub))
 
     def lmpc_feedback_gain(self, steps=1):
         """Engine.lmpc_feedback_gain over the shards of the last run (numpy arrays holding the whole batch)"""

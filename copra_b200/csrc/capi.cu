@@ -1188,12 +1188,13 @@ int download_outputs(copra_b200_handle* h, const std::vector<OutItem>& items, si
     return run_download(h, D, COPRA_B200_HOST);
 }
 
-// K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs, _vjp_model): the outputs are zeroed first and k8_adjoint only
-// writes the entries it owns; with `costs`, k8_cost_grad follows k8_adjoint on each chunk and writes the cost gradients;
-// with `model`, the KKT solve takes the forward solve as a second right-hand side (its multipliers) and k8_model_grad
-// follows them and writes the model gradients.
+// K8 for the last solve (copra_b200_lmpc_vjp, _vjp_costs, _vjp_model, _vjp_initial_state): the outputs are zeroed first and
+// k8_adjoint only writes the entries it owns; with `costs`, k8_cost_grad follows k8_adjoint on each chunk and writes the cost
+// gradients; with `model`, the KKT solve takes the forward solve as a second right-hand side (its multipliers) and
+// k8_model_grad follows them and writes the model gradients.  `init` (initial-state builds) adds R, r, x0lb and x0ub to
+// k8_adjoint's outputs.
 int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, int memory, const copra_b200_vjp_out* out,
-    const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model)
+    const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model, const copra_b200_vjp_initial_out* init = nullptr)
 {
     const BuildParams& P = h->bp;
     const size_t B = P.batch, nx = P.nx, nu = P.nu;
@@ -1256,7 +1257,14 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
             want_model |= E || G;
         }
     }
-    if ((want_costs || want_model) && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
+    if (init) {
+        items.push_back({ init->R, &V.dR, nx * nx });
+        items.push_back({ init->r, &V.dr, nx });
+        items.push_back({ init->x0lb, &V.dx0lb, nx });
+        items.push_back({ init->x0ub, &V.dx0ub, nx });
+    }
+    const bool want_x = want_costs || want_model || (init && init->R);
+    if (want_x && (rc = ws(h, "res_x", B * P.nvar, &V.U))) return rc;
     if ((rc = bind_outputs(h, items, B, memory))) return rc;
     V.dcontrol = dc; V.sdc = P.nU; V.dtraj = dt; V.sdt = P.X;
     rc = sens_run(h, V, P.nvar, P.batch, want_model ? 2 : 1, 0, [&](int b0, int, SensFactor& F) { return lmpc_factor(h, b0, F); },
@@ -1280,11 +1288,12 @@ int do_vjp(copra_b200_handle* h, const double* dcontrol, const double* dtraj, in
     return download_outputs(h, items, B, memory);
 }
 
-// K9 for the last solve (copra_b200_lmpc_jvp, copra_b200_lmpc_feedback_gain): k tangent directions described by `in`, or
-// (gain) the columns of the identity on x0.  k9_output writes every entry of the first ru rows of dU and the first rx rows of
-// dtrajectory of each direction (zeros for an instance whose status is not 0).
+// K9 for the last solve (copra_b200_lmpc_jvp, copra_b200_lmpc_feedback_gain, copra_b200_lmpc_jvp_initial_state): k tangent
+// directions described by `in` (and, initial-state builds, `init`), or (gain) the columns of the identity on x0.  k9_output
+// writes every entry of the first ru rows of dU and the first rx rows of dtrajectory of each direction (zeros for an instance
+// whose status is not 0).
 int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, int memory, double* dcontrol, int ru,
-    double* dtraj, int rx)
+    double* dtraj, int rx, const copra_b200_jvp_initial_in* init = nullptr)
 {
     const BuildParams& P = h->bp;
     const size_t B = P.batch, nx = P.nx, K = size_t(k);
@@ -1293,7 +1302,7 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
     J.gain = gain ? 1 : 0;
     // tangents: the caller's device arrays, or HOST arrays packed into the staging buffer and uploaded in one copy
     Upload U;
-    DArr tx0{}, tp[kMaxCost]{}, tf[kMaxFam]{}, tlo{}, tup{};
+    DArr tx0{}, tp[kMaxCost]{}, tf[kMaxFam]{}, tlo{}, tup{}, tR{}, tr{}, tx0lb{}, tx0ub{};
     auto add = [&](const double* a, size_t len, DArr* dst) { U.add(copra_b200_array{ a, (long long)(len * K) }, len * K, dst); };
     if (in) {
         add(in->x0, nx, &tx0);
@@ -1313,7 +1322,15 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
             add(in->upper ? in->upper[h->bound_cstr] : nullptr, size_t(J.cblen), &tup);
         }
     }
+    if (init) {
+        add(init->R, nx * nx, &tR);
+        add(init->r, nx, &tr);
+        add(init->x0lb, nx, &tx0lb);
+        add(init->x0ub, nx, &tx0ub);
+    }
     if ((rc = run_upload(h, U, P.batch, memory, "jvp_in"))) return rc;
+    J.tR = tR.p; J.tr = tr.p; J.tx0lb = tx0lb.p; J.tx0ub = tx0ub.p;
+    if (J.tR && (rc = ws(h, "res_x", B * P.nvar, const_cast<double**>(&J.x)))) return rc;
     J.tx0 = tx0.p;
     for (int ci = 0; ci < P.ncost; ++ci) J.tp[ci] = tp[ci].p;
     for (int fi = 0; fi < P.nfam; ++fi) J.tf[fi] = tf[fi].p;
@@ -1398,11 +1415,10 @@ int do_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b2
 }
 
 // the resident build takes its vectors only through the vector part of K2 / K4, which retarget re-runs and the sensitivities
-// differentiate: LMPC mode, and no full-size entry other than the control bound
-int vector_inputs_check(copra_b200_handle* h, const char* name)
+// differentiate: no full-size entry other than the control bound
+int full_size_check(copra_b200_handle* h, const char* name)
 {
     const BuildParams& P = h->bp;
-    if (P.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s is defined for LMPC mode only", name);
     for (int i = 0; i < P.ncost; ++i)
         if (P.cost[i].dense) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: cost %d is a full-size entry (its f comes out of the dense GEMMs)", name, i);
     for (int k = 0; k < P.nfam; ++k)
@@ -1411,11 +1427,44 @@ int vector_inputs_check(copra_b200_handle* h, const char* name)
     return 0;
 }
 
+// the same, and LMPC mode
+int vector_inputs_check(copra_b200_handle* h, const char* name)
+{
+    if (h->bp.initial_state) return fail(h, COPRA_B200_E_UNSUPPORTED, "%s is defined for LMPC mode only", name);
+    return full_size_check(h, name);
+}
+
 // the preconditions of the sensitivities of the last solve (copra_b200_lmpc_vjp, _jvp, _feedback_gain)
 int sens_check(copra_b200_handle* h, const char* name)
 {
     if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_%s needs a solve of the resident build on this handle", name);
     return vector_inputs_check(h, name);
+}
+
+// the preconditions of the initial-state sensitivities (copra_b200_lmpc_vjp_initial_state, _jvp_initial_state), k right-hand
+// sides: a solved initial-state build, R / r / x0lb / x0ub gradients or tangents only for the arrays the build was given, and
+// k8_adjoint's and sens_solve's shared memory (the active set has at most nvar rows) within the device's limit
+int initial_state_check(copra_b200_handle* h, const char* name, const void* R, const void* r, const void* x0lb, const void* x0ub, int k)
+{
+    if (!h->built || !h->solved) return fail(h, COPRA_B200_E_STATE, "copra_b200_%s needs a solve of the resident build on this handle", name);
+    const BuildParams& P = h->bp;
+    if (!P.initial_state)
+        return fail(h, COPRA_B200_E_UNSUPPORTED, "%s is defined for initial-state builds; an LMPC-mode build takes copra_b200_lmpc_vjp / "
+            "copra_b200_lmpc_jvp", name);
+    int rc = full_size_check(h, name);
+    if (rc) return rc;
+    const struct { const void* want; const void* given; const char* what; } arg[] = {
+        { R, P.R.p, "R" }, { r, P.r.p, "r" }, { x0lb, P.x0lb.p, "x0lb" }, { x0ub, P.x0ub.p, "x0ub" } };
+    for (const auto& a : arg)
+        if (a.want && !a.given)
+            return fail(h, COPRA_B200_E_ARG, "%s: the build was not given %s (the reference default is used), it has no sensitivity",
+                name, a.what);
+    const size_t solve = sizeof(double) * 2 * size_t(std::min(k, 8)) * size_t(P.nvar);
+    const size_t need = std::max(k8_adjoint_smem(P), solve);
+    if (need > h->smem_optin)
+        return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: nvar = %d needs %zu bytes of shared memory per block, the device allows %zu", name,
+            P.nvar, need, h->smem_optin);
+    return 0;
 }
 
 } // namespace
@@ -1798,6 +1847,36 @@ int copra_b200_lmpc_feedback_gain(copra_b200_handle* h, int steps, double* Ku, d
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
     return do_jvp(h, nullptr, P.nx, true, memory, Ku, P.nu * steps, Kx, P.nx * (steps + 1));
+}
+
+int copra_b200_lmpc_vjp_initial_state(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_initial_out* init)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    static const copra_b200_vjp_initial_out none{};
+    const copra_b200_vjp_initial_out& in = init ? *init : none;
+    int rc = initial_state_check(h, "lmpc_vjp_initial_state", in.R, in.r, in.x0lb, in.x0ub, 1);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_vjp(h, dcontrol, dtrajectory, memory, out, nullptr, nullptr, &in);
+}
+
+int copra_b200_lmpc_jvp_initial_state(copra_b200_handle* h, const copra_b200_jvp_in* in, const copra_b200_jvp_initial_in* init,
+    int memory, double* dcontrol, double* dtrajectory)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!in) return fail(h, COPRA_B200_E_ARG, "lmpc_jvp_initial_state: null tangent description");
+    if (in->ndir < 1) return fail(h, COPRA_B200_E_ARG, "lmpc_jvp_initial_state: ndir = %d, needs at least one direction", in->ndir);
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    static const copra_b200_jvp_initial_in none{};
+    const copra_b200_jvp_initial_in& ti = init ? *init : none;
+    int rc = initial_state_check(h, "lmpc_jvp_initial_state", ti.R, ti.r, ti.x0lb, ti.x0ub, in->ndir);
+    if (rc) return rc;
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_jvp(h, in, in->ndir, false, memory, dcontrol, h->bp.nU, dtrajectory, h->bp.X, &ti);
 }
 
 int copra_b200_set_warm_start(copra_b200_handle* h, int on)

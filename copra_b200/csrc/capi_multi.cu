@@ -60,6 +60,53 @@ template <class F> int run_shards(copra_b200_multi* m, F body)
     return 0;
 }
 
+// a copra_b200_vjp_out of whole-batch arrays advanced to instance lo of a shard (nx, plen, clen: cb_vjp_lengths)
+struct VjpOutSlice {
+    std::vector<double*> p, f, lower, upper;
+    copra_b200_vjp_out o{};
+    VjpOutSlice(const copra_b200_vjp_out& out, long long lo, int nx, const std::vector<int>& plen, const std::vector<int>& clen)
+        : p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size())
+    {
+        for (size_t i = 0; i < plen.size(); ++i) p[i] = (out.p && out.p[i]) ? out.p[i] + lo * plen[i] : nullptr;
+        for (size_t i = 0; i < clen.size(); ++i) {
+            f[i] = (out.f && out.f[i]) ? out.f[i] + lo * clen[i] : nullptr;
+            lower[i] = (out.lower && out.lower[i]) ? out.lower[i] + lo * clen[i] : nullptr;
+            upper[i] = (out.upper && out.upper[i]) ? out.upper[i] + lo * clen[i] : nullptr;
+        }
+        o.x0 = out.x0 ? out.x0 + lo * nx : nullptr;
+        o.p = out.p ? p.data() : nullptr;
+        o.f = out.f ? f.data() : nullptr;
+        o.lower = out.lower ? lower.data() : nullptr;
+        o.upper = out.upper ? upper.data() : nullptr;
+    }
+};
+
+// a copra_b200_jvp_in of whole-batch tangents (len x k per instance) advanced to instance lo of a shard
+struct JvpInSlice {
+    std::vector<const double*> p, f, lower, upper;
+    copra_b200_jvp_in t{};
+    JvpInSlice(const copra_b200_jvp_in& in, long long lo, int nx, const std::vector<int>& plen, const std::vector<int>& clen)
+        : p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size())
+    {
+        const long long k = in.ndir;
+        auto at = [&](const double* const* arr, size_t i, int len) -> const double* {
+            return (arr && arr[i]) ? arr[i] + lo * len * k : nullptr;
+        };
+        for (size_t i = 0; i < plen.size(); ++i) p[i] = at(in.p, i, plen[i]);
+        for (size_t i = 0; i < clen.size(); ++i) {
+            f[i] = at(in.f, i, clen[i]);
+            lower[i] = at(in.lower, i, clen[i]);
+            upper[i] = at(in.upper, i, clen[i]);
+        }
+        t = in;
+        t.x0 = in.x0 ? in.x0 + lo * nx * k : nullptr;
+        t.p = in.p ? p.data() : nullptr;
+        t.f = in.f ? f.data() : nullptr;
+        t.lower = in.lower ? lower.data() : nullptr;
+        t.upper = in.upper ? upper.data() : nullptr;
+    }
+};
+
 } // namespace
 
 // per-instance lengths of x0 and of every cost's p / constraint's vector of the resident build (capi.cu)
@@ -226,19 +273,8 @@ int copra_b200_multi_lmpc_vjp_model(copra_b200_multi* m, const double* dcontrol,
         cb_vjp_lengths(m->h[g], nx, plen, clen);
         const long long lo = m->lo[g];
         // every array of the whole batch, advanced to this shard's first instance
-        std::vector<double*> p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size());
-        for (size_t i = 0; i < plen.size(); ++i) p[i] = (out->p && out->p[i]) ? out->p[i] + lo * plen[i] : nullptr;
-        for (size_t i = 0; i < clen.size(); ++i) {
-            f[i] = (out->f && out->f[i]) ? out->f[i] + lo * clen[i] : nullptr;
-            lower[i] = (out->lower && out->lower[i]) ? out->lower[i] + lo * clen[i] : nullptr;
-            upper[i] = (out->upper && out->upper[i]) ? out->upper[i] + lo * clen[i] : nullptr;
-        }
-        copra_b200_vjp_out o{};
-        o.x0 = out->x0 ? out->x0 + lo * nx : nullptr;
-        o.p = out->p ? p.data() : nullptr;
-        o.f = out->f ? f.data() : nullptr;
-        o.lower = out->lower ? lower.data() : nullptr;
-        o.upper = out->upper ? upper.data() : nullptr;
+        VjpOutSlice os(*out, lo, nx, plen, clen);
+        const copra_b200_vjp_out& o = os.o;
         // the cost gradients likewise: rows, rows x nx and rows x nu per instance
         int nu = 0;
         std::vector<int> rows;
@@ -290,24 +326,64 @@ int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, 
         cb_vjp_lengths(m->h[g], nx, plen, clen);
         const long long lo = m->lo[g], k = in->ndir;
         // every array of the whole batch (len x k per instance), advanced to this shard's first instance
-        auto at = [&](const double* const* arr, size_t i, int len) -> const double* {
-            return (arr && arr[i]) ? arr[i] + lo * len * k : nullptr;
-        };
-        std::vector<const double*> p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size());
-        for (size_t i = 0; i < plen.size(); ++i) p[i] = at(in->p, i, plen[i]);
-        for (size_t i = 0; i < clen.size(); ++i) {
-            f[i] = at(in->f, i, clen[i]);
-            lower[i] = at(in->lower, i, clen[i]);
-            upper[i] = at(in->upper, i, clen[i]);
-        }
-        copra_b200_jvp_in t = *in;
-        t.x0 = in->x0 ? in->x0 + lo * nx * k : nullptr;
-        t.p = in->p ? p.data() : nullptr;
-        t.f = in->f ? f.data() : nullptr;
-        t.lower = in->lower ? lower.data() : nullptr;
-        t.upper = in->upper ? upper.data() : nullptr;
-        return copra_b200_lmpc_jvp(m->h[g], &t, COPRA_B200_HOST, dcontrol ? dcontrol + lo * sz.nU * k : nullptr,
+        JvpInSlice ts(*in, lo, nx, plen, clen);
+        return copra_b200_lmpc_jvp(m->h[g], &ts.t, COPRA_B200_HOST, dcontrol ? dcontrol + lo * sz.nU * k : nullptr,
             dtrajectory ? dtrajectory + lo * sz.X * k : nullptr);
+    });
+}
+
+int copra_b200_multi_lmpc_vjp_initial_state(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_initial_out* init)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    static const copra_b200_vjp_out none{};
+    if (!out) out = &none;
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp_initial_state needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        std::vector<int> plen, clen;
+        int nx = 0;
+        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const long long lo = m->lo[g];
+        VjpOutSlice os(*out, lo, nx, plen, clen);
+        copra_b200_vjp_initial_out io{};
+        if (init) {
+            io.R = init->R ? init->R + lo * nx * nx : nullptr;
+            io.r = init->r ? init->r + lo * nx : nullptr;
+            io.x0lb = init->x0lb ? init->x0lb + lo * nx : nullptr;
+            io.x0ub = init->x0ub ? init->x0ub + lo * nx : nullptr;
+        }
+        return copra_b200_lmpc_vjp_initial_state(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
+            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &os.o, init ? &io : nullptr);
+    });
+}
+
+int copra_b200_multi_lmpc_jvp_initial_state(copra_b200_multi* m, const copra_b200_jvp_in* in, const copra_b200_jvp_initial_in* init,
+    double* dcontrol, double* dtrajectory)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!in) return mfail(m, COPRA_B200_E_ARG, "lmpc_jvp_initial_state: null tangent description");
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_jvp_initial_state needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        std::vector<int> plen, clen;
+        int nx = 0;
+        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const long long lo = m->lo[g], k = in->ndir;
+        JvpInSlice ts(*in, lo, nx, plen, clen);
+        copra_b200_jvp_initial_in ti{};
+        if (init) {
+            ti.R = init->R ? init->R + lo * nx * nx * k : nullptr;
+            ti.r = init->r ? init->r + lo * nx * k : nullptr;
+            ti.x0lb = init->x0lb ? init->x0lb + lo * nx * k : nullptr;
+            ti.x0ub = init->x0ub ? init->x0ub + lo * nx * k : nullptr;
+        }
+        return copra_b200_lmpc_jvp_initial_state(m->h[g], &ts.t, init ? &ti : nullptr, COPRA_B200_HOST,
+            dcontrol ? dcontrol + lo * sz.nU * k : nullptr, dtrajectory ? dtrajectory + lo * sz.X * k : nullptr);
     });
 }
 

@@ -35,6 +35,13 @@
 //               Aeq / Aineq, and dc = -v, dQ = -(v x' + x v') / 2, dbeta_j = mu_j, da_j = -lambda_j v - mu_j x (k = 2 when the
 //               Aeq / Aineq gradients are wanted, lambda again from the forward solve as second right-hand side)
 //   k9_output  the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
+// Initial-state mode (copra_b200_lmpc_vjp_initial_state / _jvp_initial_state): the decision vector is z = [x0*; U] (n = nx + nU)
+// with the per-instance Hessian of the build, and x0 enters only as the default of a bound that was not given.  The same
+// kernels take the branch off = nx: a general row is [Y_row | EGx row] with b = z (no -Y x0 term), gbar = [Phi' dtraj;
+// dcontrol + Psi' dtraj], c = [r; sum f], so dr = c^[0:nx], dR = (c^_0 x0*' + x0* c^_0') / 2 (the top-left block of
+// -(v z' + z v') / 2), dp / df / the control bounds read c^[nx:] and the bound rows nx.., dx0lb / dx0ub are the multipliers of
+// the bound rows 0..nx-1 and dx0 their sum over the bounds that defaulted.  Forward: cdot = [rdot + sym(Rdot) x0*; sum fdot],
+// bdot of bound row k < nx is x0lbdot_k / x0ubdot_k (x0dot_k when that bound defaulted), dtraj = Phi zdot[0:nx] + Psi zdot[nx:].
 // Every sum runs in a fixed order.  Instances whose status is not 0 get zeros; a Hessian or Gram factorisation that failed
 // gives NaN instead of silently wrong results.
 #include "common.cuh"
@@ -82,6 +89,16 @@ __device__ __forceinline__ double general_row_entry(const BuildParams& P, int b,
     return v;
 }
 
+// entry col < nx of general row idx in initial-state mode: the row's Y = E Phi_i block, resident from the build (K3's
+// dev_fill_row copies the same values into Aeq / Aineq)
+__device__ __forceinline__ double initial_row_entry(const BuildParams& P, int b, int idx, int col)
+{
+    const bool iseq = idx < P.meq;
+    const int mtot = iseq ? P.meq : P.mineq;
+    const double* Y = (iseq ? P.Yeq : P.Yin) + (long long)b * mtot * P.nx;
+    return Y[(iseq ? idx : idx - P.meq) + (long long)col * mtot];
+}
+
 // zero the lds x (nm + k) slab of chunk instance lb (batch instance b) and write its active rows as the first nact columns:
 // row(idx, col) gives entry `col` of general row idx < mg, a bound row (upper rows first, then lower rows) is a unit vector.
 // The caller writes the k right-hand-side columns
@@ -122,9 +139,12 @@ __device__ __forceinline__ double active_beta(int idx, int meq, int mg, int n, c
 __global__ void __launch_bounds__(kSensThreads) k8_gather_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ VjpParams V)
 {
     const int lb = blockIdx.x, b = V.b0 + lb;
-    const int n = V.n, nu = P.nu, N = P.N, nx = P.nx, nm = V.nm, mg = P.meq + P.mineq;
+    const int n = V.n, nu = P.nu, N = P.N, nx = P.nx, nm = V.nm, mg = P.meq + P.mineq, X = P.X;
+    const int off = P.initial_state ? nx : 0;
     const long long NX = (long long)N * nx;
-    double* slab = sens_gather(V, lb, b, mg, [&](int idx, int col) { return general_row_entry(P, b, nu, idx, col); });
+    double* slab = sens_gather(V, lb, b, mg, [&](int idx, int col) {
+        return col < off ? initial_row_entry(P, b, idx, col) : general_row_entry(P, b, nu, idx, col - off);
+    });
     vjp_rhs(V, lb, b, [&](int idx) {
         return active_beta(idx, P.meq, mg, n, P.beq + (long long)b * P.meq, P.bineq + (long long)b * P.mineq,
             P.ub + (long long)b * P.nvar, P.lb + (long long)b * P.nvar);
@@ -132,12 +152,24 @@ __global__ void __launch_bounds__(kSensThreads) k8_gather_kernel(const __grid_co
     if (V.status[b] != 0) return;
     if (V.k == 2)
         for (int col = threadIdx.x; col < n; col += blockDim.x) slab[col + (long long)(nm + 1) * V.lds] = -P.c[(long long)b * P.nvar + col];
-    // gbar = dcontrol + Psi' dtraj, Psi' applied as the transposed block-Toeplitz product over the compact Gs
+    // gbar = dcontrol + Psi' dtraj, Psi' applied as the transposed block-Toeplitz product over the compact Gs; in initial-state
+    // mode the first nx entries are Phi' dtraj (x0* enters the trajectory through Phi)
     const double* Gs = P.Gs + (long long)b * NX * nu;
     for (int col = threadIdx.x; col < n; col += blockDim.x) {
-        double g = V.dcontrol ? V.dcontrol[(long long)b * V.sdc + col] : 0.0;
+        if (col < off) {
+            double g = 0.0;
+            if (V.dtraj) {
+                const double* Phi = P.Phi + (long long)b * X * nx + (long long)col * X;
+                const double* dt = V.dtraj + (long long)b * V.sdt;
+                for (int r = 0; r < X; ++r) g += Phi[r] * dt[r];
+            }
+            slab[col + (long long)nm * V.lds] = g;
+            continue;
+        }
+        const int cu = col - off;
+        double g = V.dcontrol ? V.dcontrol[(long long)b * V.sdc + cu] : 0.0;
         if (V.dtraj) {
-            const int j = col / nu, bb = col % nu;
+            const int j = cu / nu, bb = cu % nu;
             const double* dt = V.dtraj + (long long)b * V.sdt;
             double s = 0.0;
             for (int i = j + 1; i <= N; ++i) {
@@ -160,16 +192,33 @@ __device__ __forceinline__ double x0_tangent(const JvpParams& J, int b, int nx, 
 __global__ void __launch_bounds__(kSensThreads) k9_tangent_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ JvpParams J)
 {
     const int lb = blockIdx.x, b = J.b0 + lb;
-    const int n = J.n, nu = P.nu, nx = P.nx, mg = P.meq + P.mineq, nm = J.nm, k = J.k;
-    double* slab = sens_gather(J, lb, b, mg, [&](int idx, int col) { return general_row_entry(P, b, nu, idx, col); });
+    const int n = J.n, nu = P.nu, nx = P.nx, nU = P.nU, mg = P.meq + P.mineq, nm = J.nm, k = J.k;
+    const int off = P.initial_state ? nx : 0;
+    double* slab = sens_gather(J, lb, b, mg, [&](int idx, int col) {
+        return col < off ? initial_row_entry(P, b, idx, col) : general_row_entry(P, b, nu, idx, col - off);
+    });
     if (J.status[b] != 0) return;
     const int na = J.nact[b];
     const int* iact = J.iact + (long long)b * n;
-    const bool has_x0 = J.gain || J.tx0;
+    const bool has_x0 = !off && (J.gain || J.tx0); // initial-state mode: x0 moves only the bounds that defaulted to it
     // -cdot_d: cdot[col] = sum_costs (sum_s E[s, col] x0dot[s] + fdot[col]),  fdot[(j, bb)] = -sum_{i >= j} sum_l
-    // w[l] pdot_i[l] MGx[l, bb, i - j]  (the tangent of dev_ef's f through res_i = M xi_i - p_i)
+    // w[l] pdot_i[l] MGx[l, bb, i - j]  (the tangent of dev_ef's f through res_i = M xi_i - p_i); in initial-state mode
+    // cdot[s < nx] = rdot[s] + sum_a (Rdot[s, a] + Rdot[a, s]) / 2 x0*[a]
     for (int t = threadIdx.x; t < n * k; t += blockDim.x) {
-        const int col = t % n, d = t / n;
+        const int cl = t % n, d = t / n;
+        if (cl < off) {
+            double c = J.tr ? J.tr[((long long)b * k + d) * nx + cl] : 0.0;
+            if (J.tR) {
+                const double* Rd = J.tR + ((long long)b * k + d) * nx * nx;
+                const double* xs = J.x + (long long)b * n;
+                double s = 0.0;
+                for (int a = 0; a < nx; ++a) s += 0.5 * (Rd[cl + a * nx] + Rd[a + cl * nx]) * xs[a];
+                c += s;
+            }
+            slab[cl + (long long)(nm + d) * J.lds] = -c;
+            continue;
+        }
+        const int col = cl - off;
         const int j = col / nu, bb = col % nu;
         double c = 0.0;
         for (int ci = 0; ci < P.ncost; ++ci) {
@@ -188,9 +237,10 @@ __global__ void __launch_bounds__(kSensThreads) k9_tangent_kernel(const __grid_c
                 for (int l = 0; l < r; ++l) fd += w[l] * pd[i * F.pstep + l] * MG[l + r * (bb + nu * (i - j))];
             c -= fd;
         }
-        slab[col + (long long)(nm + d) * J.lds] = -c;
+        slab[cl + (long long)(nm + d) * J.lds] = -c;
     }
-    // bdot_act (nm x k): an Aeq / Aineq row's fdot at its (step, line) minus Y_row x0dot; a bound row's lbdot / ubdot
+    // bdot_act (nm x k): an Aeq / Aineq row's fdot at its (step, line) minus Y_row x0dot (LMPC mode); a bound row's lbdot /
+    // ubdot, in initial-state mode x0lbdot / x0ubdot for the rows k < nx (x0dot where that bound defaulted to x0)
     for (int t = threadIdx.x; t < nm * k; t += blockDim.x) {
         const int a = t % nm, d = t / nm;
         double v = 0.0;
@@ -211,8 +261,15 @@ __global__ void __launch_bounds__(kSensThreads) k9_tangent_kernel(const __grid_c
                 }
             } else {
                 const int var = (idx - mg) % n;
-                const double* src = (idx - mg) < n ? J.tupper : J.tlower; // upper rows first, then lower rows
-                if (src) v = src[((long long)b * k + d) * J.cblen + (J.cblen == n ? var : var % nu)];
+                const bool up = (idx - mg) < n; // upper rows first, then lower rows
+                if (var < off) {
+                    const double* src = up ? (P.x0ub.p ? J.tx0ub : J.tx0) : (P.x0lb.p ? J.tx0lb : J.tx0);
+                    if (src) v = src[((long long)b * k + d) * nx + var];
+                } else {
+                    const int vu = var - off;
+                    const double* src = up ? J.tupper : J.tlower;
+                    if (src) v = src[((long long)b * k + d) * J.cblen + (J.cblen == nU ? vu : vu % nu)];
+                }
             }
         }
         J.rhs[(long long)lb * nm * k + t] = v;
@@ -327,6 +384,7 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
     const int lb = blockIdx.x, b = V.b0 + lb;
     if (V.status[b] != 0) return; // gradients stay at the zeros they were initialised to
     const int n = V.n, nx = P.nx, nu = P.nu, N = P.N, X = P.X, meq = P.meq, mineq = P.mineq, mg = meq + mineq, nm = V.nm;
+    const int nU = P.nU, off = P.initial_state ? nx : 0;
     const int na = V.nact[b];
     const int tid = threadIdx.x, T = blockDim.x;
     double* ch = sens_sm;          // n    c^ = -v
@@ -338,8 +396,26 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
     const int* iact = V.iact + (long long)b * n;
     for (int k = tid; k < na; k += T) bh[iact[k] - 1] = V.rhs[(long long)lb * nm * V.k + k]; // mu, from sens_solve
     __syncthreads();
-    // dx0 = sum_costs E c^ - Yeq' b^eq - Yin' b^in + Phi' dtraj
-    if (V.dx0) {
+    if (off) {
+        // initial-state mode: c[0:nx] = r, Q_tl = R + E Qb^-1 E', the bound rows 0..nx-1 are [x0lb, x0ub] (x0 where not given)
+        const double* ubh = bh + mg;
+        const double* lbh = bh + mg + n;
+        const double* xs = V.U + (long long)b * n; // x0* = the solution's first nx entries
+        for (int s = tid; s < nx; s += T) {
+            if (V.dr) V.dr[(long long)b * nx + s] = ch[s];
+            if (V.dx0lb) V.dx0lb[(long long)b * nx + s] = lbh[s];
+            if (V.dx0ub) V.dx0ub[(long long)b * nx + s] = ubh[s];
+            if (V.dx0) V.dx0[(long long)b * nx + s] = (P.x0lb.p ? 0.0 : lbh[s]) + (P.x0ub.p ? 0.0 : ubh[s]);
+        }
+        if (V.dR)
+            for (int q = tid; q < nx * nx; q += T) {
+                const int s = q % nx, u = q / nx;
+                // no contraction, so that dR is exactly symmetric
+                V.dR[(long long)b * nx * nx + q] = 0.5 * __dadd_rn(__dmul_rn(ch[s], xs[u]), __dmul_rn(xs[s], ch[u]));
+            }
+    }
+    // dx0 = sum_costs E c^ - Yeq' b^eq - Yin' b^in + Phi' dtraj (LMPC mode)
+    if (V.dx0 && !off) {
         const double* Yeq = P.Yeq + (long long)b * meq * nx;
         const double* Yin = P.Yin + (long long)b * mineq * nx;
         const double* Phi = P.Phi + (long long)b * X * nx;
@@ -359,6 +435,7 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
         }
     }
     // dp_i = -W T_i c^ with T_i[l, (j, bb)] = MGx[l, bb, i - j] (j <= i); a step-size p receives the sum over its steps
+    const double* cu = ch + off; // c^ of U
     for (int ci = 0; ci < P.ncost; ++ci) {
         double* out = V.dp[ci];
         if (!out) continue;
@@ -372,7 +449,7 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
             const int l = t % r, i = F.i0 + t / r;
             double acc = 0.0;
             for (int j = 0; j <= min(i, N - 1); ++j)
-                for (int bb = 0; bb < nu; ++bb) acc += MG[l + r * (bb + nu * (i - j))] * ch[j * nu + bb];
+                for (int bb = 0; bb < nu; ++bb) acc += MG[l + r * (bb + nu * (i - j))] * cu[j * nu + bb];
             const double v = -w[l] * acc;
             if (F.pstep) out[(long long)i * F.pstep + l] = v;
             else tmp[t] = v;
@@ -406,18 +483,18 @@ __global__ void __launch_bounds__(kSensThreads) k8_adjoint_kernel(const __grid_c
             }
         }
     }
-    // control bounds: lb[k] = lower[cb_full ? k : k % nu] (dev_finalize)
+    // control bounds: lb[off + k] = lower[cb_full ? k : k % nu] (dev_finalize)
     for (int side = 0; side < 2; ++side) {
         double* out = side == 0 ? V.dlower : V.dupper;
         if (!out) continue;
-        const double* g = bh + mg + (side == 0 ? n : 0);
+        const double* g = bh + mg + (side == 0 ? n : 0) + off;
         out += (long long)b * V.cblen;
-        if (V.cblen == n)
-            for (int k = tid; k < n; k += T) out[k] = g[k];
+        if (V.cblen == nU)
+            for (int k = tid; k < nU; k += T) out[k] = g[k];
         else
             for (int e = tid; e < nu; e += T) {
                 double acc = 0.0;
-                for (int k = e; k < n; k += nu) acc += g[k];
+                for (int k = e; k < nU; k += nu) acc += g[k];
                 out[e] = acc;
             }
     }
@@ -761,13 +838,15 @@ __global__ void __launch_bounds__(kSensThreads) qp_grad_kernel(const __grid_cons
 }
 
 // dcontrol = the first ru rows of Udot; dtraj = the first rx rows of Phi x0dot + Psi Udot, Psi applied as the block-Toeplitz
-// product over the compact Gs (K7 without xi).  Zeros for an instance whose status is not 0.
+// product over the compact Gs (K7 without xi).  In initial-state mode Udot = zdot[nx:] and x0dot = zdot[0:nx].  Zeros for an
+// instance whose status is not 0.
 __global__ void __launch_bounds__(kSensThreads) k9_output_kernel(const __grid_constant__ BuildParams P, const __grid_constant__ JvpParams J)
 {
     const int lb = blockIdx.x, b = J.b0 + lb, k = J.k;
-    const int nx = P.nx, nu = P.nu, X = P.X, NX = P.N * P.nx;
+    const int nx = P.nx, nu = P.nu, X = P.X, NX = P.N * P.nx, off = P.initial_state ? nx : 0;
     const bool live = J.status[b] == 0;
-    const double* Ud = J.V + (long long)lb * J.lds * k;
+    const double* Zd = J.V + (long long)lb * J.lds * k;
+    const double* Ud = Zd + off;
     if (J.dcontrol) {
         double* out = J.dcontrol + (long long)b * J.ru * k;
         for (int t = threadIdx.x; t < J.ru * k; t += blockDim.x) {
@@ -785,8 +864,9 @@ __global__ void __launch_bounds__(kSensThreads) k9_output_kernel(const __grid_co
         double v = 0.0;
         if (live) {
             const double* u = Ud + (long long)d * J.lds;
+            const double* z = Zd + (long long)d * J.lds;
             double s1 = 0.0;
-            for (int a = 0; a < nx; ++a) s1 += Phi[row + (long long)a * X] * x0_tangent(J, b, nx, d, a);
+            for (int a = 0; a < nx; ++a) s1 += Phi[row + (long long)a * X] * (off ? z[a] : x0_tangent(J, b, nx, d, a));
             double s2 = 0.0;
             int go = (i - 1) * nx + r; // G_{i-1-j}[r, :]
             for (int j = 0; j < i; ++j, go -= nx)

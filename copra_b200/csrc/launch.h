@@ -66,7 +66,7 @@ int k7_results_launch(const BuildParams& P, const double* x, double* control, do
 // the chunk of instances [b0, b0 + nb).  Buffers marked "chunk" hold nb instances; the others are indexed by the instance
 // number in the batch.  SensChunk is what the VJP and the JVP share; per-instance vectors are len x k column-major.
 struct SensChunk {
-    int n;                           // decision variables (nU: LMPC mode)
+    int n;                           // decision variables (nU: LMPC mode, nx + nU: initial-state mode)
     int nm;                          // the largest active-set size of the chunk (the padded width of slab, Y and G)
     int k;                           // right-hand sides: 1 for the VJP (2 with model gradients), the tangent directions for the JVP
     int lds, ldy, ldg;               // leading dimensions of slab / W / V, Y, J_G
@@ -118,6 +118,12 @@ struct VjpParams : SensChunk {
     double* dd;                      // nx per instance
     double* dE[kMaxFam];             // per row family (not the trajectory-bound selectors): rows x nx per instance, column-major
     double* dG[kMaxFam];             // rows x nu per instance, column-major
+    // initial-state mode (k8_adjoint; whole batch, zeroed by the caller; null = not wanted; dR needs U).  dx0 is then the sum
+    // of the multipliers of the x0 bounds that defaulted to x0
+    double* dR;                      // nx x nx per instance, column-major
+    double* dr;                      // nx
+    double* dx0lb;                   // nx
+    double* dx0ub;                   // nx
 };
 int k8_gather_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 int k8_adjoint_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
@@ -126,6 +132,8 @@ size_t k8_cost_grad_smem(const BuildParams& P);
 int k8_cost_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 // the same for k8_model_grad
 size_t k8_model_grad_smem(const BuildParams& P);
+// shared memory of k8_adjoint for the resident build
+size_t k8_adjoint_smem(const BuildParams& P);
 int k8_model_grad_launch(const BuildParams& P, const VjpParams& V, int nb, cudaStream_t st);
 
 // K8 for a raw QP batch (copra_b200_qp_vjp): the same KKT core with the active rows read from the caller's dense Aeq / Aineq
@@ -151,6 +159,13 @@ struct JvpParams : SensChunk {
     const double* tf[kMaxFam];
     const double* tlower;            // control bound
     const double* tupper;
+    // initial-state mode: tangents of R (nx x nx, column-major, used through its symmetric part), r, x0lb and x0ub, and the
+    // solution z = [x0*; U] (n per instance; needed with tR).  tx0 moves the x0 bounds that were not given
+    const double* tR;
+    const double* tr;
+    const double* tx0lb;
+    const double* tx0ub;
+    const double* x;
     // outputs (whole batch, every entry written; null = not wanted)
     double* dcontrol;                // ru x k per instance: the first ru rows of Udot
     int ru;

@@ -1243,6 +1243,30 @@ public:
         if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
         b200::check(rc);
     }
+    // Sensitivities of the last solve of an initial-state controller (copra_b200_lmpc_vjp_initial_state): the vector-Jacobian
+    // product with respect to x0 (through the x0 bounds that default to it) and every entry's vectors (`out`), and to R, r,
+    // x0lb and x0ub (`init`: nx x nx, nx, nx, nx per instance; null = not wanted), batch-major HOST arrays.
+    // std::runtime_error on an LMPC-mode controller or when another controller has built on the engine since this solve;
+    // std::domain_error for full-size entries other than the control bound and for a gradient of an R, r, x0lb or x0ub the
+    // controller was not given.
+    void initialStateVjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out,
+        const copra_b200_vjp_initial_out& init)
+    {
+        initialStateGuard("initialStateVjp");
+        const int rc = multi_ ? copra_b200_multi_lmpc_vjp_initial_state(multi_, dcontrol, dtrajectory, &out, &init)
+                              : copra_b200_lmpc_vjp_initial_state(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, &init);
+        initialStateCheck(rc);
+    }
+    // Forward mode of the same (copra_b200_lmpc_jvp_initial_state): dU (nU x k per instance) and dtrajectory (X x k) along the
+    // in.ndir tangent directions of `in` and `init` (R: nx x nx x k, r / x0lb / x0ub: nx x k per instance; null = zero).
+    // Errors as initialStateVjp, plus std::domain_error for in.ndir < 1.
+    void initialStateJvp(const copra_b200_jvp_in& in, const copra_b200_jvp_initial_in& init, double* dcontrol, double* dtrajectory)
+    {
+        initialStateGuard("initialStateJvp");
+        const int rc = multi_ ? copra_b200_multi_lmpc_jvp_initial_state(multi_, &in, &init, dcontrol, dtrajectory)
+                              : copra_b200_lmpc_jvp_initial_state(b200::handle(), &in, &init, COPRA_B200_HOST, dcontrol, dtrajectory);
+        initialStateCheck(rc);
+    }
     const std::vector<double>& controls() const { return controls_; }         // nU x batch, column-major
     const std::vector<double>& trajectories() const { return trajectories_; } // X x batch
     const std::vector<int>& status() const { return status_; }
@@ -1275,6 +1299,19 @@ private:
         const int rc = copra_b200_lmpc_vjp_model(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, costs, model);
         if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
         b200::check(rc);
+    }
+    void initialStateGuard(const char* name) const
+    {
+        if (!p_.initial_state) throw std::runtime_error(std::string("BatchedLMPC::") + name + " needs an initial-state controller; use vjp / jvp");
+        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR(std::string("BatchedLMPC::") + name + " takes HOST arrays");
+        if (multi_ ? !multiBuilt_ : myEpoch_ != b200::buildEpoch())
+            throw std::runtime_error(std::string("BatchedLMPC::") + name + ": no solve of this controller is resident on the engine");
+    }
+    void initialStateCheck(int rc) const
+    {
+        const char* msg = multi_ ? copra_b200_multi_last_error(multi_) : copra_b200_last_error(b200::handle());
+        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(msg);
+        if (rc) throw std::runtime_error(msg);
     }
     copra_b200_problem p_{};
     std::vector<copra_b200_cost> costs_;

@@ -358,6 +358,47 @@ int copra_b200_lmpc_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int m
  * (nx*(steps+1)) x nx, both column-major; either may be NULL.  A loop running faster than the MPC applies
  * u0 + Ku (x - x0) with steps = 1.  E_ARG for steps outside [1, N]; otherwise as copra_b200_lmpc_jvp. */
 int copra_b200_lmpc_feedback_gain(copra_b200_handle* h, int steps, double* Ku, double* Kx, int memory);
+/* Sensitivities of the last solve of an initial-state build (copra::InitialStateLMPC, decision vector z = [x0*; U]): the
+ * vector-Jacobian product of (control, trajectory) with respect to the vectors of copra_b200_lmpc_vjp and to R, r, x0lb and
+ * x0ub.  The trajectory is Phi x0* + Psi U + xi with the optimised x0* (its first nx entries are x0*).  On the final active
+ * set, with gbar = [Phi' dL/dtrajectory; dL/dcontrol + Psi' dL/dtrajectory], [Q A'; A 0] [v; mu] = [gbar; 0] and c^ = -v:
+ *   dL/dr = c^[0:nx],  dL/dR = (c^_0 x0*' + x0* c^_0') / 2 with c^_0 = c^[0:nx] (R is read through its symmetric part),
+ *   dL/dx0lb / dL/dx0ub = mu of the bound rows 0..nx-1, and p, f, lower and upper as copra_b200_lmpc_vjp on c^[nx:] and
+ *   the multipliers of the general rows (b = z: no x0 term) and of the control bound rows nx...
+ * x0 enters an initial-state build only as the default of an x0 bound that was not given (x0lb = x0ub = x0), so
+ * out->x0 receives the sum of the multipliers of those bounds: zeros when both x0lb and x0ub were given.
+ * `out` and `init` may be NULL; NULL pointers mark gradients that are not wanted.  Gradients are per instance even for
+ * inputs given with stride 0.  Instances whose status is not 0 get zeros; a Hessian (with the default R = 0 it is only
+ * semidefinite) or Gram factor that is not positive definite gives NaN.  E_STATE without a solve of the resident build
+ * (or after a raw QP batch); E_UNSUPPORTED for an LMPC-mode build (use copra_b200_lmpc_vjp), for a full-size cost, row
+ * constraint or trajectory bound (a full-size control bound is fine) and for a problem needing more shared memory per
+ * block than the device allows; E_ARG for a gradient of R, r, x0lb or x0ub the build was not given (a NULL array, the
+ * reference default).  Gradients with respect to w, M, N, A, B, d, E and G are not available in initial-state mode.
+ * Leaves the resident build, the factor caches and the warm-start seed untouched. */
+typedef struct {
+    double* R;      /* nx x nx per instance, column-major (symmetric) */
+    double* r;      /* nx per instance */
+    double* x0lb;   /* nx per instance */
+    double* x0ub;   /* nx per instance */
+} copra_b200_vjp_initial_out;
+int copra_b200_lmpc_vjp_initial_state(copra_b200_handle* h, const double* dcontrol, const double* dtrajectory, int memory,
+    const copra_b200_vjp_out* out /* x0, p, f, lower, upper; may be NULL */, const copra_b200_vjp_initial_out* init /* may be NULL */);
+/* Forward mode of the same: the Jacobian-vector product of (control, trajectory) of the last solve of an initial-state
+ * build along in->ndir = k tangent directions of the vectors of copra_b200_jvp_in and of R, r, x0lb and x0ub (nx x nx x k
+ * and nx x k per instance; NULL = zero).  cdot = [rdot + sym(Rdot) x0*; sum_costs fdot(pdot)], the bound rows 0..nx-1 move
+ * with x0lbdot / x0ubdot, or with in->x0 where that bound defaulted to x0; dtrajectory = Phi zdot[0:nx] + Psi zdot[nx:].
+ * Rdot enters through its symmetric part, so this is the exact adjoint of copra_b200_lmpc_vjp_initial_state.
+ * `dcontrol` receives nU x k doubles per instance, `dtrajectory` X x k; either may be NULL.  Errors as
+ * copra_b200_lmpc_vjp_initial_state (E_ARG for a tangent of R, r, x0lb or x0ub the build was not given), plus E_ARG for a
+ * NULL `in` or ndir < 1. */
+typedef struct {
+    const double* R;     /* nx x nx x k per instance */
+    const double* r;     /* nx x k per instance */
+    const double* x0lb;  /* nx x k per instance */
+    const double* x0ub;  /* nx x k per instance */
+} copra_b200_jvp_initial_in;
+int copra_b200_lmpc_jvp_initial_state(copra_b200_handle* h, const copra_b200_jvp_in* in, const copra_b200_jvp_initial_in* init /* may be NULL */,
+    int memory, double* dcontrol, double* dtrajectory);
 /* SolverInterface::SI_warmStart(bool) / SI_warmStart() (include/SolverInterface.h:42-45; QuadProg has none, the reference
  * prints "No warmStart() function for this qp").  Opt-in: with it on, copra_b200_lmpc_resolve seeds every instance with the
  * inequality / bound rows that were active at its previous solve on the resident build, solves that equality-constrained
@@ -414,6 +455,12 @@ int copra_b200_multi_lmpc_vjp_model(copra_b200_multi* m, const double* dcontrol,
 /* copra_b200_lmpc_jvp / copra_b200_lmpc_feedback_gain on every shard of the last run; HOST arrays holding the whole batch */
 int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory);
 int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx);
+/* copra_b200_lmpc_vjp_initial_state / copra_b200_lmpc_jvp_initial_state on every shard of the last run; HOST arrays holding
+ * the whole batch */
+int copra_b200_multi_lmpc_vjp_initial_state(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_initial_out* init);
+int copra_b200_multi_lmpc_jvp_initial_state(copra_b200_multi* m, const copra_b200_jvp_in* in, const copra_b200_jvp_initial_in* init,
+    double* dcontrol, double* dtrajectory);
 /* copra_b200_set_warm_start on every shard's handle */
 int copra_b200_multi_set_warm_start(copra_b200_multi* m, int on);
 
