@@ -75,6 +75,13 @@ cudaError_t gt_psit_fill_launch(const double* Gs, double* PsiT, int nx, int nu, 
 
 int gt_cluster_capacity(const GtPlan& plan, int csize); // k6_thin_cluster.cu
 
+// Global workspace per CTA: Q1 (or P, ld x n) then S (n x n).  The kernels read Q1 with 128-bit loads, so every CTA's slice
+// starts on a 16-byte boundary: for odd n, ld n + n n is odd and is rounded up.
+static long long gt_ws_stride(const GtShape& sh)
+{
+    return ((long long)sh.ld * sh.n + (long long)sh.n * sh.n + 1) & ~1LL;
+}
+
 GtPlan gt_plan(const GtShape& sh, int batch, int sms, size_t smem_optin)
 {
     GtPlan p{};
@@ -90,7 +97,7 @@ GtPlan gt_plan(const GtShape& sh, int batch, int sms, size_t smem_optin)
         p.q1s = 0;
         p.per_sm = 1;
         p.smem_bytes = base;
-        p.ws_stride = (long long)sh.ld * sh.n + (long long)sh.n * sh.n;
+        p.ws_stride = gt_ws_stride(sh);
         const int cap = gt_cluster_capacity(p, sh.cluster);
         if (cap <= 0) { p.ok = 0; return p; }
         p.grid = std::max(1, std::min(batch, cap)) * sh.cluster;
@@ -107,7 +114,7 @@ GtPlan gt_plan(const GtShape& sh, int batch, int sms, size_t smem_optin)
     p.smem_bytes = gt_layout(sh.n, sh.meq, sh.m, sh.tab_doubles, p.threads, q1s, sh.ss_doubles).bytes;
     p.per_sm = per_sm;
     p.grid = std::max(1, std::min(batch, sms * per_sm));
-    p.ws_stride = (long long)sh.ld * sh.n + (long long)sh.n * sh.n; // Q1 (or P), S
+    p.ws_stride = gt_ws_stride(sh);
     return p;
 }
 
