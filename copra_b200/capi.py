@@ -78,6 +78,10 @@ class QpVjpOut(C.Structure):
     _fields_ = [(k, C.c_void_p) for k in ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")]
 
 
+class QpJvpIn(C.Structure):
+    _fields_ = [("ndir", C.c_int)] + [(k, Array) for k in ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")]
+
+
 class JvpIn(C.Structure):
     _fields_ = [("ndir", C.c_int), ("x0", C.c_void_p), ("p", C.POINTER(C.c_void_p)), ("f", C.POINTER(C.c_void_p)),
                 ("lower", C.POINTER(C.c_void_p)), ("upper", C.POINTER(C.c_void_p))]
@@ -110,13 +114,15 @@ EXPORTS = ["copra_b200_abi_version", "copra_b200_device_count", "copra_b200_crea
            "copra_b200_multi_lmpc_jvp", "copra_b200_multi_lmpc_feedback_gain", "copra_b200_lmpc_vjp_costs",
            "copra_b200_multi_lmpc_vjp_costs", "copra_b200_lmpc_vjp_model", "copra_b200_multi_lmpc_vjp_model",
            "copra_b200_qp_vjp", "copra_b200_lmpc_vjp_initial_state", "copra_b200_lmpc_jvp_initial_state",
-           "copra_b200_multi_lmpc_vjp_initial_state", "copra_b200_multi_lmpc_jvp_initial_state"]
+           "copra_b200_multi_lmpc_vjp_initial_state", "copra_b200_multi_lmpc_jvp_initial_state", "copra_b200_qp_jvp",
+           "copra_b200_qp_jacobian"]
 VJP_WANT = ("x0", "p", "f", "lower", "upper")
 VJP_COST_WANT = ("w", "M", "N")  # gradients with respect to the cost weights and matrices: requested by name only
 VJP_MODEL_WANT = ("A", "B", "d", "E", "G")  # ... and to the dynamics and the row constraints' matrices: by name only
 QP_VJP_WANT = ("Q", "c", "Aeq", "beq", "Aineq", "bineq", "lb", "ub")  # gradients of a raw QP batch (copra_b200_qp_vjp)
 INITIAL_KEYS = ("R", "r", "x0lb", "x0ub")  # initial-state builds: the x0 cost and box (copra_b200_lmpc_vjp_initial_state)
 QP_BASE_NDIM = dict(Q=2, c=1, Aeq=2, beq=1, Aineq=2, bineq=1, lb=1, ub=1)
+QP_WRT = dict(c=0, beq=1, bineq=2, lb=3, ub=4)  # COPRA_B200_QP_WRT_*: the inputs copra_b200_qp_jacobian differentiates by
 
 _lib = None
 
@@ -192,6 +198,8 @@ def load():
         lib.copra_b200_multi_lmpc_vjp_model.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(VjpOut),
                                                         C.POINTER(VjpCostOut), C.POINTER(VjpModelOut)]
         lib.copra_b200_qp_vjp.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(QpVjpOut)]
+        lib.copra_b200_qp_jvp.argtypes = [C.c_void_p, C.POINTER(QpJvpIn), C.c_int, C.c_void_p]
+        lib.copra_b200_qp_jacobian.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int]
         lib.copra_b200_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_int, C.c_void_p, C.c_void_p]
         lib.copra_b200_lmpc_feedback_gain.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]
         lib.copra_b200_multi_lmpc_jvp.argtypes = [C.c_void_p, C.POINTER(JvpIn), C.c_void_p, C.c_void_p]
@@ -794,6 +802,98 @@ class Engine:
         self._check(self.lib.copra_b200_qp_vjp(self.h, d.ctypes.data, HOST, C.byref(o)))
         return {k: None if a is None else (np.ascontiguousarray(a.transpose(0, 2, 1)) if a.ndim == 3 else a)
                 for k, a in raw.items()}
+
+    def _qp_tangents(self, tangents):
+        """check raw-QP tangents against the last batch's shapes: each is (batch, k, *base) or (k, *base) (one tangent for the
+        batch), every given one with the same k.  Returns (k, {name: (array, shared)}, device or None)"""
+        if getattr(self, "_last_qp", None) is None:
+            raise CopraB200Error(-5, "qp_jvp needs a previous solve_qp_batch on this engine")
+        q = self._last_qp
+        n, meq, m, B = q["n"], q["meq"], q["m"], q["batch"]
+        base = dict(Q=(n, n), c=(n,), Aeq=(meq, n), beq=(meq,), Aineq=(m, n), bineq=(m,), lb=(n,), ub=(n,))
+        given = {k: a for k, a in tangents.items() if a is not None}
+        if not given:
+            raise CopraB200Error(-1, "qp_jvp: no tangent given")
+        dev = next((a.device for a in given.values() if hasattr(a, "data_ptr")), None)
+        ks, out = set(), {}
+        for name, a in given.items():
+            if dev is not None:
+                import torch
+                a = torch.as_tensor(a, dtype=torch.float64, device=dev)
+            else:
+                a = np.asarray(a, dtype=np.float64)
+            shape, b = tuple(a.shape), base[name]
+            if len(shape) == len(b) + 2 and shape[0] == B and shape[2:] == b:
+                shared = False
+            elif len(shape) == len(b) + 1 and shape[1:] == b:
+                shared = True
+            else:
+                raise CopraB200Error(-1, "qp_jvp: the %s tangent has shape %s, expected (%d, k) + %s or (k,) + %s"
+                                     % (name, shape, B, b, b))
+            if 0 in b:
+                raise CopraB200Error(-1, "qp_jvp: a %s tangent for a batch without those rows" % name)
+            ks.add(shape[0] if shared else shape[1])
+            out[name] = (a, shared)
+        if len(ks) != 1 or min(ks) < 1:
+            raise CopraB200Error(-1, "qp_jvp: the tangents disagree on the number of directions k (%s)" % sorted(ks))
+        return ks.pop(), out, dev
+
+    def qp_jvp(self, Q=None, c=None, Aeq=None, beq=None, Aineq=None, bineq=None, lb=None, ub=None):
+        """Jacobian-vector products of the last raw QP batch (copra_b200_qp_jvp) along k tangent directions: each tangent is
+        (batch, k, *shape of the input) or (k, *shape) for one tangent shared by the batch, numpy arrays or CUDA float64
+        tensors; None is a zero tangent.  Returns xdot (batch, k, n) of the same kind.  Q is read through its symmetric part.
+        Instances whose status is not 0 get zeros."""
+        k, ts, dev = self._qp_tangents(dict(Q=Q, c=c, Aeq=Aeq, beq=beq, Aineq=Aineq, bineq=bineq, lb=lb, ub=ub))
+        q = self._last_qp
+        n, B = q["n"], q["batch"]
+        t = QpJvpIn()
+        t.ndir = k
+        keep = []
+        for name, (a, shared) in ts.items():
+            o = getattr(t, name)
+            if QP_BASE_NDIM[name] == 2:  # each direction column-major
+                a = a.transpose(-1, -2) if dev is not None else np.swapaxes(a, -1, -2)
+            buf = a.contiguous() if dev is not None else np.ascontiguousarray(a)
+            keep.append(buf)
+            o.ptr = buf.data_ptr() if dev is not None else buf.ctypes.data
+            o.stride = 0 if shared else (buf[0].numel() if dev is not None else buf[0].size)
+        if dev is not None:
+            import torch
+            dx = torch.empty((B, k, n), dtype=torch.float64, device=dev)
+            torch.cuda.synchronize(dev)
+            try:
+                self._check(self.lib.copra_b200_qp_jvp(self.h, C.byref(t), DEVICE, dx.data_ptr()))
+            finally:
+                self.synchronize()
+            return dx
+        dx = np.zeros((B, k, n))
+        self._check(self.lib.copra_b200_qp_jvp(self.h, C.byref(t), HOST, dx.ctypes.data))
+        return dx
+
+    def qp_jacobian(self, wrt, device=None):
+        """The Jacobian of the last raw QP batch's solutions with respect to one vector input (copra_b200_qp_jacobian): wrt in
+        "c", "beq", "bineq", "lb", "ub".  Returns (batch, n, len) -- numpy, or a CUDA tensor on `device`.  dx/dc is symmetric;
+        the columns of inactive rows are exactly zero."""
+        if getattr(self, "_last_qp", None) is None:
+            raise CopraB200Error(-5, "qp_jacobian needs a previous solve_qp_batch on this engine")
+        if wrt not in QP_WRT:
+            raise CopraB200Error(-1, "qp_jacobian: wrt must be one of %s, got %r" % (sorted(QP_WRT), wrt))
+        q = self._last_qp
+        n, B = q["n"], q["batch"]
+        ln = dict(c=n, beq=q["meq"], bineq=q["m"], lb=n, ub=n)[wrt]
+        # the engine writes each instance's n x len Jacobian column-major: allocated as (batch, len, n)
+        if device is not None:
+            import torch
+            J = torch.empty((B, ln, n), dtype=torch.float64, device=device)
+            torch.cuda.synchronize(device)
+            try:
+                self._check(self.lib.copra_b200_qp_jacobian(self.h, QP_WRT[wrt], J.data_ptr() if J.numel() else None, DEVICE))
+            finally:
+                self.synchronize()
+            return J.transpose(1, 2).contiguous()
+        J = np.zeros((B, ln, n))
+        self._check(self.lib.copra_b200_qp_jacobian(self.h, QP_WRT[wrt], J.ctypes.data if J.size else None, HOST))
+        return np.ascontiguousarray(J.transpose(0, 2, 1))
 
     # ---- K1..K7 ----
     def sizes(self, hb):

@@ -1358,10 +1358,38 @@ int do_jvp(copra_b200_handle* h, const copra_b200_jvp_in* in, int k, bool gain, 
     return 0;
 }
 
-// K8 for the last raw QP batch (copra_b200_qp_vjp): the same KKT core, fed by qp_gather and finished by qp_grad.  Its factor
-// of Q has workspace of its own, so the resident LMPC build's factors survive: one factorisation for a stride-0 Q, else one
-// per chunk (counted in the chunk's bytes instead of 2 ld n doubles for the whole batch).  With dAeq / dAineq the forward
-// solve is the second right-hand side (k = 2) and its multipliers lambda enter.
+// The factor source of the last raw QP batch for sens_run: R^-1 of its Q in workspace of its own (`prefix`_Jt, _JtT, _pd), so
+// the resident LMPC build's factors survive: one factorisation for a stride-0 Q (at the first chunk), else one per chunk
+// (counted in the chunk's bytes instead of 2 ld n doubles for the whole batch)
+int qp_factor(copra_b200_handle* h, const std::string& prefix, int b0, int nb, SensFactor& F)
+{
+    const GiBatch& G = h->qp;
+    const size_t n = G.n;
+    const int ldj = gt_even(G.n);
+    const bool shared_q = G.Q.s == 0;
+    double *J = nullptr, *JT = nullptr;
+    int* pd = nullptr;
+    const size_t count = shared_q ? 1 : size_t(nb); // the first chunk is the largest: later ones reuse its workspace
+    int rc;
+    if ((rc = ws(h, (prefix + "_Jt").c_str(), count * ldj * n, &J))) return rc;
+    if ((rc = ws(h, (prefix + "_JtT").c_str(), count * ldj * n, &JT))) return rc;
+    if ((rc = ws(h, (prefix + "_pd").c_str(), shared_q ? 1 : size_t(G.batch), &pd))) return rc;
+    if (!shared_q || b0 == 0) {
+        cudaError_t e = gt_factor_launch(DArr{ G.Q.at(shared_q ? 0 : b0), G.Q.s }, G.n, ldj, int(count), J, JT,
+            shared_q ? pd : pd + b0, h->plan_sms, h->stream);
+        if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
+        h->launches += 1; h->call_launches += 1;
+    }
+    F.Jt = J;
+    F.sJ = shared_q ? 0 : (long long)ldj * (long long)n;
+    F.qpd = pd;
+    F.qpd_stride = shared_q ? 0 : 1;
+    return 0;
+}
+
+// K8 for the last raw QP batch (copra_b200_qp_vjp): the same KKT core, fed by qp_gather and finished by qp_grad, with the
+// factor of Q from qp_factor.  With dAeq / dAineq the forward solve is the second right-hand side (k = 2) and its multipliers
+// lambda enter.
 int do_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b200_qp_vjp_out* out)
 {
     const GiBatch& G = h->qp;
@@ -1387,31 +1415,56 @@ int do_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b2
     if ((rc = ws(h, "res_x", B * n, &x))) return rc;
     V.x = x;
     const bool shared_q = G.Q.s == 0;
-    auto factor = [&](int b0, int nb, SensFactor& F) {
-        double *J = nullptr, *JT = nullptr;
-        int* pd = nullptr;
-        const size_t count = shared_q ? 1 : size_t(nb); // the first chunk is the largest: later ones reuse its workspace
-        int rc2;
-        if ((rc2 = ws(h, "qpv_Jt", count * ldj * n, &J))) return rc2;
-        if ((rc2 = ws(h, "qpv_JtT", count * ldj * n, &JT))) return rc2;
-        if ((rc2 = ws(h, "qpv_pd", shared_q ? 1 : B, &pd))) return rc2;
-        if (!shared_q || b0 == 0) {
-            cudaError_t e = gt_factor_launch(DArr{ G.Q.at(shared_q ? 0 : b0), G.Q.s }, G.n, ldj, int(count), J, JT,
-                shared_q ? pd : pd + b0, h->plan_sms, h->stream);
-            if (e != cudaSuccess) return fail(h, COPRA_B200_E_CUDA, "gt_factor_launch: %s", cudaGetErrorString(e));
-            h->launches += 1; h->call_launches += 1;
-        }
-        F.Jt = J;
-        F.sJ = shared_q ? 0 : (long long)ldj * (long long)n;
-        F.qpd = pd;
-        F.qpd_stride = shared_q ? 0 : 1;
-        return 0;
-    };
+    auto factor = [&](int b0, int nb, SensFactor& F) { return qp_factor(h, "qpv", b0, nb, F); };
     const bool want_rows = out->Aeq || out->Aineq;
     rc = sens_run(h, V, G.n, G.batch, want_rows ? 2 : 1, shared_q ? 0 : 2 * size_t(ldj) * n, factor,
         [&](int nb) { return qp_gather_launch(V, nb, h->stream); }, [&](int nb) { return qp_grad_launch(V, nb, h->stream); });
     if (rc) return rc;
     return download_outputs(h, items, B, memory);
+}
+
+// K9 for the last raw QP batch (copra_b200_qp_jvp, copra_b200_qp_jacobian): k tangent directions described by `in`, or (in
+// == NULL) the columns of the identity on the input `wrt`.  Q's factor comes from qp_factor with workspace of its own.  With
+// Aeq / Aineq tangents a k = 1 pass on the forward right-hand side first leaves lambda in qpj_lam (its own chunking, so its
+// own factorisation); without them there is one pass.  qp_output writes every entry of dx (n x k per instance).
+int do_qp_jvp(copra_b200_handle* h, const copra_b200_qp_jvp_in* in, int k, int wrt, int memory, double* dx)
+{
+    const GiBatch& G = h->qp;
+    const size_t B = G.batch, n = G.n, meq = G.meq, m = G.m, K = size_t(k);
+    int rc;
+    QpJvpParams J{};
+    J.wrt = in ? -1 : wrt;
+    // tangents: the caller's device arrays, or HOST arrays packed into the staging buffer and uploaded in one copy
+    Upload U;
+    if (in) {
+        const struct { copra_b200_array a; size_t len; DArr* dst; } t[] = { { in->Q, n * n, &J.tQ }, { in->c, n, &J.tc },
+            { in->Aeq, meq * n, &J.tAeq }, { in->beq, meq, &J.tbeq }, { in->Aineq, m * n, &J.tAineq }, { in->bineq, m, &J.tbineq },
+            { in->lb, n, &J.tlb }, { in->ub, n, &J.tub } };
+        for (const auto& it : t) U.add(it.a, it.len * K, it.dst);
+    }
+    if ((rc = run_upload(h, U, G.batch, memory, "qpj_in"))) return rc;
+    J.meq = G.meq; J.m = G.m;
+    J.c = G.c; J.Aeq = G.Aeq; J.beq = G.beq; J.Aineq = G.Aineq; J.bineq = G.bineq; J.lb = G.lb; J.ub = G.ub;
+    if ((rc = ws(h, "res_x", B * n, const_cast<double**>(&J.x)))) return rc;
+    J.dx = dx;
+    if (memory == COPRA_B200_HOST && (rc = ws(h, "qpj_out", B * n * K, &J.dx))) return rc;
+    const size_t factor_per = G.Q.s == 0 ? 0 : 2 * size_t(gt_even(G.n)) * n;
+    auto factor = [&](int b0, int nb, SensFactor& F) { return qp_factor(h, "qpj", b0, nb, F); };
+    if (J.tAeq.p || J.tAineq.p) {
+        if ((rc = ws(h, "qpj_lam", B * n, &J.lam))) return rc;
+        rc = sens_run(h, J, G.n, G.batch, 1, factor_per, factor, [&](int nb) { return qp_lambda_gather_launch(J, nb, h->stream); },
+            [&](int nb) { return qp_lambda_store_launch(J, nb, h->stream); });
+        if (rc) return rc;
+    }
+    rc = sens_run(h, J, G.n, G.batch, k, factor_per, factor, [&](int nb) { return qp_tangent_launch(J, nb, h->stream); },
+        [&](int nb) { return qp_output_launch(J, nb, h->stream); });
+    if (rc) return rc;
+    if (memory == COPRA_B200_HOST) {
+        Download D;
+        D.add(J.dx, dx, B * n * K * sizeof(double));
+        if ((rc = run_download(h, D, COPRA_B200_HOST))) return rc;
+    }
+    return 0;
 }
 
 // the resident build takes its vectors only through the vector part of K2 / K4, which retarget re-runs and the sensitivities
@@ -2108,6 +2161,62 @@ int copra_b200_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const 
     CU(cudaSetDevice(h->device));
     h->call_launches = 0;
     return do_qp_vjp(h, dx, memory, out);
+}
+
+// the shared preconditions of copra_b200_qp_jvp / copra_b200_qp_jacobian with k directions: sens_solve's shared memory for k
+// right-hand sides (the active set has at most n rows) and gt_factor's for Q within the device's limit
+static int qp_jvp_check(copra_b200_handle* h, const char* name, int k)
+{
+    const GiBatch& G = h->qp;
+    const size_t smem = std::max(sens_solve_smem(k, G.n), gt_factor_smem(G.n));
+    if (smem > h->smem_optin)
+        return fail(h, COPRA_B200_E_UNSUPPORTED, "%s: n = %d needs %zu bytes of shared memory per block, the device allows %zu",
+            name, G.n, smem, h->smem_optin);
+    return 0;
+}
+
+int copra_b200_qp_jvp(copra_b200_handle* h, const copra_b200_qp_jvp_in* in, int memory, double* dx)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!h->qp_solved)
+        return fail(h, COPRA_B200_E_STATE, "copra_b200_qp_jvp needs a raw QP batch (copra_b200_solve_qp_batch) as the last solve on this handle");
+    if (!in) return fail(h, COPRA_B200_E_ARG, "qp_jvp: the tangents are required");
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    if (in->ndir < 1) return fail(h, COPRA_B200_E_ARG, "qp_jvp: ndir = %d, needs at least one direction", in->ndir);
+    const copra_b200_array* t[] = { &in->Q, &in->c, &in->Aeq, &in->beq, &in->Aineq, &in->bineq, &in->lb, &in->ub };
+    for (const copra_b200_array* a : t)
+        if (a->ptr && a->stride < 0) return fail(h, COPRA_B200_E_ARG, "qp_jvp: negative tangent stride %lld", a->stride);
+    const GiBatch& G = h->qp;
+    if ((in->Aeq.ptr || in->beq.ptr) && G.meq == 0) return fail(h, COPRA_B200_E_ARG, "qp_jvp: Aeq / beq tangents for a batch without equality rows");
+    if ((in->Aineq.ptr || in->bineq.ptr) && G.m == 0) return fail(h, COPRA_B200_E_ARG, "qp_jvp: Aineq / bineq tangents for a batch without inequality rows");
+    int rc = qp_jvp_check(h, "qp_jvp", in->ndir);
+    if (rc || !dx) return rc;
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_qp_jvp(h, in, in->ndir, -1, memory, dx);
+}
+
+int copra_b200_qp_jacobian(copra_b200_handle* h, int wrt, double* J, int memory)
+{
+    if (!h) return COPRA_B200_E_ARG;
+    if (!h->qp_solved)
+        return fail(h, COPRA_B200_E_STATE, "copra_b200_qp_jacobian needs a raw QP batch (copra_b200_solve_qp_batch) as the last solve on this handle");
+    if (memory != COPRA_B200_HOST && memory != COPRA_B200_DEVICE) return fail(h, COPRA_B200_E_ARG, "bad memory kind");
+    const GiBatch& G = h->qp;
+    int len;
+    switch (wrt) {
+    case COPRA_B200_QP_WRT_C: len = G.n; break;
+    case COPRA_B200_QP_WRT_BEQ: len = G.meq; break;
+    case COPRA_B200_QP_WRT_BINEQ: len = G.m; break;
+    case COPRA_B200_QP_WRT_LB: case COPRA_B200_QP_WRT_UB: len = G.n; break;
+    default: return fail(h, COPRA_B200_E_ARG, "qp_jacobian: unknown wrt %d", wrt);
+    }
+    if (len == 0) return fail(h, COPRA_B200_E_ARG, "qp_jacobian: wrt %d names rows the batch does not have", wrt);
+    int rc = qp_jvp_check(h, "qp_jacobian", len);
+    if (rc || !J) return rc;
+    CU(cudaSetDevice(h->device));
+    h->call_launches = 0;
+    return do_qp_jvp(h, nullptr, len, wrt, memory, J);
 }
 
 } // extern "C"

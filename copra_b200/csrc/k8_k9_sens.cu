@@ -34,6 +34,10 @@
 //   qp_gather / qp_grad  the same VJP for a raw QP batch (copra_b200_qp_vjp): the active rows come from the caller's dense
 //               Aeq / Aineq, and dc = -v, dQ = -(v x' + x v') / 2, dbeta_j = mu_j, da_j = -lambda_j v - mu_j x (k = 2 when the
 //               Aeq / Aineq gradients are wanted, lambda again from the forward solve as second right-hand side)
+//   qp_tangent / qp_output  the JVP of a raw QP batch (copra_b200_qp_jvp, copra_b200_qp_jacobian): r = -cdot_eff with
+//               cdot_eff = cdot + sym(Qdot) x + sum_active lambda_j adot_j, bdot_act of a general row bdot_j - adot_j' x, of a
+//               bound row lbdot / ubdot, and x = xdot (n x k per instance).  With Aeq / Aineq tangents lambda comes first, from
+//               a k = 1 pass on the forward right-hand side (qp_lambda_gather: -c and beta; qp_lambda_store keeps rhs = lambda)
 //   k9_output  the caller's layout: the first ru rows of Udot, and the first rx rows of Phi x0dot + Toeplitz(Gs) Udot
 // Initial-state mode (copra_b200_lmpc_vjp_initial_state / _jvp_initial_state): the decision vector is z = [x0*; U] (n = nx + nU)
 // with the per-instance Hessian of the build, and x0 enters only as the default of a bound that was not given.  The same
@@ -837,6 +841,127 @@ __global__ void __launch_bounds__(kSensThreads) qp_grad_kernel(const __grid_cons
         }
 }
 
+// The values of COPRA_B200_QP_WRT_*: the input whose identity columns qp_tangent writes (QpJvpParams::wrt)
+constexpr int kWrtC = 0, kWrtBeq = 1, kWrtBineq = 2, kWrtLb = 3, kWrtUb = 4;
+
+// entry `col` of general row idx (< meq + m) of a raw QP: the caller's column-major Aeq / Aineq of one instance
+struct QpRows {
+    const double* Aeq;
+    const double* Aineq;
+    int meq, m;
+    __device__ double operator()(int idx, int col) const
+    {
+        return idx < meq ? Aeq[idx + (long long)meq * col] : Aineq[idx - meq + (long long)m * col];
+    }
+};
+
+// direction d of a raw-QP tangent (len doubles per direction, column-major) of instance b, null when not given
+__device__ __forceinline__ const double* qp_dir(const DArr& t, int b, long long len, int d)
+{
+    return t.p ? t.at(b) + len * d : nullptr;
+}
+
+// The raw QP's lambda pass (k = 1): [A_act' | -c] into the slab and beta of the active rows in rhs, so that sens_solve leaves
+// the forward multipliers lambda in rhs
+__global__ void __launch_bounds__(kSensThreads) qp_lambda_gather_kernel(const __grid_constant__ QpJvpParams J)
+{
+    const int lb = blockIdx.x, b = J.b0 + lb;
+    const int n = J.n, meq = J.meq, m = J.m, mg = meq + m, nm = J.nm;
+    double* slab = sens_gather(J, lb, b, mg, QpRows{ J.Aeq.at(b), J.Aineq.at(b), meq, m });
+    const int na = sens_nact(J, b);
+    const int* iact = J.iact + (long long)b * n;
+    for (int a = threadIdx.x; a < nm; a += blockDim.x)
+        J.rhs[(long long)lb * nm + a] = a < na ? active_beta(iact[a] - 1, meq, mg, n, J.beq.at(b), J.bineq.at(b), J.ub.at(b), J.lb.at(b)) : 0.0;
+    if (J.status[b] != 0) return;
+    const double* c = J.c.at(b);
+    for (int col = threadIdx.x; col < n; col += blockDim.x) slab[col + (long long)nm * J.lds] = -c[col];
+}
+
+// lambda (rhs after sens_solve, k = 1) into the whole-batch workspace, by active position
+__global__ void __launch_bounds__(kSensThreads) qp_lambda_store_kernel(const __grid_constant__ QpJvpParams J)
+{
+    const int lb = blockIdx.x, b = J.b0 + lb, na = sens_nact(J, b);
+    for (int a = threadIdx.x; a < na; a += blockDim.x) J.lam[(long long)b * J.n + a] = J.rhs[(long long)lb * J.nm + a];
+}
+
+// The raw QP's tangent pass: [A_act' | -cdot_eff,1 .. -cdot_eff,k] into the slab and bdot_eff (nm x k) in rhs, with
+//   cdot_eff = cdot + sym(Qdot) x + sum_active lambda_j adot_j,   bdot_eff,j = bdot_j - adot_j' x (general row), lbdot / ubdot
+// (bound row); in identity mode (wrt >= 0) cdot or bdot of direction d is the unit vector e_d and every other tangent is zero.
+// The symmetric-part product is formed without contraction, so that Qdot and Qdot' give the same bits.
+__global__ void __launch_bounds__(kSensThreads) qp_tangent_kernel(const __grid_constant__ QpJvpParams J)
+{
+    const int lb = blockIdx.x, b = J.b0 + lb;
+    const int n = J.n, meq = J.meq, m = J.m, mg = meq + m, nm = J.nm, k = J.k, wrt = J.wrt;
+    double* slab = sens_gather(J, lb, b, mg, QpRows{ J.Aeq.at(b), J.Aineq.at(b), meq, m });
+    if (J.status[b] != 0) return; // sens_gram zeroes the rhs of an instance without an active set
+    const int na = J.nact[b];
+    const int* iact = J.iact + (long long)b * n;
+    const double* x = J.x + (long long)b * n;
+    const double* lam = J.lam ? J.lam + (long long)b * n : nullptr;
+    const long long nn = (long long)n * n;
+    for (int t = threadIdx.x; t < n * k; t += blockDim.x) {
+        const int i = t % n, d = t / n;
+        const double* tc = qp_dir(J.tc, b, n, d);
+        double c = wrt == kWrtC ? (i == d ? 1.0 : 0.0) : tc ? tc[i] : 0.0;
+        if (const double* Qd = qp_dir(J.tQ, b, nn, d)) {
+            double s = 0.0;
+            for (int a = 0; a < n; ++a)
+                s = __dadd_rn(s, __dmul_rn(__dmul_rn(0.5, __dadd_rn(Qd[i + (long long)a * n], Qd[a + (long long)i * n])), x[a]));
+            c += s;
+        }
+        if (lam) {
+            const double* Ae = qp_dir(J.tAeq, b, (long long)meq * n, d);
+            const double* Ai = qp_dir(J.tAineq, b, (long long)m * n, d);
+            for (int a = 0; a < na; ++a) {
+                const int idx = iact[a] - 1;
+                if (idx < meq) {
+                    if (Ae) c += lam[a] * Ae[idx + (long long)meq * i];
+                } else if (idx < mg && Ai) {
+                    c += lam[a] * Ai[idx - meq + (long long)m * i];
+                }
+            }
+        }
+        slab[i + (long long)(nm + d) * J.lds] = -c;
+    }
+    for (int t = threadIdx.x; t < nm * k; t += blockDim.x) {
+        const int a = t % nm, d = t / nm;
+        double v = 0.0;
+        if (a < na) {
+            const int idx = iact[a] - 1;
+            if (idx < mg) {
+                const bool eq = idx < meq;
+                const int r = eq ? idx : idx - meq, rows = eq ? meq : m;
+                const double* tb = qp_dir(eq ? J.tbeq : J.tbineq, b, rows, d);
+                const double* tA = qp_dir(eq ? J.tAeq : J.tAineq, b, (long long)rows * n, d);
+                if (wrt == (eq ? kWrtBeq : kWrtBineq)) v = r == d ? 1.0 : 0.0;
+                else if (tb) v = tb[r];
+                if (tA) {
+                    double s = 0.0;
+                    for (int i = 0; i < n; ++i) s += tA[r + (long long)rows * i] * x[i];
+                    v -= s;
+                }
+            } else {
+                const int var = (idx - mg) % n;
+                const bool up = idx - mg < n; // upper rows first, then lower rows
+                const double* tv = qp_dir(up ? J.tub : J.tlb, b, n, d);
+                if (wrt == (up ? kWrtUb : kWrtLb)) v = var == d ? 1.0 : 0.0;
+                else if (tv) v = tv[var];
+            }
+        }
+        J.rhs[(long long)lb * nm * k + t] = v;
+    }
+}
+
+// xdot = V, n x k per instance (column-major); zeros for an instance whose status is not 0
+__global__ void __launch_bounds__(kSensThreads) qp_output_kernel(const __grid_constant__ QpJvpParams J)
+{
+    const int lb = blockIdx.x, b = J.b0 + lb, n = J.n, k = J.k;
+    const bool live = J.status[b] == 0;
+    const double* V = J.V + (long long)lb * J.lds * k;
+    double* out = J.dx + (long long)b * n * k;
+    for (int t = threadIdx.x; t < n * k; t += blockDim.x) out[t] = live ? V[t % n + (long long)(t / n) * J.lds] : 0.0;
+}
+
 // dcontrol = the first ru rows of Udot; dtraj = the first rx rows of Phi x0dot + Psi Udot, Psi applied as the block-Toeplitz
 // product over the compact Gs (K7 without xi).  In initial-state mode Udot = zdot[nx:] and x0dot = zdot[0:nx].  Zeros for an
 // instance whose status is not 0.
@@ -899,11 +1024,16 @@ int sens_gram_launch(const SensChunk& S, int nb, cudaStream_t st)
     return launched(cudaGetLastError());
 }
 
+size_t sens_solve_smem(int k, int nm)
+{
+    const int tile = k <= 2 ? k : kDirTile;
+    return sizeof(double) * 2 * std::min(k, tile) * size_t(std::max(nm, 1));
+}
+
 int sens_solve_launch(const SensChunk& S, int nb, cudaStream_t st)
 {
-    const int tile = S.k <= 2 ? S.k : kDirTile;
     const auto kernel = S.k == 1 ? sens_solve_kernel<1> : S.k == 2 ? sens_solve_kernel<2> : sens_solve_kernel<kDirTile>;
-    const size_t smem = sizeof(double) * 2 * std::min(S.k, tile) * size_t(std::max(S.nm, 1));
+    const size_t smem = sens_solve_smem(S.k, S.nm);
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return -int(e);
     kernel<<<nb, kSensThreads, smem, st>>>(S);
@@ -976,6 +1106,30 @@ int qp_grad_launch(const QpVjpParams& V, int nb, cudaStream_t st)
     cudaError_t e = cudaFuncSetAttribute(qp_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
     if (e != cudaSuccess) return -int(e);
     qp_grad_kernel<<<nb, kSensThreads, smem, st>>>(V);
+    return launched(cudaGetLastError());
+}
+
+int qp_lambda_gather_launch(const QpJvpParams& J, int nb, cudaStream_t st)
+{
+    qp_lambda_gather_kernel<<<nb, kSensThreads, 0, st>>>(J);
+    return launched(cudaGetLastError());
+}
+
+int qp_lambda_store_launch(const QpJvpParams& J, int nb, cudaStream_t st)
+{
+    qp_lambda_store_kernel<<<nb, kSensThreads, 0, st>>>(J);
+    return launched(cudaGetLastError());
+}
+
+int qp_tangent_launch(const QpJvpParams& J, int nb, cudaStream_t st)
+{
+    qp_tangent_kernel<<<nb, kSensThreads, 0, st>>>(J);
+    return launched(cudaGetLastError());
+}
+
+int qp_output_launch(const QpJvpParams& J, int nb, cudaStream_t st)
+{
+    qp_output_kernel<<<nb, kSensThreads, 0, st>>>(J);
     return launched(cudaGetLastError());
 }
 

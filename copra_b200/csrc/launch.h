@@ -149,6 +149,29 @@ struct QpVjpParams : SensChunk {
 int qp_gather_launch(const QpVjpParams& V, int nb, cudaStream_t st);
 size_t qp_grad_smem(int n);
 int qp_grad_launch(const QpVjpParams& V, int nb, cudaStream_t st);
+// shared memory of sens_solve for k right-hand sides and an active set of at most nm rows
+size_t sens_solve_smem(int k, int nm);
+
+// K9 for a raw QP batch (copra_b200_qp_jvp, copra_b200_qp_jacobian): the KKT core with the active rows read as qp_gather
+// reads them.  When an Aeq / Aineq tangent is given, a k = 1 pass on the forward right-hand side (-c, beta_act) first leaves
+// the forward multipliers lambda in `lam` (qp_lambda_gather, then qp_lambda_store); the tangent pass then runs qp_tangent and
+// qp_output around the core.
+struct QpJvpParams : SensChunk {
+    int meq, m;
+    DArr c, Aeq, beq, Aineq, bineq, lb, ub; // the inputs of the solve
+    const double* x;                 // the solution, n per instance
+    double* lam;                     // lambda of the active rows by active position, n per instance (whole batch)
+    int wrt;                         // -1: the tangents below; else the columns of the identity on c / beq / bineq / lb / ub
+                                     // (the values of COPRA_B200_QP_WRT_*), every tangent null
+    // tangents: per instance len x k, each direction column-major in the layout of the input (s = 0: one for the batch;
+    // p null: zero)
+    DArr tQ, tc, tAeq, tbeq, tAineq, tbineq, tlb, tub;
+    double* dx;                      // output, whole batch: n x k per instance, every entry written
+};
+int qp_lambda_gather_launch(const QpJvpParams& J, int nb, cudaStream_t st);
+int qp_lambda_store_launch(const QpJvpParams& J, int nb, cudaStream_t st);
+int qp_tangent_launch(const QpJvpParams& J, int nb, cudaStream_t st);
+int qp_output_launch(const QpJvpParams& J, int nb, cudaStream_t st);
 
 // K9: Jacobian-vector products along k tangent directions, or the feedback gain
 struct JvpParams : SensChunk {

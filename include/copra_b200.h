@@ -228,6 +228,41 @@ typedef struct {
  * and its warm-start seed untouched. */
 int copra_b200_qp_vjp(copra_b200_handle* h, const double* dx, int memory, const copra_b200_qp_vjp_out* out);
 
+/* Forward mode on the last raw QP batch: Jacobian-vector products of its solutions x along k tangent directions, exact on the
+ * final active set.  With the active rows a_j'x = beta_j written as for copra_b200_qp_vjp and lambda the forward multipliers,
+ * one KKT solve per instance with k right-hand sides,
+ *   [Q A_act'; A_act 0] [xdot; lambdadot] = [-cdot_eff; bdot_eff],
+ *   cdot_eff = cdot + (Qdot + Qdot') x / 2 + sum_active lambda_j adot_j,
+ *   bdot_eff_j = bdot_j - adot_j' x (an active Aeq / Aineq row),  ubdot_k / lbdot_k (an active bound row),
+ * gives xdot.  Q is read through its symmetric part, as by copra_b200_qp_vjp.  lambda is computed (one more KKT solve with one
+ * right-hand side) only when an Aeq or Aineq tangent is given.  A weakly active row gives the one-sided derivative on the final
+ * active set. */
+typedef struct {
+    int ndir;                                      /* k >= 1 tangent directions */
+    copra_b200_array Q, c, Aeq, beq, Aineq, bineq, lb, ub;
+    /* per instance len x k: the k directions one after the other, each in the layout copra_b200_solve_qp_batch takes for the
+     * input (Q n x n, Aeq meq x n, Aineq m x n, column-major); stride in doubles between instances, 0 = one tangent for every
+     * instance; ptr NULL = zero tangent */
+} copra_b200_qp_jvp_in;
+/* `dx` receives n x k doubles per instance (column-major: direction d at d * n); it and the tangents live in `memory`.
+ * Instances whose status is not 0 get zeros; a Q or a Gram matrix of the active rows that is not positive definite gives NaN.
+ * With DEVICE inputs the solve's input arrays are read again: the caller leaves them unchanged until this call.  E_STATE when
+ * the last solve on the handle was not a raw QP batch; E_ARG for a NULL `in`, ndir < 1, a negative stride, Aeq / beq tangents
+ * with meq = 0 or Aineq / bineq tangents with m = 0; E_UNSUPPORTED when n needs more shared memory per block than the device
+ * allows.  A NULL `dx` returns 0 after these checks.  Leaves a resident LMPC build, its factor caches, its warm-start seed and
+ * a later copra_b200_qp_vjp untouched. */
+int copra_b200_qp_jvp(copra_b200_handle* h, const copra_b200_qp_jvp_in* in, int memory, double* dx);
+
+/* The Jacobian of the last raw QP batch's solutions x with respect to one vector input: copra_b200_qp_jvp along the columns of
+ * the identity on that input (never materialised).  wrt = c gives dx/dc (n x n, the projected inverse Hessian
+ * -Z (Z'QZ)^-1 Z' on the active set, symmetric); beq, bineq, lb, ub give n x meq, n x m, n x n, n x n, whose columns of
+ * inactive rows are exactly zero.  `J` receives n x len doubles per instance, column-major, in `memory`.  Errors and
+ * conventions as copra_b200_qp_jvp; E_ARG for an unknown wrt, or beq with meq = 0 or bineq with m = 0.  A NULL `J` returns 0
+ * after the checks. */
+enum { COPRA_B200_QP_WRT_C = 0, COPRA_B200_QP_WRT_BEQ = 1, COPRA_B200_QP_WRT_BINEQ = 2, COPRA_B200_QP_WRT_LB = 3,
+       COPRA_B200_QP_WRT_UB = 4 };
+int copra_b200_qp_jacobian(copra_b200_handle* h, int wrt, double* J, int memory);
+
 /* Dense assembly primitive -- batched FP64 GEMM on the tensor cores (DMMA m8n8k4 fed through shared memory, TMA
  * bulk loads for aligned operands): C[b] = alpha * op(A[b]) * B[b] + beta * C[b], column-major, strides in doubles.
  * It is what full-size (autoSpan'd) entries use for M*Psi, T'WT, E*Psi (src/costFunctions.cpp:65-69,
