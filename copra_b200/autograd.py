@@ -44,20 +44,20 @@ import torch
 from . import capi
 
 
-def _vec_entries(bp):
-    """(kind, index) of every vector input after x0, in the order of the Function's arguments"""
+def _vector_entries(bp):
+    """(kind, index) of every cost's p and every constraint's f or lower / upper"""
     keys = [("p", i) for i in range(len(bp["costs"]))]
     for j, c in enumerate(bp["constraints"]):
         keys += [("lower", j), ("upper", j)] if c["kind"] in ("trajectory_bound", "control_bound") else [("f", j)]
-    keys += [(k, i) for i in range(len(bp["costs"])) for k in _COST_KEYS]
-    return keys + [(k, 0) for k in _SYSTEM_KEYS] + [(k, j) for j in range(len(bp["constraints"])) for k in ("E", "G")]
+    return keys
 
 
 _COST_KEYS = ("w", "M", "N")
 _SYSTEM_KEYS = ("A", "B", "d")
 _MODEL_KEYS = _SYSTEM_KEYS + ("E", "G")
 _MATRIX_KEYS = _COST_KEYS + _MODEL_KEYS  # reverse mode only
-_BASE_NDIM = dict(w=1, M=2, N=2, A=2, B=2, d=1, E=2, G=2)
+_TOP_KEYS = _SYSTEM_KEYS + capi.INITIAL_KEYS  # one per problem, not per cost / constraint
+_BASE_NDIM = dict(w=1, M=2, N=2, A=2, B=2, d=1, E=2, G=2, R=2, r=1, x0lb=1, x0ub=1)
 
 
 def _point(arr, t, base):
@@ -83,7 +83,8 @@ def _patch_cost_matrix(problem, pr, kind, i, t):
 
 
 def _patch_model_matrix(bp, pr, kind, i, t):
-    """point A, B or d, or constraint i's E or G, of the packed problem at the tensor t (batched or shared)"""
+    """point A, B, d, R, r, x0lb or x0ub, or constraint i's E or G, of the packed problem at the tensor t (batched or
+    shared)"""
     nx, nu = int(bp["nx"]), int(bp["nu"])
     if kind in ("E", "G"):
         rows, has_e, has_g = capi.cstr_shapes(bp)[i]
@@ -91,13 +92,22 @@ def _patch_model_matrix(bp, pr, kind, i, t):
             raise ValueError("constraint %d (%s) has no %s" % (i, bp["constraints"][i]["kind"], kind))
         shape = (rows, nx if kind == "E" else nu)
     else:
-        shape = dict(A=(nx, nx), B=(nx, nu), d=(nx,))[kind]
+        shape = dict(A=(nx, nx), B=(nx, nu), d=(nx,), R=(nx, nx), r=(nx,), x0lb=(nx,), x0ub=(nx,))[kind]
     if t.dim() not in (len(shape), len(shape) + 1) or tuple(t.shape[t.dim() - len(shape):]) != shape:
         raise ValueError("%s has shape %s, expected %s (with an optional leading batch axis)" % (kind, tuple(t.shape), shape))
     return _point(getattr(pr.cstrs[i] if kind in ("E", "G") else pr, kind), t, len(shape))
 
 
+def _check_resident(ctx, what):
+    if ctx.engine.solve_count != ctx.count:
+        raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the %s needs the active "
+                           "sets of the solve being differentiated" % what)
+
+
 class _LMPC(torch.autograd.Function):
+    """an LMPC-mode or an initial-state build (bp["initial_state"]): the forward solves it, the backward and the
+    forward-mode tangent run the engine's VJP and JVP of that build mode"""
+
     @staticmethod
     def forward(ctx, engine, bp, keys, x0, *vecs):
         B = int(bp["batch"])
@@ -109,7 +119,7 @@ class _LMPC(torch.autograd.Function):
         for (kind, i), v in zip(keys, vecs):
             if v is None:  # shape only: the tensor itself is patched in below
                 continue
-            if kind in _SYSTEM_KEYS:
+            if kind in _TOP_KEYS:
                 problem[kind] = np.zeros(tuple(v.shape))
             else:
                 (problem["costs"] if kind in ("p",) + _COST_KEYS else problem["constraints"])[i][kind] = np.zeros(tuple(v.shape))
@@ -123,7 +133,7 @@ class _LMPC(torch.autograd.Function):
             if kind in _COST_KEYS:
                 live.append(_patch_cost_matrix(problem, pr, kind, i, v))
                 continue
-            if kind in _MODEL_KEYS:
+            if kind in _BASE_NDIM:
                 live.append(_patch_model_matrix(bp, pr, kind, i, v))
                 continue
             t = v.detach().contiguous()
@@ -145,46 +155,55 @@ class _LMPC(torch.autograd.Function):
         ctx.engine, ctx.count, ctx.keys, ctx.present = engine, engine.solve_count, keys, [v is not None for v in vecs]
         # the build reads x0 and the matrices where they live: the VJP of the cost and model matrices reads them again
         ctx.live = (hb, live)
-        ctx.shared = [v is not None and kind in _MATRIX_KEYS and v.dim() == _BASE_NDIM[kind] for (kind, _), v in zip(keys, vecs)]
-        ctx.counts = (len(bp["costs"]), len(bp["constraints"]))
+        ctx.shared = [v is not None and kind in _BASE_NDIM and v.dim() == _BASE_NDIM[kind] for (kind, _), v in zip(keys, vecs)]
+        ctx.initial = bool(bp.get("initial_state"))
+        ctx.counts = (B, len(bp["costs"]), len(bp["constraints"]))
         ctx.mark_non_differentiable()
         return control, traj
 
     @staticmethod
     def jvp(ctx, _engine, _bp, _keys, dx0, *dvecs):
-        # forward mode: one tangent direction through copra_b200_lmpc_jvp (K9); the engine holds everything it needs
-        eng = ctx.engine
-        if eng.solve_count != ctx.count:
-            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the JVP needs the "
-                               "active sets of the solve being differentiated")
-        ncost, ncstr = ctx.counts
+        # forward mode: one tangent direction through copra_b200_lmpc_jvp (_initial_state) (K9); the engine holds everything
+        # it needs
+        _check_resident(ctx, "JVP")
+        B, ncost, ncstr = ctx.counts
         tangents = dict(p=[None] * ncost, f=[None] * ncstr, lower=[None] * ncstr, upper=[None] * ncstr)
-        for (kind, i), t in zip(ctx.keys, dvecs):
+        init = {}
+        for (kind, i), t, shared in zip(ctx.keys, dvecs, ctx.shared):
+            if t is None:
+                continue
             if kind in _MATRIX_KEYS:
-                if t is not None and bool(torch.count_nonzero(t)):
+                if bool(torch.count_nonzero(t)):
                     raise NotImplementedError("copra_b200.autograd: forward-mode derivatives with respect to the cost weights "
                                               "and matrices (w, M, N) and the model (A, B, d, E, G) are not implemented; "
                                               "reverse mode (backward) is")
-                continue
-            if t is not None:
+            elif kind in capi.INITIAL_KEYS:
+                init[kind] = (t.expand(B, *t.shape) if shared else t).unsqueeze(1)
+            else:
                 tangents[kind][i] = t.unsqueeze(1)
-        du, dx = eng.lmpc_jvp(x0=dx0.unsqueeze(1) if dx0 is not None else None, **tangents)
+        dx0 = dx0.unsqueeze(1) if dx0 is not None else None
+        eng = ctx.engine
+        du, dx = eng.initial_state_jvp(x0=dx0, **init, **tangents) if ctx.initial else eng.lmpc_jvp(x0=dx0, **tangents)
         return du[:, 0], dx[:, 0]
 
     @staticmethod
     def backward(ctx, dcontrol, dtraj):
-        eng = ctx.engine
-        if eng.solve_count != ctx.count:
-            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the VJP needs the "
-                               "active sets of the solve being differentiated")
-        want = capi.VJP_WANT + tuple(k for k in _MATRIX_KEYS
-                                     if any(p and kind == k for (kind, _), p in zip(ctx.keys, ctx.present)))
-        g = eng.lmpc_vjp(dcontrol=dcontrol, dtrajectory=dtraj, want=want)  # ordered against torch's stream on both sides
+        _check_resident(ctx, "VJP")
+        want = capi.VJP_WANT + tuple(k for k in _BASE_NDIM if any(p and kind == k for (kind, _), p in zip(ctx.keys, ctx.present)))
+        vjp = ctx.engine.initial_state_vjp if ctx.initial else ctx.engine.lmpc_vjp
+        g = vjp(dcontrol=dcontrol, dtrajectory=dtraj, want=want)  # ordered against torch's stream on both sides
         grads = [g["x0"]]
         for (kind, i), present, shared in zip(ctx.keys, ctx.present, ctx.shared):
-            grad = (g[kind] if kind in _SYSTEM_KEYS else g[kind][i]) if present else None
+            grad = (g[kind] if kind in _TOP_KEYS else g[kind][i]) if present else None
             grads.append(grad.sum(0) if shared else grad)  # a shared input's gradient sums its instances'
         return (None, None, None, *grads)
+
+
+def _apply(engine, bp, keys, x0, given):
+    """_LMPC of the inputs `given` (lists indexed by cost / constraint, None entries keep bp's values) in the order of
+    `keys`"""
+    vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
+    return _LMPC.apply(engine, bp, keys, x0, *vecs)
 
 
 def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None, w=None, M=None, N=None, A=None, B=None, d=None, E=None,
@@ -193,110 +212,11 @@ def lmpc(engine, bp, x0, p=None, f=None, lower=None, upper=None, w=None, M=None,
     vector, weight and matrix given (lists indexed by cost / constraint, None entries keep bp's values).  w, M and N are
     (rows,), (rows, nx) and (rows, nu) per cost, A, B and d (nx, nx), (nx, nu) and (nx,), E and G (rows, nx) and (rows, nu)
     per row constraint, each with an optional leading batch axis; reverse mode only for these."""
-    keys = _vec_entries(bp)
-    given = dict(p=p or [], f=f or [], lower=lower or [], upper=upper or [], w=w or [], M=M or [], N=N or [], A=[A], B=[B],
-                 d=[d], E=E or [], G=G or [])
-    vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
-    return _LMPC.apply(engine, bp, keys, x0, *vecs)
-
-
-_INITIAL_BASE = dict(R=2, r=1, x0lb=1, x0ub=1)
-
-
-def _initial_entries(bp):
-    """(kind, index) of every input after x0 of an initial-state build: R, r, x0lb, x0ub, then the vectors"""
-    keys = [(k, 0) for k in capi.INITIAL_KEYS] + [("p", i) for i in range(len(bp["costs"]))]
-    for j, c in enumerate(bp["constraints"]):
-        keys += [("lower", j), ("upper", j)] if c["kind"] in ("trajectory_bound", "control_bound") else [("f", j)]
-    return keys
-
-
-class _InitialStateLMPC(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, engine, bp, keys, x0, *vecs):
-        B, nx = int(bp["batch"]), int(bp["nx"])
-        dev = x0.device
-        problem = dict(bp)
-        problem["costs"] = [dict(c) for c in bp["costs"]]
-        problem["constraints"] = [dict(c) for c in bp["constraints"]]
-        problem["x0"] = np.zeros((B, nx))
-        for (kind, i), v in zip(keys, vecs):
-            if v is None:  # shape only: the tensor itself is patched in below
-                continue
-            if kind in _INITIAL_BASE:
-                problem[kind] = np.zeros(tuple(v.shape))
-            else:
-                (problem["costs"] if kind == "p" else problem["constraints"])[i][kind] = np.zeros(tuple(v.shape))
-        hb = capi.HostBatch(problem, device_tensors=dev)
-        live = [x0.detach().contiguous()]
-        pr = hb.problem
-        pr.x0.ptr, pr.x0.stride = live[0].data_ptr(), live[0].shape[1]
-        for (kind, i), v in zip(keys, vecs):
-            if v is None:
-                continue
-            if kind in _INITIAL_BASE:
-                base = _INITIAL_BASE[kind]
-                if v.dim() not in (base, base + 1) or tuple(v.shape[v.dim() - base:]) != (nx,) * base:
-                    raise ValueError("%s has shape %s, expected %s (with an optional leading batch axis)"
-                                     % (kind, tuple(v.shape), (nx,) * base))
-                live.append(_point(getattr(pr, kind), v, base))
-                continue
-            t = v.detach().contiguous()
-            live.append(t)
-            arr = getattr(pr.costs[i] if kind == "p" else pr.cstrs[i], kind)
-            arr.ptr, arr.stride = t.data_ptr(), t.shape[1]
-        s = engine.sizes(hb)
-        control = torch.empty((B, s["nU"]), dtype=torch.float64, device=dev)
-        traj = torch.empty((B, s["X"]), dtype=torch.float64, device=dev)
-        r = capi.Results()
-        r.memory = capi.DEVICE
-        r.control, r.trajectory = control.data_ptr(), traj.data_ptr()
-        torch.cuda.synchronize(dev)
-        engine.solve_count += 1
-        engine._last_bp = None
-        engine._check(engine.lib.copra_b200_lmpc_run(engine.h, C.byref(pr), C.byref(r)))
-        engine._last_bp = problem
-        engine.synchronize()
-        ctx.engine, ctx.count, ctx.keys, ctx.present = engine, engine.solve_count, keys, [v is not None for v in vecs]
-        ctx.live = (hb, live)
-        ctx.shared = [v is not None and kind in _INITIAL_BASE and v.dim() == _INITIAL_BASE[kind] for (kind, _), v in zip(keys, vecs)]
-        ctx.counts = (B, len(bp["costs"]), len(bp["constraints"]))
-        ctx.mark_non_differentiable()
-        return control, traj
-
-    @staticmethod
-    def jvp(ctx, _engine, _bp, _keys, dx0, *dvecs):
-        # forward mode: one tangent direction through copra_b200_lmpc_jvp_initial_state (K9)
-        eng = ctx.engine
-        if eng.solve_count != ctx.count:
-            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the JVP needs the "
-                               "active sets of the solve being differentiated")
-        B, ncost, ncstr = ctx.counts
-        tangents = dict(p=[None] * ncost, f=[None] * ncstr, lower=[None] * ncstr, upper=[None] * ncstr)
-        init = {}
-        for (kind, i), t, shared in zip(ctx.keys, dvecs, ctx.shared):
-            if t is None:
-                continue
-            if kind in _INITIAL_BASE:
-                init[kind] = (t.expand(B, *t.shape) if shared else t).unsqueeze(1)
-            else:
-                tangents[kind][i] = t.unsqueeze(1)
-        du, dx = eng.initial_state_jvp(x0=dx0.unsqueeze(1) if dx0 is not None else None, **init, **tangents)
-        return du[:, 0], dx[:, 0]
-
-    @staticmethod
-    def backward(ctx, dcontrol, dtraj):
-        eng = ctx.engine
-        if eng.solve_count != ctx.count:
-            raise RuntimeError("copra_b200.autograd: another solve ran on this engine since the forward; the VJP needs the "
-                               "active sets of the solve being differentiated")
-        want = capi.VJP_WANT + tuple(k for (k, _), p in zip(ctx.keys, ctx.present) if p and k in _INITIAL_BASE)
-        g = eng.initial_state_vjp(dcontrol=dcontrol, dtrajectory=dtraj, want=want)  # ordered against torch's stream
-        grads = [g["x0"]]
-        for (kind, i), present, shared in zip(ctx.keys, ctx.present, ctx.shared):
-            grad = (g[kind] if kind in _INITIAL_BASE else g[kind][i]) if present else None
-            grads.append(grad.sum(0) if shared else grad)  # a shared input's gradient sums its instances'
-        return (None, None, None, *grads)
+    ncost, ncstr = len(bp["costs"]), len(bp["constraints"])
+    keys = (_vector_entries(bp) + [(k, i) for i in range(ncost) for k in _COST_KEYS] + [(k, 0) for k in _SYSTEM_KEYS]
+            + [(k, j) for j in range(ncstr) for k in ("E", "G")])
+    return _apply(engine, bp, keys, x0, dict(p=p or [], f=f or [], lower=lower or [], upper=upper or [], w=w or [], M=M or [],
+                                             N=N or [], A=[A], B=[B], d=[d], E=E or [], G=G or []))
 
 
 def initial_state_lmpc(engine, bp, x0, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
@@ -305,10 +225,9 @@ def initial_state_lmpc(engine, bp, x0, R=None, r=None, x0lb=None, x0ub=None, p=N
     vector given (lists indexed by cost / constraint, as lmpc); None keeps bp's value, which then gets no gradient"""
     if not bp.get("initial_state"):
         raise ValueError("initial_state_lmpc takes an initial-state problem; copra_b200.autograd.lmpc takes LMPC-mode ones")
-    keys = _initial_entries(bp)
-    given = dict(R=[R], r=[r], x0lb=[x0lb], x0ub=[x0ub], p=p or [], f=f or [], lower=lower or [], upper=upper or [])
-    vecs = [given[k][i] if i < len(given[k]) else None for k, i in keys]
-    return _InitialStateLMPC.apply(engine, bp, keys, x0, *vecs)
+    keys = [(k, 0) for k in capi.INITIAL_KEYS] + _vector_entries(bp)
+    return _apply(engine, bp, keys, x0, dict(R=[R], r=[r], x0lb=[x0lb], x0ub=[x0ub], p=p or [], f=f or [], lower=lower or [],
+                                             upper=upper or []))
 
 
 class _QP(torch.autograd.Function):

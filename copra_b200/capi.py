@@ -352,16 +352,83 @@ class HostBatch:
         return out
 
 
-def _result_buffers(B, s):
-    """host result arrays for B instances of sizes `s` and the Results struct pointing at them"""
+def _result_buffers(B, s, want=None):
+    """host result arrays for B instances of sizes `s` and the Results struct pointing at those in `want` (default: all)"""
     out = dict(control=np.zeros((B, s["nU"])), trajectory=np.zeros((B, s["X"])), x=np.zeros((B, s["nvar"])),
                status=np.full(B, -1, np.int32), iters=np.zeros((B, 2), np.int32), nact=np.zeros(B, np.int32),
                iact=np.zeros((B, s["nvar"]), np.int32))
     r = Results()
     r.memory = HOST
-    for k, v in out.items():
-        setattr(r, k, v.ctypes.data)
+    for k in out if want is None else want:
+        setattr(r, k, out[k].ctypes.data)
     return out, r
+
+
+class _Memory:
+    """Where the arrays of one call live: HOST numpy arrays, or CUDA float64 tensors on the device of its torch inputs (or
+    on `device`).  Outputs are allocated the same way.  With tensors the engine runs on its own stream: `run` makes the
+    inputs complete before the call (device synchronise) and waits for the engine's stream (`sync`) before the outputs
+    are handed back."""
+
+    def __init__(self, *inputs, device=None):
+        self.device = next((a.device for a in inputs if hasattr(a, "data_ptr")), device)
+        self.kind = HOST if self.device is None else DEVICE
+        self.keep = []  # input copies and pointer arrays, alive for the call
+
+    def array(self, a):
+        """`a` as a float64 array of this memory"""
+        if self.device is None:
+            return np.asarray(a, dtype=np.float64)
+        import torch
+        return torch.as_tensor(a, dtype=torch.float64, device=self.device).detach()
+
+    def buffer(self, a):
+        """the pointer to a contiguous float64 copy of `a` kept for the call (None for None)"""
+        if a is None:
+            return None
+        a = self.array(a)
+        a = np.ascontiguousarray(a) if self.device is None else a.contiguous()
+        self.keep.append(a)
+        return self.ptr(a)
+
+    def empty(self, *shape, dtype=np.float64):
+        """an output array; the engine writes (or zeroes) every entry of what it is handed"""
+        if self.device is None:
+            return np.zeros(shape, dtype)
+        import torch
+        return torch.empty(shape, dtype=getattr(torch, np.dtype(dtype).name), device=self.device)
+
+    def ptr(self, a):
+        """the data pointer of `a`, None for None or an empty array"""
+        if a is None or 0 in a.shape:
+            return None
+        return a.ctypes.data if self.device is None else a.data_ptr()
+
+    def pointers(self, arrs):
+        """a C array of the pointers of `arrs`, kept for the call"""
+        p = (C.c_void_p * max(1, len(arrs)))(*[self.ptr(a) for a in arrs])
+        self.keep.append(p)
+        return C.cast(p, C.POINTER(C.c_void_p))
+
+    def rowmajor(self, a):
+        """(batch, cols, rows) as the engine writes matrices (column-major) -> contiguous (batch, rows, cols)"""
+        if a is None:
+            return None
+        return np.ascontiguousarray(a.transpose(0, 2, 1)) if self.device is None else a.transpose(1, 2).contiguous()
+
+    def run(self, call, sync=None):
+        if self.device is None:
+            return call()
+        import torch
+        torch.cuda.synchronize(self.device)
+        try:
+            return call()
+        finally:
+            if sync is not None:
+                sync()
+
+
+_MEM = object()  # stands where a single-device entry takes the memory kind; a multi-device entry has no such argument
 
 
 def vjp_lengths(bp):
@@ -406,121 +473,51 @@ def _vjp_call(bp, B, dcontrol, dtrajectory, want, call, sync=None, initial=False
     VjpOut (and, when w, M or N are wanted, a VjpCostOut; when A, B, d, E or G are, a VjpModelOut) and run
     `call(dcontrol_ptr, dtrajectory_ptr, memory, out, cost_out, model_out)`, cost_out / model_out None unless such gradients
     are wanted.  With `initial` (an initial-state build) it runs `call(dcontrol_ptr, dtrajectory_ptr, memory, out, init_out)`
-    instead, init_out a VjpInitialOut for R, r, x0lb and x0ub.  With torch tensors the engine runs on its own stream:
-    the cotangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the
-    gradients (written, zero-initialised, by the engine itself) and the input copies are handed back."""
+    instead, init_out a VjpInitialOut for R, r, x0lb and x0ub.  With torch tensors the call runs as _Memory.run orders it."""
+    mem = _Memory(dcontrol, dtrajectory)
+    nu = int(bp["nu"])
     nx, plen, clen = vjp_lengths(bp)
-    dev = next((t.device for t in (dcontrol, dtrajectory) if t is not None and hasattr(t, "data_ptr")), None)
-    keep = []
-    if dev is not None:
-        import torch
 
-        def zeros(k):  # the engine zeroes every requested gradient on its stream
-            return torch.empty((B, k), dtype=torch.float64, device=dev)
-
-        def ptr(a):
-            return a.data_ptr()
-
-        def inp(a):
-            if a is None:
-                return None
-            a = a.detach().to(torch.float64).contiguous()
-            keep.append(a)
-            return a.data_ptr()
-        mem = DEVICE
-    else:
-        def zeros(k):
-            return np.zeros((B, k))
-
-        def ptr(a):
-            return a.ctypes.data
-
-        def inp(a):
-            if a is None:
-                return None
-            a = np.ascontiguousarray(np.asarray(a, dtype=np.float64))
-            keep.append(a)
-            return a.ctypes.data
-        mem = HOST
-    res = dict(x0=zeros(nx) if "x0" in want else None)
-    o = VjpOut()
-    o.x0 = ptr(res["x0"]) if res["x0"] is not None else None
-    kinds = [c["kind"] for c in bp["constraints"]]
-    bound = [k in ("trajectory_bound", "control_bound") for k in kinds]
-    lists = dict(p=[zeros(k) if "p" in want else None for k in plen],
-                 f=[zeros(k) if "f" in want and not b else None for k, b in zip(clen, bound)],
-                 lower=[zeros(k) if "lower" in want and b else None for k, b in zip(clen, bound)],
-                 upper=[zeros(k) if "upper" in want and b else None for k, b in zip(clen, bound)])
-    for key, arrs in lists.items():
-        ptrs = (C.c_void_p * max(1, len(arrs)))(*[ptr(a) if a is not None else None for a in arrs])
-        keep.append(ptrs)
-        setattr(o, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
-        res[key] = arrs
-    co = None
+    def zeros(*shape):  # the engine zeroes every requested gradient on its stream
+        return mem.empty(B, *shape)
+    bound = [c["kind"] in ("trajectory_bound", "control_bound") for c in bp["constraints"]]
+    res = dict(x0=zeros(nx) if "x0" in want else None,
+               p=[zeros(k) if "p" in want else None for k in plen],
+               f=[zeros(k) if "f" in want and not b else None for k, b in zip(clen, bound)],
+               lower=[zeros(k) if "lower" in want and b else None for k, b in zip(clen, bound)],
+               upper=[zeros(k) if "upper" in want and b else None for k, b in zip(clen, bound)])
+    o = VjpOut(x0=mem.ptr(res["x0"]), **{k: mem.pointers(res[k]) for k in ("p", "f", "lower", "upper")})
+    # the engine writes every matrix column-major: allocated as (batch, cols, rows), handed back as (batch, rows, cols)
+    co = mo = io = None
     if any(k in want for k in VJP_COST_WANT):
-        # the engine writes M (rows x nx) and N (rows x nu) column-major: allocated as (batch, cols, rows)
-        nu = int(bp["nu"])
         shapes = cost_shapes(bp)
-        raw = dict(w=[zeros(r) if "w" in want else None for r, _, _ in shapes],
-                   M=[zeros(nx * r).reshape(B, nx, r) if "M" in want and hm else None for r, hm, _ in shapes],
-                   N=[zeros(nu * r).reshape(B, nu, r) if "N" in want and hn else None for r, _, hn in shapes])
-        co = VjpCostOut()
-        for key, arrs in raw.items():
-            ptrs = (C.c_void_p * max(1, len(arrs)))(*[ptr(a) if a is not None else None for a in arrs])
-            keep.append(ptrs)
-            setattr(co, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
-    mo = None
+        res.update(w=[zeros(r) if "w" in want else None for r, _, _ in shapes],
+                   M=[zeros(nx, r) if "M" in want and hm else None for r, hm, _ in shapes],
+                   N=[zeros(nu, r) if "N" in want and hn else None for r, _, hn in shapes])
+        co = VjpCostOut(**{k: mem.pointers(res[k]) for k in VJP_COST_WANT})
     if any(k in want for k in VJP_MODEL_WANT):
-        # column-major matrices again: A as (batch, nx, nx) transposed, B (batch, nu, nx), E (batch, nx, rows), G (batch, nu, rows)
-        nu = int(bp["nu"])
         shapes = cstr_shapes(bp)
-        mraw = dict(A=zeros(nx * nx).reshape(B, nx, nx) if "A" in want else None,
-                    B=zeros(nx * nu).reshape(B, nu, nx) if "B" in want else None,
-                    d=zeros(nx) if "d" in want else None,
-                    E=[zeros(nx * r).reshape(B, nx, r) if "E" in want and he else None for r, he, _ in shapes],
-                    G=[zeros(nu * r).reshape(B, nu, r) if "G" in want and hg else None for r, _, hg in shapes])
-        mo = VjpModelOut()
-        for key in ("A", "B", "d"):
-            setattr(mo, key, ptr(mraw[key]) if mraw[key] is not None else None)
-        for key in ("E", "G"):
-            ptrs = (C.c_void_p * max(1, len(mraw[key])))(*[ptr(a) if a is not None else None for a in mraw[key]])
-            keep.append(ptrs)
-            setattr(mo, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
-    io = None
+        res.update(A=zeros(nx, nx) if "A" in want else None, B=zeros(nu, nx) if "B" in want else None,
+                   d=zeros(nx) if "d" in want else None,
+                   E=[zeros(nx, r) if "E" in want and he else None for r, he, _ in shapes],
+                   G=[zeros(nu, r) if "G" in want and hg else None for r, _, hg in shapes])
+        mo = VjpModelOut(A=mem.ptr(res["A"]), B=mem.ptr(res["B"]), d=mem.ptr(res["d"]), E=mem.pointers(res["E"]),
+                         G=mem.pointers(res["G"]))
     if initial:
         if co is not None or mo is not None:
             raise CopraB200Error(-4, "initial-state builds have no gradients with respect to w, M, N, A, B, d, E or G")
-        # R is written column-major; it is symmetric, so its logical layout is the same
-        iraw = dict(R=zeros(nx * nx).reshape(B, nx, nx) if "R" in want else None,
-                    **{k: zeros(nx) if k in want else None for k in ("r", "x0lb", "x0ub")})
-        io = VjpInitialOut()
-        for key, a in iraw.items():
-            setattr(io, key, ptr(a) if a is not None else None)
-            res[key] = a
-    dc, dt = inp(dcontrol), inp(dtrajectory)
-    if dev is not None:
-        torch.cuda.synchronize(dev)
-    try:
-        if initial:
-            call(dc, dt, mem, o, io)
-        else:
-            call(dc, dt, mem, o, co, mo)
-    finally:
-        if dev is not None and sync is not None:
-            sync()
-    if co is not None:
-        res["w"] = raw["w"]
-        for key in ("M", "N"):
-            res[key] = [None if a is None else (a.transpose(1, 2).contiguous() if dev is not None
-                                                else np.ascontiguousarray(a.transpose(0, 2, 1))) for a in raw[key]]
-
-    def logical(a):  # (batch, cols, rows) column-major -> (batch, rows, cols)
-        if a is None:
-            return None
-        return a.transpose(1, 2).contiguous() if dev is not None else np.ascontiguousarray(a.transpose(0, 2, 1))
-    if mo is not None:
-        res["A"], res["B"], res["d"] = logical(mraw["A"]), logical(mraw["B"]), mraw["d"]
-        res["E"], res["G"] = [logical(a) for a in mraw["E"]], [logical(a) for a in mraw["G"]]
+        # R is symmetric: its column-major layout is its logical one
+        res.update(R=zeros(nx, nx) if "R" in want else None,
+                   **{k: zeros(nx) if k in want else None for k in ("r", "x0lb", "x0ub")})
+        io = VjpInitialOut(**{k: mem.ptr(res[k]) for k in INITIAL_KEYS})
+    dc, dt = mem.buffer(dcontrol), mem.buffer(dtrajectory)
+    mem.run(lambda: call(dc, dt, mem.kind, o, io) if initial else call(dc, dt, mem.kind, o, co, mo), sync)
+    for k in ("M", "N", "E", "G"):
+        if k in res:
+            res[k] = [mem.rowmajor(a) for a in res[k]]
+    for k in ("A", "B"):
+        if k in res:
+            res[k] = mem.rowmajor(res[k])
     return res
 
 
@@ -528,12 +525,10 @@ def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None, init=None):
     """describe the tangents (each (batch, k, len), numpy or CUDA float64 tensors; None = zero) in a JvpIn, allocate dU
     (batch, k, nU) and dtrajectory (batch, k, X) of the same kind and run `call(jvp_in, memory, dU_ptr, dX_ptr)`.  With
     `init` (a dict of the R (batch, k, nx, nx), r, x0lb and x0ub (batch, k, nx) tangents of an initial-state build) it runs
-    `call(jvp_in, jvp_initial_in, memory, dU_ptr, dX_ptr)` instead.  With torch tensors the engine runs on its own stream: the
-    tangents are complete before the call (device synchronise) and `sync()` waits for the engine's stream before the results
-    are handed back."""
+    `call(jvp_in, jvp_initial_in, memory, dU_ptr, dX_ptr)` instead.  With torch tensors the call runs as _Memory.run
+    orders it."""
     nx, plen, clen = vjp_lengths(bp)
-    kinds = [c["kind"] for c in bp["constraints"]]
-    bound = [kd in ("trajectory_bound", "control_bound") for kd in kinds]
+    bound = [c["kind"] in ("trajectory_bound", "control_bound") for c in bp["constraints"]]
     lists = dict(p=list(p or []), f=list(f or []), lower=list(lower or []), upper=list(upper or []))
     initial = init is not None
     init = dict(init or {})
@@ -541,38 +536,24 @@ def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None, init=None):
     if R is not None and len(R.shape) == 4:  # (batch, k, nx, nx) -> column-major nx x nx per direction
         R = R.transpose(2, 3) if hasattr(R, "data_ptr") else np.swapaxes(np.asarray(R, dtype=np.float64), 2, 3)
         init["R"] = R.reshape(R.shape[0], R.shape[1], nx * nx)
-    given = [x0] + [t for v in lists.values() for t in v] + [t for t in init.values()]
-    given = [t for t in given if t is not None]
+    given = [t for t in [x0] + [t for v in lists.values() for t in v] + list(init.values()) if t is not None]
     if not given:
         raise CopraB200Error(-1, "lmpc_jvp needs at least one tangent")
     k = int(given[0].shape[1]) if len(given[0].shape) == 3 else 0
-    dev = next((t.device for t in given if hasattr(t, "data_ptr")), None)
-    if dev is not None:
-        import torch
-    keep = []
+    mem = _Memory(*given)
 
     def inp(a, n, what):
-        if a is None:
-            return None
-        if tuple(a.shape) != (B, k, n):
+        if a is not None and tuple(a.shape) != (B, k, n):
             raise CopraB200Error(-1, "lmpc_jvp: the %s tangent has shape %s, expected (batch, k, len) = %s"
                                  % (what, tuple(a.shape), (B, k, n)))
-        if dev is not None:
-            a = a.detach().to(device=dev, dtype=torch.float64).contiguous()
-            keep.append(a)
-            return a.data_ptr()
-        if hasattr(a, "data_ptr"):
-            raise CopraB200Error(-1, "lmpc_jvp: numpy and torch tangents cannot be mixed")
-        a = np.ascontiguousarray(np.asarray(a, dtype=np.float64))
-        keep.append(a)
-        return a.ctypes.data
+        return mem.buffer(a)
 
     t = JvpIn()
     t.ndir = k
     t.x0 = inp(x0, nx, "x0")
     lens = dict(p=plen, f=clen, lower=clen, upper=clen)
     for key, arrs in lists.items():
-        n = len(plen) if key == "p" else len(clen)
+        n = len(lens[key])
         if len(arrs) > n:
             raise CopraB200Error(-1, "lmpc_jvp: %d %s tangents for %d entries" % (len(arrs), key, n))
         arrs = arrs + [None] * (n - len(arrs))
@@ -581,53 +562,108 @@ def _jvp_call(bp, B, x0, p, f, lower, upper, call, sync=None, init=None):
                 if a is not None and bound[j] == (key == "f"):
                     raise CopraB200Error(-1, "lmpc_jvp: constraint %d has no %s vector" % (j, key))
         ptrs = (C.c_void_p * max(1, n))(*[inp(a, lens[key][j], "%s[%d]" % (key, j)) for j, a in enumerate(arrs)])
-        keep.append(ptrs)
+        mem.keep.append(ptrs)
         setattr(t, key, C.cast(ptrs, C.POINTER(C.c_void_p)))
-    ti = JvpInitialIn()
-    for key in INITIAL_KEYS:
-        setattr(ti, key, inp(init.get(key), nx * nx if key == "R" else nx, key))
+    ti = JvpInitialIn(**{key: inp(init.get(key), nx * nx if key == "R" else nx, key) for key in INITIAL_KEYS})
     nU, X = int(bp["nu"]) * int(bp["N"]), nx * (int(bp["N"]) + 1)
-    if dev is not None:
-        du = torch.empty((B, k, nU), dtype=torch.float64, device=dev)
-        dx = torch.empty((B, k, X), dtype=torch.float64, device=dev)
-        torch.cuda.synchronize(dev)
-        ptr, mem = (lambda a: a.data_ptr()), DEVICE
-    else:
-        du, dx = np.zeros((B, k, nU)), np.zeros((B, k, X))
-        ptr, mem = (lambda a: a.ctypes.data), HOST
-    try:
-        if initial:
-            call(t, ti, mem, ptr(du), ptr(dx))
-        else:
-            call(t, mem, ptr(du), ptr(dx))
-    finally:
-        if dev is not None and sync is not None:
-            sync()
+    du, dx = mem.empty(B, k, nU), mem.empty(B, k, X)
+    pu, px = mem.ptr(du), mem.ptr(dx)
+    mem.run(lambda: call(t, ti, mem.kind, pu, px) if initial else call(t, mem.kind, pu, px), sync)
     return du, dx
 
 
 def _gain_call(bp, B, steps, device, call, sync=None):
     """allocate Ku / Kx (numpy, or CUDA tensors on `device`), run `call(steps, Ku_ptr, Kx_ptr, memory)` and return them as
     (batch, nu*steps, nx) and (batch, nx*(steps+1), nx): the engine writes each instance's gain column-major"""
+    mem = _Memory(device=device)
     nx, nu = int(bp["nx"]), int(bp["nu"])
-    ru, rx = nu * int(steps), nx * (int(steps) + 1)
-    if device is not None:
-        import torch
-        ku = torch.empty((B, nx, max(ru, 0)), dtype=torch.float64, device=device)
-        kx = torch.empty((B, nx, max(rx, 0)), dtype=torch.float64, device=device)
-        torch.cuda.synchronize(device)
-        try:
-            call(int(steps), ku.data_ptr(), kx.data_ptr(), DEVICE)
-        finally:
-            if sync is not None:
-                sync()
-        return ku.transpose(1, 2).contiguous(), kx.transpose(1, 2).contiguous()
-    ku, kx = np.zeros((B, nx, max(ru, 0))), np.zeros((B, nx, max(rx, 0)))
-    call(int(steps), ku.ctypes.data, kx.ctypes.data, HOST)
-    return np.ascontiguousarray(ku.transpose(0, 2, 1)), np.ascontiguousarray(kx.transpose(0, 2, 1))
+    ku, kx = mem.empty(B, nx, max(nu * int(steps), 0)), mem.empty(B, nx, max(nx * (int(steps) + 1), 0))
+    mem.run(lambda: call(int(steps), mem.ptr(ku), mem.ptr(kx), mem.kind), sync)
+    return mem.rowmajor(ku), mem.rowmajor(kx)
 
 
-class Engine:
+class _Sensitivities:
+    """The sensitivities of the resident solve, shared by Engine and MultiEngine.  A subclass runs its C entries through
+    `_entry(memory, name, *args)` (copra_b200_<name> or copra_b200_multi_<name>, _MEM where the single-device entry takes
+    the memory kind) and names its stream synchronise `_stream_sync`; `_host_only` refuses anything but HOST numpy
+    arrays."""
+
+    _host_only = False
+    _stream_sync = None
+
+    def _resident(self, name, *inputs, device=None):
+        """the problem of the resident build"""
+        bp = self._last_bp
+        if bp is None:
+            raise CopraB200Error(-5, "%s needs a previous lmpc_run / lmpc_retarget on this engine" % name)
+        if self._host_only and (device is not None or any(hasattr(t, "data_ptr") for t in inputs)):
+            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
+        return bp
+
+    def lmpc_vjp(self, dcontrol=None, dtrajectory=None, want=VJP_WANT):
+        """Vector-Jacobian product of the last solve (copra_b200_lmpc_vjp): dcontrol (batch, nU) = dL/dcontrol and / or
+        dtrajectory (batch, X) = dL/dtrajectory, numpy arrays or CUDA float64 tensors.  Returns dict(x0=(batch, nx),
+        p=[per cost], f=[per row constraint, None for bounds], lower=/upper=[per bound constraint, None otherwise]), each
+        gradient (batch, rows) or (batch, rows x steps) for a per-step entry, of the same kind as the cotangents; a gradient
+        not in `want` is None.  Instances whose status is not 0 get zeros.
+        With "w", "M" or "N" in `want` (copra_b200_lmpc_vjp_costs, the same KKT solve) it also returns w=[(batch, rows)],
+        M=[(batch, rows, nx)] and N=[(batch, rows, nu)] per cost, None where a cost has no such matrix.
+        With "A", "B", "d", "E" or "G" in `want` (copra_b200_lmpc_vjp_model, the same KKT solve with the forward solve as a
+        second right-hand side) it also returns A=(batch, nx, nx), B=(batch, nx, nu), d=(batch, nx), and E=[(batch, rows, nx)]
+        and G=[(batch, rows, nu)] per constraint, None where a constraint has no such matrix (a trajectory bound's selector
+        has no gradient)."""
+        bp = self._resident("lmpc_vjp", dcontrol, dtrajectory)
+
+        def call(dc, dt, mem, o, co, mo):
+            if mo is not None:
+                self._entry(mem, "lmpc_vjp_model", dc, dt, _MEM, C.byref(o), co and C.byref(co), C.byref(mo))
+            elif co is None:
+                self._entry(mem, "lmpc_vjp", dc, dt, _MEM, C.byref(o))
+            else:
+                self._entry(mem, "lmpc_vjp_costs", dc, dt, _MEM, C.byref(o), C.byref(co))
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want, call, sync=self._stream_sync)
+
+    def initial_state_vjp(self, dcontrol=None, dtrajectory=None, want=None):
+        """Vector-Jacobian product of the last solve of an initial-state build (copra_b200_lmpc_vjp_initial_state): as
+        lmpc_vjp, with R=(batch, nx, nx), r=, x0lb=, x0ub=(batch, nx) as well.  x0 receives the multipliers of the x0 bounds
+        that defaulted to x0 (zeros when the build was given both x0lb and x0ub).  `want` defaults to x0, the vectors, and
+        those of R, r, x0lb and x0ub the build was given; asking for one it was not given raises (E_ARG)."""
+        bp = self._resident("initial_state_vjp", dcontrol, dtrajectory)
+        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, initial_want(bp) if want is None else want,
+                         lambda dc, dt, mem, o, io: self._entry(mem, "lmpc_vjp_initial_state", dc, dt, _MEM, C.byref(o),
+                                                                C.byref(io)),
+                         sync=self._stream_sync, initial=True)
+
+    def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
+        """Jacobian-vector product of the last solve (copra_b200_lmpc_jvp) along k tangent directions: x0 (batch, k, nx) and
+        lists indexed by cost (p) / constraint (f for row constraints, lower / upper for bounds) of (batch, k, len) tangents,
+        len as the matching lmpc_vjp gradient; None entries are zero.  numpy arrays or CUDA float64 tensors.  Returns
+        (dcontrol (batch, k, nU), dtrajectory (batch, k, X)) of the same kind.  Instances whose status is not 0 get zeros."""
+        bp = self._resident("lmpc_jvp", x0, *(p or []), *(f or []), *(lower or []), *(upper or []))
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, mem, du, dx: self._entry(mem, "lmpc_jvp", C.byref(t), _MEM, du, dx),
+                         sync=self._stream_sync)
+
+    def initial_state_jvp(self, x0=None, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
+        """Jacobian-vector product of the last solve of an initial-state build (copra_b200_lmpc_jvp_initial_state): as
+        lmpc_jvp, with tangents R (batch, k, nx, nx), r, x0lb and x0ub (batch, k, nx) as well.  The x0 tangent moves the x0
+        bounds the build was not given.  Returns (dcontrol (batch, k, nU), dtrajectory (batch, k, X))."""
+        bp = self._resident("initial_state_jvp", x0, R, r, x0lb, x0ub, *(p or []), *(f or []), *(lower or []), *(upper or []))
+        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
+                         lambda t, ti, mem, du, dx: self._entry(mem, "lmpc_jvp_initial_state", C.byref(t), C.byref(ti), _MEM,
+                                                                du, dx),
+                         sync=self._stream_sync, init=dict(R=R, r=r, x0lb=x0lb, x0ub=x0ub))
+
+    def lmpc_feedback_gain(self, steps=1, device=None):
+        """Local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): (Ku (batch, nu*steps, nx) = dU[:nu*steps]/dx0,
+        Kx (batch, nx*(steps+1), nx) = dtrajectory[:nx*(steps+1)]/dx0); numpy, or CUDA tensors on the torch `device`."""
+        bp = self._resident("lmpc_feedback_gain", device=device)
+        return _gain_call(bp, int(bp["batch"]), steps, device,
+                          lambda st, ku, kx, mem: self._entry(mem, "lmpc_feedback_gain", st, ku, kx, _MEM),
+                          sync=self._stream_sync)
+
+
+class Engine(_Sensitivities):
     """One handle == one GPU + one stream (include/copra_b200.h)."""
 
     def __init__(self, device=0, stream=None, sm_limit=0, small_variant=0):
@@ -656,6 +692,17 @@ class Engine:
     def _check(self, rc):
         if rc != 0:
             raise CopraB200Error(rc, self.lib.copra_b200_last_error(self.h).decode())
+
+    def _entry(self, memory, name, *args):
+        """copra_b200_<name> on this engine, `memory` where _MEM stands"""
+        self._check(getattr(self.lib, "copra_b200_" + name)(self.h, *[memory if a is _MEM else a for a in args]))
+
+    def _call(self, mem, name, *args):
+        """copra_b200_<name> on this engine's stream, ordered against torch's when `mem` is DEVICE memory"""
+        mem.run(lambda: self._entry(mem.kind, name, *args), self.synchronize)
+
+    def _stream_sync(self):
+        self.synchronize()
 
     def set_stream(self, stream_ptr):
         self._check(self.lib.copra_b200_set_stream(self.h, C.c_void_p(stream_ptr)))
@@ -717,57 +764,39 @@ class Engine:
         (HOST memory), or CUDA float64 tensors (DEVICE memory: the results are tensors on the same device, and the inputs are
         kept alive on this engine because qp_vjp reads them again)."""
         arrs = dict(Q=Q, c=c, Aeq=Aeq, beq=beq, Aineq=Aineq, bineq=bineq, lb=lb, ub=ub)
-        dev = next((a.device for a in arrs.values() if hasattr(a, "data_ptr")), None)
-        if dev is not None:
-            import torch
-            arrs = {k: None if a is None else torch.as_tensor(a, dtype=torch.float64, device=dev) for k, a in arrs.items()}
-        else:
-            arrs = {k: None if a is None else np.asarray(a, float) for k, a in arrs.items()}
+        mem = _Memory(*arrs.values())
+        arrs = {k: None if a is None else mem.array(a) for k, a in arrs.items()}
         n = arrs["Q"].shape[-1]
         batch = 1
         for k, a in arrs.items():
             if a is not None and a.ndim > QP_BASE_NDIM[k]:
                 batch = a.shape[0]
-        def size(a):
-            return 0 if a is None else (a.numel() if dev is not None else a.size)
-        rows = {k: int(arrs[k].shape[-2]) if size(arrs[k]) else 0 for k in ("Aeq", "Aineq")}
+
+        def given(a):
+            return a is not None and 0 not in a.shape
+        rows = {k: int(arrs[k].shape[-2]) if given(arrs[k]) else 0 for k in ("Aeq", "Aineq")}
         meq, m = rows["Aeq"], rows["Aineq"]
-        keep, cargs = [], []
+        cargs = []
         for k in QP_VJP_WANT:
             a, base = arrs[k], QP_BASE_NDIM[k]
             o = Array()
-            if size(a) and rows.get(k, 1) > 0:
-                if dev is not None:
-                    buf = (a.transpose(-1, -2) if base == 2 else a).contiguous()
-                    o.ptr = buf.data_ptr()
-                    o.stride = buf[0].numel() if a.dim() > base else 0
-                else:
-                    buf = _colmajor(a, base)
-                    o.ptr = buf.ctypes.data
-                    o.stride = int(np.prod(buf.shape[1:])) if a.ndim > base else 0
-                keep.append(buf)
+            if given(a) and rows.get(k, 1) > 0:
+                o.ptr = mem.buffer(a.swapaxes(-1, -2) if base == 2 else a)  # each instance column-major
+                o.stride = int(np.prod(a.shape[1:])) if a.ndim > base else 0
             cargs.append(o)
         self.solve_count += 1
         self._last_qp = None
-        if dev is not None:
-            x = torch.empty((batch, n), dtype=torch.float64, device=dev)
-            status, iters = torch.empty(batch, dtype=torch.int32, device=dev), torch.empty((batch, 2), dtype=torch.int32, device=dev)
-            nact, iact = torch.empty(batch, dtype=torch.int32, device=dev), torch.empty((batch, n), dtype=torch.int32, device=dev)
-            torch.cuda.synchronize(dev)
-            try:
-                self._check(self.lib.copra_b200_solve_qp_batch(self.h, n, meq, m, batch, *cargs, x.data_ptr(), status.data_ptr(),
-                                                               iters.data_ptr(), nact.data_ptr(), iact.data_ptr(), DEVICE))
-            finally:
-                self.synchronize()
-        else:
-            x = np.zeros((batch, n))
-            status, iters = np.zeros(batch, np.int32), np.zeros((batch, 2), np.int32)
-            nact, iact = np.zeros(batch, np.int32), np.zeros((batch, n), np.int32)
-            self._check(self.lib.copra_b200_solve_qp_batch(self.h, n, meq, m, batch, *cargs, x.ctypes.data, status.ctypes.data,
-                                                           iters.ctypes.data, nact.ctypes.data, iact.ctypes.data, HOST))
+        x, iters = mem.empty(batch, n), mem.empty(batch, 2, dtype=np.int32)
+        status, nact, iact = mem.empty(batch, dtype=np.int32), mem.empty(batch, dtype=np.int32), mem.empty(batch, n, dtype=np.int32)
+        self._call(mem, "solve_qp_batch", n, meq, m, batch, *cargs, *[mem.ptr(a) for a in (x, status, iters, nact, iact)], _MEM)
         # DEVICE inputs are read again by qp_vjp: they stay alive until the next raw QP batch
-        self._last_qp = dict(n=n, meq=meq, m=m, batch=batch, live=keep if dev is not None else None)
+        self._last_qp = dict(n=n, meq=meq, m=m, batch=batch, live=mem.keep if mem.device is not None else None)
         return dict(x=x, status=status, iters=iters, nact=nact, iact=iact)
+
+    def _resident_qp(self, name):
+        if getattr(self, "_last_qp", None) is None:
+            raise CopraB200Error(-5, "%s needs a previous solve_qp_batch on this engine" % name)
+        return self._last_qp
 
     def qp_vjp(self, dx, want=QP_VJP_WANT):
         """Vector-Jacobian product of the last raw QP batch (copra_b200_qp_vjp): dx (batch, n) = dL/dx, a numpy array or a
@@ -775,53 +804,30 @@ class Engine:
         Aineq=(batch, m, n), bineq=(batch, m), lb=(batch, n), ub=(batch, n)) of the same kind as dx, per instance even for
         inputs given shared; a gradient not in `want` is None, and those of absent rows (meq or m = 0) are empty.  dQ is the
         gradient along symmetric perturbations of Q.  Instances whose status is not 0 get zeros."""
-        if getattr(self, "_last_qp", None) is None:
-            raise CopraB200Error(-5, "qp_vjp needs a previous solve_qp_batch on this engine")
-        q = self._last_qp
+        q = self._resident_qp("qp_vjp")
         n, meq, m, B = q["n"], q["meq"], q["m"], q["batch"]
         # the engine writes each instance's matrices column-major: allocated as (batch, cols, rows)
         shapes = dict(Q=(n, n), c=(n,), Aeq=(n, meq), beq=(meq,), Aineq=(n, m), bineq=(m,), lb=(n,), ub=(n,))
-        dev = dx.device if hasattr(dx, "data_ptr") else None
-        o = QpVjpOut()
-        if dev is not None:
-            import torch
-            d = dx.detach().to(torch.float64).contiguous()
-            raw = {k: torch.empty((B,) + shapes[k], dtype=torch.float64, device=dev) if k in want else None for k in shapes}
-            for k, a in raw.items():
-                setattr(o, k, a.data_ptr() if a is not None and a.numel() else None)
-            torch.cuda.synchronize(dev)
-            try:
-                self._check(self.lib.copra_b200_qp_vjp(self.h, d.data_ptr(), DEVICE, C.byref(o)))
-            finally:
-                self.synchronize()
-            return {k: None if a is None else (a.transpose(1, 2).contiguous() if a.dim() == 3 else a) for k, a in raw.items()}
-        d = np.ascontiguousarray(np.asarray(dx, dtype=np.float64))
-        raw = {k: np.zeros((B,) + shapes[k]) if k in want else None for k in shapes}
-        for k, a in raw.items():
-            setattr(o, k, a.ctypes.data if a is not None and a.size else None)
-        self._check(self.lib.copra_b200_qp_vjp(self.h, d.ctypes.data, HOST, C.byref(o)))
-        return {k: None if a is None else (np.ascontiguousarray(a.transpose(0, 2, 1)) if a.ndim == 3 else a)
-                for k, a in raw.items()}
+        mem = _Memory(dx)
+        d = mem.buffer(dx)
+        raw = {k: mem.empty(B, *shapes[k]) if k in want else None for k in shapes}
+        o = QpVjpOut(**{k: mem.ptr(a) for k, a in raw.items()})
+        self._call(mem, "qp_vjp", d, _MEM, C.byref(o))
+        return {k: mem.rowmajor(a) if a is not None and a.ndim == 3 else a for k, a in raw.items()}
 
     def _qp_tangents(self, tangents):
         """check raw-QP tangents against the last batch's shapes: each is (batch, k, *base) or (k, *base) (one tangent for the
         batch), every given one with the same k.  Returns (k, {name: (array, shared)}, device or None)"""
-        if getattr(self, "_last_qp", None) is None:
-            raise CopraB200Error(-5, "qp_jvp needs a previous solve_qp_batch on this engine")
-        q = self._last_qp
+        q = self._resident_qp("qp_jvp")
         n, meq, m, B = q["n"], q["meq"], q["m"], q["batch"]
         base = dict(Q=(n, n), c=(n,), Aeq=(meq, n), beq=(meq,), Aineq=(m, n), bineq=(m,), lb=(n,), ub=(n,))
         given = {k: a for k, a in tangents.items() if a is not None}
         if not given:
             raise CopraB200Error(-1, "qp_jvp: no tangent given")
-        dev = next((a.device for a in given.values() if hasattr(a, "data_ptr")), None)
+        mem = _Memory(*given.values())
         ks, out = set(), {}
         for name, a in given.items():
-            if dev is not None:
-                import torch
-                a = torch.as_tensor(a, dtype=torch.float64, device=dev)
-            else:
-                a = np.asarray(a, dtype=np.float64)
+            a = mem.array(a)
             shape, b = tuple(a.shape), base[name]
             if len(shape) == len(b) + 2 and shape[0] == B and shape[2:] == b:
                 shared = False
@@ -836,7 +842,7 @@ class Engine:
             out[name] = (a, shared)
         if len(ks) != 1 or min(ks) < 1:
             raise CopraB200Error(-1, "qp_jvp: the tangents disagree on the number of directions k (%s)" % sorted(ks))
-        return ks.pop(), out, dev
+        return ks.pop(), out, mem.device
 
     def qp_jvp(self, Q=None, c=None, Aeq=None, beq=None, Aineq=None, bineq=None, lb=None, ub=None):
         """Jacobian-vector products of the last raw QP batch (copra_b200_qp_jvp) along k tangent directions: each tangent is
@@ -844,56 +850,31 @@ class Engine:
         tensors; None is a zero tangent.  Returns xdot (batch, k, n) of the same kind.  Q is read through its symmetric part.
         Instances whose status is not 0 get zeros."""
         k, ts, dev = self._qp_tangents(dict(Q=Q, c=c, Aeq=Aeq, beq=beq, Aineq=Aineq, bineq=bineq, lb=lb, ub=ub))
-        q = self._last_qp
-        n, B = q["n"], q["batch"]
+        q, mem = self._last_qp, _Memory(device=dev)
         t = QpJvpIn()
         t.ndir = k
-        keep = []
         for name, (a, shared) in ts.items():
             o = getattr(t, name)
-            if QP_BASE_NDIM[name] == 2:  # each direction column-major
-                a = a.transpose(-1, -2) if dev is not None else np.swapaxes(a, -1, -2)
-            buf = a.contiguous() if dev is not None else np.ascontiguousarray(a)
-            keep.append(buf)
-            o.ptr = buf.data_ptr() if dev is not None else buf.ctypes.data
-            o.stride = 0 if shared else (buf[0].numel() if dev is not None else buf[0].size)
-        if dev is not None:
-            import torch
-            dx = torch.empty((B, k, n), dtype=torch.float64, device=dev)
-            torch.cuda.synchronize(dev)
-            try:
-                self._check(self.lib.copra_b200_qp_jvp(self.h, C.byref(t), DEVICE, dx.data_ptr()))
-            finally:
-                self.synchronize()
-            return dx
-        dx = np.zeros((B, k, n))
-        self._check(self.lib.copra_b200_qp_jvp(self.h, C.byref(t), HOST, dx.ctypes.data))
+            o.ptr = mem.buffer(a.swapaxes(-1, -2) if QP_BASE_NDIM[name] == 2 else a)  # each direction column-major
+            o.stride = 0 if shared else int(np.prod(a.shape[1:]))
+        dx = mem.empty(q["batch"], k, q["n"])
+        self._call(mem, "qp_jvp", C.byref(t), _MEM, mem.ptr(dx))
         return dx
 
     def qp_jacobian(self, wrt, device=None):
         """The Jacobian of the last raw QP batch's solutions with respect to one vector input (copra_b200_qp_jacobian): wrt in
         "c", "beq", "bineq", "lb", "ub".  Returns (batch, n, len) -- numpy, or a CUDA tensor on `device`.  dx/dc is symmetric;
         the columns of inactive rows are exactly zero."""
-        if getattr(self, "_last_qp", None) is None:
-            raise CopraB200Error(-5, "qp_jacobian needs a previous solve_qp_batch on this engine")
+        q = self._resident_qp("qp_jacobian")
         if wrt not in QP_WRT:
             raise CopraB200Error(-1, "qp_jacobian: wrt must be one of %s, got %r" % (sorted(QP_WRT), wrt))
-        q = self._last_qp
-        n, B = q["n"], q["batch"]
+        n = q["n"]
         ln = dict(c=n, beq=q["meq"], bineq=q["m"], lb=n, ub=n)[wrt]
         # the engine writes each instance's n x len Jacobian column-major: allocated as (batch, len, n)
-        if device is not None:
-            import torch
-            J = torch.empty((B, ln, n), dtype=torch.float64, device=device)
-            torch.cuda.synchronize(device)
-            try:
-                self._check(self.lib.copra_b200_qp_jacobian(self.h, QP_WRT[wrt], J.data_ptr() if J.numel() else None, DEVICE))
-            finally:
-                self.synchronize()
-            return J.transpose(1, 2).contiguous()
-        J = np.zeros((B, ln, n))
-        self._check(self.lib.copra_b200_qp_jacobian(self.h, QP_WRT[wrt], J.ctypes.data if J.size else None, HOST))
-        return np.ascontiguousarray(J.transpose(0, 2, 1))
+        mem = _Memory(device=device)
+        J = mem.empty(q["batch"], ln, n)
+        self._call(mem, "qp_jacobian", QP_WRT[wrt], mem.ptr(J), _MEM)
+        return mem.rowmajor(J)
 
     # ---- K1..K7 ----
     def sizes(self, hb):
@@ -905,14 +886,7 @@ class Engine:
         """Solve a batch problem given as a workloads dict or a prepared HostBatch (HOST memory)."""
         hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
         s = self.sizes(hb)
-        B = hb.problem.batch
-        out = dict(control=np.zeros((B, s["nU"])), trajectory=np.zeros((B, s["X"])), x=np.zeros((B, s["nvar"])),
-                   status=np.full(B, -1, np.int32), iters=np.zeros((B, 2), np.int32), nact=np.zeros(B, np.int32),
-                   iact=np.zeros((B, s["nvar"]), np.int32))
-        r = Results()
-        r.memory = HOST
-        for k in want:
-            setattr(r, k, out[k].ctypes.data)
+        out, r = _result_buffers(hb.problem.batch, s, want)
         self.solve_count += 1
         self._last_bp = None
         self._check(self.lib.copra_b200_lmpc_run(self.h, C.byref(hb.problem), C.byref(r)))
@@ -942,14 +916,7 @@ class Engine:
     def lmpc_resolve(self, x0, sizes):
         """receding-horizon re-solve of the last built batch with new initial states x0 (batch, nx)"""
         x0 = np.ascontiguousarray(np.asarray(x0, dtype=np.float64))
-        B = x0.shape[0]
-        out = dict(control=np.zeros((B, sizes["nU"])), trajectory=np.zeros((B, sizes["X"])), x=np.zeros((B, sizes["nvar"])),
-                   status=np.full(B, -1, np.int32), iters=np.zeros((B, 2), np.int32), nact=np.zeros(B, np.int32),
-                   iact=np.zeros((B, sizes["nvar"]), np.int32))
-        r = Results()
-        r.memory = HOST
-        for k, v in out.items():
-            setattr(r, k, v.ctypes.data)
+        out, r = _result_buffers(x0.shape[0], sizes)
         a = Array()
         a.ptr, a.stride = x0.ctypes.data, x0.shape[1]
         self.solve_count += 1
@@ -965,79 +932,6 @@ class Engine:
         self._check(self.lib.copra_b200_lmpc_retarget(self.h, C.byref(hb.problem), C.byref(r)))
         self._last_bp = hb.bp
         return out
-
-    def lmpc_vjp(self, dcontrol=None, dtrajectory=None, want=VJP_WANT):
-        """Vector-Jacobian product of the last solve (copra_b200_lmpc_vjp): dcontrol (batch, nU) = dL/dcontrol and / or
-        dtrajectory (batch, X) = dL/dtrajectory, numpy arrays or CUDA float64 tensors.  Returns dict(x0=(batch, nx),
-        p=[per cost], f=[per row constraint, None for bounds], lower=/upper=[per bound constraint, None otherwise]), each
-        gradient (batch, rows) or (batch, rows x steps) for a per-step entry, of the same kind as the cotangents; a gradient
-        not in `want` is None.  Instances whose status is not 0 get zeros.
-        With "w", "M" or "N" in `want` (copra_b200_lmpc_vjp_costs, the same KKT solve) it also returns w=[(batch, rows)],
-        M=[(batch, rows, nx)] and N=[(batch, rows, nu)] per cost, None where a cost has no such matrix.
-        With "A", "B", "d", "E" or "G" in `want` (copra_b200_lmpc_vjp_model, the same KKT solve with the forward solve as a
-        second right-hand side) it also returns A=(batch, nx, nx), B=(batch, nx, nu), d=(batch, nx), and E=[(batch, rows, nx)]
-        and G=[(batch, rows, nu)] per constraint, None where a constraint has no such matrix (a trajectory bound's selector
-        has no gradient)."""
-        if self._last_bp is None:
-            raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run / lmpc_retarget on this engine")
-        bp = self._last_bp
-
-        def call(dc, dt, mem, o, co, mo):
-            if mo is not None:
-                self._check(self.lib.copra_b200_lmpc_vjp_model(self.h, dc, dt, mem, C.byref(o), co and C.byref(co),
-                                                               C.byref(mo)))
-            elif co is None:
-                self._check(self.lib.copra_b200_lmpc_vjp(self.h, dc, dt, mem, C.byref(o)))
-            else:
-                self._check(self.lib.copra_b200_lmpc_vjp_costs(self.h, dc, dt, mem, C.byref(o), C.byref(co)))
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want, call, sync=self.synchronize)
-
-    def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
-        """Jacobian-vector product of the last solve (copra_b200_lmpc_jvp) along k tangent directions: x0 (batch, k, nx) and
-        lists indexed by cost (p) / constraint (f for row constraints, lower / upper for bounds) of (batch, k, len) tangents,
-        len as the matching lmpc_vjp gradient; None entries are zero.  numpy arrays or CUDA float64 tensors.  Returns
-        (dcontrol (batch, k, nU), dtrajectory (batch, k, X)) of the same kind.  Instances whose status is not 0 get zeros."""
-        if self._last_bp is None:
-            raise CopraB200Error(-5, "lmpc_jvp needs a previous lmpc_run / lmpc_retarget on this engine")
-        bp = self._last_bp
-        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
-                         lambda t, mem, du, dx: self._check(self.lib.copra_b200_lmpc_jvp(self.h, C.byref(t), mem, du, dx)),
-                         sync=self.synchronize)
-
-    def initial_state_vjp(self, dcontrol=None, dtrajectory=None, want=None):
-        """Vector-Jacobian product of the last solve of an initial-state build (copra_b200_lmpc_vjp_initial_state): as
-        lmpc_vjp, with R=(batch, nx, nx), r=, x0lb=, x0ub=(batch, nx) as well.  x0 receives the multipliers of the x0 bounds
-        that defaulted to x0 (zeros when the build was given both x0lb and x0ub).  `want` defaults to x0, the vectors, and
-        those of R, r, x0lb and x0ub the build was given; asking for one it was not given raises (E_ARG)."""
-        if self._last_bp is None:
-            raise CopraB200Error(-5, "initial_state_vjp needs a previous lmpc_run on this engine")
-        bp = self._last_bp
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, initial_want(bp) if want is None else want,
-                         lambda dc, dt, mem, o, io: self._check(self.lib.copra_b200_lmpc_vjp_initial_state(
-                             self.h, dc, dt, mem, C.byref(o), C.byref(io))),
-                         sync=self.synchronize, initial=True)
-
-    def initial_state_jvp(self, x0=None, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
-        """Jacobian-vector product of the last solve of an initial-state build (copra_b200_lmpc_jvp_initial_state): as
-        lmpc_jvp, with tangents R (batch, k, nx, nx), r, x0lb and x0ub (batch, k, nx) as well.  The x0 tangent moves the x0
-        bounds the build was not given.  Returns (dcontrol (batch, k, nU), dtrajectory (batch, k, X))."""
-        if self._last_bp is None:
-            raise CopraB200Error(-5, "initial_state_jvp needs a previous lmpc_run on this engine")
-        bp = self._last_bp
-        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
-                         lambda t, ti, mem, du, dx: self._check(self.lib.copra_b200_lmpc_jvp_initial_state(
-                             self.h, C.byref(t), C.byref(ti), mem, du, dx)),
-                         sync=self.synchronize, init=dict(R=R, r=r, x0lb=x0lb, x0ub=x0ub))
-
-    def lmpc_feedback_gain(self, steps=1, device=None):
-        """Local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): (Ku (batch, nu*steps, nx) = dU[:nu*steps]/dx0,
-        Kx (batch, nx*(steps+1), nx) = dtrajectory[:nx*(steps+1)]/dx0); numpy, or CUDA tensors on the torch `device`."""
-        if self._last_bp is None:
-            raise CopraB200Error(-5, "lmpc_feedback_gain needs a previous lmpc_run / lmpc_retarget on this engine")
-        bp = self._last_bp
-        return _gain_call(bp, int(bp["batch"]), steps, device,
-                          lambda st, ku, kx, mem: self._check(self.lib.copra_b200_lmpc_feedback_gain(self.h, st, ku, kx, mem)),
-                          sync=self.synchronize)
 
     def lmpc_build(self, hb):
         self._last_bp = None
@@ -1060,13 +954,17 @@ class Engine:
         return np.swapaxes(buf, 1, 2) if len(shp) == 2 else buf
 
 
-class MultiEngine:
+class MultiEngine(_Sensitivities):
     """Data-parallel sharder (copra_b200_multi_*): one engine handle + host thread per listed device, the batch split
-    into contiguous instance ranges, results gathered by DMA into the caller's buffers."""
+    into contiguous instance ranges, results gathered by DMA into the caller's buffers.  The sensitivity methods are
+    Engine's over the shards of the last run, on HOST numpy arrays holding the whole batch."""
+
+    _host_only = True  # each shard is copied to its own device
 
     def __init__(self, devices=None):
         self.lib = load()
         self.m = C.c_void_p()
+        self._last_bp = None
         if devices is None:
             rc = self.lib.copra_b200_multi_create(None, 0, C.byref(self.m))
         else:
@@ -1111,92 +1009,20 @@ class MultiEngine:
         d["wall_ms"] = w.value
         return d
 
-    @staticmethod
-    def _outputs(B, s):
-        return dict(control=np.zeros((B, s["nU"])), trajectory=np.zeros((B, s["X"])), x=np.zeros((B, s["nvar"])),
-                    status=np.full(B, -1, np.int32), iters=np.zeros((B, 2), np.int32), nact=np.zeros(B, np.int32),
-                    iact=np.zeros((B, s["nvar"]), np.int32))
+    def _entry(self, memory, name, *args):
+        """copra_b200_multi_<name> over the shards of the last run (HOST arrays only: the entry has no memory argument)"""
+        self._check(getattr(self.lib, "copra_b200_multi_" + name)(self.m, *[a for a in args if a is not _MEM]))
 
     def lmpc_run(self, bp_or_hb, sizes, results=None):
         """`sizes` from Engine.sizes(); `results` an optional prepared ctypes Results (e.g. pinned torch buffers)."""
         hb = bp_or_hb if isinstance(bp_or_hb, HostBatch) else HostBatch(bp_or_hb)
-        if results is not None:
-            self._check(self.lib.copra_b200_multi_lmpc_run(self.m, C.byref(hb.problem), C.byref(results)))
-            self._last_bp = hb.bp
-            return None
-        out = self._outputs(hb.problem.batch, sizes)
-        r = Results()
-        r.memory = HOST
-        for k, v in out.items():
-            setattr(r, k, v.ctypes.data)
+        out, r = (None, results) if results is not None else _result_buffers(hb.problem.batch, sizes)
         self._check(self.lib.copra_b200_multi_lmpc_run(self.m, C.byref(hb.problem), C.byref(r)))
         self._last_bp = hb.bp
         return out
 
-    def lmpc_vjp(self, dcontrol=None, dtrajectory=None, want=VJP_WANT):
-        """Engine.lmpc_vjp over the shards of the last run (numpy arrays holding the whole batch)"""
-        bp = getattr(self, "_last_bp", None)
-        if bp is None:
-            raise CopraB200Error(-5, "lmpc_vjp needs a previous lmpc_run on this engine")
-        if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
-            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
-
-        def call(dc, dt, mem, o, co, mo):
-            if mo is not None:
-                self._check(self.lib.copra_b200_multi_lmpc_vjp_model(self.m, dc, dt, C.byref(o), co and C.byref(co),
-                                                                     C.byref(mo)))
-            elif co is None:
-                self._check(self.lib.copra_b200_multi_lmpc_vjp(self.m, dc, dt, C.byref(o)))
-            else:
-                self._check(self.lib.copra_b200_multi_lmpc_vjp_costs(self.m, dc, dt, C.byref(o), C.byref(co)))
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, want, call)
-
-    def lmpc_jvp(self, x0=None, p=None, f=None, lower=None, upper=None):
-        """Engine.lmpc_jvp over the shards of the last run (numpy arrays holding the whole batch)"""
-        bp = getattr(self, "_last_bp", None)
-        if bp is None:
-            raise CopraB200Error(-5, "lmpc_jvp needs a previous lmpc_run on this engine")
-        tangents = [x0] + list(p or []) + list(f or []) + list(lower or []) + list(upper or [])
-        if any(hasattr(t, "data_ptr") for t in tangents):
-            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
-        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
-                         lambda t, mem, du, dx: self._check(self.lib.copra_b200_multi_lmpc_jvp(self.m, C.byref(t), du, dx)))
-
-    def initial_state_vjp(self, dcontrol=None, dtrajectory=None, want=None):
-        """Engine.initial_state_vjp over the shards of the last run (numpy arrays holding the whole batch)"""
-        bp = getattr(self, "_last_bp", None)
-        if bp is None:
-            raise CopraB200Error(-5, "initial_state_vjp needs a previous lmpc_run on this engine")
-        if any(hasattr(t, "data_ptr") for t in (dcontrol, dtrajectory)):
-            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
-        return _vjp_call(bp, int(bp["batch"]), dcontrol, dtrajectory, initial_want(bp) if want is None else want,
-                         lambda dc, dt, mem, o, io: self._check(self.lib.copra_b200_multi_lmpc_vjp_initial_state(
-                             self.m, dc, dt, C.byref(o), C.byref(io))), initial=True)
-
-    def initial_state_jvp(self, x0=None, R=None, r=None, x0lb=None, x0ub=None, p=None, f=None, lower=None, upper=None):
-        """Engine.initial_state_jvp over the shards of the last run (numpy arrays holding the whole batch)"""
-        bp = getattr(self, "_last_bp", None)
-        if bp is None:
-            raise CopraB200Error(-5, "initial_state_jvp needs a previous lmpc_run on this engine")
-        tangents = [x0, R, r, x0lb, x0ub] + list(p or []) + list(f or []) + list(lower or []) + list(upper or [])
-        if any(hasattr(t, "data_ptr") for t in tangents):
-            raise CopraB200Error(-1, "the multi-device entry takes HOST numpy arrays (each shard is copied to its own device)")
-        return _jvp_call(bp, int(bp["batch"]), x0, p, f, lower, upper,
-                         lambda t, ti, mem, du, dx: self._check(self.lib.copra_b200_multi_lmpc_jvp_initial_state(
-                             self.m, C.byref(t), C.byref(ti), du, dx)), init=dict(R=R, r=r, x0lb=x0lb, x0ub=x0ub))
-
-    def lmpc_feedback_gain(self, steps=1):
-        """Engine.lmpc_feedback_gain over the shards of the last run (numpy arrays holding the whole batch)"""
-        bp = getattr(self, "_last_bp", None)
-        if bp is None:
-            raise CopraB200Error(-5, "lmpc_feedback_gain needs a previous lmpc_run on this engine")
-        return _gain_call(bp, int(bp["batch"]), steps, None,
-                          lambda st, ku, kx, mem: self._check(self.lib.copra_b200_multi_lmpc_feedback_gain(self.m, st, ku, kx)))
-
     def set_warm_start(self, on=True):
-        rc = self.lib.copra_b200_multi_set_warm_start(self.m, 1 if on else 0)
-        if rc:
-            raise CopraB200Error("copra_b200_multi_set_warm_start failed (%d)" % rc)
+        self._check(self.lib.copra_b200_multi_set_warm_start(self.m, 1 if on else 0))
 
     def lmpc_retarget(self, bp_or_hb, sizes):
         """copra_b200_lmpc_retarget on every shard of the last run"""
@@ -1207,11 +1033,7 @@ class MultiEngine:
 
     def lmpc_resolve(self, x0, sizes):
         x0 = np.ascontiguousarray(np.asarray(x0, dtype=np.float64))
-        out = self._outputs(x0.shape[0], sizes)
-        r = Results()
-        r.memory = HOST
-        for k, v in out.items():
-            setattr(r, k, v.ctypes.data)
+        out, r = _result_buffers(x0.shape[0], sizes)
         a = Array()
         a.ptr, a.stride = x0.ctypes.data, x0.shape[1]
         self._check(self.lib.copra_b200_multi_lmpc_resolve(self.m, a, C.byref(r)))

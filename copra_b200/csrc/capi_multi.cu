@@ -60,53 +60,6 @@ template <class F> int run_shards(copra_b200_multi* m, F body)
     return 0;
 }
 
-// a copra_b200_vjp_out of whole-batch arrays advanced to instance lo of a shard (nx, plen, clen: cb_vjp_lengths)
-struct VjpOutSlice {
-    std::vector<double*> p, f, lower, upper;
-    copra_b200_vjp_out o{};
-    VjpOutSlice(const copra_b200_vjp_out& out, long long lo, int nx, const std::vector<int>& plen, const std::vector<int>& clen)
-        : p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size())
-    {
-        for (size_t i = 0; i < plen.size(); ++i) p[i] = (out.p && out.p[i]) ? out.p[i] + lo * plen[i] : nullptr;
-        for (size_t i = 0; i < clen.size(); ++i) {
-            f[i] = (out.f && out.f[i]) ? out.f[i] + lo * clen[i] : nullptr;
-            lower[i] = (out.lower && out.lower[i]) ? out.lower[i] + lo * clen[i] : nullptr;
-            upper[i] = (out.upper && out.upper[i]) ? out.upper[i] + lo * clen[i] : nullptr;
-        }
-        o.x0 = out.x0 ? out.x0 + lo * nx : nullptr;
-        o.p = out.p ? p.data() : nullptr;
-        o.f = out.f ? f.data() : nullptr;
-        o.lower = out.lower ? lower.data() : nullptr;
-        o.upper = out.upper ? upper.data() : nullptr;
-    }
-};
-
-// a copra_b200_jvp_in of whole-batch tangents (len x k per instance) advanced to instance lo of a shard
-struct JvpInSlice {
-    std::vector<const double*> p, f, lower, upper;
-    copra_b200_jvp_in t{};
-    JvpInSlice(const copra_b200_jvp_in& in, long long lo, int nx, const std::vector<int>& plen, const std::vector<int>& clen)
-        : p(plen.size()), f(clen.size()), lower(clen.size()), upper(clen.size())
-    {
-        const long long k = in.ndir;
-        auto at = [&](const double* const* arr, size_t i, int len) -> const double* {
-            return (arr && arr[i]) ? arr[i] + lo * len * k : nullptr;
-        };
-        for (size_t i = 0; i < plen.size(); ++i) p[i] = at(in.p, i, plen[i]);
-        for (size_t i = 0; i < clen.size(); ++i) {
-            f[i] = at(in.f, i, clen[i]);
-            lower[i] = at(in.lower, i, clen[i]);
-            upper[i] = at(in.upper, i, clen[i]);
-        }
-        t = in;
-        t.x0 = in.x0 ? in.x0 + lo * nx * k : nullptr;
-        t.p = in.p ? p.data() : nullptr;
-        t.f = in.f ? f.data() : nullptr;
-        t.lower = in.lower ? lower.data() : nullptr;
-        t.upper = in.upper ? upper.data() : nullptr;
-    }
-};
-
 } // namespace
 
 // per-instance lengths of x0 and of every cost's p / constraint's vector of the resident build (capi.cu)
@@ -115,6 +68,131 @@ void cb_vjp_lengths(const copra_b200_handle* h, int& nx, std::vector<int>& cost_
 void cb_cost_shapes(const copra_b200_handle* h, int& nu, std::vector<int>& rows);
 // the rows of every row constraint's E / G of the resident build, 0 for a bound (capi.cu)
 void cb_cstr_rows(const copra_b200_handle* h, std::vector<int>& rows);
+
+namespace {
+
+// the per-instance shapes of a shard's resident build: nx, nu, the lengths of every cost's p and every constraint's
+// vector, the rows of every cost and of every row constraint's E / G (0 for a bound)
+struct ShardShapes {
+    int nx = 0, nu = 0;
+    std::vector<int> plen, clen, cost_rows, cstr_rows;
+    explicit ShardShapes(const copra_b200_handle* h)
+    {
+        cb_vjp_lengths(h, nx, plen, clen);
+        cb_cost_shapes(h, nu, cost_rows);
+        cb_cstr_rows(h, cstr_rows);
+    }
+};
+
+// arr[i] + lo * len[i] * k for every entry i of a whole-batch pointer array (null stays null)
+template <class T> std::vector<T*> advance(T* const* arr, const std::vector<int>& len, long long lo, long long k = 1)
+{
+    std::vector<T*> out(len.size());
+    for (size_t i = 0; i < len.size(); ++i) out[i] = (arr && arr[i]) ? arr[i] + lo * len[i] * k : nullptr;
+    return out;
+}
+
+// Runs a VJP over the shards: the whole-batch cotangents and outputs (vectors; cost, model and initial-state gradients
+// where asked for) are advanced to each shard's first instance and handed to copra_b200_lmpc_vjp_initial_state when
+// `initial`, to copra_b200_lmpc_vjp_model otherwise.  `name` is the entry's name in the error strings.
+int multi_vjp(copra_b200_multi* m, const char* name, bool initial, const double* dcontrol, const double* dtrajectory,
+    const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model,
+    const copra_b200_vjp_initial_out* init)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!initial && !out && !costs && !model) return mfail(m, COPRA_B200_E_ARG, std::string(name) + ": null output description");
+    static const copra_b200_vjp_out none{};
+    if (!out) out = &none;
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, std::string("copra_b200_multi_") + name + " needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        const ShardShapes s(m->h[g]);
+        const int nx = s.nx, nu = s.nu;
+        const long long lo = m->lo[g];
+        std::vector<double*> p = advance(out->p, s.plen, lo), f = advance(out->f, s.clen, lo),
+                             lower = advance(out->lower, s.clen, lo), upper = advance(out->upper, s.clen, lo);
+        copra_b200_vjp_out o{};
+        o.x0 = out->x0 ? out->x0 + lo * nx : nullptr;
+        o.p = out->p ? p.data() : nullptr;
+        o.f = out->f ? f.data() : nullptr;
+        o.lower = out->lower ? lower.data() : nullptr;
+        o.upper = out->upper ? upper.data() : nullptr;
+        // the cost gradients: rows, rows x nx and rows x nu per instance
+        std::vector<double*> cw, cM, cN;
+        copra_b200_vjp_cost_out co{};
+        if (costs) {
+            cw = advance(costs->w, s.cost_rows, lo), cM = advance(costs->M, s.cost_rows, lo, nx);
+            cN = advance(costs->N, s.cost_rows, lo, nu);
+            co.w = costs->w ? cw.data() : nullptr;
+            co.M = costs->M ? cM.data() : nullptr;
+            co.N = costs->N ? cN.data() : nullptr;
+        }
+        // the model gradients: nx x nx, nx x nu, nx, and rows x nx / rows x nu per row constraint
+        std::vector<double*> mE, mG;
+        copra_b200_vjp_model_out mo{};
+        if (model) {
+            mE = advance(model->E, s.cstr_rows, lo, nx), mG = advance(model->G, s.cstr_rows, lo, nu);
+            mo.A = model->A ? model->A + lo * nx * nx : nullptr;
+            mo.B = model->B ? model->B + lo * nx * nu : nullptr;
+            mo.d = model->d ? model->d + lo * nx : nullptr;
+            mo.E = model->E ? mE.data() : nullptr;
+            mo.G = model->G ? mG.data() : nullptr;
+        }
+        // the initial-state gradients: nx x nx, nx, nx, nx
+        copra_b200_vjp_initial_out io{};
+        if (init) {
+            io.R = init->R ? init->R + lo * nx * nx : nullptr;
+            io.r = init->r ? init->r + lo * nx : nullptr;
+            io.x0lb = init->x0lb ? init->x0lb + lo * nx : nullptr;
+            io.x0ub = init->x0ub ? init->x0ub + lo * nx : nullptr;
+        }
+        const double* dc = dcontrol ? dcontrol + lo * sz.nU : nullptr;
+        const double* dt = dtrajectory ? dtrajectory + lo * sz.X : nullptr;
+        if (initial) return copra_b200_lmpc_vjp_initial_state(m->h[g], dc, dt, COPRA_B200_HOST, &o, init ? &io : nullptr);
+        return copra_b200_lmpc_vjp_model(m->h[g], dc, dt, COPRA_B200_HOST, &o, costs ? &co : nullptr, model ? &mo : nullptr);
+    });
+}
+
+// Runs a JVP over the shards: the whole-batch tangents (len x k per instance: vectors, and R, r, x0lb, x0ub where given)
+// and outputs are advanced to each shard's first instance and handed to copra_b200_lmpc_jvp_initial_state when
+// `initial`, to copra_b200_lmpc_jvp otherwise.  `name` is the entry's name in the error strings.
+int multi_jvp(copra_b200_multi* m, const char* name, bool initial, const copra_b200_jvp_in* in,
+    const copra_b200_jvp_initial_in* init, double* dcontrol, double* dtrajectory)
+{
+    if (!m) return COPRA_B200_E_ARG;
+    if (!in) return mfail(m, COPRA_B200_E_ARG, std::string(name) + ": null tangent description");
+    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, std::string("copra_b200_multi_") + name + " needs a previous run");
+    return run_shards(m, [&](int g) {
+        copra_b200_sizes sz{};
+        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
+        if (rc) return rc;
+        const ShardShapes s(m->h[g]);
+        const long long nx = s.nx, lo = m->lo[g], k = in->ndir;
+        std::vector<const double*> p = advance(in->p, s.plen, lo, k), f = advance(in->f, s.clen, lo, k),
+                                   lower = advance(in->lower, s.clen, lo, k), upper = advance(in->upper, s.clen, lo, k);
+        copra_b200_jvp_in t = *in;
+        t.x0 = in->x0 ? in->x0 + lo * nx * k : nullptr;
+        t.p = in->p ? p.data() : nullptr;
+        t.f = in->f ? f.data() : nullptr;
+        t.lower = in->lower ? lower.data() : nullptr;
+        t.upper = in->upper ? upper.data() : nullptr;
+        copra_b200_jvp_initial_in ti{};
+        if (init) {
+            ti.R = init->R ? init->R + lo * nx * nx * k : nullptr;
+            ti.r = init->r ? init->r + lo * nx * k : nullptr;
+            ti.x0lb = init->x0lb ? init->x0lb + lo * nx * k : nullptr;
+            ti.x0ub = init->x0ub ? init->x0ub + lo * nx * k : nullptr;
+        }
+        double* du = dcontrol ? dcontrol + lo * sz.nU * k : nullptr;
+        double* dx = dtrajectory ? dtrajectory + lo * sz.X * k : nullptr;
+        if (initial) return copra_b200_lmpc_jvp_initial_state(m->h[g], &t, init ? &ti : nullptr, COPRA_B200_HOST, du, dx);
+        return copra_b200_lmpc_jvp(m->h[g], &t, COPRA_B200_HOST, du, dx);
+    });
+}
+
+} // namespace
 
 extern "C" {
 
@@ -259,132 +337,24 @@ int copra_b200_multi_lmpc_vjp_costs(copra_b200_multi* m, const double* dcontrol,
 int copra_b200_multi_lmpc_vjp_model(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
     const copra_b200_vjp_out* out, const copra_b200_vjp_cost_out* costs, const copra_b200_vjp_model_out* model)
 {
-    if (!m) return COPRA_B200_E_ARG;
-    if (!out && !costs && !model) return mfail(m, COPRA_B200_E_ARG, "lmpc_vjp: null output description");
-    static const copra_b200_vjp_out none{};
-    if (!out) out = &none;
-    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp needs a previous run");
-    return run_shards(m, [&](int g) {
-        copra_b200_sizes sz{};
-        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
-        if (rc) return rc;
-        std::vector<int> plen, clen;
-        int nx = 0;
-        cb_vjp_lengths(m->h[g], nx, plen, clen);
-        const long long lo = m->lo[g];
-        // every array of the whole batch, advanced to this shard's first instance
-        VjpOutSlice os(*out, lo, nx, plen, clen);
-        const copra_b200_vjp_out& o = os.o;
-        // the cost gradients likewise: rows, rows x nx and rows x nu per instance
-        int nu = 0;
-        std::vector<int> rows;
-        cb_cost_shapes(m->h[g], nu, rows);
-        std::vector<double*> cw(rows.size()), cM(rows.size()), cN(rows.size());
-        for (size_t i = 0; i < rows.size() && costs; ++i) {
-            cw[i] = (costs->w && costs->w[i]) ? costs->w[i] + lo * rows[i] : nullptr;
-            cM[i] = (costs->M && costs->M[i]) ? costs->M[i] + lo * rows[i] * nx : nullptr;
-            cN[i] = (costs->N && costs->N[i]) ? costs->N[i] + lo * rows[i] * nu : nullptr;
-        }
-        copra_b200_vjp_cost_out co{};
-        if (costs) {
-            co.w = costs->w ? cw.data() : nullptr;
-            co.M = costs->M ? cM.data() : nullptr;
-            co.N = costs->N ? cN.data() : nullptr;
-        }
-        // and the model gradients: nx x nx, nx x nu, nx, and rows x nx / rows x nu per row constraint
-        std::vector<int> crows;
-        cb_cstr_rows(m->h[g], crows);
-        std::vector<double*> mE(crows.size()), mG(crows.size());
-        for (size_t i = 0; i < crows.size() && model; ++i) {
-            mE[i] = (model->E && model->E[i]) ? model->E[i] + lo * crows[i] * nx : nullptr;
-            mG[i] = (model->G && model->G[i]) ? model->G[i] + lo * crows[i] * nu : nullptr;
-        }
-        copra_b200_vjp_model_out mo{};
-        if (model) {
-            mo.A = model->A ? model->A + lo * nx * nx : nullptr;
-            mo.B = model->B ? model->B + lo * nx * nu : nullptr;
-            mo.d = model->d ? model->d + lo * nx : nullptr;
-            mo.E = model->E ? mE.data() : nullptr;
-            mo.G = model->G ? mG.data() : nullptr;
-        }
-        return copra_b200_lmpc_vjp_model(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
-            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &o, costs ? &co : nullptr, model ? &mo : nullptr);
-    });
+    return multi_vjp(m, "lmpc_vjp", false, dcontrol, dtrajectory, out, costs, model, nullptr);
 }
 
 int copra_b200_multi_lmpc_jvp(copra_b200_multi* m, const copra_b200_jvp_in* in, double* dcontrol, double* dtrajectory)
 {
-    if (!m) return COPRA_B200_E_ARG;
-    if (!in) return mfail(m, COPRA_B200_E_ARG, "lmpc_jvp: null tangent description");
-    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_jvp needs a previous run");
-    return run_shards(m, [&](int g) {
-        copra_b200_sizes sz{};
-        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
-        if (rc) return rc;
-        std::vector<int> plen, clen;
-        int nx = 0;
-        cb_vjp_lengths(m->h[g], nx, plen, clen);
-        const long long lo = m->lo[g], k = in->ndir;
-        // every array of the whole batch (len x k per instance), advanced to this shard's first instance
-        JvpInSlice ts(*in, lo, nx, plen, clen);
-        return copra_b200_lmpc_jvp(m->h[g], &ts.t, COPRA_B200_HOST, dcontrol ? dcontrol + lo * sz.nU * k : nullptr,
-            dtrajectory ? dtrajectory + lo * sz.X * k : nullptr);
-    });
+    return multi_jvp(m, "lmpc_jvp", false, in, nullptr, dcontrol, dtrajectory);
 }
 
 int copra_b200_multi_lmpc_vjp_initial_state(copra_b200_multi* m, const double* dcontrol, const double* dtrajectory,
     const copra_b200_vjp_out* out, const copra_b200_vjp_initial_out* init)
 {
-    if (!m) return COPRA_B200_E_ARG;
-    static const copra_b200_vjp_out none{};
-    if (!out) out = &none;
-    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_vjp_initial_state needs a previous run");
-    return run_shards(m, [&](int g) {
-        copra_b200_sizes sz{};
-        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
-        if (rc) return rc;
-        std::vector<int> plen, clen;
-        int nx = 0;
-        cb_vjp_lengths(m->h[g], nx, plen, clen);
-        const long long lo = m->lo[g];
-        VjpOutSlice os(*out, lo, nx, plen, clen);
-        copra_b200_vjp_initial_out io{};
-        if (init) {
-            io.R = init->R ? init->R + lo * nx * nx : nullptr;
-            io.r = init->r ? init->r + lo * nx : nullptr;
-            io.x0lb = init->x0lb ? init->x0lb + lo * nx : nullptr;
-            io.x0ub = init->x0ub ? init->x0ub + lo * nx : nullptr;
-        }
-        return copra_b200_lmpc_vjp_initial_state(m->h[g], dcontrol ? dcontrol + lo * sz.nU : nullptr,
-            dtrajectory ? dtrajectory + lo * sz.X : nullptr, COPRA_B200_HOST, &os.o, init ? &io : nullptr);
-    });
+    return multi_vjp(m, "lmpc_vjp_initial_state", true, dcontrol, dtrajectory, out, nullptr, nullptr, init);
 }
 
 int copra_b200_multi_lmpc_jvp_initial_state(copra_b200_multi* m, const copra_b200_jvp_in* in, const copra_b200_jvp_initial_in* init,
     double* dcontrol, double* dtrajectory)
 {
-    if (!m) return COPRA_B200_E_ARG;
-    if (!in) return mfail(m, COPRA_B200_E_ARG, "lmpc_jvp_initial_state: null tangent description");
-    if (m->lo.size() != m->h.size()) return mfail(m, COPRA_B200_E_STATE, "copra_b200_multi_lmpc_jvp_initial_state needs a previous run");
-    return run_shards(m, [&](int g) {
-        copra_b200_sizes sz{};
-        int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
-        if (rc) return rc;
-        std::vector<int> plen, clen;
-        int nx = 0;
-        cb_vjp_lengths(m->h[g], nx, plen, clen);
-        const long long lo = m->lo[g], k = in->ndir;
-        JvpInSlice ts(*in, lo, nx, plen, clen);
-        copra_b200_jvp_initial_in ti{};
-        if (init) {
-            ti.R = init->R ? init->R + lo * nx * nx * k : nullptr;
-            ti.r = init->r ? init->r + lo * nx * k : nullptr;
-            ti.x0lb = init->x0lb ? init->x0lb + lo * nx * k : nullptr;
-            ti.x0ub = init->x0ub ? init->x0ub + lo * nx * k : nullptr;
-        }
-        return copra_b200_lmpc_jvp_initial_state(m->h[g], &ts.t, init ? &ti : nullptr, COPRA_B200_HOST,
-            dcontrol ? dcontrol + lo * sz.nU * k : nullptr, dtrajectory ? dtrajectory + lo * sz.X * k : nullptr);
-    });
+    return multi_jvp(m, "lmpc_jvp_initial_state", true, in, init, dcontrol, dtrajectory);
 }
 
 int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* Ku, double* Kx)
@@ -395,9 +365,7 @@ int copra_b200_multi_lmpc_feedback_gain(copra_b200_multi* m, int steps, double* 
         copra_b200_sizes sz{};
         int rc = copra_b200_lmpc_built_sizes(m->h[g], &sz);
         if (rc) return rc;
-        std::vector<int> plen, clen;
-        int nx = 0;
-        cb_vjp_lengths(m->h[g], nx, plen, clen);
+        const int nx = ShardShapes(m->h[g]).nx;
         const int N = sz.X / nx - 1, nu = N > 0 ? sz.nU / N : 0;
         if (steps < 1 || steps > N) return copra_b200_lmpc_feedback_gain(m->h[g], steps, nullptr, nullptr, COPRA_B200_HOST); // E_ARG
         const long long lo = m->lo[g];

@@ -1211,37 +1211,18 @@ public:
     // output may be null).  Errors as vjp, plus std::domain_error for in.ndir < 1.
     void jvp(const copra_b200_jvp_in& in, double* dcontrol, double* dtrajectory)
     {
-        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::jvp takes HOST arrays");
-        if (multi_) {
-            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::jvp needs a previous solve");
-            const int rc = copra_b200_multi_lmpc_jvp(multi_, &in, dcontrol, dtrajectory);
-            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
-            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
-            return;
-        }
-        if (myEpoch_ != b200::buildEpoch()) throw std::runtime_error("BatchedLMPC::jvp: another controller has built on the engine since this solve");
-        const int rc = copra_b200_lmpc_jvp(b200::handle(), &in, COPRA_B200_HOST, dcontrol, dtrajectory);
-        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
-        b200::check(rc);
+        sensGuard("jvp", false);
+        sensCheck(multi_ ? copra_b200_multi_lmpc_jvp(multi_, &in, dcontrol, dtrajectory)
+                         : copra_b200_lmpc_jvp(b200::handle(), &in, COPRA_B200_HOST, dcontrol, dtrajectory));
     }
     // The local feedback gain of the last solve (copra_b200_lmpc_feedback_gain): Ku = dU[0 : nu*steps]/dx0 ((nu*steps) x nx
     // per instance) and Kx = dtrajectory[0 : nx*(steps+1)]/dx0 ((nx*(steps+1)) x nx), column-major, batch-major HOST arrays;
     // either may be null.  Errors as jvp, with std::domain_error for steps outside [1, N].
     void feedbackGain(int steps, double* Ku, double* Kx)
     {
-        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::feedbackGain takes HOST arrays");
-        if (multi_) {
-            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::feedbackGain needs a previous solve");
-            const int rc = copra_b200_multi_lmpc_feedback_gain(multi_, steps, Ku, Kx);
-            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
-            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
-            return;
-        }
-        if (myEpoch_ != b200::buildEpoch())
-            throw std::runtime_error("BatchedLMPC::feedbackGain: another controller has built on the engine since this solve");
-        const int rc = copra_b200_lmpc_feedback_gain(b200::handle(), steps, Ku, Kx, COPRA_B200_HOST);
-        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
-        b200::check(rc);
+        sensGuard("feedbackGain", false);
+        sensCheck(multi_ ? copra_b200_multi_lmpc_feedback_gain(multi_, steps, Ku, Kx)
+                         : copra_b200_lmpc_feedback_gain(b200::handle(), steps, Ku, Kx, COPRA_B200_HOST));
     }
     // Sensitivities of the last solve of an initial-state controller (copra_b200_lmpc_vjp_initial_state): the vector-Jacobian
     // product with respect to x0 (through the x0 bounds that default to it) and every entry's vectors (`out`), and to R, r,
@@ -1252,20 +1233,18 @@ public:
     void initialStateVjp(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out,
         const copra_b200_vjp_initial_out& init)
     {
-        initialStateGuard("initialStateVjp");
-        const int rc = multi_ ? copra_b200_multi_lmpc_vjp_initial_state(multi_, dcontrol, dtrajectory, &out, &init)
-                              : copra_b200_lmpc_vjp_initial_state(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, &init);
-        initialStateCheck(rc);
+        sensGuard("initialStateVjp", true);
+        sensCheck(multi_ ? copra_b200_multi_lmpc_vjp_initial_state(multi_, dcontrol, dtrajectory, &out, &init)
+                         : copra_b200_lmpc_vjp_initial_state(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, &init));
     }
     // Forward mode of the same (copra_b200_lmpc_jvp_initial_state): dU (nU x k per instance) and dtrajectory (X x k) along the
     // in.ndir tangent directions of `in` and `init` (R: nx x nx x k, r / x0lb / x0ub: nx x k per instance; null = zero).
     // Errors as initialStateVjp, plus std::domain_error for in.ndir < 1.
     void initialStateJvp(const copra_b200_jvp_in& in, const copra_b200_jvp_initial_in& init, double* dcontrol, double* dtrajectory)
     {
-        initialStateGuard("initialStateJvp");
-        const int rc = multi_ ? copra_b200_multi_lmpc_jvp_initial_state(multi_, &in, &init, dcontrol, dtrajectory)
-                              : copra_b200_lmpc_jvp_initial_state(b200::handle(), &in, &init, COPRA_B200_HOST, dcontrol, dtrajectory);
-        initialStateCheck(rc);
+        sensGuard("initialStateJvp", true);
+        sensCheck(multi_ ? copra_b200_multi_lmpc_jvp_initial_state(multi_, &in, &init, dcontrol, dtrajectory)
+                         : copra_b200_lmpc_jvp_initial_state(b200::handle(), &in, &init, COPRA_B200_HOST, dcontrol, dtrajectory));
     }
     const std::vector<double>& controls() const { return controls_; }         // nU x batch, column-major
     const std::vector<double>& trajectories() const { return trajectories_; } // X x batch
@@ -1287,31 +1266,28 @@ private:
     void vjpImpl(const double* dcontrol, const double* dtrajectory, const copra_b200_vjp_out& out, const copra_b200_vjp_cost_out* costs,
         const copra_b200_vjp_model_out* model)
     {
-        if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR("BatchedLMPC::vjp takes HOST arrays");
-        if (multi_) {
-            if (!multiBuilt_) throw std::runtime_error("BatchedLMPC::vjp needs a previous solve");
-            const int rc = copra_b200_multi_lmpc_vjp_model(multi_, dcontrol, dtrajectory, &out, costs, model);
-            if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_multi_last_error(multi_));
-            if (rc) throw std::runtime_error(copra_b200_multi_last_error(multi_));
-            return;
-        }
-        if (myEpoch_ != b200::buildEpoch()) throw std::runtime_error("BatchedLMPC::vjp: another controller has built on the engine since this solve");
-        const int rc = copra_b200_lmpc_vjp_model(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, costs, model);
-        if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(copra_b200_last_error(b200::handle()));
-        b200::check(rc);
+        sensGuard("vjp", false);
+        sensCheck(multi_ ? copra_b200_multi_lmpc_vjp_model(multi_, dcontrol, dtrajectory, &out, costs, model)
+                         : copra_b200_lmpc_vjp_model(b200::handle(), dcontrol, dtrajectory, COPRA_B200_HOST, &out, costs, model));
     }
-    void initialStateGuard(const char* name) const
+    // What every sensitivity method checks before it calls the engine: an initial-state controller for the initialState*
+    // methods (std::runtime_error), HOST arrays (std::domain_error), and this controller's solve still resident on the
+    // engine (std::runtime_error: another controller may have built on the shared engine since)
+    void sensGuard(const char* name, bool initial) const
     {
-        if (!p_.initial_state) throw std::runtime_error(std::string("BatchedLMPC::") + name + " needs an initial-state controller; use vjp / jvp");
+        if (initial && !p_.initial_state) throw std::runtime_error(std::string("BatchedLMPC::") + name + " needs an initial-state controller; use vjp / jvp");
         if (p_.memory != COPRA_B200_HOST) COPRA_DOMAIN_ERROR(std::string("BatchedLMPC::") + name + " takes HOST arrays");
         if (multi_ ? !multiBuilt_ : myEpoch_ != b200::buildEpoch())
             throw std::runtime_error(std::string("BatchedLMPC::") + name + ": no solve of this controller is resident on the engine");
     }
-    void initialStateCheck(int rc) const
+    // The engine's error of a sensitivity call: E_ARG and E_UNSUPPORTED (a request this build cannot serve) as
+    // std::domain_error, any other failure as std::runtime_error
+    void sensCheck(int rc) const
     {
+        if (!rc) return;
         const char* msg = multi_ ? copra_b200_multi_last_error(multi_) : copra_b200_last_error(b200::handle());
         if (rc == COPRA_B200_E_UNSUPPORTED || rc == COPRA_B200_E_ARG) COPRA_DOMAIN_ERROR(msg);
-        if (rc) throw std::runtime_error(msg);
+        throw std::runtime_error(msg);
     }
     copra_b200_problem p_{};
     std::vector<copra_b200_cost> costs_;

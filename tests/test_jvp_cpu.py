@@ -2,6 +2,7 @@
 against central differences of the CPU oracle, its adjoint identity with the VJP reference, the host-side refusals of
 copra_b200_lmpc_jvp / copra_b200_lmpc_feedback_gain and their exported symbols."""
 import ctypes as C
+import types
 
 import numpy as np
 import pytest
@@ -141,3 +142,13 @@ def test_feedback_gain_layout():
     assert ku.shape == (2, 6, 6) and kx.shape == (2, 24, 6)
     # instance 1, row r, column s sits at 1 * 36 + s * 6 + r
     assert ku[1, 4, 2] == 36 + 2 * 6 + 4
+
+
+def test_multi_set_warm_start_raises_the_engine_error():
+    me = capi.MultiEngine.__new__(capi.MultiEngine)  # no device handles: only the host-side error path
+    me.m = None
+    me.lib = types.SimpleNamespace(copra_b200_multi_set_warm_start=lambda m, on: -1,
+                                   copra_b200_multi_last_error=lambda m: b"null handle")
+    with pytest.raises(capi.CopraB200Error) as e:
+        me.set_warm_start(True)
+    assert e.value.code == -1
